@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA backend
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's frame to DIR/*.npy
 
 A step is one full render of the workload (one pass of Tracer.render's pixel loop):
   N = 1 : BASELINE config 2 — RTOW final scene (randomBouncing, scene seed 42, 485 spheres),
@@ -35,6 +36,30 @@ sys.path.insert(0, ROOT)
 METRIC = "Mpaths/s"
 ENTRY_BYTES = 64   # one queue entry of the staged K1 (rz_search.cuh: rz_queue_push)
 NOMINAL_FP32_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12  # 74.45: SMs x lanes x 2 flop x max SM clock
+DUMP_BYTES = 60 << 20   # --dump-outputs: data bytes in all; with the .npy headers the files stay under 64 MB (10^6 bytes)
+
+
+def dump_outputs(out_dir: str, frames: dict):
+    """--dump-outputs: writes each [H, W, C] frame of the last timed step as out_dir/<name>.npy, float64 data as float64 and
+    everything else as float32, so that two builds can be compared output for output.  When the frames would exceed
+    DUMP_BYTES together, every file holds the same fixed, seeded sample of pixels instead: [n, C], pixels in row-major order."""
+    os.makedirs(out_dir, exist_ok=True)
+    import numpy as np
+    frames = {k: np.asarray(v) for k, v in frames.items()}
+    h, w = next(iter(frames.values())).shape[:2]
+    as_dtype = {k: np.float64 if v.dtype == np.float64 else np.float32 for k, v in frames.items()}
+    per_px = sum(np.dtype(as_dtype[k]).itemsize * v[0, 0].size for k, v in frames.items())
+    pick = None
+    if per_px * h * w > DUMP_BYTES:
+        pick = np.sort(np.random.default_rng(0).choice(h * w, DUMP_BYTES // per_px, replace=False))
+    for k, v in frames.items():
+        assert v.shape[:2] == (h, w), (k, v.shape)
+        out = v.astype(as_dtype[k])
+        if pick is not None:
+            out = out.reshape(h * w, -1)[pick]
+        np.save(os.path.join(out_dir, k + ".npy"), out)
+    print(f"bench.py: wrote {', '.join(k + '.npy' for k in frames)} to {out_dir}"
+          + (f" ({len(pick)} of {h * w} pixels, seeded sample)" if pick is not None else ""), file=sys.stderr)
 
 
 def workload(n_gpus: int, args) -> dict:
@@ -127,8 +152,10 @@ def run_reference(args, rank: int, world: int):
         scene.render(cam, w["width"], h, spp, w["depth"], seed=100 + i, threads=threads)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        scene.render(cam, w["width"], h, spp, w["depth"], seed=200 + i, threads=threads)
-    dt = (time.perf_counter() - t0) / max(1, args.steps)
+        img, _ = scene.render(cam, w["width"], h, spp, w["depth"], seed=200 + i, threads=threads)
+    dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"linear": img})
     v = paths / dt / 1e6
     sample = f"{w['width']}x{h} at {spp} spp of the {w['spp']}-spp workload per step (rate is spp-independent)"
     print(json.dumps({
@@ -217,7 +244,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-variants", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the frame the last timed step computed to DIR/<name>.npy (float32 / float64, <= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -276,9 +307,12 @@ def main():
     gather_lin = SlabGather(H, (W, 4), torch.float32, dev, band) if world > 1 else None
     gather_rgb = SlabGather(H, (W, 3), torch.uint8, dev, band) if world > 1 else None
 
+    last_frame = [None, None]   # device pointers of the latest step's linear and RGB8 frames (world == 1)
+
     def step_device():
         """One render, inputs resident in HBM, result left in HBM on GPU0 (after the NCCL gather for N>1)."""
         dl, d8, n = be.render_device(cam, p, sync=False)
+        last_frame[:] = dl, d8
         if world == 1:
             return n
         lin = torch.as_tensor(DevArray(dl, (my_rows, W, 4), "<f4"), device=dev)
@@ -331,6 +365,14 @@ def main():
     barrier()
     t_wall1 = time.time()
     step_ms = [a.elapsed_time(b) for a, b in ev]
+    # the last timed step's frame, as a caller of the timed path receives it, before any later render reuses the buffers
+    if args.dump_outputs and rank == 0:
+        if world == 1:
+            lin = torch.as_tensor(DevArray(last_frame[0], (H, W, 4), "<f4"), device=dev)
+            rgb = torch.as_tensor(DevArray(last_frame[1], (H, W, 3), "|u1"), device=dev)
+        else:
+            lin, rgb = gather_lin.final, gather_rgb.final
+        dump_outputs(args.dump_outputs, {"linear": lin.cpu().numpy(), "rgb8": rgb.cpu().numpy()})
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)

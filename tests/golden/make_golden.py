@@ -9,7 +9,9 @@ ids_config4_960x540.npz     same for BASELINE config 4's scene (randomBouncing w
 scene_seed42.npz            the flat scene arrays of randomBouncing(seed 42) (RzScene field names)
 config2_oracle_500spp.npz   (--full) 1200x675, 500 spp, depth 50 oracle render (row-stream mode,
                             seed 2024) reduced to 4x4 and 16x16 block means + global means
-The full 500-spp float image is cached under oracle/_cache/ (git-ignored) for local use.
+config2_oracle_500spp_pixels.npz
+                            (--full) the same render at every PIXEL_STEP-th pixel in row-major order: `idx` (flat
+                            pixel index), `rgb` (linear float32) — the per-pixel comparison at full resolution
 """
 import os
 import sys
@@ -22,6 +24,7 @@ sys.path.insert(0, ROOT)
 import oracle  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+PIXEL_STEP = 49   # 16,531 of 810,000 pixels; coprime to the width, so the sample moves across the columns row by row
 
 
 def block_means(img, b):
@@ -48,10 +51,11 @@ def main():
     if "--full" in sys.argv:
         cam, h = oracle.default_camera(1200)
         t = time.time()
-        img, st = sc.render(cam, 1200, h, 500, 50, seed=2024, threads=0, stats=True)
+        img, st = sc.render(cam, 1200, h, 500, 50, seed=2024, threads=0, row_streams=True, stats=True)
         print("500 spp oracle render:", time.time() - t, "s", st)
-        os.makedirs(os.path.join(ROOT, "oracle", "_cache"), exist_ok=True)
-        np.save(os.path.join(ROOT, "oracle", "_cache", "config2_oracle_500spp_f32.npy"), img.astype(np.float32))
+        idx = np.arange(0, 1200 * h, PIXEL_STEP, dtype=np.uint32)
+        np.savez_compressed(os.path.join(HERE, "config2_oracle_500spp_pixels.npz"), idx=idx,
+                            rgb=img.reshape(-1, 3)[idx].astype(np.float32), seed=2024, spp=500)
         np.savez_compressed(os.path.join(HERE, "config2_oracle_500spp.npz"),
                             block4=block_means(img, 4).astype(np.float32), block16=block_means(img, 16).astype(np.float32),
                             mean=img.mean(axis=(0, 1)), stats=np.array([st[k] for k in oracle.STAT_NAMES], dtype=np.uint64),

@@ -160,12 +160,11 @@ def test_image_parity_config2_against_golden_blocks(be, scene42):
     assert b16 <= 0.002
     # 4x4 block means average 16 pixels: floor ~ 39.7 dB + 10log10(16) ~ 51.7 dB at 500 vs 500 spp
     assert psnr4 >= 49.0
-    full = os.path.join(os.path.dirname(GOLDEN), "..", "oracle", "_cache", "config2_oracle_500spp_f32.npy")
-    if os.path.exists(full):
-        ref = np.load(full)
-        got = compare(img, ref)
-        print("full-res", got)
-        assert got["psnr"] >= 38.0 and max(got["mae"]) <= 0.008 and got["block_mae"] <= 0.002
+    # per pixel, at the committed sample of the same oracle render (its 16x16 block MAE is b16 above)
+    px = np.load(os.path.join(GOLDEN, "config2_oracle_500spp_pixels.npz"))
+    got = compare(img.reshape(-1, 1, 3)[px["idx"]], px["rgb"][:, None])
+    print("full-res pixel sample", got)
+    assert got["psnr"] >= 38.0 and max(got["mae"]) <= 0.008
 
 
 def test_glass_heavy_scene_parity(be, orc):
