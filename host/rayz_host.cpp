@@ -2,12 +2,14 @@
 //
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
-//               [--dump-scene file] [--dump-linear file] [--ppm-bench]
+//               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N]]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
 // The pixel loop runs in librayz_cuda.so; the timed region covers what the reference's covers
-// (hittables + BVH build == scene upload, and the render).
+// (hittables + BVH build == scene upload, and the render).  --noise-target X (displayed-value rms error, 1/255 = one 8-bit
+// step) starts at --spp samples and doubles them until the frame reaches X or --max-spp (default 4096); the samples reached
+// and the error go to stderr, the report line and the P3 output are unchanged.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -34,6 +36,8 @@ int main(int argc, char **argv) {
     uint32_t variant = RZ_VARIANT_AUTO;
     const char *dump_scene = nullptr, *dump_linear = nullptr;
     bool ppm_bench = false, penultimate = false;
+    float noise_target = 0;
+    uint32_t max_spp = 4096;
     for (int i = 2; i < argc; i++) {
         const std::string a = argv[i];
         auto val = [&]() -> const char * { if (i + 1 >= argc) { std::fprintf(stderr, "missing value for %s\n", a.c_str()); std::exit(2); } return argv[++i]; };
@@ -46,6 +50,8 @@ int main(int argc, char **argv) {
         else if (a == "--dump-scene") dump_scene = val();
         else if (a == "--dump-linear") dump_linear = val();
         else if (a == "--ppm-bench") ppm_bench = true;
+        else if (a == "--noise-target") noise_target = std::strtof(val(), nullptr);
+        else if (a == "--max-spp") max_spp = (uint32_t)std::strtoul(val(), nullptr, 10);
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -62,6 +68,8 @@ int main(int argc, char **argv) {
         tracer.max_bounces = depth;
         tracer.render_seed = render_seed;
         tracer.variant = variant;
+        tracer.noise_target = noise_target;
+        tracer.max_spp = max_spp;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);
@@ -74,6 +82,10 @@ int main(int argc, char **argv) {
         std::fprintf(stderr, "  [rayz_cuda] path kernel %.3f ms, resolve %.3f ms, %u launches, %u static + %u moving spheres, variant %u, %d GPU(s)\n",
                      tracer.timing.kernel_ms, tracer.timing.resolve_ms, tracer.timing.launches, tracer.timing.n_static, tracer.timing.n_moving,
                      tracer.timing.variant, gpus);
+        if (noise_target > 0)
+            std::fprintf(stderr, "  [rayz_cuda] noise target %.5f: %llu spp reached, rms error %.5f (%.2f 8-bit steps), mean %.5f, max %.5f, %u of %u pixels above\n",
+                         noise_target, (unsigned long long)tracer.noise.samples, tracer.noise.rms_err, tracer.noise.rms_err * 255.0, tracer.noise.mean_err,
+                         tracer.noise.max_err, tracer.noise.n_above, tracer.noise.n_pixels);
         if (dump_scene && !dumpScene(tracer, dump_scene)) { std::perror(dump_scene); return 1; }
         if (dump_linear) {
             FILE *f = std::fopen(dump_linear, "wb");

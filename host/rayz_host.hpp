@@ -241,6 +241,9 @@ struct Tracer {
     std::vector<int> devices{0};
     RzContext *ctx = nullptr;
     RzTiming timing{};
+    float noise_target = 0;       // > 0: render from samples_per_px, doubling, until the frame's rms error reaches it (rayz_cuda_render_to_noise)
+    uint32_t max_spp = 4096;      // ... or this many samples are in
+    RzNoise noise{};              // summary of the last render with a noise target
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
         : rng(seed) {
@@ -315,7 +318,8 @@ struct Tracer {
         lin.assign(img.w * img.h * 4, 0.f);
         img.rgb8.resize(img.w * img.h * 3);
         uint64_t rays = 0;
-        check(rayz_cuda_render(ctx, &cam, &p, lin.data(), img.rgb8.data(), &rays));
+        if (noise_target > 0) check(rayz_cuda_render_to_noise(ctx, &cam, &p, noise_target, max_spp, lin.data(), img.rgb8.data(), &rays, &noise));
+        else check(rayz_cuda_render(ctx, &cam, &p, lin.data(), img.rgb8.data(), &rays));
         for (size_t i = 0; i < img.w * img.h; i++) img.pixels[i] = {lin[4 * i], lin[4 * i + 1], lin[4 * i + 2]};
         rayz_cuda_timing(ctx, &timing);
         return (size_t)rays;

@@ -121,7 +121,7 @@ typedef struct RzRenderParams {
     uint32_t spp;           /* Tracer.samples_per_px (renderer.zig:24)          */
     uint32_t max_depth;     /* Tracer.max_bounces   (renderer.zig:23)           */
     uint64_t seed;          /* Philox key                                        */
-    uint32_t sample_offset; /* first sample index (progressive accumulation)     */
+    uint32_t sample_offset; /* first sample index (batches: RZ_RENDER_ACCUMULATE) */
     uint32_t variant;       /* RZ_VARIANT_*                                      */
     float t_min;            /* FP32 stand-in for renderer.zig:107's 1e-10; 0 => 1e-4 */
     uint32_t shard_index;
@@ -135,6 +135,34 @@ typedef struct RzRenderParams {
 #define RZ_RENDER_SERIAL_PASSES 1u /* staged K1: run the passes back to back on one stream instead of
                                     * overlapping them on two, so that RzTiming.primary_ms and
                                     * kernel_ms - primary_ms are clean per-kernel durations (profiling) */
+#define RZ_RENDER_MOMENTS 2u       /* also sum each path's luminance squared (Y = 0.2126 r + 0.7152 g + 0.0722 b) in the
+                                    * fourth accumulator slot, so that rayz_cuda_noise can estimate the per-pixel error;
+                                    * changes no pixel of the image (one more atomic per path that ends in the sky) */
+#define RZ_RENDER_ACCUMULATE 4u    /* progressive rendering: add this batch to the sums of the previous render instead of
+                                    * starting over, and resolve by the cumulative sample count.  Radiance is summed in
+                                    * integers, so batches [0,a) + [a,b) + ... reproduce one render of all the samples bit
+                                    * for bit when every batch runs the same kernel family (brute force: MEGA, MEGA_SINGLE,
+                                    * WAVEFRONT; or BVH).  AUTO picks each batch's family by that batch's frame size, and the
+                                    * two families agree up to a pixel or two (see RZ_VARIANT_AUTO): pin the variant where
+                                    * bit equality matters.  Refused with RZ_ERR_INVALID_ARG, the sums untouched, unless the
+                                    * previous render succeeded with the same width, height, shard_index/count, band_rows,
+                                    * seed, max_depth, t_min, camera and RZ_RENDER_MOMENTS bit on this context, no scene
+                                    * upload or differently shaped reserve came in between, sample_offset equals the previous
+                                    * batch's sample_offset + spp, and the cumulative count stays below 2^32.  A render that
+                                    * fails ends the accumulation.  *out_paths counts this call's paths only.  With
+                                    * rayz_cuda_render_device(sync = 0), the next batch checks the previous one's device
+                                    * error word before it adds to its sums. */
+
+/* Noise summary of the accumulated frame (rayz_cuda_noise).  Errors are standard errors of the DISPLAYED value
+ * (gamma 2, as writePPM shows it) in units of [0, 1]: one 8-bit step is 1/255.  +inf while samples < 2. */
+typedef struct RzNoise {
+    uint64_t samples;  /* samples per pixel summed so far (cumulative over RZ_RENDER_ACCUMULATE batches) */
+    uint32_t n_pixels; /* pixels of the context's rows                                                   */
+    uint32_t n_above;  /* pixels whose error exceeds the caller's target                                */
+    double mean_err;   /* mean over the pixels                                                           */
+    double rms_err;    /* root mean square over the pixels                                               */
+    double max_err;
+} RzNoise;
 
 typedef struct RzConfig {
     int32_t n_devices;     /* 0 => 1 */
@@ -217,6 +245,25 @@ int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *params);
  * destroy) are returned instead of copied.  With `sync` == 0 the call only enqueues. */
 int rayz_cuda_render_device(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params,
                             void **d_linear_rgba, void **d_rgb8, uint64_t *out_paths, int sync);
+
+/*
+ * Per-pixel noise of the accumulated frame of the last render(s): the standard error of the displayed value
+ *   Ybar = (0.2126 q0 + 0.7152 q1 + 0.0722 q2) / n,  s^2 = (q3 / n - Ybar^2) n / (n - 1)  (q: per-pixel sums, n: samples),
+ *   e = sqrt(s^2 / n) / (2 sqrt(max(Ybar, 1e-4)))
+ * out_err (nullable): rows of the context * width floats, laid out like out_linear_rgba.  out (nullable): the frame summary,
+ * n_above counting pixels with e > target.  RZ_ERR_INVALID_ARG unless the accumulated render(s) ran with RZ_RENDER_MOMENTS.
+ */
+int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzNoise *out);
+
+/*
+ * Render until the frame is clean enough: the first batch is p->spp samples from p->sample_offset (RZ_RENDER_MOMENTS
+ * implied), each next batch doubles the accumulated count (capped at max_spp) with RZ_RENDER_ACCUMULATE; stops when
+ * rms_err <= target or max_spp samples are reached.  RZ_OK either way: *out_noise says which (its samples and rms_err).
+ * The host buffers (each nullable, as in rayz_cuda_render) are written once, at the end; *out_paths counts every batch.
+ * RZ_ERR_INVALID_ARG if max_spp < p->spp.
+ */
+int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float target, uint32_t max_spp,
+                              float *out_linear_rgba, uint8_t *out_rgb8, uint64_t *out_paths, RzNoise *out_noise);
 
 /* Number of image rows a shard owns under the banding rule above. */
 uint32_t rayz_cuda_shard_rows(uint32_t height, uint32_t shard_index, uint32_t shard_count,

@@ -19,6 +19,7 @@ TEX_CHECKER, TEX_SOLID = 0, 1
 DIFFUSE_UNIT_SPHERE, DIFFUSE_UNIT_SPHERE_SURFACE, DIFFUSE_HEMISPHERE = 0, 1, 2
 VARIANT_AUTO, VARIANT_MEGA, VARIANT_WAVEFRONT, VARIANT_BVH = 0, 1, 2, 3
 VARIANTS = {"auto": 0, "mega": 1, "wavefront": 2, "bvh": 3, "mega_single": 4}
+RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE = 1, 2, 4   # RzRenderParams.flags (RZ_RENDER_*)
 
 _dp, _up = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 
@@ -64,6 +65,14 @@ class RzTiming(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved0"}
 
 
+class RzNoise(C.Structure):
+    _fields_ = [("samples", C.c_uint64), ("n_pixels", C.c_uint32), ("n_above", C.c_uint32), ("mean_err", C.c_double),
+                ("rms_err", C.c_double), ("max_err", C.c_double)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 class RzTuning(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("rays_per_thread", C.c_int32), ("chunk", C.c_uint32), ("chunk_primary", C.c_uint32),
                 ("queue_log2", C.c_int32), ("second_stages", C.c_int32), ("bvh_stages", C.c_int32), ("tail_brute", C.c_int32),
@@ -88,6 +97,9 @@ SYMBOLS = {
                                    C.POINTER(C.c_uint64)]),
     "rayz_cuda_render_device": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.POINTER(C.c_void_p),
                                           C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.c_int]),
+    "rayz_cuda_noise": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p, C.POINTER(RzNoise)]),
+    "rayz_cuda_render_to_noise": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_float, C.c_uint32,
+                                            C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(RzNoise)]),
     "rayz_cuda_shard_rows": (C.c_uint32, [C.c_uint32] * 4),
     "rayz_cuda_context_rows": (C.c_uint32, [C.c_void_p] + [C.c_uint32] * 4),
     "rayz_cuda_primary_ids": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]),

@@ -24,7 +24,7 @@ struct RzIdsArgs {
     uint32_t width, height; int use_bvh; int32_t *out; unsigned int *err;
 };
 struct RzResolveArgs {
-    const unsigned long long *accum; float4 *out_linear; uint8_t *out_rgb8;
+    const unsigned long long *accum; float4 *out_linear; uint8_t *out_rgb8; float *out_err;
     uint32_t n_local_px, width; uint32_t spp; uint32_t dev_index, dev_count, band_rows;
 };
 extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, int collect_stats, int sm_count,
@@ -52,6 +52,9 @@ extern "C" size_t rz_bvh_wide_scratch_bytes(uint32_t n_nodes);
 extern "C" cudaError_t rz_bvh_wide_collapse(const RzBvhNode *n2, uint32_t n_nodes, void *scratch, RzBvh4Node *out, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_ids(const RzIdsArgs *a, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
+extern "C" uint32_t rz_noise_grid(void);
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, uint32_t n_local_px, uint32_t n, double target, void *out,
+                                              cudaStream_t stream);
 extern "C" cudaError_t rz_launch_ffma_peak(float *sink, int grid, int iters, int mode, cudaStream_t stream);
 extern "C" cudaError_t rz_wavefront_render(const RzPathArgs *a, int sm_count, int collect_stats, cudaStream_t stream,
                                            void **scratch, size_t *scratch_bytes, uint32_t *launches);
@@ -152,6 +155,8 @@ struct Dev {
     DBuf<RzStatsDev> stats;
     DBuf<float4> out_linear;
     DBuf<uint8_t> out_rgb8;
+    DBuf<float> out_err;              // rayz_cuda_noise: per-pixel error of the context's rows (gather root only)
+    DBuf<double> noise_part;          // rayz_cuda_noise: the reduction's per-CTA partials of this device
     DBuf<float4> loc_linear;          // multi-device render into HOST buffers: this device's own rows, copied out over its own PCIe link
     DBuf<uint8_t> loc_rgb8;
     uint32_t loc_rows = 0;            // rows of the last such render
@@ -167,8 +172,22 @@ struct Dev {
     bool serial_passes = false;
 };
 
+// What the accumulators of the context's devices hold (RZ_RENDER_ACCUMULATE, include/rayz_cuda.h): the frame, shard and
+// sampling parameters a next batch must repeat, and the samples summed so far.  The device set is the context's own.
+struct AccumRecord {
+    bool valid = false;
+    bool pending = false;   // enqueued by rayz_cuda_render_device(sync = 0): the device error words are not checked yet
+    uint32_t width = 0, height = 0, shard_index = 0, shard_count = 1, band_rows = 4, max_depth = 0, moments = 0;
+    uint64_t seed = 0;
+    float t_min = 0;
+    RzCamera cam{};
+    uint32_t first_offset = 0;
+    uint64_t samples = 0;
+};
+
 struct RzContext {
     std::vector<Dev> devs;
+    AccumRecord acc;
     bool have_scene = false;
     uint32_t n_spheres = 0;
     RzStats stats{};
@@ -331,6 +350,7 @@ extern "C" void rayz_cuda_destroy(RzContext *ctx) {
         for (int sd = 0; sd < 2; sd++) { D.q1[sd].release(); D.q2[sd].release(); D.keys[sd].release(); D.idx_sorted[sd].release(); D.bins[sd].release(); }
         D.bin_lists.release();
         D.stats.release(); D.out_linear.release(); D.out_rgb8.release(); D.loc_linear.release(); D.loc_rgb8.release();
+        D.out_err.release(); D.noise_part.release();
         D.ids.release(); D.sink.release();
         if (D.wf_scratch) rz_wavefront_free(D.wf_scratch);
         for (auto &ev : D.ev) if (ev) cudaEventDestroy(ev);
@@ -404,6 +424,7 @@ static const uint32_t RZ_SMEM_BUDGET = 180u * 1024u;  // of 227 KB per CTA on sm
 
 extern "C" int rayz_cuda_upload_scene(RzContext *ctx, const RzScene *sc) {
     if (!ctx || !sc) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: NULL argument");
+    ctx->acc.valid = false;   // sums of the old scene: a next batch may not add to them
     const uint32_t n = sc->n_spheres, nm = sc->n_materials, nt = sc->n_textures;
     if (n == 0) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: empty scene (BVH.build asserts nobjs > 0, hit.zig:132)");
     if (n >= (1u << 28)) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: too many spheres (K3 leaf references hold 28 bits)");
@@ -765,8 +786,31 @@ static int collect_timing_and_stats(RzContext *ctx, bool collect_stats) {
     return RZ_OK;
 }
 
+// An accumulation left pending by rayz_cuda_render_device(sync = 0): wait for it and read the device error words, so that a
+// batch that dropped paths ends the accumulation before anything is added to its sums.
+static int settle_accumulation(RzContext *ctx) {
+    if (!ctx->acc.valid || !ctx->acc.pending) return RZ_OK;
+    ctx->acc.valid = false;
+    for (Dev &D : ctx->devs) {
+        unsigned int ew = 0;
+        RZ_CUDA(cudaSetDevice(D.id));
+        RZ_CUDA(cudaStreamSynchronize(D.stream));
+        RZ_CUDA(cudaMemcpy(&ew, D.errword.p, sizeof ew, cudaMemcpyDeviceToHost));
+        if (ew) return RZ_OK;   // stays invalid
+    }
+    ctx->acc.valid = true;
+    ctx->acc.pending = false;
+    return RZ_OK;
+}
+
 static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, bool sync, bool host_direct = false) {
     if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "render: NULL argument");
+    // Every render ends what the accumulators held unless it succeeds (the record is committed at the end) or it is an
+    // RZ_RENDER_ACCUMULATE batch that is refused before anything was touched (the record is restored).
+    const bool accumulate = (p->flags & RZ_RENDER_ACCUMULATE) != 0;
+    if (accumulate) { DeviceGuard g; const int rc = settle_accumulation(ctx); if (rc) return rc; }
+    const AccumRecord prev = ctx->acc;
+    ctx->acc.valid = false;
     if (!ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "render: rayz_cuda_upload_scene has not been called");
     if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "render: width, height and spp must be > 0");
     if ((uint64_t)p->width * p->height >= (1ull << 31)) return rz_fail(RZ_ERR_INVALID_ARG, "render: image too large");
@@ -793,6 +837,27 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
         return rz_fail(RZ_ERR_INVALID_ARG, "render: unknown variant %u", p->variant);
     if (variant == RZ_VARIANT_MEGA && brute_smem > RZ_SMEM_BUDGET)
         return rz_fail(RZ_ERR_UNSUPPORTED, "render: scene needs %u B of shared memory for the brute-force kernel (budget %u); use RZ_VARIANT_BVH", brute_smem, RZ_SMEM_BUDGET);
+
+    AccumRecord next;
+    next.width = p->width; next.height = p->height; next.shard_index = s; next.shard_count = S; next.band_rows = band;
+    next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
+    next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
+    next.first_offset = p->sample_offset; next.samples = p->spp;
+    if (accumulate) {
+        auto refuse = [&](const char *why) { ctx->acc = prev; return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ACCUMULATE refused: %s", why); };
+        if (!prev.valid) return refuse("no previous render to add to (none, it failed, or a scene upload or reserve came in between)");
+        if (prev.width != next.width || prev.height != next.height || prev.shard_index != s || prev.shard_count != S || prev.band_rows != band)
+            return refuse("frame size, shard or band_rows differ from the accumulated render");
+        if (prev.seed != next.seed || prev.max_depth != next.max_depth || memcmp(&prev.t_min, &next.t_min, sizeof(float)) != 0)
+            return refuse("seed, max_depth or t_min differ from the accumulated render");
+        if (memcmp(&prev.cam, cam, sizeof(RzCamera)) != 0) return refuse("the camera differs from the accumulated render");
+        if (prev.moments != next.moments) return refuse("the RZ_RENDER_MOMENTS bit differs from the accumulated render");
+        if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
+            return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
+        if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
+        next.first_offset = prev.first_offset;
+        next.samples = prev.samples + p->spp;
+    }
 
     const auto t_host0 = std::chrono::steady_clock::now();
     DeviceGuard guard;
@@ -821,7 +886,7 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
         if ((rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4))) return rc;
         if ((rc = D.stats.alloc(3))) return rc;   // [0] whole render / primary kernel, [1] sorted stages, [2] persistent tail kernel
         RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
-        RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
+        if (!accumulate) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
         RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
         RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
         if (p->collect_stats) RZ_CUDA(cudaMemsetAsync(D.stats.p, 0, 3 * sizeof(RzStatsDev), D.stream));
@@ -851,6 +916,7 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
         a.unit_entries = ctx->tun.unit_entries;
         a.bvh_active_min = (uint32_t)ctx->tun.bvh_active_min; a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
         a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
+        a.moments = next.moments;
 
         RZ_CUDA(cudaEventRecord(D.ev[1], D.stream));
         D.passes = 0;
@@ -994,8 +1060,8 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
         RZ_CUDA(cudaEventRecord(D.ev[2], D.stream));
 
         RzResolveArgs r;
-        r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p;
-        r.n_local_px = n_local; r.width = p->width; r.spp = p->spp;
+        r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p; r.out_err = nullptr;
+        r.n_local_px = n_local; r.width = p->width; r.spp = (uint32_t)next.samples;   // cumulative with RZ_RENDER_ACCUMULATE
         r.dev_index = d; r.dev_count = ND; r.band_rows = band;
         if (host_direct) {   // every device resolves into its OWN compact buffers; rayz_cuda_render copies them out in parallel
             if ((rc = D.loc_linear.alloc((size_t)n_local)) || (rc = D.loc_rgb8.alloc((size_t)n_local * 3))) return rc;
@@ -1039,6 +1105,9 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
         { const int rc = collect_timing_and_stats(ctx, p->collect_stats != 0); if (rc) return rc; }
         ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host0).count();
     }
+    ctx->acc = next;
+    ctx->acc.valid = true;
+    ctx->acc.pending = !sync;
     return RZ_OK;
 }
 
@@ -1051,6 +1120,8 @@ extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     const uint32_t S = p->shard_count <= 1 ? 1 : p->shard_count, s = p->shard_count <= 1 ? 0 : p->shard_index;
     if (s >= S) return rz_fail(RZ_ERR_INVALID_ARG, "reserve: shard_index %u >= shard_count %u", s, S);
     const uint32_t band = p->band_rows ? p->band_rows : 4, ND = (uint32_t)ctx->devs.size();
+    if (p->width != ctx->acc.width || p->height != ctx->acc.height || s != ctx->acc.shard_index || S != ctx->acc.shard_count || band != ctx->acc.band_rows)
+        ctx->acc.valid = false;   // another frame shape: a next batch may not add to the sums
     DeviceGuard guard;
     int rc;
     Dev &D0 = ctx->devs[0];
@@ -1099,8 +1170,21 @@ static bool host_pinned(const void *p) {
     return at.type == cudaMemoryTypeHost;
 }
 
+static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba, uint8_t *out_rgb8,
+                       uint64_t *out_paths);
+
 extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba,
                                 uint8_t *out_rgb8, uint64_t *out_paths) {
+    const int rc = render_host(ctx, cam, params, out_linear_rgba, out_rgb8, out_paths);
+    if (ctx) {
+        if (rc != RZ_OK && ctx->acc.pending) ctx->acc.valid = false;   // the paths ran but the call failed: the sums are not to be added to
+        ctx->acc.pending = false;
+    }
+    return rc;
+}
+
+static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba, uint8_t *out_rgb8,
+                       uint64_t *out_paths) {
     const auto t0 = std::chrono::steady_clock::now();
     if (!ctx || !params) return rz_fail(RZ_ERR_INVALID_ARG, "render: NULL argument");
     // Several devices and page-locked host buffers: no gather to device 0 at all.  Every device resolves its own rows and
@@ -1146,6 +1230,99 @@ extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRen
     { const int rc2 = collect_timing_and_stats(ctx, params->collect_stats != 0); if (rc2) return rc2; }
     ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (out_paths) *out_paths = (uint64_t)npx * params->spp;
+    return RZ_OK;
+}
+
+// Noise of the accumulated frame: every device computes its pixels' errors from its own accumulators with the resolve kernel
+// (rows scattered into the gather root's buffer like the image) and reduces them in a fixed order; the host adds the partials
+// device by device, CTA by CTA.
+extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzNoise *out) {
+    if (!ctx) return rz_fail(RZ_ERR_INVALID_ARG, "noise: ctx is NULL");
+    DeviceGuard guard;
+    { const int rc = settle_accumulation(ctx); if (rc) return rc; }
+    const AccumRecord &A = ctx->acc;
+    if (!A.valid) return rz_fail(RZ_ERR_INVALID_ARG, "noise: no accumulated render (none, it failed, or a scene upload or reserve came in between)");
+    if (!A.moments) return rz_fail(RZ_ERR_INVALID_ARG, "noise: the accumulated render(s) ran without RZ_RENDER_MOMENTS");
+    const uint32_t ND = (uint32_t)ctx->devs.size(), G = rz_noise_grid();
+    Dev &D0 = ctx->devs[0];
+    const uint32_t rows_ctx = rayz_cuda_context_rows(ctx, A.height, A.shard_index, A.shard_count, A.band_rows);
+    int rc;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if (out_err && (rc = D0.out_err.alloc((size_t)rows_ctx * A.width))) return rc;
+    for (uint32_t d = 0; d < ND; d++) {   // every device enqueues before the first wait
+        Dev &D = ctx->devs[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        const uint32_t n_local = rayz_cuda_shard_rows(A.height, A.shard_index * ND + d, A.shard_count * ND, A.band_rows) * A.width;
+        if ((rc = D.noise_part.alloc(4 * (size_t)G))) return rc;
+        if (out_err) {
+            RzResolveArgs r;
+            r.accum = D.accum.p; r.out_linear = nullptr; r.out_rgb8 = nullptr; r.out_err = D0.out_err.p;
+            r.n_local_px = n_local; r.width = A.width; r.spp = (uint32_t)A.samples;
+            r.dev_index = d; r.dev_count = ND; r.band_rows = A.band_rows;
+            RZ_CUDA(rz_launch_resolve(&r, D.stream));
+        }
+        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, n_local, (uint32_t)A.samples, (double)target, D.noise_part.p, D.stream));
+    }
+    double sum = 0, sum2 = 0, mx = 0;
+    uint64_t above = 0;
+    std::vector<double> part(4 * (size_t)G);
+    for (Dev &D : ctx->devs) {
+        RZ_CUDA(cudaSetDevice(D.id));
+        RZ_CUDA(cudaMemcpyAsync(part.data(), D.noise_part.p, part.size() * sizeof(double), cudaMemcpyDeviceToHost, D.stream));
+        RZ_CUDA(cudaStreamSynchronize(D.stream));
+        for (uint32_t g = 0; g < G; g++) {
+            uint64_t cnt;
+            memcpy(&cnt, &part[4 * (size_t)g + 3], sizeof cnt);
+            sum += part[4 * (size_t)g]; sum2 += part[4 * (size_t)g + 1]; mx = std::max(mx, part[4 * (size_t)g + 2]); above += cnt;
+        }
+    }
+    if (out_err) {
+        RZ_CUDA(cudaSetDevice(D0.id));
+        RZ_CUDA(cudaMemcpyAsync(out_err, D0.out_err.p, (size_t)rows_ctx * A.width * sizeof(float), cudaMemcpyDeviceToHost, D0.stream));
+        RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    }
+    if (out) {
+        const double npx = (double)rows_ctx * A.width;
+        out->samples = A.samples;
+        out->n_pixels = rows_ctx * A.width;
+        out->n_above = (uint32_t)above;
+        out->mean_err = npx > 0 ? sum / npx : 0.0;
+        out->rms_err = npx > 0 ? std::sqrt(sum2 / npx) : 0.0;
+        out->max_err = mx;
+    }
+    return RZ_OK;
+}
+
+// The stopping policy of progressive rendering, in one place for every host: batches that double the accumulated sample count
+// until the frame's rms error reaches the target or max_spp samples are in.
+extern "C" int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float target, uint32_t max_spp,
+                                         float *out_linear_rgba, uint8_t *out_rgb8, uint64_t *out_paths, RzNoise *out_noise) {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "render_to_noise: NULL argument");
+    if (p->spp == 0 || max_spp < p->spp) return rz_fail(RZ_ERR_INVALID_ARG, "render_to_noise: need 0 < spp <= max_spp (spp %u, max_spp %u)", p->spp, max_spp);
+    RzRenderParams q = *p;
+    q.flags = (p->flags & ~RZ_RENDER_ACCUMULATE) | RZ_RENDER_MOMENTS;
+    RzNoise nz;
+    memset(&nz, 0, sizeof nz);
+    for (;;) {
+        int rc = render_impl(ctx, cam, &q, true);
+        if (rc) return rc;
+        if ((rc = rayz_cuda_noise(ctx, target, nullptr, &nz))) return rc;
+        if (nz.rms_err <= (double)target || nz.samples >= max_spp) break;
+        q.sample_offset = p->sample_offset + (uint32_t)nz.samples;
+        q.spp = (uint32_t)std::min<uint64_t>(nz.samples, max_spp - nz.samples);
+        q.flags |= RZ_RENDER_ACCUMULATE;
+    }
+    DeviceGuard guard;
+    Dev &D0 = ctx->devs[0];
+    const size_t npx = (size_t)rayz_cuda_context_rows(ctx, p->height, p->shard_index, p->shard_count, p->band_rows) * p->width;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if (out_linear_rgba) RZ_CUDA(cudaMemcpyAsync(out_linear_rgba, D0.out_linear.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
+    if (out_rgb8) RZ_CUDA(cudaMemcpyAsync(out_rgb8, D0.out_rgb8.p, npx * 3, cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    if (out_paths) *out_paths = (uint64_t)npx * nz.samples;
+    if (out_noise) *out_noise = nz;
+    ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return RZ_OK;
 }
 

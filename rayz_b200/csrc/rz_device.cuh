@@ -126,7 +126,7 @@ struct RzPathArgs {
     const void *bvh;             // K3 only: RzBvhNode[] (or RzBvh4Node[] in the RZ_BVH_WIDE experiment)
     uint32_t bvh_nodes;
     RzCamF32 cam;
-    unsigned long long *accum;   // [n_local_px_pad][4] u64 fixed point (2^-32), rgb + pad
+    unsigned long long *accum;   // [n_local_px_pad][4] u64 fixed point (2^-32), rgb + sum of Y^2 (only with `moments`)
     unsigned int *unit_counter;  // persistent-kernel work counter (zeroed before launch)
     RzStatsDev *stats;           // STATS builds only
     uint32_t width, height;      // full image
@@ -169,7 +169,44 @@ struct RzPathArgs {
     uint32_t bvh_active_min;     // K3: lanes that must still be traversing for a burst to go on (ray replacement threshold)
     uint32_t bvh_descend_min;    // K3: a descend round ends once fewer lanes than this are still descending
     uint32_t tile_w;             // K3 camera stage: 0 = a work unit's 32 pixels are consecutive in a row; 8 = an 8 x 4 block (tile lists: the narrower cone)
+    uint32_t moments;            // != 0 (RZ_RENDER_MOMENTS): a path that ends in the sky also adds its luminance squared to accum slot 3
 };
+
+// ---------------------------------------------------------------------------------------------
+// Per-pixel noise (RZ_RENDER_MOMENTS, DESIGN.md "Progressive rendering").  Slot 3 of a pixel's accumulator sums Y^2 over its
+// paths in the 2^-32 fixed point of slots 0..2, Y = Rec. 709 luminance of the same clamped radiance the three colour atomics
+// add.  Paths that end absorbed or at the depth limit add zero to all four slots, as their radiance is zero.
+// ---------------------------------------------------------------------------------------------
+// Luminance floor of the displayed-value error: the gamma-2 slope 1 / (2 sqrt(Y)) grows without bound at black, where a pixel
+// with no variance would otherwise read as 0 / 0.  1e-4 linear is 0.01 displayed, 2.6 steps of 8 bits.
+#define RZ_NOISE_Y_FLOOR 1e-4
+
+RZ_HD float rz_clamp_radiance(float v) { return fminf(fmaxf(v, 0.f), 1048576.f); }
+// fixed-point sample of a clamped value (the kernels' atomics round to nearest, __float2ull_rn)
+RZ_HD unsigned long long rz_fixed32(float v) {
+#ifdef __CUDA_ARCH__
+    return __float2ull_rn(v * 4294967296.f);
+#else
+    return (unsigned long long)nearbyint((double)(v * 4294967296.f));
+#endif
+}
+// Y^2 of a path's clamped radiance, clamped like the colour channels; the FMAs are explicit so host and device agree bit for bit
+RZ_HD float rz_luma_sq(float r, float g, float b) {
+    const float y = fmaf(0.0722f, b, fmaf(0.7152f, g, 0.2126f * r));
+    return rz_clamp_radiance(y * y);
+}
+
+// Standard error of the DISPLAYED value (gamma 2: sqrt of the linear mean, as writePPM shows it) of one pixel from its four
+// accumulator slots after n samples, in units of the displayed range [0, 1] (one 8-bit step = 1/255).  f64:
+//   Ybar = (0.2126 q0 + 0.7152 q1 + 0.0722 q2) 2^-32 / n,  s^2 = max(0, q3 2^-32 / n - Ybar^2) n / (n - 1),
+//   sigma = sqrt(s^2 / n),  e = sigma / (2 sqrt(max(Ybar, RZ_NOISE_Y_FLOOR))).   n < 2 has no variance estimate: +inf.
+RZ_HD double rz_pixel_err(unsigned long long q0, unsigned long long q1, unsigned long long q2, unsigned long long q3, uint32_t n) {
+    if (n < 2u) return INFINITY;
+    const double s = 2.3283064365386962890625e-10, inv = 1.0 / (double)n;   // 2^-32
+    const double y = (0.2126 * (double)q0 + 0.7152 * (double)q1 + 0.0722 * (double)q2) * s * inv;
+    const double s2 = fmax(0.0, (double)q3 * s * inv - y * y) * ((double)n / (double)(n - 1u));
+    return sqrt(s2 * inv) / (2.0 * sqrt(fmax(y, RZ_NOISE_Y_FLOOR)));
+}
 
 // ---------------------------------------------------------------------------------------------
 // Philox4x32 (Salmon et al., SC'11), seven rounds.  key = 64-bit seed; counter = (global pixel, sample,

@@ -11,13 +11,17 @@
 // Output rows may live on ANOTHER GPU (peer pointers): with out_row_stride/out_row_offset the
 // kernel scatters this device's compact band-interleaved rows straight into the gather root's
 // full-shard buffers over NVLink, i.e. resolve and gather are one kernel.
+// The same kernel writes the per-pixel noise estimate (out_err: rz_pixel_err of the four slots) when asked.
 // ---------------------------------------------------------------------------------------------
+#include "rz_device.cuh"   // rz_pixel_err
+
 struct RzResolveArgs {
     const unsigned long long *accum;  // [n_local_px][4]
     float4 *out_linear;               // nullable
     uint8_t *out_rgb8;                // nullable
+    float *out_err;                   // nullable: displayed-value standard error per pixel (needs slot 3, RZ_RENDER_MOMENTS)
     uint32_t n_local_px, width;
-    uint32_t spp;
+    uint32_t spp;                     // samples summed in the accumulators (cumulative over RZ_RENDER_ACCUMULATE batches)
     // local row lr of this device -> destination row ((lr / band) * dev_count + dev_index) * band + lr % band
     uint32_t dev_index, dev_count, band_rows;
 };
@@ -27,15 +31,16 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
     if (lp >= a.n_local_px) return;
     const ulonglong2 q0 = *reinterpret_cast<const ulonglong2 *>(a.accum + (size_t)lp * 4);
     const unsigned long long q1 = a.accum[(size_t)lp * 4 + 2];
-    const double inv = 1.0 / (double)a.spp;
-    const double s = 2.3283064365386962890625e-10;  // 2^-32
-    const double r = (double)q0.x * s * inv, g = (double)q0.y * s * inv, b = (double)q1 * s * inv;
     size_t dst = lp;
     if (a.dev_count > 1u) {
         const uint32_t lr = lp / a.width, i = lp - lr * a.width;
         const uint32_t lb = lr / a.band_rows, within = lr - lb * a.band_rows;
         dst = (size_t)((lb * a.dev_count + a.dev_index) * a.band_rows + within) * a.width + i;
     }
+    if (a.out_err) a.out_err[dst] = (float)rz_pixel_err(q0.x, q0.y, q1, a.accum[(size_t)lp * 4 + 3], a.spp);
+    const double inv = 1.0 / (double)a.spp;
+    const double s = 2.3283064365386962890625e-10;  // 2^-32
+    const double r = (double)q0.x * s * inv, g = (double)q0.y * s * inv, b = (double)q1 * s * inv;
     if (a.out_linear) a.out_linear[dst] = make_float4((float)r, (float)g, (float)b, 1.0f);
     if (a.out_rgb8) {
         const double sr = r > 0 ? sqrt(r) : 0, sg = g > 0 ? sqrt(g) : 0, sb = b > 0 ? sqrt(b) : 0;
@@ -49,6 +54,45 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream) {
     if (a->n_local_px == 0) return cudaSuccess;
     rz_resolve_kernel<<<(a->n_local_px + 255) / 256, 256, 0, stream>>>(*a);
+    return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------
+// Frame summary of the noise estimate: per CTA of a FIXED grid (RZ_NOISE_GRID x 256), sum of e, sum of e^2, max e and the
+// count of pixels with e > target over the pixels lp = cta * 256 + tid + k * grid * 256, reduced in a fixed tree.  The host
+// adds the CTAs' partials in order: no floating-point atomics, so two identical calls give identical summaries.
+// ---------------------------------------------------------------------------------------------
+#define RZ_NOISE_GRID 256
+struct RzNoisePartial { double sum, sum2, max; unsigned long long above; };
+
+__global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned long long *__restrict__ accum, uint32_t n_local_px, uint32_t n,
+                                                              double target, RzNoisePartial *__restrict__ out) {
+    __shared__ double s_sum[256], s_sum2[256], s_max[256];
+    __shared__ unsigned long long s_above[256];
+    double sum = 0, sum2 = 0, mx = 0;
+    unsigned long long above = 0;
+    for (uint32_t lp = blockIdx.x * 256u + threadIdx.x; lp < n_local_px; lp += RZ_NOISE_GRID * 256u) {
+        const unsigned long long *q = accum + (size_t)lp * 4;
+        const double e = (double)(float)rz_pixel_err(q[0], q[1], q[2], q[3], n);   // the value out_err shows
+        sum += e; sum2 += e * e; mx = fmax(mx, e); above += e > target ? 1u : 0u;
+    }
+    s_sum[threadIdx.x] = sum; s_sum2[threadIdx.x] = sum2; s_max[threadIdx.x] = mx; s_above[threadIdx.x] = above;
+    __syncthreads();
+    for (uint32_t h = 128; h > 0; h >>= 1) {
+        if (threadIdx.x < h) {
+            s_sum[threadIdx.x] += s_sum[threadIdx.x + h]; s_sum2[threadIdx.x] += s_sum2[threadIdx.x + h];
+            s_max[threadIdx.x] = fmax(s_max[threadIdx.x], s_max[threadIdx.x + h]); s_above[threadIdx.x] += s_above[threadIdx.x + h];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) out[blockIdx.x] = RzNoisePartial{s_sum[0], s_sum2[0], s_max[0], s_above[0]};
+}
+
+extern "C" uint32_t rz_noise_grid(void) { return RZ_NOISE_GRID; }
+// out: RZ_NOISE_GRID x 4 words (sum, sum2, max as doubles, then the count as an integer)
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, uint32_t n_local_px, uint32_t n, double target, void *out,
+                                              cudaStream_t stream) {
+    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_local_px, n, target, (RzNoisePartial *)out);
     return cudaGetLastError();
 }
 

@@ -363,6 +363,8 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
         atomicAdd(acc + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.f), 1048576.f) * 4294967296.f));
         atomicAdd(acc + 1, __float2ull_rn(fminf(fmaxf(L.y, 0.f), 1048576.f) * 4294967296.f));
         atomicAdd(acc + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.f), 1048576.f) * 4294967296.f));
+        // the noise estimate's second moment (the only accumulation site besides the three above: every kernel shades here)
+        if (a.moments) atomicAdd(acc + 3, rz_fixed32(rz_luma_sq(rz_clamp_radiance(L.x), rz_clamp_radiance(L.y), rz_clamp_radiance(L.z))));
         return RZ_END_SKY;
     }
     const int k = bk & ~RZ_FAR_BIT;

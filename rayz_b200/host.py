@@ -225,6 +225,7 @@ class Backend:
         abi.check(self.lib.rayz_cuda_create(C.byref(cfg), C.byref(h)))
         self._h = h
         self.devices = tuple(devices)
+        self._acc_shape = None   # (height, width, shard_index, shard_count, band_rows) of the last successful render: noise()'s rows
 
     def close(self):
         if getattr(self, "_h", None):
@@ -276,7 +277,10 @@ class Backend:
 
     @staticmethod
     def params(width, height, spp, max_depth=50, seed=1, sample_offset=0, variant="auto", t_min=0.0, shard_index=0,
-               shard_count=1, band_rows=0, collect_stats=False, serial_passes=False) -> abi.RzRenderParams:
+               shard_count=1, band_rows=0, collect_stats=False, serial_passes=False, accumulate=False,
+               moments=False) -> abi.RzRenderParams:
+        """RzRenderParams.  accumulate: add this batch to the previous render's sums (RZ_RENDER_ACCUMULATE; sample_offset must
+        continue where they end); moments: also sum each path's luminance squared, so that noise() can estimate the error."""
         p = abi.RzRenderParams()
         p.width, p.height, p.spp, p.max_depth = width, height, spp, max_depth
         p.seed, p.sample_offset = seed, sample_offset
@@ -284,7 +288,8 @@ class Backend:
         p.t_min = t_min
         p.shard_index, p.shard_count, p.band_rows = shard_index, shard_count, band_rows
         p.collect_stats = 1 if collect_stats else 0
-        p.flags = 1 if serial_passes else 0   # RZ_RENDER_SERIAL_PASSES
+        p.flags = ((abi.RENDER_SERIAL_PASSES if serial_passes else 0) | (abi.RENDER_ACCUMULATE if accumulate else 0)
+                   | (abi.RENDER_MOMENTS if moments else 0))
         return p
 
     def reserve(self, p: abi.RzRenderParams):
@@ -306,6 +311,7 @@ class Backend:
         abi.check(self.lib.rayz_cuda_render(self._h, C.byref(cam), C.byref(p),
                                             out_linear.ctypes.data if want_linear else None,
                                             out_rgb8.ctypes.data if want_rgb8 else None, C.byref(n)))
+        self._acc_shape = (p.height, p.width, p.shard_index, p.shard_count, p.band_rows)
         return (out_linear if want_linear else None), (out_rgb8 if want_rgb8 else None), n.value
 
     def render_device(self, cam: abi.RzCamera, p: abi.RzRenderParams, sync=True):
@@ -313,7 +319,33 @@ class Backend:
         dl, d8, n = C.c_void_p(), C.c_void_p(), C.c_uint64()
         abi.check(self.lib.rayz_cuda_render_device(self._h, C.byref(cam), C.byref(p), C.byref(dl), C.byref(d8), C.byref(n),
                                                    1 if sync else 0))
+        self._acc_shape = (p.height, p.width, p.shard_index, p.shard_count, p.band_rows)
         return dl.value, d8.value, n.value
+
+    def noise(self, target: float = 0.0):
+        """rayz_cuda_noise: per-pixel standard error of the displayed value of the accumulated frame (needs moments=True) ->
+        (err [rows,w] f32, summary dict: samples, n_pixels, n_above (pixels with err > target), mean_err, rms_err, max_err)."""
+        nz = abi.RzNoise()
+        if self._acc_shape is None:   # nothing rendered: the library says why
+            abi.check(self.lib.rayz_cuda_noise(self._h, float(target), None, C.byref(nz)))
+        rows, w = int(self.lib.rayz_cuda_context_rows(self._h, self._acc_shape[0], *self._acc_shape[2:])), self._acc_shape[1]
+        err = np.empty((rows, w), dtype=np.float32)
+        abi.check(self.lib.rayz_cuda_noise(self._h, float(target), err.ctypes.data, C.byref(nz)))
+        return err, nz.as_dict()
+
+    def render_to_noise(self, cam: abi.RzCamera, p: abi.RzRenderParams, target: float, max_spp: int, want_linear=True,
+                        want_rgb8=True):
+        """rayz_cuda_render_to_noise: p.spp samples, then batches doubling the count until rms_err <= target or max_spp.
+        Returns (linear [rows,w,4] f32, rgb8 [rows,w,3] u8, paths, summary dict as noise())."""
+        rows = self.shard_rows(p)
+        lin = np.empty((rows, p.width, 4), dtype=np.float32) if want_linear else None
+        rgb8 = np.empty((rows, p.width, 3), dtype=np.uint8) if want_rgb8 else None
+        n, nz = C.c_uint64(), abi.RzNoise()
+        abi.check(self.lib.rayz_cuda_render_to_noise(self._h, C.byref(cam), C.byref(p), float(target), int(max_spp),
+                                                     lin.ctypes.data if want_linear else None,
+                                                     rgb8.ctypes.data if want_rgb8 else None, C.byref(n), C.byref(nz)))
+        self._acc_shape = (p.height, p.width, p.shard_index, p.shard_count, p.band_rows)
+        return lin, rgb8, n.value, nz.as_dict()
 
     def primary_ids(self, cam: abi.RzCamera, width: int, height: int, use_bvh=True) -> np.ndarray:
         out = np.empty((height, width), dtype=np.int32)
@@ -375,6 +407,7 @@ class Tracer:
         self.seed = seed           # the reference seeds from the OS (renderer.zig:55-59)
         self.variant = "auto"
         self.devices = devices
+        self.noise = None          # summary of the last render(noise_target=...) (rayz_cuda_render_to_noise)
         self._backend = None
 
     @property
@@ -383,11 +416,17 @@ class Tracer:
             self._backend = Backend(self.devices)
         return self._backend
 
-    def render(self) -> int:
+    def render(self, noise_target: float | None = None, max_spp: int = 4096) -> int:
+        """noise_target (displayed-value rms error, 1/255 = one 8-bit step): start at samples_per_px and double the samples
+        until the frame's rms error reaches it or max_spp samples are in (rayz_cuda_render_to_noise); `self.noise` then holds
+        the summary.  Without it, one render of samples_per_px, as the reference."""
         b = self.backend
         b.upload_scene(self.pool.arrays())  # initHittables + bvh.build (renderer.zig:76-78)
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant)
-        lin, rgb8, rays = b.render(self.camera.rz, p)
+        if noise_target is None:
+            lin, rgb8, rays = b.render(self.camera.rz, p)
+        else:
+            lin, rgb8, rays, self.noise = b.render_to_noise(self.camera.rz, p, noise_target, max_spp)
         self.img.pixels[:] = lin.reshape(-1, 4)[:, :3]
         self.img.rgb8 = rgb8
         return rays

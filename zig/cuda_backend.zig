@@ -71,6 +71,18 @@ pub const RzConfig = extern struct {
     flags: u32 = 0,
 };
 
+pub const RZ_RENDER_MOMENTS: u32 = 2; // sum each path's luminance squared: rayz_cuda_noise
+pub const RZ_RENDER_ACCUMULATE: u32 = 4; // add this batch to the previous render's sums (progressive rendering)
+
+pub const RzNoise = extern struct {
+    samples: u64,
+    n_pixels: u32,
+    n_above: u32,
+    mean_err: f64,
+    rms_err: f64,
+    max_err: f64,
+};
+
 pub const RzContext = opaque {};
 
 pub extern fn rayz_cuda_create(cfg: ?*const RzConfig, out: *?*RzContext) c_int;
@@ -79,6 +91,8 @@ pub extern fn rayz_cuda_reserve(ctx: *RzContext, params: *const RzRenderParams) 
 pub extern fn rayz_cuda_upload_scene(ctx: *RzContext, scene: *const RzScene) c_int;
 pub extern fn rayz_cuda_render(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8, out_paths: ?*u64) c_int;
 pub extern fn rayz_cuda_primary_ids(ctx: *RzContext, cam: *const RzCamera, width: u32, height: u32, use_bvh: c_int, out_ids: [*]i32) c_int;
+pub extern fn rayz_cuda_noise(ctx: *RzContext, target: f32, out_err: ?[*]f32, out: ?*RzNoise) c_int;
+pub extern fn rayz_cuda_render_to_noise(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, target: f32, max_spp: u32, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8, out_paths: ?*u64, out_noise: ?*RzNoise) c_int;
 pub extern fn rayz_cuda_last_error() [*:0]const u8;
 
 pub const Error = error{ CudaBackend, OutOfMemory };
