@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -84,10 +85,17 @@ struct DeviceGuard {
 };
 
 // ------------------------------------------------------------------------------ device state
+static const uint32_t RZ_MAX_DEVICES = 8;   // RzConfig::device_ids
+
+// A device allocation that frees itself; whoever destroys one makes its device current (Dev::~Dev).
 template <class T>
 struct DBuf {
     T *p = nullptr;
     size_t n = 0;
+    DBuf() = default;
+    DBuf(DBuf &&o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+    DBuf &operator=(DBuf &&o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+    ~DBuf() { release(); }
     int alloc(size_t count) {
         if (count <= n && p) return RZ_OK;
         release();
@@ -117,7 +125,6 @@ struct SetBufs {
         s.n = n; s.n_static = n_static; s.n_static_pad = n_static_pad; s.n_pad = n_pad;
         return s;
     }
-    void release() { cr.release(); vel.release(); pk.release(); c64.release(); v64.release(); mat.release(); orig.release(); }
 };
 
 struct Dev {
@@ -170,6 +177,21 @@ struct Dev {
     uint32_t queue_entries = 0;         // entries per queue buffer of the last render (0 = not the staged form)
     uint32_t passes = 0;                // passes of the last render (0 = not the staged form)
     bool serial_passes = false;
+
+    // With the device current and its streams drained; the DBuf members free themselves after this body.
+    ~Dev() {
+        if (!own_stream || cudaSetDevice(id) != cudaSuccess) return;   // (own_stream is the first handle rayz_cuda_create makes)
+        cudaStreamSynchronize(own_stream);
+        if (stream2) cudaStreamSynchronize(stream2);
+        if (wf_scratch) rz_wavefront_free(wf_scratch);
+        for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
+        for (cudaEvent_t e : pass_ev) cudaEventDestroy(e);
+        for (cudaEvent_t e : stage_ev) cudaEventDestroy(e);
+        if (ev_s2) cudaEventDestroy(ev_s2);
+        if (ev_tab) cudaEventDestroy(ev_tab);
+        if (stream2) cudaStreamDestroy(stream2);
+        cudaStreamDestroy(own_stream);
+    }
 };
 
 // What the accumulators of the context's devices hold (RZ_RENDER_ACCUMULATE, include/rayz_cuda.h): the frame, shard and
@@ -186,6 +208,7 @@ struct AccumRecord {
 };
 
 struct RzContext {
+    explicit RzContext(int n_devices) : devs(n_devices) {}
     std::vector<Dev> devs;
     AccumRecord acc;
     bool have_scene = false;
@@ -213,12 +236,18 @@ extern "C" uint32_t rayz_cuda_shard_rows(uint32_t height, uint32_t shard_index, 
     return rows;
 }
 
+// RzRenderParams' shard fields as every render reads them: shard_count 0 or 1 is the whole frame, band_rows 0 means 4.
+struct Shard {
+    uint32_t S, s, band;
+    Shard(uint32_t index, uint32_t count, uint32_t band_rows) : S(count <= 1 ? 1u : count), s(count <= 1 ? 0u : index), band(band_rows ? band_rows : 4u) {}
+};
+
 extern "C" uint32_t rayz_cuda_context_rows(const RzContext *ctx, uint32_t height, uint32_t shard_index, uint32_t shard_count,
                                            uint32_t band_rows) {
-    const uint32_t S = shard_count <= 1 ? 1 : shard_count, s = shard_count <= 1 ? 0 : shard_index;
+    const Shard sh(shard_index, shard_count, band_rows);
     const uint32_t nd = ctx ? (uint32_t)ctx->devs.size() : 1u;
     uint32_t rows = 0;
-    for (uint32_t d = 0; d < nd; d++) rows += rayz_cuda_shard_rows(height, s * nd + d, S * nd, band_rows ? band_rows : 4);
+    for (uint32_t d = 0; d < nd; d++) rows += rayz_cuda_shard_rows(height, sh.s * nd + d, sh.S * nd, sh.band);
     return rows;
 }
 
@@ -295,72 +324,49 @@ extern "C" int rayz_cuda_create(const RzConfig *cfg, RzContext **out) {
                        e == cudaSuccess ? "device count 0" : cudaGetErrorString(e));
     int nd = cfg ? cfg->n_devices : 1;
     if (nd <= 0) nd = 1;
-    if (nd > 8) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_create: n_devices %d > 8", nd);
+    if (nd > (int)RZ_MAX_DEVICES) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_create: n_devices %d > %u", nd, RZ_MAX_DEVICES);
     DeviceGuard guard;
-    RzContext *ctx = new RzContext();
+    std::unique_ptr<RzContext> ctx(new RzContext(nd));   // an error return tears down what was made so far (Dev::~Dev)
     ctx->flags = cfg ? cfg->flags : 0u;
     ctx->tun = default_tuning();
-    ctx->devs.resize(nd);
     for (int d = 0; d < nd; d++) {
         Dev &D = ctx->devs[d];
         D.id = cfg ? cfg->device_ids[d] : 0;
-        if (D.id < 0 || D.id >= count) { delete ctx; return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_create: device id %d out of range (have %d)", D.id, count); }
+        if (D.id < 0 || D.id >= count) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_create: device id %d out of range (have %d)", D.id, count);
         for (int q = 0; q < d; q++)
-            if (ctx->devs[q].id == D.id) { delete ctx; return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_create: device id %d listed twice", D.id); }
+            if (ctx->devs[q].id == D.id) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_create: device id %d listed twice", D.id);
     }
     for (int d = 0; d < nd; d++) {
         Dev &D = ctx->devs[d];
-        if ((e = cudaSetDevice(D.id)) != cudaSuccess) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "cudaSetDevice(%d): %s", D.id, cudaGetErrorString(e)); }
+        if ((e = cudaSetDevice(D.id)) != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "cudaSetDevice(%d): %s", D.id, cudaGetErrorString(e));
         cudaDeviceProp prop;
-        if ((e = cudaGetDeviceProperties(&prop, D.id)) != cudaSuccess) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "cudaGetDeviceProperties: %s", cudaGetErrorString(e)); }
-        if (prop.major < 10) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_UNSUPPORTED, "device %d is sm_%d%d; this library carries sm_100a code only", D.id, prop.major, prop.minor); }
+        if ((e = cudaGetDeviceProperties(&prop, D.id)) != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "cudaGetDeviceProperties: %s", cudaGetErrorString(e));
+        if (prop.major < 10) return rz_fail(RZ_ERR_UNSUPPORTED, "device %d is sm_%d%d; this library carries sm_100a code only", D.id, prop.major, prop.minor);
         D.sms = prop.multiProcessorCount;
-        if ((e = cudaStreamCreateWithFlags(&D.own_stream, cudaStreamNonBlocking)) != cudaSuccess) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e)); }
+        if ((e = cudaStreamCreateWithFlags(&D.own_stream, cudaStreamNonBlocking)) != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
         D.stream = D.own_stream;
         if ((e = cudaStreamCreateWithFlags(&D.stream2, cudaStreamNonBlocking)) != cudaSuccess || (e = cudaEventCreateWithFlags(&D.ev_s2, cudaEventDisableTiming)) != cudaSuccess ||
-            (e = cudaEventCreateWithFlags(&D.ev_tab, cudaEventDisableTiming)) != cudaSuccess) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e)); }
+            (e = cudaEventCreateWithFlags(&D.ev_tab, cudaEventDisableTiming)) != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
         for (auto &ev : D.ev)
-            if ((e = cudaEventCreate(&ev)) != cudaSuccess) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "cudaEventCreate: %s", cudaGetErrorString(e)); }
-        if ((e = rz_path_warm()) != cudaSuccess || (e = rz_bvh_warm()) != cudaSuccess || (e = rz_sort_warm()) != cudaSuccess) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "loading the path kernels: %s", cudaGetErrorString(e)); }
+            if ((e = cudaEventCreate(&ev)) != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "cudaEventCreate: %s", cudaGetErrorString(e));
+        if ((e = rz_path_warm()) != cudaSuccess || (e = rz_bvh_warm()) != cudaSuccess || (e = rz_sort_warm()) != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "loading the path kernels: %s", cudaGetErrorString(e));
         if (d > 0) {
             // the resolve kernel of device d stores straight into device 0's buffers (NVLink P2P)
             int can = 0;
             cudaDeviceCanAccessPeer(&can, D.id, ctx->devs[0].id);
-            if (!can) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_UNSUPPORTED, "device %d cannot access peer %d", D.id, ctx->devs[0].id); }
+            if (!can) return rz_fail(RZ_ERR_UNSUPPORTED, "device %d cannot access peer %d", D.id, ctx->devs[0].id);
             e = cudaDeviceEnablePeerAccess(ctx->devs[0].id, 0);
-            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) { rayz_cuda_destroy(ctx); return rz_fail(RZ_ERR_CUDA, "cudaDeviceEnablePeerAccess: %s", cudaGetErrorString(e)); }
+            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return rz_fail(RZ_ERR_CUDA, "cudaDeviceEnablePeerAccess: %s", cudaGetErrorString(e));
             cudaGetLastError();
         }
     }
-    *out = ctx;
+    *out = ctx.release();
     return RZ_OK;
 }
 
 extern "C" void rayz_cuda_destroy(RzContext *ctx) {
     if (!ctx) return;
     DeviceGuard guard;
-    for (Dev &D : ctx->devs) {
-        if (cudaSetDevice(D.id) != cudaSuccess) continue;
-        if (D.own_stream) cudaStreamSynchronize(D.own_stream);
-        D.brute.release(); D.bvhset.release(); D.bvh.release(); D.bvh4.release(); D.wide_scratch.release(); D.brute_to_bvh.release(); D.refnodes.release(); D.reforder.release();
-        D.c64_orig.release(); D.v64_orig.release(); D.mat_orig.release(); D.lbvh_scratch.release();
-        D.m_rec.release(); D.m_kind.release(); D.m_tex.release(); D.m_method.release(); D.t_kind.release(); D.t_even.release(); D.t_odd.release();
-        D.m_fuzz.release(); D.m_ior.release(); D.t_color.release(); D.t_inv_scale.release();
-        D.accum.release(); D.counter.release(); D.errword.release();
-        for (int sd = 0; sd < 2; sd++) { D.q1[sd].release(); D.q2[sd].release(); D.keys[sd].release(); D.idx_sorted[sd].release(); D.bins[sd].release(); }
-        D.bin_lists.release();
-        D.stats.release(); D.out_linear.release(); D.out_rgb8.release(); D.loc_linear.release(); D.loc_rgb8.release();
-        D.out_err.release(); D.noise_part.release();
-        D.ids.release(); D.sink.release();
-        if (D.wf_scratch) rz_wavefront_free(D.wf_scratch);
-        for (auto &ev : D.ev) if (ev) cudaEventDestroy(ev);
-        for (auto &ev : D.pass_ev) if (ev) cudaEventDestroy(ev);
-        for (auto &ev : D.stage_ev) if (ev) cudaEventDestroy(ev);
-        if (D.ev_s2) cudaEventDestroy(D.ev_s2);
-        if (D.ev_tab) cudaEventDestroy(D.ev_tab);
-        if (D.stream2) { cudaStreamSynchronize(D.stream2); cudaStreamDestroy(D.stream2); }
-        if (D.own_stream) cudaStreamDestroy(D.own_stream);
-    }
     delete ctx;
 }
 
@@ -421,6 +427,24 @@ extern "C" int rayz_cuda_set_tuning(RzContext *ctx, const RzTuning *t) {
 }
 
 static const uint32_t RZ_SMEM_BUDGET = 180u * 1024u;  // of 227 KB per CTA on sm_100: the set, + 25 % for the primary kernel's pair lists
+
+// Runs fn(d) for every device d of the context: inline for one device, else on one host thread PER DEVICE.  ~90 launches per
+// pass and device issued from a single thread made device 7 start milliseconds after device 0 (e2e 5 % below the
+// device-resident rate at 8 GPUs).  Returns the first failure in device order, with its message.
+template <class F>
+static int for_each_device(RzContext *ctx, F &&fn) {
+    const uint32_t nd = (uint32_t)ctx->devs.size();
+    if (nd == 1) return fn(0u);
+    int rcs[RZ_MAX_DEVICES] = {};
+    std::string errs[RZ_MAX_DEVICES];
+    std::thread workers[RZ_MAX_DEVICES];
+    for (uint32_t d = 0; d < nd; d++)
+        workers[d] = std::thread([&, d] { rcs[d] = fn(d); if (rcs[d]) errs[d] = g_err; });   // g_err is thread-local: hand the text over
+    for (uint32_t d = 0; d < nd; d++) workers[d].join();
+    for (uint32_t d = 0; d < nd; d++)
+        if (rcs[d]) return rz_fail(rcs[d], "%s", errs[d].c_str());
+    return RZ_OK;
+}
 
 extern "C" int rayz_cuda_upload_scene(RzContext *ctx, const RzScene *sc) {
     if (!ctx || !sc) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: NULL argument");
@@ -567,12 +591,13 @@ extern "C" int rayz_cuda_upload_scene(RzContext *ctx, const RzScene *sc) {
     }
 
     DeviceGuard guard;
-    // one host thread per device (as in render_impl): ~25 small copies and allocations each
-    auto upload_device = [&](Dev &D) -> int {
+    // one host thread per device (for_each_device): ~25 small copies and allocations each
+    auto upload_device = [&](uint32_t d) -> int {
+        Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
         int rc;
         if (upload_brute) { if ((rc = upload_set(D.brute, bs, D.stream))) return rc; }
-        else { D.brute.release(); D.brute.n = bs.n; D.brute.n_static = bs.n_static; D.brute.n_static_pad = bs.n_static_pad; D.brute.n_pad = bs.n_pad; }
+        else { D.brute = SetBufs(); D.brute.n = bs.n; D.brute.n_static = bs.n_static; D.brute.n_static_pad = bs.n_static_pad; D.brute.n_pad = bs.n_pad; }
         if ((rc = D.c64_orig.upload(c64o, D.stream))) return rc;
         if ((rc = D.v64_orig.upload(v64o, D.stream))) return rc;
         if ((rc = D.mat_orig.upload(mato, D.stream))) return rc;
@@ -610,21 +635,7 @@ extern "C" int rayz_cuda_upload_scene(RzContext *ctx, const RzScene *sc) {
             return rc;
         return RZ_OK;
     };
-    if (ctx->devs.size() == 1) {
-        const int rc = upload_device(ctx->devs[0]);
-        if (rc) return rc;
-    } else {
-        const size_t nd = ctx->devs.size();
-        std::vector<int> rcs(nd, RZ_OK);
-        std::vector<std::string> errs(nd);
-        std::vector<std::thread> workers;
-        workers.reserve(nd);
-        for (size_t d = 0; d < nd; d++)
-            workers.emplace_back([&, d] { rcs[d] = upload_device(ctx->devs[d]); if (rcs[d]) errs[d] = g_err; });
-        for (std::thread &w : workers) w.join();
-        for (size_t d = 0; d < nd; d++)
-            if (rcs[d]) return rz_fail(rcs[d], "%s", errs[d].c_str());
-    }
+    { const int rc = for_each_device(ctx, upload_device); if (rc) return rc; }
     for (Dev &D : ctx->devs) {   // every device's copies are in flight before the first wait
         RZ_CUDA(cudaSetDevice(D.id));
         RZ_CUDA(cudaStreamSynchronize(D.stream));  // host vectors die at return: copy semantics
@@ -655,7 +666,7 @@ static RzCamF32 cam_to_f32(const RzCamera *c) {
 }
 
 
-// Pass/queue sizing of the staged K1 (see render_impl).
+// Pass/queue sizing of the staged K1 (see enqueue_staged).
 struct QueuePlan {
     uint64_t unit_paths = 0, cap = 0;
     uint32_t units_per_pass = 1, n_pass = 1;
@@ -721,6 +732,20 @@ static int plan_and_alloc_queues(const RzTuning &tun, Dev &D, QueuePlan &qp, uin
     }
 }
 
+// Every device's error word (RZ_DEV_ERR_*), read behind everything enqueued on its streams: RZ_ERR_INTERNAL if one is set, as
+// a device-side capacity was exceeded and work was dropped.
+static int read_error_words(RzContext *ctx) {
+    for (Dev &D : ctx->devs) {
+        unsigned int ew = 0;
+        RZ_CUDA(cudaSetDevice(D.id));
+        RZ_CUDA(cudaMemcpyAsync(&ew, D.errword.p, sizeof ew, cudaMemcpyDeviceToHost, D.stream));
+        RZ_CUDA(cudaStreamSynchronize(D.stream));
+        if (ew) return rz_fail(RZ_ERR_INTERNAL, "render: device %d reported%s%s (error word 0x%x): paths were dropped, result withheld", D.id,
+                               (ew & RZ_DEV_ERR_QUEUE_OVERFLOW) ? " a queue overflow" : "", (ew & RZ_DEV_ERR_STACK_OVERFLOW) ? " a traversal-stack overflow" : "", ew);
+    }
+    return RZ_OK;
+}
+
 // Device timings (CUDA events) and, if asked for, the counters of the render that just finished on every stream.
 static int collect_timing_and_stats(RzContext *ctx, bool collect_stats) {
     float kmax = 0, rmax = 0, pmax = 0, smax = 0, somax = 0;
@@ -747,13 +772,7 @@ static int collect_timing_and_stats(RzContext *ctx, bool collect_stats) {
         kmax = std::max(kmax, k); rmax = std::max(rmax, r); pmax = std::max(pmax, pr); smax = std::max(smax, se); somax = std::max(somax, so);
         passes = std::max(passes, D.passes);
     }
-    for (Dev &D : ctx->devs) {   // a device-side capacity was exceeded: work was dropped, the result is not to be used
-        unsigned int ew = 0;
-        RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaMemcpy(&ew, D.errword.p, sizeof ew, cudaMemcpyDeviceToHost));
-        if (ew) return rz_fail(RZ_ERR_INTERNAL, "render: device %d reported%s%s (error word 0x%x): paths were dropped, result withheld", D.id,
-                               (ew & RZ_DEV_ERR_QUEUE_OVERFLOW) ? " a queue overflow" : "", (ew & RZ_DEV_ERR_STACK_OVERFLOW) ? " a traversal-stack overflow" : "", ew);
-    }
+    if (const int rc = read_error_words(ctx)) return rc;   // the result is not to be used
     ctx->timing.kernel_ms = kmax;
     ctx->timing.resolve_ms = rmax;
     ctx->timing.primary_ms = pmax;
@@ -791,15 +810,318 @@ static int collect_timing_and_stats(RzContext *ctx, bool collect_stats) {
 static int settle_accumulation(RzContext *ctx) {
     if (!ctx->acc.valid || !ctx->acc.pending) return RZ_OK;
     ctx->acc.valid = false;
-    for (Dev &D : ctx->devs) {
-        unsigned int ew = 0;
-        RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaStreamSynchronize(D.stream));
-        RZ_CUDA(cudaMemcpy(&ew, D.errword.p, sizeof ew, cudaMemcpyDeviceToHost));
-        if (ew) return RZ_OK;   // stays invalid
-    }
+    const int rc = read_error_words(ctx);
+    if (rc) return rc == RZ_ERR_INTERNAL ? RZ_OK : rc;   // an error word: stays invalid
     ctx->acc.valid = true;
     ctx->acc.pending = false;
+    return RZ_OK;
+}
+
+// ------------------------------------------------------------------------------ render plan
+struct DevPlan {
+    uint32_t rows = 0, n_local = 0, n_tiles = 0, n_units = 0;   // n_units: work units of the first kernel
+    QueuePlan qp;                                                // staged: the passes alloc_render could allocate
+};
+
+// What a render runs and needs, decided before any device is touched: render_impl is plan_render -> alloc_render -> enqueue,
+// rayz_cuda_reserve is plan_render -> alloc_render.
+struct RenderPlan {
+    const RzRenderParams *p = nullptr;
+    const RzCamera *cam = nullptr;   // nullptr: planned for rayz_cuda_reserve
+    bool host_direct = false;        // every device resolves into its OWN compact buffers; rayz_cuda_render copies them out in parallel
+    Shard sh{0, 1, 0};
+    uint32_t variant = 0, rows_ctx = 0;   // variant: resolved to RZ_VARIANT_MEGA, _BVH or _WAVEFRONT; rows_ctx: of all the devices
+    bool mega_single = false, staged = false;   // staged: enqueue_staged; else one kernel, or the wavefront's own loop
+    bool bvh_family = false, bvh_tail = false, enough_spheres = false, serial = false;   // the staged form's plan_queues inputs
+    uint32_t chunk = 0, n_chunks = 0, tile_w = 0;   // the first kernel's work-unit size; tile_w: staged K3's camera-stage blocks
+    DevPlan dev[RZ_MAX_DEVICES];
+    AccumRecord next;                   // what the render commits to ctx->acc when it succeeds
+    bool refused = false;               // an RZ_RENDER_ACCUMULATE batch that does not continue `prev`
+};
+
+// Plans a render of these parameters, with the validations (and messages) of rayz_cuda_render.  cam == nullptr plans for
+// rayz_cuda_reserve: no scene is needed and no accumulation record is made.
+static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, const AccumRecord &prev, RenderPlan &P) {
+    P.p = p;
+    P.cam = cam;
+    const char *who = cam ? "render" : "reserve";
+    if (cam && !ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "render: rayz_cuda_upload_scene has not been called");
+    if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "%s: width, height and spp must be > 0", who);
+    if ((uint64_t)p->width * p->height >= (1ull << 31)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: image too large", who);
+    P.sh = Shard(p->shard_index, p->shard_count, p->band_rows);
+    const uint32_t S = P.sh.S, s = P.sh.s, band = P.sh.band, ND = (uint32_t)ctx->devs.size();
+    if (s >= S) return rz_fail(RZ_ERR_INVALID_ARG, "%s: shard_index %u >= shard_count %u", who, s, S);
+    const Dev &D0 = ctx->devs[0];
+    const uint32_t brute_smem = (D0.brute.n_pad * 2 - D0.brute.n_static_pad) * 16u;
+    // Every kernel choice looks at the WHOLE FRAME (width x height x spp), never at this shard's or device's share of it: every
+    // shard of a frame runs the same kernels, so a sharded render equals the full-frame one bit for bit.
+    const uint64_t frame_paths = (uint64_t)p->width * p->height * p->spp;
+    P.variant = p->variant;
+    if (P.variant == RZ_VARIANT_AUTO) {
+        // AUTO picks by cost: the staged brute-force K1 when the sphere set fits shared memory AND the frame is big enough to
+        // amortise its ~25 launches per pass (measured one-shot, 485 spheres: 0.9 M paths 3.9 ms vs 0.8 ms for the BVH kernel,
+        // 8 M 6.3 vs 2.8, 81 M 23.8 vs 25.3, 405 M 104 vs 125); else the BVH kernel.  (The two kernel families themselves can
+        // differ in a pixel or two: FP32 sphere test against exact boxes, tests/test_gpu_parity.py.)
+        P.variant = (brute_smem <= RZ_SMEM_BUDGET && frame_paths >= (1ull << 26)) ? RZ_VARIANT_MEGA : RZ_VARIANT_BVH;
+    }
+    P.mega_single = P.variant == RZ_VARIANT_MEGA_SINGLE;
+    if (P.mega_single) P.variant = RZ_VARIANT_MEGA;
+    if (P.variant != RZ_VARIANT_MEGA && P.variant != RZ_VARIANT_BVH && P.variant != RZ_VARIANT_WAVEFRONT)
+        return rz_fail(RZ_ERR_INVALID_ARG, "%s: unknown variant %u", who, p->variant);
+    if (P.variant == RZ_VARIANT_MEGA && brute_smem > RZ_SMEM_BUDGET)
+        return rz_fail(RZ_ERR_UNSUPPORTED, "%s: scene needs %u B of shared memory for the brute-force kernel (budget %u); use RZ_VARIANT_BVH", who, brute_smem, RZ_SMEM_BUDGET);
+
+    if (cam) {
+        AccumRecord &next = P.next;
+        next.width = p->width; next.height = p->height; next.shard_index = s; next.shard_count = S; next.band_rows = band;
+        next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
+        next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
+        next.first_offset = p->sample_offset; next.samples = p->spp;
+        if (p->flags & RZ_RENDER_ACCUMULATE) {
+            auto refuse = [&](const char *why) { P.refused = true; return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ACCUMULATE refused: %s", why); };
+            if (!prev.valid) return refuse("no previous render to add to (none, it failed, or a scene upload or reserve came in between)");
+            if (prev.width != next.width || prev.height != next.height || prev.shard_index != s || prev.shard_count != S || prev.band_rows != band)
+                return refuse("frame size, shard or band_rows differ from the accumulated render");
+            if (prev.seed != next.seed || prev.max_depth != next.max_depth || memcmp(&prev.t_min, &next.t_min, sizeof(float)) != 0)
+                return refuse("seed, max_depth or t_min differ from the accumulated render");
+            if (memcmp(&prev.cam, cam, sizeof(RzCamera)) != 0) return refuse("the camera differs from the accumulated render");
+            if (prev.moments != next.moments) return refuse("the RZ_RENDER_MOMENTS bit differs from the accumulated render");
+            if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
+                return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
+            if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
+            next.first_offset = prev.first_offset;
+            next.samples = prev.samples + p->spp;
+        }
+    }
+
+    if (P.variant == RZ_VARIANT_BVH) {
+        // K3 on a big job: the same staged pipeline with BVH traversal instead of culled lists (sorted rays stay converged); the
+        // staged camera stage searches block lists, the unstaged kernel walks the tree
+        P.staged = ctx->tun.bvh_staged && frame_paths >= (1ull << 26);
+    } else if (P.variant == RZ_VARIANT_MEGA) {
+        // one persistent kernel for RZ_VARIANT_MEGA_SINGLE, or for a set whose pair lists do not fit beside the primary kernel
+        RzPathArgs probe;
+        memset(&probe, 0, sizeof probe);
+        probe.set = D0.brute.view();
+        P.staged = !P.mega_single && rz_primary_smem_bytes(&probe) <= 227u * 1024u;
+    }
+    if (P.staged) {
+        P.bvh_family = P.variant == RZ_VARIANT_BVH;
+        // The tail of the paths (whatever survives the sorted stages: incoherent, few) goes to the BVH kernel when the host-built
+        // tree is there — ~28 node + sphere tests per segment instead of every sphere of the set (config 2: 29.2 -> 11.1 ms
+        // behind four sorted stages).
+        P.bvh_tail = !P.bvh_family && D0.brute_to_bvh.p != nullptr && !ctx->tun.tail_brute;
+        P.enough_spheres = ctx->n_spheres >= 64u;
+        P.serial = (p->flags & RZ_RENDER_SERIAL_PASSES) != 0;
+        // The one guess: a reserve before the scene upload cannot know the set, the sphere count or whether there is a BVH tail.
+        // It plans the largest staged form (brute force with sorted stages and a BVH tail, both tilings' units); the first
+        // render still sizes the sorted stages' pair lists (a function of the set) and, if it runs more passes, their events.
+        if (!ctx->have_scene) { P.bvh_family = false; P.bvh_tail = true; P.enough_spheres = true; }
+        P.tile_w = P.bvh_family ? rz_bvh_camera_tile_w() : 0u;
+    }
+    const uint32_t chunk = std::min(ctx->tun.chunk, p->spp), n_chunks = (p->spp + chunk - 1) / chunk;
+    P.chunk = P.staged ? std::min(ctx->tun.chunk_primary, p->spp) : chunk;   // the camera-stage kernels build a culled sphere list per unit: their own, larger work-unit size
+    P.n_chunks = (p->spp + P.chunk - 1) / P.chunk;
+    for (uint32_t d = 0; d < ND; d++) {
+        DevPlan &dp = P.dev[d];
+        dp.rows = rayz_cuda_shard_rows(p->height, s * ND + d, S * ND, band);
+        dp.n_local = dp.rows * p->width;
+        dp.n_tiles = (dp.n_local + 31u) / 32u;
+        P.rows_ctx += dp.rows;
+        if ((uint64_t)dp.n_tiles * n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: too many work units", who);
+        uint64_t tiles = dp.n_tiles;
+        const uint64_t blocks = (uint64_t)((p->width + 7u) / 8u) * ((dp.rows + 3u) / 4u);   // K3's camera stage works on 8 x 4 pixel blocks
+        if (P.tile_w) tiles = blocks;
+        else if (P.staged && !ctx->have_scene) tiles = std::max(tiles, blocks);
+        if (tiles * P.n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: too many work units", who);
+        dp.n_units = (uint32_t)tiles * P.n_chunks;
+    }
+    return RZ_OK;
+}
+
+// Everything the plan needs on every device, so that enqueueing it allocates nothing.  The one exception is the wavefront
+// form's scratch, which rz_wavefront_render sizes itself.
+static int alloc_render(RzContext *ctx, RenderPlan &P) {
+    const uint32_t width = P.p->width;
+    int rc;
+    if (!P.host_direct) {   // the gather root's frame, into which every device's resolve scatters its rows
+        Dev &D0 = ctx->devs[0];
+        RZ_CUDA(cudaSetDevice(D0.id));
+        if ((rc = D0.out_linear.alloc((size_t)P.rows_ctx * width)) || (rc = D0.out_rgb8.alloc((size_t)P.rows_ctx * width * 3))) return rc;
+    }
+    for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {
+        Dev &D = ctx->devs[d];
+        DevPlan &dp = P.dev[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        if ((rc = D.accum.alloc((size_t)dp.n_tiles * 32u * 4u))) return rc;
+        if ((rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4))) return rc;
+        if ((rc = D.stats.alloc(3))) return rc;   // [0] whole render / primary kernel, [1] sorted stages, [2] persistent tail kernel
+        if (P.staged && dp.n_local > 0) {
+            if ((rc = plan_and_alloc_queues(ctx->tun, D, dp.qp, dp.n_units, P.chunk, P.serial, P.enough_spheres, P.bvh_family, P.bvh_tail))) return rc;
+            // the sorted-segment kernel's pair lists, one row per sort group
+            if (dp.qp.second_stage && !P.bvh_family && ctx->have_scene && (rc = D.bin_lists.alloc((size_t)RZ_SORT_BINS * rz_bin_row_bytes(D.brute.n_pad)))) return rc;
+            for (cudaEvent_t e = nullptr; D.pass_ev.size() < 3 * (size_t)dp.qp.n_pass; D.pass_ev.push_back(e)) RZ_CUDA(cudaEventCreate(&e));
+            for (cudaEvent_t e = nullptr; D.stage_ev.size() < 2 * (size_t)dp.qp.n_pass * dp.qp.n_second; D.stage_ev.push_back(e)) RZ_CUDA(cudaEventCreate(&e));
+        }
+        if (P.host_direct && ((rc = D.loc_linear.alloc((size_t)dp.n_local)) || (rc = D.loc_rgb8.alloc((size_t)dp.n_local * 3)))) return rc;
+    }
+    return RZ_OK;
+}
+
+// The staged form on one device: primary kernel (tile-culled camera segments; K3: the block-culled camera stage) -> queue ->
+// [sort -> sorted-segment kernel (culled per unit) -> queue] x n_second -> persistent tail kernel (BVH, or brute force).
+// Passes are sized by the queues (RzTuning::queue_log2, default 2^27 entries per buffer; two buffers per side, two sides).
+// collect_timing_and_stats reads pass_ev and stage_ev by index: their records belong to the streams and places they have here.
+static int enqueue_staged(RzContext *ctx, Dev &D, RzPathArgs a, const RenderPlan &P, const QueuePlan &qp, uint32_t &launches) {
+    const RzCamera *cam = P.cam;
+    const RzRenderParams *p = P.p;
+    const int n_sides = qp.n_sides, n_second = qp.n_second;
+    const double pcx = cam->px_origin[0] + 0.5 * (p->width - 1) * cam->px_du[0] + 0.5 * (p->height - 1) * cam->px_dv[0] - cam->look_from[0];
+    const double pcy = cam->px_origin[1] + 0.5 * (p->width - 1) * cam->px_du[1] + 0.5 * (p->height - 1) * cam->px_dv[1] - cam->look_from[1];
+    const double pcz = cam->px_origin[2] + 0.5 * (p->width - 1) * cam->px_du[2] + 0.5 * (p->height - 1) * cam->px_dv[2] - cam->look_from[2];
+    a.focus_dist = (float)std::sqrt(pcx * pcx + pcy * pcy + pcz * pcz);   // look_from -> centre of the focus plane
+    const double lu = std::sqrt(cam->defocus_u[0] * cam->defocus_u[0] + cam->defocus_u[1] * cam->defocus_u[1] + cam->defocus_u[2] * cam->defocus_u[2]);
+    const double lv = std::sqrt(cam->defocus_v[0] * cam->defocus_v[0] + cam->defocus_v[1] * cam->defocus_v[1] + cam->defocus_v[2] * cam->defocus_v[2]);
+    a.lens_radius = cam->defocus ? (float)(std::max(lu, lv) * 1.001) : 0.f;
+    a.queue_cap = ctx->tun.debug_queue_cap ? std::min((uint32_t)qp.cap, ctx->tun.debug_queue_cap) : (uint32_t)qp.cap;
+    rz_key_grid(a, ctx->sb_lo, ctx->sb_hi, ctx->tun.cell_bits, ctx->tun.key_sectors);
+    a.huge_radius = ctx->huge_radius;
+    uint32_t ue_div = 0;
+    if (qp.second_stage && !P.bvh_family) {
+        // the sorted-segment kernel's pair lists, one row per sort group: a function of the set and the key grid
+        a.bin_row = rz_bin_row_bytes(a.set.n_pad);
+        a.bin_lists = D.bin_lists.p;
+        RZ_CUDA(rz_launch_bin_lists(&a, D.sms, D.stream));
+        launches += 1;
+        int grid2 = 0;
+        RZ_CUDA(rz_second_grid(&a, (int)p->collect_stats, D.sms, &grid2));
+        ue_div = 16u * (uint32_t)grid2;
+    }
+    RZ_CUDA(cudaEventRecord(D.ev_tab, D.stream));
+    D.passes = qp.n_pass;
+    D.n_second = (uint32_t)n_second;
+    D.queue_entries = (uint32_t)qp.cap;
+    D.serial_passes = P.serial;
+    // Passes alternate between two streams and two sets of buffers: the persistent kernel ends with a tail of a few long paths
+    // (measured ~2 ms per pass), which the next pass's kernels fill.
+    if (n_sides > 1) RZ_CUDA(cudaStreamWaitEvent(D.stream2, D.ev_tab, 0));   // (recorded after ev[1] on the same stream)
+    uint32_t pass = 0;
+    for (uint32_t u0 = 0; u0 < a.n_units; u0 += qp.units_per_pass, pass++) {
+        const int side = n_sides > 1 ? (int)(pass & 1u) : 0;
+        cudaStream_t st = side ? D.stream2 : D.stream;
+        unsigned int *ctr = D.counter.p + 8 * side;   // [0..2] unit counters of K1a/K1c/K1b, [3] entries in q1, [4] entries in q2
+        if (pass >= (uint32_t)n_sides) RZ_CUDA(cudaMemsetAsync(ctr, 0, 8 * sizeof(unsigned int), st));
+        const uint32_t pass_units = std::min(qp.units_per_pass, a.n_units - u0);
+        RzPathArgs a1 = a;
+        a1.q_out = D.q1[side].p; a1.q_out_count = ctr + 3; a1.q_out_keys = qp.second_stage ? D.keys[side].p : nullptr;
+        a1.unit_base = u0; a1.n_units = pass_units; a1.unit_counter = ctr;
+        if (P.bvh_family) RZ_CUDA(rz_launch_bvh_stage(&a1, (int)p->collect_stats, D.sms, st));
+        else RZ_CUDA(rz_launch_primary(&a1, (int)p->collect_stats, D.sms, st));
+        RZ_CUDA(cudaEventRecord(D.pass_ev[3 * pass], st));
+        launches += 1;
+        RzPathArgs a3 = a;
+        a3.q_in = D.q1[side].p; a3.q_in_count = ctr + 3;
+        // sorted, culled stages for the next `n_second` segments: q1 -> q2 -> q1 -> ...
+        float4 *qa = D.q1[side].p, *qb = qp.second_stage ? D.q2[side].p : nullptr;
+        unsigned int *ca = ctr + 3, *cb = ctr + 4;
+        for (int stg = 0; stg < n_second; stg++) {
+            const bool more = stg + 1 < n_second;
+            // group the entries by key (rz_sort.cu: count / scan / scatter, sized on the device from the live count)
+            RZ_CUDA(rz_bin_sort(D.keys[side].p, ca, a.queue_cap, D.bins[side].p, nullptr, D.idx_sorted[side].p, a.unit_entries, ue_div, D.sms, st));
+            RZ_CUDA(cudaEventRecord(D.stage_ev[2 * ((size_t)pass * n_second + stg)], st));
+            if (stg > 0) RZ_CUDA(cudaMemsetAsync(cb, 0, sizeof(unsigned int), st));           // recycled output counter
+            if (stg > 0) RZ_CUDA(cudaMemsetAsync(ctr + 1, 0, sizeof(unsigned int), st));      // the stage's unit counter
+            RzPathArgs a2 = a;
+            a2.q_in = qa; a2.q_in_count = ca; a2.q_in_idx = D.idx_sorted[side].p; a2.q_in_bins = D.bins[side].p;
+            a2.q_out = qb; a2.q_out_count = cb; a2.q_out_keys = more ? D.keys[side].p : nullptr; a2.unit_counter = ctr + 1;
+            a2.stats = D.stats.p + 1;
+            if (P.bvh_family) RZ_CUDA(rz_launch_bvh_stage(&a2, (int)p->collect_stats, D.sms, st));
+            else RZ_CUDA(rz_launch_second(&a2, (int)p->collect_stats, D.sms, st));
+            RZ_CUDA(cudaEventRecord(D.stage_ev[2 * ((size_t)pass * n_second + stg) + 1], st));
+            launches += 4;   // count + scan + scatter (rz_sort.cu) + the sorted-segment kernel
+            std::swap(qa, qb); std::swap(ca, cb);
+        }
+        a3.q_in = qa; a3.q_in_count = ca;
+        RZ_CUDA(cudaEventRecord(D.pass_ev[3 * pass + 1], st));
+        a3.unit_counter = ctr + 2;
+        a3.stats = D.stats.p + 2;
+        if (P.bvh_tail) { a3.set = D.bvhset.view(); a3.self_map = D.brute_to_bvh.p; }
+        if (P.bvh_family || P.bvh_tail) RZ_CUDA(rz_launch_bvh(&a3, (int)p->collect_stats, D.sms, st));
+        else RZ_CUDA(rz_launch_path(&a3, ctx->tun.rays_per_thread, (int)p->collect_stats, D.sms, st, nullptr));
+        RZ_CUDA(cudaEventRecord(D.pass_ev[3 * pass + 2], st));
+        launches += 1;
+    }
+    if (n_sides > 1) {   // join the second stream before the resolve
+        RZ_CUDA(cudaEventRecord(D.ev_s2, D.stream2));
+        RZ_CUDA(cudaStreamWaitEvent(D.stream, D.ev_s2, 0));
+    }
+    return RZ_OK;
+}
+
+// Everything device d does for this render, enqueued on its streams into what alloc_render allocated.
+static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint32_t &launches) {
+    const RzRenderParams *p = P.p;
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    Dev &D = ctx->devs[d], &D0 = ctx->devs[0];
+    const DevPlan &dp = P.dev[d];
+    RZ_CUDA(cudaSetDevice(D.id));
+    RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
+    if (!(p->flags & RZ_RENDER_ACCUMULATE)) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
+    RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
+    RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
+    if (p->collect_stats) RZ_CUDA(cudaMemsetAsync(D.stats.p, 0, 3 * sizeof(RzStatsDev), D.stream));
+
+    RzPathArgs a;
+    memset(&a, 0, sizeof a);
+    a.set = (P.variant == RZ_VARIANT_BVH) ? D.bvhset.view() : D.brute.view();
+    a.mats.kind = D.m_kind.p; a.mats.fuzz = D.m_fuzz.p; a.mats.ior = D.m_ior.p; a.mats.tex = D.m_tex.p; a.mats.method = D.m_method.p; a.mats.rec = D.m_rec.p;
+    a.texs.kind = D.t_kind.p; a.texs.color = D.t_color.p; a.texs.inv_scale = D.t_inv_scale.p; a.texs.even = D.t_even.p; a.texs.odd = D.t_odd.p;
+#ifdef RZ_BVH_WIDE
+    a.bvh = D.bvh4.p; a.bvh_nodes = D.bvh_nodes;
+#else
+    a.bvh = D.bvh.p; a.bvh_nodes = D.bvh_nodes;
+#endif
+    a.cam = cam_to_f32(P.cam);
+    a.accum = D.accum.p; a.unit_counter = D.counter.p; a.stats = D.stats.p;
+    a.width = p->width; a.height = p->height; a.n_local_px = dp.n_local;
+    a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;
+    a.chunk = P.chunk; a.n_chunks = P.n_chunks; a.n_units = dp.n_units; a.tile_w = P.tile_w;
+    a.shard_index = P.sh.s * ND + d; a.shard_count = P.sh.S * ND; a.band_rows = P.sh.band;
+    a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
+    a.t_min = p->t_min > 0 ? p->t_min : 1e-4f;
+    a.err = D.errword.p;
+    a.unit_entries = ctx->tun.unit_entries;
+    a.bvh_active_min = (uint32_t)ctx->tun.bvh_active_min; a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
+    a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
+    a.moments = P.next.moments;
+
+    RZ_CUDA(cudaEventRecord(D.ev[1], D.stream));
+    D.passes = 0;
+    D.n_second = 0;
+    D.queue_entries = 0;
+    if (dp.n_local > 0 && P.staged) {
+        const int rc = enqueue_staged(ctx, D, a, P, dp.qp, launches);
+        if (rc) return rc;
+    } else if (dp.n_local > 0) {   // one kernel (the wavefront form counts its own launches)
+        uint32_t l = 1;
+        if (P.variant == RZ_VARIANT_WAVEFRONT) RZ_CUDA(rz_wavefront_render(&a, D.sms, (int)p->collect_stats, D.stream, &D.wf_scratch, &D.wf_scratch_bytes, &l));
+        else if (P.variant == RZ_VARIANT_BVH) RZ_CUDA(rz_launch_bvh(&a, (int)p->collect_stats, D.sms, D.stream));
+        else RZ_CUDA(rz_launch_path(&a, ctx->tun.rays_per_thread, (int)p->collect_stats, D.sms, D.stream, nullptr));
+        launches += l;
+    }
+    RZ_CUDA(cudaEventRecord(D.ev[2], D.stream));
+
+    RzResolveArgs r;
+    r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p; r.out_err = nullptr;
+    r.n_local_px = dp.n_local; r.width = p->width; r.spp = (uint32_t)P.next.samples;   // cumulative with RZ_RENDER_ACCUMULATE
+    r.dev_index = d; r.dev_count = ND; r.band_rows = P.sh.band;
+    if (P.host_direct) {
+        r.out_linear = D.loc_linear.p; r.out_rgb8 = D.loc_rgb8.p; r.dev_index = 0; r.dev_count = 1;
+        D.loc_rows = dp.rows;
+    }
+    RZ_CUDA(rz_launch_resolve(&r, D.stream));
+    if (dp.n_local > 0) launches += 1;
+    RZ_CUDA(cudaEventRecord(D.ev[3], D.stream));
     return RZ_OK;
 }
 
@@ -807,305 +1129,43 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "render: NULL argument");
     // Every render ends what the accumulators held unless it succeeds (the record is committed at the end) or it is an
     // RZ_RENDER_ACCUMULATE batch that is refused before anything was touched (the record is restored).
-    const bool accumulate = (p->flags & RZ_RENDER_ACCUMULATE) != 0;
-    if (accumulate) { DeviceGuard g; const int rc = settle_accumulation(ctx); if (rc) return rc; }
+    if (p->flags & RZ_RENDER_ACCUMULATE) { DeviceGuard g; const int rc = settle_accumulation(ctx); if (rc) return rc; }
     const AccumRecord prev = ctx->acc;
     ctx->acc.valid = false;
-    if (!ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "render: rayz_cuda_upload_scene has not been called");
-    if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "render: width, height and spp must be > 0");
-    if ((uint64_t)p->width * p->height >= (1ull << 31)) return rz_fail(RZ_ERR_INVALID_ARG, "render: image too large");
-    const uint32_t S = p->shard_count <= 1 ? 1 : p->shard_count;
-    const uint32_t s = p->shard_count <= 1 ? 0 : p->shard_index;
-    if (s >= S) return rz_fail(RZ_ERR_INVALID_ARG, "render: shard_index %u >= shard_count %u", s, S);
-    const uint32_t band = p->band_rows ? p->band_rows : 4;
-    const uint32_t ND = (uint32_t)ctx->devs.size();
-    uint32_t variant = p->variant;
-    const uint32_t brute_smem = (ctx->devs[0].brute.n_pad * 2 - ctx->devs[0].brute.n_static_pad) * 16u;
-    if (variant == RZ_VARIANT_AUTO) {
-        // AUTO picks by cost: the staged brute-force K1 when the sphere set fits shared memory AND the frame is big enough to
-        // amortise its ~25 launches per pass (measured one-shot, 485 spheres: 0.9 M paths 3.9 ms vs 0.8 ms for the BVH kernel,
-        // 8 M 6.3 vs 2.8, 81 M 23.8 vs 25.3, 405 M 104 vs 125); else the BVH kernel.  The choice looks at the WHOLE FRAME
-        // (width x height x spp), never at this shard's or device's share of it: every shard of a frame runs the same
-        // kernels, so a sharded render equals the full-frame one bit for bit (the two kernel families themselves can
-        // differ in a pixel or two: FP32 sphere test against exact boxes, tests/test_gpu_parity.py).
-        const uint64_t frame_paths = (uint64_t)p->width * p->height * p->spp;
-        variant = (brute_smem <= RZ_SMEM_BUDGET && frame_paths >= (1ull << 26)) ? RZ_VARIANT_MEGA : RZ_VARIANT_BVH;
+    RenderPlan P;
+    if (const int rc = plan_render(ctx, cam, p, prev, P)) {
+        if (P.refused) ctx->acc = prev;
+        return rc;
     }
-    const bool mega_single = variant == RZ_VARIANT_MEGA_SINGLE;
-    if (mega_single) variant = RZ_VARIANT_MEGA;
-    if (variant != RZ_VARIANT_MEGA && variant != RZ_VARIANT_BVH && variant != RZ_VARIANT_WAVEFRONT)
-        return rz_fail(RZ_ERR_INVALID_ARG, "render: unknown variant %u", p->variant);
-    if (variant == RZ_VARIANT_MEGA && brute_smem > RZ_SMEM_BUDGET)
-        return rz_fail(RZ_ERR_UNSUPPORTED, "render: scene needs %u B of shared memory for the brute-force kernel (budget %u); use RZ_VARIANT_BVH", brute_smem, RZ_SMEM_BUDGET);
-
-    AccumRecord next;
-    next.width = p->width; next.height = p->height; next.shard_index = s; next.shard_count = S; next.band_rows = band;
-    next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
-    next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
-    next.first_offset = p->sample_offset; next.samples = p->spp;
-    if (accumulate) {
-        auto refuse = [&](const char *why) { ctx->acc = prev; return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ACCUMULATE refused: %s", why); };
-        if (!prev.valid) return refuse("no previous render to add to (none, it failed, or a scene upload or reserve came in between)");
-        if (prev.width != next.width || prev.height != next.height || prev.shard_index != s || prev.shard_count != S || prev.band_rows != band)
-            return refuse("frame size, shard or band_rows differ from the accumulated render");
-        if (prev.seed != next.seed || prev.max_depth != next.max_depth || memcmp(&prev.t_min, &next.t_min, sizeof(float)) != 0)
-            return refuse("seed, max_depth or t_min differ from the accumulated render");
-        if (memcmp(&prev.cam, cam, sizeof(RzCamera)) != 0) return refuse("the camera differs from the accumulated render");
-        if (prev.moments != next.moments) return refuse("the RZ_RENDER_MOMENTS bit differs from the accumulated render");
-        if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
-            return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
-        if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
-        next.first_offset = prev.first_offset;
-        next.samples = prev.samples + p->spp;
-    }
+    P.host_direct = host_direct;
 
     const auto t_host0 = std::chrono::steady_clock::now();
     DeviceGuard guard;
-    const uint32_t rows_ctx = [&] { uint32_t r = 0; for (uint32_t d = 0; d < ND; d++) r += rayz_cuda_shard_rows(p->height, s * ND + d, S * ND, band); return r; }();
-    Dev &D0 = ctx->devs[0];
-    RZ_CUDA(cudaSetDevice(D0.id));
-    if (!host_direct) {
-        int rc;
-        if ((rc = D0.out_linear.alloc((size_t)rows_ctx * p->width))) return rc;
-        if ((rc = D0.out_rgb8.alloc((size_t)rows_ctx * p->width * 3))) return rc;
-    }
-    // Everything one device needs for this render, enqueued on its streams.  A context with several devices runs this on one
-    // host thread PER DEVICE: ~90 launches per pass and device issued from a single thread made device 7 start milliseconds
-    // after device 0 (e2e 5 % below the device-resident rate at 8 GPUs).
-    std::vector<uint32_t> launches_dev(ND, 0u);
-    auto per_device = [&](uint32_t d) -> int {
-        uint32_t &launches = launches_dev[d];
-        Dev &D = ctx->devs[d];
-        RZ_CUDA(cudaSetDevice(D.id));
-        const uint32_t sh_index = s * ND + d, sh_count = S * ND;
-        const uint32_t rows = rayz_cuda_shard_rows(p->height, sh_index, sh_count, band);
-        const uint32_t n_local = rows * p->width;
-        const uint32_t n_tiles = (n_local + 31u) / 32u;
-        int rc;
-        if ((rc = D.accum.alloc((size_t)n_tiles * 32u * 4u))) return rc;
-        if ((rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4))) return rc;
-        if ((rc = D.stats.alloc(3))) return rc;   // [0] whole render / primary kernel, [1] sorted stages, [2] persistent tail kernel
-        RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
-        if (!accumulate) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
-        RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
-        RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
-        if (p->collect_stats) RZ_CUDA(cudaMemsetAsync(D.stats.p, 0, 3 * sizeof(RzStatsDev), D.stream));
-
-        RzPathArgs a;
-        memset(&a, 0, sizeof a);
-        a.set = (variant == RZ_VARIANT_BVH) ? D.bvhset.view() : D.brute.view();
-        a.mats.kind = D.m_kind.p; a.mats.fuzz = D.m_fuzz.p; a.mats.ior = D.m_ior.p; a.mats.tex = D.m_tex.p; a.mats.method = D.m_method.p; a.mats.rec = D.m_rec.p;
-        a.texs.kind = D.t_kind.p; a.texs.color = D.t_color.p; a.texs.inv_scale = D.t_inv_scale.p; a.texs.even = D.t_even.p; a.texs.odd = D.t_odd.p;
-#ifdef RZ_BVH_WIDE
-        a.bvh = D.bvh4.p; a.bvh_nodes = D.bvh_nodes;
-#else
-        a.bvh = D.bvh.p; a.bvh_nodes = D.bvh_nodes;
-#endif
-        a.cam = cam_to_f32(cam);
-        a.accum = D.accum.p; a.unit_counter = D.counter.p; a.stats = D.stats.p;
-        a.width = p->width; a.height = p->height; a.n_local_px = n_local;
-        a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;
-        a.chunk = std::min(ctx->tun.chunk, p->spp);
-        a.n_chunks = (p->spp + a.chunk - 1) / a.chunk;
-        if ((uint64_t)n_tiles * a.n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "render: too many work units");
-        a.n_units = n_tiles * a.n_chunks;
-        a.shard_index = sh_index; a.shard_count = sh_count; a.band_rows = band;
-        a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
-        a.t_min = p->t_min > 0 ? p->t_min : 1e-4f;
-        a.err = D.errword.p;
-        a.unit_entries = ctx->tun.unit_entries;
-        a.bvh_active_min = (uint32_t)ctx->tun.bvh_active_min; a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
-        a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
-        a.moments = next.moments;
-
-        RZ_CUDA(cudaEventRecord(D.ev[1], D.stream));
-        D.passes = 0;
-        D.n_second = 0;
-        D.queue_entries = 0;
-        if (n_local > 0) {
-            if (variant == RZ_VARIANT_WAVEFRONT) {
-                uint32_t l = 0;
-                RZ_CUDA(rz_wavefront_render(&a, D.sms, (int)p->collect_stats, D.stream, &D.wf_scratch, &D.wf_scratch_bytes, &l));
-                launches += l;
-            } else {
-                // K3 on a big job: the same staged pipeline with BVH traversal instead of culled lists (sorted rays stay converged)
-                const bool bvh_family = variant == RZ_VARIANT_BVH;
-                const bool bvh_staged = bvh_family && ctx->tun.bvh_staged && (uint64_t)p->width * p->height * p->spp >= (1ull << 26);   // by the FRAME's size, never a shard's: every shard of a frame runs the same kernels (the staged camera stage searches block lists, the unstaged kernel walks the tree)
-                if (bvh_family && !bvh_staged) {
-                    RZ_CUDA(rz_launch_bvh(&a, (int)p->collect_stats, D.sms, D.stream));
-                    launches += 1;
-                } else if (!bvh_family && (mega_single || rz_primary_smem_bytes(&a) > 227u * 1024u)) {
-                    // one persistent kernel (RZ_VARIANT_MEGA_SINGLE, or a set whose pair lists do not fit beside it)
-                    RZ_CUDA(rz_launch_path(&a, ctx->tun.rays_per_thread, (int)p->collect_stats, D.sms, D.stream, nullptr));
-                    launches += 1;
-                } else {
-                    // staged K1: primary kernel (tile-culled camera segments) -> queue -> [sort -> sorted-segment kernel (culled per
-                    // unit) -> queue] x n_second -> persistent tail kernel (BVH, or brute force).  Passes are sized by the queues
-                    // (RzTuning::queue_log2, default 2^27 entries per buffer; two buffers per side, two sides).
-                    const bool serial = (p->flags & RZ_RENDER_SERIAL_PASSES) != 0;
-                    {   // the camera-stage kernels build a culled sphere list per unit: their own, larger work-unit size
-                        a.chunk = std::min(ctx->tun.chunk_primary, p->spp);
-                        a.n_chunks = (p->spp + a.chunk - 1) / a.chunk;
-                        uint64_t tiles = n_tiles;
-                        if (bvh_family && rz_bvh_camera_tile_w()) {   // K3's camera stage works on 8 x 4 pixel blocks
-                            a.tile_w = rz_bvh_camera_tile_w();
-                            tiles = (uint64_t)((p->width + 7u) / 8u) * ((n_local / p->width + 3u) / 4u);
-                        }
-                        if (tiles * a.n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "render: too many work units");
-                        a.n_units = (uint32_t)tiles * a.n_chunks;
-                    }
-                    // The tail of the paths (whatever survives the sorted stages: incoherent, few) goes to the BVH kernel when the
-                    // host-built tree is there — ~28 node + sphere tests per segment instead of every sphere of the set
-                    // (config 2: 29.2 -> 11.1 ms behind four sorted stages).
-                    const bool bvh_tail = !bvh_family && D.brute_to_bvh.p != nullptr && !ctx->tun.tail_brute;
-                    QueuePlan qp;
-                    if ((rc = plan_and_alloc_queues(ctx->tun, D, qp, a.n_units, a.chunk, serial, ctx->n_spheres >= 64u, bvh_family, bvh_tail))) return rc;
-                    const uint64_t unit_paths = qp.unit_paths, cap = qp.cap;
-                    const uint32_t units_per_pass = qp.units_per_pass, total_units = a.n_units, n_pass = qp.n_pass;
-                    const int n_sides = qp.n_sides, n_second = qp.n_second;
-                    const bool second_stage = qp.second_stage;
-                    const double pcx = cam->px_origin[0] + 0.5 * (p->width - 1) * cam->px_du[0] + 0.5 * (p->height - 1) * cam->px_dv[0] - cam->look_from[0];
-                    const double pcy = cam->px_origin[1] + 0.5 * (p->width - 1) * cam->px_du[1] + 0.5 * (p->height - 1) * cam->px_dv[1] - cam->look_from[1];
-                    const double pcz = cam->px_origin[2] + 0.5 * (p->width - 1) * cam->px_du[2] + 0.5 * (p->height - 1) * cam->px_dv[2] - cam->look_from[2];
-                    a.focus_dist = (float)std::sqrt(pcx * pcx + pcy * pcy + pcz * pcz);   // look_from -> centre of the focus plane
-                    const double lu = std::sqrt(cam->defocus_u[0] * cam->defocus_u[0] + cam->defocus_u[1] * cam->defocus_u[1] + cam->defocus_u[2] * cam->defocus_u[2]);
-                    const double lv = std::sqrt(cam->defocus_v[0] * cam->defocus_v[0] + cam->defocus_v[1] * cam->defocus_v[1] + cam->defocus_v[2] * cam->defocus_v[2]);
-                    a.lens_radius = cam->defocus ? (float)(std::max(lu, lv) * 1.001) : 0.f;
-                    a.queue_cap = ctx->tun.debug_queue_cap ? std::min((uint32_t)cap, ctx->tun.debug_queue_cap) : (uint32_t)cap;
-                    rz_key_grid(a, ctx->sb_lo, ctx->sb_hi, ctx->tun.cell_bits, ctx->tun.key_sectors);
-                    a.huge_radius = ctx->huge_radius;
-                    uint32_t ue_div = 0;
-                    if (second_stage && !bvh_family) {
-                        // the sorted-segment kernel's pair lists, one row per sort group: a function of the set and the key grid
-                        a.bin_row = rz_bin_row_bytes(a.set.n_pad);
-                        if (int rc = D.bin_lists.alloc((size_t)RZ_SORT_BINS * a.bin_row)) return rc;
-                        a.bin_lists = D.bin_lists.p;
-                        RZ_CUDA(rz_launch_bin_lists(&a, D.sms, D.stream));
-                        launches += 1;
-                        int grid2 = 0;
-                        RZ_CUDA(rz_second_grid(&a, (int)p->collect_stats, D.sms, &grid2));
-                        ue_div = 16u * (uint32_t)grid2;
-                    }
-                    RZ_CUDA(cudaEventRecord(D.ev_tab, D.stream));
-                    while (D.pass_ev.size() < 3 * (size_t)n_pass) {
-                        cudaEvent_t e = nullptr;
-                        RZ_CUDA(cudaEventCreate(&e));
-                        D.pass_ev.push_back(e);
-                    }
-                    while (D.stage_ev.size() < 2 * (size_t)n_pass * (size_t)n_second) {
-                        cudaEvent_t e = nullptr;
-                        RZ_CUDA(cudaEventCreate(&e));
-                        D.stage_ev.push_back(e);
-                    }
-                    D.passes = n_pass;
-                    D.n_second = (uint32_t)n_second;
-                    D.queue_entries = (uint32_t)cap;
-                    D.serial_passes = serial;
-                    // Passes alternate between two streams and two sets of buffers: the persistent kernel ends with a tail of a
-                    // few long paths (measured ~2 ms per pass), which the next pass's kernels fill.
-                    if (n_sides > 1) RZ_CUDA(cudaStreamWaitEvent(D.stream2, D.ev_tab, 0));   // (recorded after ev[1] on the same stream)
-                    uint32_t pass = 0;
-                    for (uint32_t u0 = 0; u0 < total_units; u0 += units_per_pass, pass++) {
-                        const int side = n_sides > 1 ? (int)(pass & 1u) : 0;
-                        cudaStream_t st = side ? D.stream2 : D.stream;
-                        unsigned int *ctr = D.counter.p + 8 * side;   // [0..2] unit counters of K1a/K1c/K1b, [3] entries in q1, [4] entries in q2
-                        if (pass >= (uint32_t)n_sides) RZ_CUDA(cudaMemsetAsync(ctr, 0, 8 * sizeof(unsigned int), st));
-                        const uint32_t pass_units = std::min(units_per_pass, total_units - u0);
-                        RzPathArgs a1 = a;
-                        a1.q_out = D.q1[side].p; a1.q_out_count = ctr + 3; a1.q_out_keys = second_stage ? D.keys[side].p : nullptr;
-                        a1.unit_base = u0; a1.n_units = pass_units; a1.unit_counter = ctr;
-                        if (bvh_family) RZ_CUDA(rz_launch_bvh_stage(&a1, (int)p->collect_stats, D.sms, st));
-                        else RZ_CUDA(rz_launch_primary(&a1, (int)p->collect_stats, D.sms, st));
-                        RZ_CUDA(cudaEventRecord(D.pass_ev[3 * pass], st));
-                        launches += 1;
-                        RzPathArgs a3 = a;
-                        a3.q_in = D.q1[side].p; a3.q_in_count = ctr + 3;
-                        // sorted, culled stages for the next `n_second` segments: q1 -> q2 -> q1 -> ...
-                        float4 *qa = D.q1[side].p, *qb = second_stage ? D.q2[side].p : nullptr;
-                        unsigned int *ca = ctr + 3, *cb = ctr + 4;
-                        for (int stg = 0; stg < n_second; stg++) {
-                            const bool more = stg + 1 < n_second;
-                            // group the entries by key (rz_sort.cu: count / scan / scatter, sized on the device from the live count)
-                            RZ_CUDA(rz_bin_sort(D.keys[side].p, ca, a.queue_cap, D.bins[side].p, nullptr, D.idx_sorted[side].p, a.unit_entries, ue_div, D.sms, st));
-                            RZ_CUDA(cudaEventRecord(D.stage_ev[2 * ((size_t)pass * n_second + stg)], st));
-                            if (stg > 0) RZ_CUDA(cudaMemsetAsync(cb, 0, sizeof(unsigned int), st));           // recycled output counter
-                            if (stg > 0) RZ_CUDA(cudaMemsetAsync(ctr + 1, 0, sizeof(unsigned int), st));      // the stage's unit counter
-                            RzPathArgs a2 = a;
-                            a2.q_in = qa; a2.q_in_count = ca; a2.q_in_idx = D.idx_sorted[side].p; a2.q_in_bins = D.bins[side].p;
-                            a2.q_out = qb; a2.q_out_count = cb; a2.q_out_keys = more ? D.keys[side].p : nullptr; a2.unit_counter = ctr + 1;
-                            a2.stats = D.stats.p + 1;
-                            if (bvh_family) RZ_CUDA(rz_launch_bvh_stage(&a2, (int)p->collect_stats, D.sms, st));
-                            else RZ_CUDA(rz_launch_second(&a2, (int)p->collect_stats, D.sms, st));
-                            RZ_CUDA(cudaEventRecord(D.stage_ev[2 * ((size_t)pass * n_second + stg) + 1], st));
-                            launches += 4;   // count + scan + scatter (rz_sort.cu) + the sorted-segment kernel
-                            std::swap(qa, qb); std::swap(ca, cb);
-                        }
-                        a3.q_in = qa; a3.q_in_count = ca;
-                        RZ_CUDA(cudaEventRecord(D.pass_ev[3 * pass + 1], st));
-                        a3.unit_counter = ctr + 2;
-                        a3.stats = D.stats.p + 2;
-                        if (bvh_tail) { a3.set = D.bvhset.view(); a3.self_map = D.brute_to_bvh.p; }
-                        if (bvh_family || bvh_tail) RZ_CUDA(rz_launch_bvh(&a3, (int)p->collect_stats, D.sms, st));
-                        else RZ_CUDA(rz_launch_path(&a3, ctx->tun.rays_per_thread, (int)p->collect_stats, D.sms, st, nullptr));
-                        RZ_CUDA(cudaEventRecord(D.pass_ev[3 * pass + 2], st));
-                        launches += 1;
-                    }
-                    if (n_sides > 1) {   // join the second stream before the resolve
-                        RZ_CUDA(cudaEventRecord(D.ev_s2, D.stream2));
-                        RZ_CUDA(cudaStreamWaitEvent(D.stream, D.ev_s2, 0));
-                    }
-                }
-            }
-        }
-        RZ_CUDA(cudaEventRecord(D.ev[2], D.stream));
-
-        RzResolveArgs r;
-        r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p; r.out_err = nullptr;
-        r.n_local_px = n_local; r.width = p->width; r.spp = (uint32_t)next.samples;   // cumulative with RZ_RENDER_ACCUMULATE
-        r.dev_index = d; r.dev_count = ND; r.band_rows = band;
-        if (host_direct) {   // every device resolves into its OWN compact buffers; rayz_cuda_render copies them out in parallel
-            if ((rc = D.loc_linear.alloc((size_t)n_local)) || (rc = D.loc_rgb8.alloc((size_t)n_local * 3))) return rc;
-            r.out_linear = D.loc_linear.p; r.out_rgb8 = D.loc_rgb8.p; r.dev_index = 0; r.dev_count = 1;
-            D.loc_rows = rows;
-        }
-        RZ_CUDA(rz_launch_resolve(&r, D.stream));
-        if (n_local > 0) launches += 1;
-        RZ_CUDA(cudaEventRecord(D.ev[3], D.stream));
-        return RZ_OK;
-    };
-    if (ND == 1) {
-        const int rc = per_device(0);
-        if (rc) return rc;
-    } else {
-        std::vector<int> rcs(ND, RZ_OK);
-        std::vector<std::string> errs(ND);
-        std::vector<std::thread> workers;
-        workers.reserve(ND);
-        for (uint32_t d = 0; d < ND; d++)
-            workers.emplace_back([&, d] { rcs[d] = per_device(d); if (rcs[d]) errs[d] = g_err; });   // g_err is thread-local: hand the text over
-        for (std::thread &w : workers) w.join();
-        for (uint32_t d = 0; d < ND; d++)
-            if (rcs[d]) return rz_fail(rcs[d], "%s", errs[d].c_str());
-    }
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    uint32_t launches_dev[RZ_MAX_DEVICES] = {};
+    int rc = alloc_render(ctx, P);
+    if (!rc) rc = for_each_device(ctx, [&](uint32_t d) { return enqueue_device(ctx, P, d, launches_dev[d]); });
+    if (rc) return rc;
     uint32_t launches = 0;
     for (uint32_t d = 0; d < ND; d++) launches += launches_dev[d];
     // gather root waits for every peer's resolve (which already wrote into its memory)
+    Dev &D0 = ctx->devs[0];
     RZ_CUDA(cudaSetDevice(D0.id));
     for (uint32_t d = 1; d < ND; d++) RZ_CUDA(cudaStreamWaitEvent(D0.stream, ctx->devs[d].ev[3], 0));
     RZ_CUDA(cudaEventRecord(D0.ev[4], D0.stream));
 
     ctx->timing.launches = launches;
-    ctx->timing.variant = mega_single ? (uint32_t)RZ_VARIANT_MEGA_SINGLE : variant;
+    ctx->timing.variant = P.mega_single ? (uint32_t)RZ_VARIANT_MEGA_SINGLE : P.variant;
     ctx->stats_valid = false;
     if (sync) {
         for (uint32_t d = 0; d < ND; d++) {
             RZ_CUDA(cudaSetDevice(ctx->devs[d].id));
             RZ_CUDA(cudaStreamSynchronize(ctx->devs[d].stream));
         }
-        { const int rc = collect_timing_and_stats(ctx, p->collect_stats != 0); if (rc) return rc; }
+        if ((rc = collect_timing_and_stats(ctx, p->collect_stats != 0))) return rc;
         ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host0).count();
     }
-    ctx->acc = next;
+    ctx->acc = P.next;
     ctx->acc.valid = true;
     ctx->acc.pending = !sync;
     return RZ_OK;
@@ -1113,36 +1173,20 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
 
 // Pre-allocates what a render with these parameters will need (accumulators, result buffers, the staged K1's queues), so
 // that the first render does not pay cudaMalloc for ~40 GB: the counterpart of Image.initEmpty in Tracer.init
-// (renderer.zig:29-64, image.zig:10-17), which the reference also does before main starts its timer.
+// (renderer.zig:29-64, image.zig:10-17), which the reference also does before main starts its timer.  A first render still
+// allocates the wavefront scratch, its own rows when several devices render into page-locked host buffers (render_host) and,
+// after a reserve made before the scene upload, what plan_render's one guess could not know.
 extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     if (!ctx || !p) return rz_fail(RZ_ERR_INVALID_ARG, "reserve: NULL argument");
-    if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "reserve: width, height and spp must be > 0");
-    const uint32_t S = p->shard_count <= 1 ? 1 : p->shard_count, s = p->shard_count <= 1 ? 0 : p->shard_index;
-    if (s >= S) return rz_fail(RZ_ERR_INVALID_ARG, "reserve: shard_index %u >= shard_count %u", s, S);
-    const uint32_t band = p->band_rows ? p->band_rows : 4, ND = (uint32_t)ctx->devs.size();
-    if (p->width != ctx->acc.width || p->height != ctx->acc.height || s != ctx->acc.shard_index || S != ctx->acc.shard_count || band != ctx->acc.band_rows)
+    RenderPlan P;
+    int rc = plan_render(ctx, nullptr, p, ctx->acc, P);
+    if (rc) return rc;
+    if (p->width != ctx->acc.width || p->height != ctx->acc.height || P.sh.s != ctx->acc.shard_index || P.sh.S != ctx->acc.shard_count || P.sh.band != ctx->acc.band_rows)
         ctx->acc.valid = false;   // another frame shape: a next batch may not add to the sums
     DeviceGuard guard;
-    int rc;
-    Dev &D0 = ctx->devs[0];
-    RZ_CUDA(cudaSetDevice(D0.id));
-    const uint32_t rows_ctx = rayz_cuda_context_rows(ctx, p->height, p->shard_index, p->shard_count, p->band_rows);
-    if ((rc = D0.out_linear.alloc((size_t)rows_ctx * p->width)) || (rc = D0.out_rgb8.alloc((size_t)rows_ctx * p->width * 3))) return rc;
-    for (uint32_t d = 0; d < ND; d++) {
-        Dev &D = ctx->devs[d];
+    if ((rc = alloc_render(ctx, P))) return rc;
+    for (Dev &D : ctx->devs) {
         RZ_CUDA(cudaSetDevice(D.id));
-        const uint32_t rows = rayz_cuda_shard_rows(p->height, s * ND + d, S * ND, band);
-        const uint32_t n_tiles = (rows * p->width + 31u) / 32u;
-        if ((rc = D.accum.alloc((size_t)n_tiles * 32u * 4u)) || (rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4)) || (rc = D.stats.alloc(3))) return rc;
-        if (p->variant == RZ_VARIANT_AUTO || p->variant == RZ_VARIANT_MEGA || (p->variant == RZ_VARIANT_BVH && (uint64_t)rows * p->width * p->spp >= (1ull << 26))) {
-            const uint32_t chunk = std::min(ctx->tun.chunk_primary, p->spp), n_chunks = (p->spp + chunk - 1) / chunk;
-            const uint64_t tiles = std::max<uint64_t>(n_tiles, (uint64_t)((p->width + 7u) / 8u) * ((rows + 3u) / 4u));   // K3's camera stage: 8 x 4 blocks
-            if (tiles * n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "reserve: too many work units");
-            QueuePlan qp;
-            if ((rc = plan_and_alloc_queues(ctx->tun, D, qp, (uint32_t)tiles * n_chunks, chunk, (p->flags & RZ_RENDER_SERIAL_PASSES) != 0,
-                                            !ctx->have_scene || ctx->n_spheres >= 64u, false, true)))
-                return rc;
-        }
         RZ_CUDA(cudaStreamSynchronize(D.stream));
     }
     return RZ_OK;
@@ -1170,17 +1214,13 @@ static bool host_pinned(const void *p) {
     return at.type == cudaMemoryTypeHost;
 }
 
-static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba, uint8_t *out_rgb8,
-                       uint64_t *out_paths);
-
-extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba,
-                                uint8_t *out_rgb8, uint64_t *out_paths) {
-    const int rc = render_host(ctx, cam, params, out_linear_rgba, out_rgb8, out_paths);
-    if (ctx) {
-        if (rc != RZ_OK && ctx->acc.pending) ctx->acc.valid = false;   // the paths ran but the call failed: the sums are not to be added to
-        ctx->acc.pending = false;
-    }
-    return rc;
+// Enqueues the copy of the gathered frame (npx pixels on device 0) into the caller's buffers on device 0's stream.
+static int copy_frame_to_host(RzContext *ctx, size_t npx, float *out_linear_rgba, uint8_t *out_rgb8) {
+    Dev &D0 = ctx->devs[0];
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if (out_linear_rgba) RZ_CUDA(cudaMemcpyAsync(out_linear_rgba, D0.out_linear.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
+    if (out_rgb8) RZ_CUDA(cudaMemcpyAsync(out_rgb8, D0.out_rgb8.p, npx * 3, cudaMemcpyDeviceToHost, D0.stream));
+    return RZ_OK;
 }
 
 static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba, uint8_t *out_rgb8,
@@ -1196,11 +1236,10 @@ static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     const int rc = render_impl(ctx, cam, params, false, direct);
     if (rc) return rc;
     DeviceGuard guard;
-    Dev &D0 = ctx->devs[0];
     const uint32_t rows = rayz_cuda_context_rows(ctx, params->height, params->shard_index, params->shard_count, params->band_rows);
     const size_t npx = (size_t)rows * params->width;
     if (direct) {
-        const uint32_t band = params->band_rows ? params->band_rows : 4, W = params->width;
+        const uint32_t band = Shard(params->shard_index, params->shard_count, params->band_rows).band, W = params->width;
         for (uint32_t d = 0; d < ND; d++) {
             Dev &D = ctx->devs[d];
             RZ_CUDA(cudaSetDevice(D.id));
@@ -1219,9 +1258,8 @@ static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams
             if (out_rgb8) RZ_CUDA(copy(out_rgb8, D.loc_rgb8.p, 3));
         }
     } else {
-        RZ_CUDA(cudaSetDevice(D0.id));
-        if (out_linear_rgba) RZ_CUDA(cudaMemcpyAsync(out_linear_rgba, D0.out_linear.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
-        if (out_rgb8) RZ_CUDA(cudaMemcpyAsync(out_rgb8, D0.out_rgb8.p, npx * 3, cudaMemcpyDeviceToHost, D0.stream));
+        const int rc2 = copy_frame_to_host(ctx, npx, out_linear_rgba, out_rgb8);
+        if (rc2) return rc2;
     }
     for (Dev &D : ctx->devs) {
         RZ_CUDA(cudaSetDevice(D.id));
@@ -1231,6 +1269,16 @@ static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (out_paths) *out_paths = (uint64_t)npx * params->spp;
     return RZ_OK;
+}
+
+extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba,
+                                uint8_t *out_rgb8, uint64_t *out_paths) {
+    const int rc = render_host(ctx, cam, params, out_linear_rgba, out_rgb8, out_paths);
+    if (ctx) {
+        if (rc != RZ_OK && ctx->acc.pending) ctx->acc.valid = false;   // the paths ran but the call failed: the sums are not to be added to
+        ctx->acc.pending = false;
+    }
+    return rc;
 }
 
 // Noise of the accumulated frame: every device computes its pixels' errors from its own accumulators with the resolve kernel
@@ -1314,12 +1362,9 @@ extern "C" int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, co
         q.flags |= RZ_RENDER_ACCUMULATE;
     }
     DeviceGuard guard;
-    Dev &D0 = ctx->devs[0];
     const size_t npx = (size_t)rayz_cuda_context_rows(ctx, p->height, p->shard_index, p->shard_count, p->band_rows) * p->width;
-    RZ_CUDA(cudaSetDevice(D0.id));
-    if (out_linear_rgba) RZ_CUDA(cudaMemcpyAsync(out_linear_rgba, D0.out_linear.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
-    if (out_rgb8) RZ_CUDA(cudaMemcpyAsync(out_rgb8, D0.out_rgb8.p, npx * 3, cudaMemcpyDeviceToHost, D0.stream));
-    RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    { const int rc = copy_frame_to_host(ctx, npx, out_linear_rgba, out_rgb8); if (rc) return rc; }
+    RZ_CUDA(cudaStreamSynchronize(ctx->devs[0].stream));
     if (out_paths) *out_paths = (uint64_t)npx * nz.samples;
     if (out_noise) *out_noise = nz;
     ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1382,17 +1427,14 @@ extern "C" int rayz_cuda_debug_sort_keys(RzContext *ctx, const unsigned short *k
     DBuf<uint32_t> io;
     DBuf<unsigned int> bins, cnt;
     int rc;
-    if ((rc = ki.alloc(n)) || (rc = ko.alloc(n)) || (rc = io.alloc(n)) || (rc = bins.alloc(rz_bin_scratch_bytes() / sizeof(unsigned int))) || (rc = cnt.alloc(1))) {
-        ki.release(); ko.release(); io.release(); bins.release(); cnt.release();
+    if ((rc = ki.alloc(n)) || (rc = ko.alloc(n)) || (rc = io.alloc(n)) || (rc = bins.alloc(rz_bin_scratch_bytes() / sizeof(unsigned int))) || (rc = cnt.alloc(1)))
         return rc;
-    }
     cudaError_t e = cudaMemcpyAsync(ki.p, keys, (size_t)n * sizeof(unsigned short), cudaMemcpyHostToDevice, D.stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(cnt.p, &n, sizeof n, cudaMemcpyHostToDevice, D.stream);
     if (e == cudaSuccess) e = rz_bin_sort(ki.p, cnt.p, n, bins.p, ko.p, io.p, 1024u, 0u, D.sms, D.stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(keys_out, ko.p, (size_t)n * sizeof(unsigned short), cudaMemcpyDeviceToHost, D.stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(idx_out, io.p, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, D.stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(D.stream);
-    ki.release(); ko.release(); io.release(); bins.release(); cnt.release();
     if (e != cudaSuccess) return rz_fail(RZ_ERR_CUDA, "debug_sort_keys: %s", cudaGetErrorString(e));
     return RZ_OK;
 }

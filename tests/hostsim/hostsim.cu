@@ -230,7 +230,7 @@ extern "C" int hostsim_tile_cull_check(const RzCamera *cam, uint32_t w, uint32_t
     C.defocus_u = make_float3((float)cam->defocus_u[0], (float)cam->defocus_u[1], (float)cam->defocus_u[2]);
     C.defocus_v = make_float3((float)cam->defocus_v[0], (float)cam->defocus_v[1], (float)cam->defocus_v[2]);
     C.defocus = cam->defocus;
-    // the two thin-lens numbers the library derives from the camera (rz_context.cu, render_impl)
+    // the two thin-lens numbers the library derives from the camera (rz_context.cu, enqueue_staged)
     double pcd[3], lu = 0, lv = 0, f2 = 0;
     for (int ax = 0; ax < 3; ax++) {
         pcd[ax] = cam->px_origin[ax] + 0.5 * (w - 1) * cam->px_du[ax] + 0.5 * (h - 1) * cam->px_dv[ax] - cam->look_from[ax];

@@ -733,7 +733,8 @@ def test_staged_kernels_on_oddly_shaped_sphere_sets(kind):
 @pytest.mark.gpu
 def test_reserve_then_render_and_auto_policy(scene42):
     """rayz_cuda_reserve pre-allocates the per-render buffers (before or after the scene upload) without changing results;
-    RZ_VARIANT_AUTO resolves to the BVH kernel for small jobs and to the staged K1 for large ones (same image)."""
+    RZ_VARIANT_AUTO resolves to the BVH kernel for small jobs and to the staged K1 for large ones (same image).  A staged
+    BVH frame rendered as one shard of two, whose shard alone is below 2^26 paths: reserved by the frame's size too."""
     w, spp = 256, 8
     cam, h = cam_for(w)
     fresh = Backend((0,))
@@ -747,6 +748,19 @@ def test_reserve_then_render_and_auto_policy(scene42):
     assert np.array_equal(a, b)
     with pytest.raises(abi.BackendError):
         fresh.reserve(Backend.params(0, h, spp))
+    w, spp = 1200, 100
+    cam, h = cam_for(w)
+    assert w * h * spp >= 1 << 26 > w * h * spp // 2
+    p = Backend.params(w, h, spp, 50, seed=3, variant="bvh", shard_index=0, shard_count=2)
+    fresh.reserve(p)
+    c, c8, _ = fresh.render(cam, p)
+    assert fresh.timing()["passes"] >= 1               # staged by the frame's size
+    other = Backend((0,))
+    other.upload_scene(scene42)
+    d, d8, _ = other.render(cam, p)                    # no reserve
+    assert np.array_equal(c, d) and np.array_equal(c8, d8)
+    other.close()
+    fresh.close()
 
 
 @pytest.mark.gpu
