@@ -2,14 +2,16 @@
 //
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
-//               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N]]
+//               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
 // The pixel loop runs in librayz_cuda.so; the timed region covers what the reference's covers
 // (hittables + BVH build == scene upload, and the render).  --noise-target X (displayed-value rms error, 1/255 = one 8-bit
 // step) starts at --spp samples and doubles them until the frame reaches X or --max-spp (default 4096); the samples reached
-// and the error go to stderr, the report line and the P3 output are unchanged.
+// and the error go to stderr, the report line and the P3 output are unchanged.  With --adaptive, X bounds every pixel's error
+// and only the pixels still above it get more samples (RZ_RENDER_ADAPTIVE); stderr then also reports the paths traced and the
+// mean and max samples per pixel.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -35,7 +37,7 @@ int main(int argc, char **argv) {
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
     const char *dump_scene = nullptr, *dump_linear = nullptr;
-    bool ppm_bench = false, penultimate = false;
+    bool ppm_bench = false, penultimate = false, adaptive = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
     for (int i = 2; i < argc; i++) {
@@ -52,6 +54,7 @@ int main(int argc, char **argv) {
         else if (a == "--ppm-bench") ppm_bench = true;
         else if (a == "--noise-target") noise_target = std::strtof(val(), nullptr);
         else if (a == "--max-spp") max_spp = (uint32_t)std::strtoul(val(), nullptr, 10);
+        else if (a == "--adaptive") adaptive = true;
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -70,6 +73,7 @@ int main(int argc, char **argv) {
         tracer.variant = variant;
         tracer.noise_target = noise_target;
         tracer.max_spp = max_spp;
+        tracer.adaptive = adaptive;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);
@@ -86,6 +90,10 @@ int main(int argc, char **argv) {
             std::fprintf(stderr, "  [rayz_cuda] noise target %.5f: %llu spp reached, rms error %.5f (%.2f 8-bit steps), mean %.5f, max %.5f, %u of %u pixels above\n",
                          noise_target, (unsigned long long)tracer.noise.samples, tracer.noise.rms_err, tracer.noise.rms_err * 255.0, tracer.noise.mean_err,
                          tracer.noise.max_err, tracer.noise.n_above, tracer.noise.n_pixels);
+        if (noise_target > 0 && adaptive)
+            std::fprintf(stderr, "  [rayz_cuda] adaptive: %.0f paths, mean %.2f spp, max %llu spp, max error %.5f (%.2f 8-bit steps)\n", rays_traced,
+                         rays_traced / std::max<double>(1.0, tracer.noise.n_pixels), (unsigned long long)tracer.noise.samples, tracer.noise.max_err,
+                         tracer.noise.max_err * 255.0);
         if (dump_scene && !dumpScene(tracer, dump_scene)) { std::perror(dump_scene); return 1; }
         if (dump_linear) {
             FILE *f = std::fopen(dump_linear, "wb");

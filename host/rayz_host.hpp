@@ -244,6 +244,7 @@ struct Tracer {
     float noise_target = 0;       // > 0: render from samples_per_px, doubling, until the frame's rms error reaches it (rayz_cuda_render_to_noise)
     uint32_t max_spp = 4096;      // ... or this many samples are in
     RzNoise noise{};              // summary of the last render with a noise target
+    bool adaptive = false;        // with noise_target: it bounds every pixel's error, and only pixels above it get more samples (RZ_RENDER_ADAPTIVE)
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
         : rng(seed) {
@@ -276,6 +277,7 @@ struct Tracer {
         std::memset(&p, 0, sizeof p);
         p.width = (uint32_t)img.w; p.height = (uint32_t)img.h; p.spp = (uint32_t)samples_per_px; p.max_depth = (uint32_t)max_bounces;
         p.seed = render_seed; p.variant = variant;
+        if (adaptive && noise_target > 0) p.flags |= RZ_RENDER_ADAPTIVE;
         return p;
     }
 

@@ -152,6 +152,18 @@ typedef struct RzRenderParams {
                                     * fails ends the accumulation.  *out_paths counts this call's paths only.  With
                                     * rayz_cuda_render_device(sync = 0), the next batch checks the previous one's device
                                     * error word before it adds to its sums. */
+#define RZ_RENDER_ADAPTIVE 0x8u    /* adaptive sampling, honoured by rayz_cuda_render_to_noise only (rayz_cuda_render and
+                                    * rayz_cuda_render_device refuse it with RZ_ERR_INVALID_ARG; rayz_cuda_reserve also allocates
+                                    * the per-pixel counts and lists, 8 bytes per pixel).  The doubling schedule runs per pixel:
+                                    * after the first round, a round traces only the pixels that took part in every earlier round
+                                    * and whose error (as rayz_cuda_noise's out_err shows it) is above the target.  A pixel that
+                                    * ends with c samples equals the same pixel of a uniform c-spp render bit for bit (linear,
+                                    * rgb8, error), as every path is a function of (seed, pixel, sample index).  AUTO runs the BVH
+                                    * family; a pinned MEGA, MEGA_SINGLE or WAVEFRONT runs its first round as pinned and the
+                                    * others with the single-form brute-force kernel (the same family: for exactness, not speed).
+                                    * Whether a pixel is active depends on its own sums only, so sharding changes no count.
+                                    * rayz_cuda_noise and rayz_cuda_pixel_samples read the frame with each pixel's own count; an
+                                    * RZ_RENDER_ACCUMULATE batch after it is refused, the sums untouched. */
 
 /* Noise summary of the accumulated frame (rayz_cuda_noise).  Errors are standard errors of the DISPLAYED value
  * (gamma 2, as writePPM shows it) in units of [0, 1]: one 8-bit step is 1/255.  +inf while samples < 2. */
@@ -261,9 +273,21 @@ int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzNoise *out);
  * rms_err <= target or max_spp samples are reached.  RZ_OK either way: *out_noise says which (its samples and rms_err).
  * The host buffers (each nullable, as in rayz_cuda_render) are written once, at the end; *out_paths counts every batch.
  * RZ_ERR_INVALID_ARG if max_spp < p->spp.
+ * With RZ_RENDER_ADAPTIVE in p->flags, `target` bounds EACH pixel's error instead of the rms: with N the count after a
+ * round, the next round gives the pixels still active (count N, error > target) the samples [N, N + b) past sample_offset,
+ * b = min(N, max_spp - N); the call ends when no pixel is active or N reaches max_spp.  *out_paths is the sum of the per-pixel
+ * counts; *out_noise is over all pixels, each with its own count, and its samples is the largest count: max_err <= target
+ * unless samples == max_spp.  RzStats and RzTiming describe the last round, except total_ms, which covers the call.
  */
 int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float target, uint32_t max_spp,
                               float *out_linear_rgba, uint8_t *out_rgb8, uint64_t *out_paths, RzNoise *out_noise);
+
+/*
+ * Per-pixel sample counts of the accumulated frame: out_spp holds rows of the context * width counts, laid out like
+ * rayz_cuda_noise's out_err.  After a uniform render (or batches) every count is the frame's; after an adaptive
+ * rayz_cuda_render_to_noise, each pixel's own.  RZ_ERR_INVALID_ARG if there is no accumulated render.
+ */
+int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp);
 
 /* Number of image rows a shard owns under the banding rule above. */
 uint32_t rayz_cuda_shard_rows(uint32_t height, uint32_t shard_index, uint32_t shard_count,

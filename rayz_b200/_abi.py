@@ -19,7 +19,7 @@ TEX_CHECKER, TEX_SOLID = 0, 1
 DIFFUSE_UNIT_SPHERE, DIFFUSE_UNIT_SPHERE_SURFACE, DIFFUSE_HEMISPHERE = 0, 1, 2
 VARIANT_AUTO, VARIANT_MEGA, VARIANT_WAVEFRONT, VARIANT_BVH = 0, 1, 2, 3
 VARIANTS = {"auto": 0, "mega": 1, "wavefront": 2, "bvh": 3, "mega_single": 4}
-RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE = 1, 2, 4   # RzRenderParams.flags (RZ_RENDER_*)
+RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE, RENDER_ADAPTIVE = 1, 2, 4, 8   # RzRenderParams.flags (RZ_RENDER_*)
 
 _dp, _up = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 
@@ -100,6 +100,7 @@ SYMBOLS = {
     "rayz_cuda_noise": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p, C.POINTER(RzNoise)]),
     "rayz_cuda_render_to_noise": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_float, C.c_uint32,
                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(RzNoise)]),
+    "rayz_cuda_pixel_samples": (C.c_int, [C.c_void_p, C.c_void_p]),
     "rayz_cuda_shard_rows": (C.c_uint32, [C.c_uint32] * 4),
     "rayz_cuda_context_rows": (C.c_uint32, [C.c_void_p] + [C.c_uint32] * 4),
     "rayz_cuda_primary_ids": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]),

@@ -25,6 +25,7 @@ UNITS = {
     "rz_path.cu": ["--use_fast_math"],
     "rz_wavefront.cu": ["--use_fast_math"],
     "rz_misc.cu": [],
+    "rz_adaptive.cu": [],
     "rz_ids.cu": ["--fmad=false"],
     "rz_bvh_build.cu": [],
     "rz_bvh_wide.cu": [],

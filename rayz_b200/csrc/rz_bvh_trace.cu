@@ -217,7 +217,8 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
     }
 }
 
-template <bool STATS, bool QUEUE, int UNIT = 512>
+// LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list).
+template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -308,8 +309,9 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
                         start_traversal();
                         need = false;
                     } else {
-                        const uint32_t nlp = unit_lp0 + (k & 31u);
-                        if (nlp < a.n_local_px) {
+                        uint32_t nlp = unit_lp0 + (k & 31u);
+                        if (nlp < (LIST ? a.n_list : a.n_local_px)) {
+                            if (LIST) nlp = __ldg(a.px_list + nlp);
                             uint32_t pi, pj;
                             rz_local_to_global(nlp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
                             lp = nlp;
@@ -623,13 +625,16 @@ static void rz_bvh_tuning(RzPathArgs &b) {   // defaults are the measured optimu
     if (b.stack_cap < 1u || b.stack_cap > (uint32_t)RZ_STACK) b.stack_cap = (uint32_t)RZ_STACK;
 }
 
-// The persistent kernel: whole paths from the camera (q_in == nullptr) or the tails of paths from a queue.
+// The persistent kernel: whole paths from the camera (q_in == nullptr; only the pixels of px_list when it is set) or the tails
+// of paths from a queue.
 extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream) {
     RzPathArgs b = *a;
     rz_bvh_tuning(b);
     if (b.q_in && b.self_map)   // the tail of the staged K1 (entries written by a brute-force stage): a short queue, small units
         return collect_stats ? launch_kernel(rz_bvh_kernel<true, true, 64>, b, sm_count, stream) : launch_kernel(rz_bvh_kernel<false, true, 64>, b, sm_count, stream);
     if (b.q_in) return collect_stats ? launch_kernel(rz_bvh_kernel<true, true>, b, sm_count, stream) : launch_kernel(rz_bvh_kernel<false, true>, b, sm_count, stream);
+    if (b.px_list)
+        return collect_stats ? launch_kernel(rz_bvh_kernel<true, false, 512, true>, b, sm_count, stream) : launch_kernel(rz_bvh_kernel<false, false, 512, true>, b, sm_count, stream);
     return collect_stats ? launch_kernel(rz_bvh_kernel<true, false>, b, sm_count, stream) : launch_kernel(rz_bvh_kernel<false, false>, b, sm_count, stream);
 }
 

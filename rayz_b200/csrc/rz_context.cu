@@ -25,7 +25,7 @@ struct RzIdsArgs {
     uint32_t width, height; int use_bvh; int32_t *out; unsigned int *err;
 };
 struct RzResolveArgs {
-    const unsigned long long *accum; float4 *out_linear; uint8_t *out_rgb8; float *out_err;
+    const unsigned long long *accum; float4 *out_linear; uint8_t *out_rgb8; float *out_err; uint32_t *out_spp; const uint32_t *n_px;
     uint32_t n_local_px, width; uint32_t spp; uint32_t dev_index, dev_count, band_rows;
 };
 extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, int collect_stats, int sm_count,
@@ -54,8 +54,13 @@ extern "C" cudaError_t rz_bvh_wide_collapse(const RzBvhNode *n2, uint32_t n_node
 extern "C" cudaError_t rz_launch_ids(const RzIdsArgs *a, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
 extern "C" uint32_t rz_noise_grid(void);
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, uint32_t n_local_px, uint32_t n, double target, void *out,
-                                              cudaStream_t stream);
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, uint32_t n_local_px, uint32_t n,
+                                              double target, void *out, cudaStream_t stream);
+extern "C" size_t rz_list_scratch_words(uint32_t n_local_px);
+extern "C" size_t rz_list_count_word(uint32_t n_local_px);
+extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, uint32_t *n_px, uint32_t n_local_px, uint32_t n_cur, uint32_t add,
+                                            float target, uint32_t *list, uint32_t *scratch, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_fill_u32(uint32_t *p, uint32_t n, uint32_t v, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_ffma_peak(float *sink, int grid, int iters, int mode, cudaStream_t stream);
 extern "C" cudaError_t rz_wavefront_render(const RzPathArgs *a, int sm_count, int collect_stats, cudaStream_t stream,
                                            void **scratch, size_t *scratch_bytes, uint32_t *launches);
@@ -164,6 +169,10 @@ struct Dev {
     DBuf<uint8_t> out_rgb8;
     DBuf<float> out_err;              // rayz_cuda_noise: per-pixel error of the context's rows (gather root only)
     DBuf<double> noise_part;          // rayz_cuda_noise: the reduction's per-CTA partials of this device
+    DBuf<uint32_t> out_spp;           // rayz_cuda_pixel_samples: per-pixel sample counts of the context's rows (gather root only)
+    DBuf<uint32_t> n_px;              // RZ_RENDER_ADAPTIVE: every local pixel's sample count
+    DBuf<uint32_t> px_list;           // RZ_RENDER_ADAPTIVE: the local pixels the next round traces, in increasing order
+    DBuf<uint32_t> list_scratch;      // RZ_RENDER_ADAPTIVE: the list kernels' mask words, block offsets and list length (rz_adaptive.cu)
     DBuf<float4> loc_linear;          // multi-device render into HOST buffers: this device's own rows, copied out over its own PCIe link
     DBuf<uint8_t> loc_rgb8;
     uint32_t loc_rows = 0;            // rows of the last such render
@@ -204,7 +213,8 @@ struct AccumRecord {
     float t_min = 0;
     RzCamera cam{};
     uint32_t first_offset = 0;
-    uint64_t samples = 0;
+    uint64_t samples = 0;      // adaptive: the largest per-pixel count (the pixels still active in the last round)
+    bool adaptive = false;     // RZ_RENDER_ADAPTIVE: the pixels' counts differ (Dev::n_px), no RZ_RENDER_ACCUMULATE batch continues them
 };
 
 struct RzContext {
@@ -820,6 +830,7 @@ static int settle_accumulation(RzContext *ctx) {
 // ------------------------------------------------------------------------------ render plan
 struct DevPlan {
     uint32_t rows = 0, n_local = 0, n_tiles = 0, n_units = 0;   // n_units: work units of the first kernel
+    uint32_t n_list = 0;                                         // adaptive round: the pixels listed on this device
     QueuePlan qp;                                                // staged: the passes alloc_render could allocate
 };
 
@@ -837,13 +848,17 @@ struct RenderPlan {
     DevPlan dev[RZ_MAX_DEVICES];
     AccumRecord next;                   // what the render commits to ctx->acc when it succeeds
     bool refused = false;               // an RZ_RENDER_ACCUMULATE batch that does not continue `prev`
+    bool list = false;                  // an adaptive round after the first: only the pixels of each device's list (Dev::px_list)
 };
 
 // Plans a render of these parameters, with the validations (and messages) of rayz_cuda_render.  cam == nullptr plans for
-// rayz_cuda_reserve: no scene is needed and no accumulation record is made.
-static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, const AccumRecord &prev, RenderPlan &P) {
+// rayz_cuda_reserve: no scene is needed and no accumulation record is made.  n_list (rayz_cuda_render_to_noise's adaptive
+// rounds after the first, RZ_RENDER_ADAPTIVE | RZ_RENDER_ACCUMULATE): per device, the length of its pixel list.
+static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, const AccumRecord &prev, RenderPlan &P,
+                       const uint32_t *n_list = nullptr) {
     P.p = p;
     P.cam = cam;
+    P.list = n_list != nullptr;
     const char *who = cam ? "render" : "reserve";
     if (cam && !ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "render: rayz_cuda_upload_scene has not been called");
     if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "%s: width, height and spp must be > 0", who);
@@ -862,8 +877,13 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         // amortise its ~25 launches per pass (measured one-shot, 485 spheres: 0.9 M paths 3.9 ms vs 0.8 ms for the BVH kernel,
         // 8 M 6.3 vs 2.8, 81 M 23.8 vs 25.3, 405 M 104 vs 125); else the BVH kernel.  (The two kernel families themselves can
         // differ in a pixel or two: FP32 sphere test against exact boxes, tests/test_gpu_parity.py.)
-        P.variant = (brute_smem <= RZ_SMEM_BUDGET && frame_paths >= (1ull << 26)) ? RZ_VARIANT_MEGA : RZ_VARIANT_BVH;
+        // An adaptive render runs the BVH family: its rounds after the first are small jobs of scattered pixels.
+        P.variant = (p->flags & RZ_RENDER_ADAPTIVE) ? RZ_VARIANT_BVH
+                    : (brute_smem <= RZ_SMEM_BUDGET && frame_paths >= (1ull << 26)) ? RZ_VARIANT_MEGA : RZ_VARIANT_BVH;
     }
+    // The listed rounds of an adaptive render run the unstaged kernel of the first round's family: K3 for BVH, the single-form
+    // K1b for the brute-force family (MEGA, MEGA_SINGLE, WAVEFRONT).  Same family, so every pixel stays exact.
+    if (P.list && (P.variant == RZ_VARIANT_MEGA || P.variant == RZ_VARIANT_WAVEFRONT)) P.variant = RZ_VARIANT_MEGA_SINGLE;
     P.mega_single = P.variant == RZ_VARIANT_MEGA_SINGLE;
     if (P.mega_single) P.variant = RZ_VARIANT_MEGA;
     if (P.variant != RZ_VARIANT_MEGA && P.variant != RZ_VARIANT_BVH && P.variant != RZ_VARIANT_WAVEFRONT)
@@ -877,9 +897,12 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
+        next.adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
         if (p->flags & RZ_RENDER_ACCUMULATE) {
             auto refuse = [&](const char *why) { P.refused = true; return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ACCUMULATE refused: %s", why); };
             if (!prev.valid) return refuse("no previous render to add to (none, it failed, or a scene upload or reserve came in between)");
+            if (prev.adaptive != next.adaptive)
+                return refuse("the accumulated frame was rendered adaptively: its pixels hold different sample counts, so no sample_offset continues it");
             if (prev.width != next.width || prev.height != next.height || prev.shard_index != s || prev.shard_count != S || prev.band_rows != band)
                 return refuse("frame size, shard or band_rows differ from the accumulated render");
             if (prev.seed != next.seed || prev.max_depth != next.max_depth || memcmp(&prev.t_min, &next.t_min, sizeof(float)) != 0)
@@ -897,7 +920,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
     if (P.variant == RZ_VARIANT_BVH) {
         // K3 on a big job: the same staged pipeline with BVH traversal instead of culled lists (sorted rays stay converged); the
         // staged camera stage searches block lists, the unstaged kernel walks the tree
-        P.staged = ctx->tun.bvh_staged && frame_paths >= (1ull << 26);
+        P.staged = !P.list && ctx->tun.bvh_staged && frame_paths >= (1ull << 26);
     } else if (P.variant == RZ_VARIANT_MEGA) {
         // one persistent kernel for RZ_VARIANT_MEGA_SINGLE, or for a set whose pair lists do not fit beside the primary kernel
         RzPathArgs probe;
@@ -930,6 +953,10 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         P.rows_ctx += dp.rows;
         if ((uint64_t)dp.n_tiles * n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: too many work units", who);
         uint64_t tiles = dp.n_tiles;
+        if (P.list) {   // work unit u: list entries [tile * 32, tile * 32 + 32) x one chunk of samples
+            dp.n_list = n_list[d];
+            tiles = (dp.n_list + 31u) / 32u;
+        }
         const uint64_t blocks = (uint64_t)((p->width + 7u) / 8u) * ((dp.rows + 3u) / 4u);   // K3's camera stage works on 8 x 4 pixel blocks
         if (P.tile_w) tiles = blocks;
         else if (P.staged && !ctx->have_scene) tiles = std::max(tiles, blocks);
@@ -964,6 +991,9 @@ static int alloc_render(RzContext *ctx, RenderPlan &P) {
             for (cudaEvent_t e = nullptr; D.stage_ev.size() < 2 * (size_t)dp.qp.n_pass * dp.qp.n_second; D.stage_ev.push_back(e)) RZ_CUDA(cudaEventCreate(&e));
         }
         if (P.host_direct && ((rc = D.loc_linear.alloc((size_t)dp.n_local)) || (rc = D.loc_rgb8.alloc((size_t)dp.n_local * 3)))) return rc;
+        if ((P.p->flags & RZ_RENDER_ADAPTIVE) &&
+            ((rc = D.n_px.alloc(dp.n_local)) || (rc = D.px_list.alloc(dp.n_local)) || (rc = D.list_scratch.alloc(rz_list_scratch_words(dp.n_local)))))
+            return rc;
     }
     return RZ_OK;
 }
@@ -1064,9 +1094,12 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     const uint32_t ND = (uint32_t)ctx->devs.size();
     Dev &D = ctx->devs[d], &D0 = ctx->devs[0];
     const DevPlan &dp = P.dev[d];
+    const bool adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
+    const bool trace = dp.n_local > 0 && (!P.list || dp.n_list > 0);   // a device with an empty list launches nothing
     RZ_CUDA(cudaSetDevice(D.id));
     RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
     if (!(p->flags & RZ_RENDER_ACCUMULATE)) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
+    if (adaptive && !P.list) RZ_CUDA(rz_launch_fill_u32(D.n_px.p, dp.n_local, p->spp, D.stream));   // first round: every pixel
     RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
     RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
     if (p->collect_stats) RZ_CUDA(cudaMemsetAsync(D.stats.p, 0, 3 * sizeof(RzStatsDev), D.stream));
@@ -1094,15 +1127,16 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     a.bvh_active_min = (uint32_t)ctx->tun.bvh_active_min; a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
     a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
     a.moments = P.next.moments;
+    if (P.list) { a.px_list = D.px_list.p; a.n_list = dp.n_list; }
 
     RZ_CUDA(cudaEventRecord(D.ev[1], D.stream));
     D.passes = 0;
     D.n_second = 0;
     D.queue_entries = 0;
-    if (dp.n_local > 0 && P.staged) {
+    if (trace && P.staged) {
         const int rc = enqueue_staged(ctx, D, a, P, dp.qp, launches);
         if (rc) return rc;
-    } else if (dp.n_local > 0) {   // one kernel (the wavefront form counts its own launches)
+    } else if (trace) {   // one kernel (the wavefront form counts its own launches)
         uint32_t l = 1;
         if (P.variant == RZ_VARIANT_WAVEFRONT) RZ_CUDA(rz_wavefront_render(&a, D.sms, (int)p->collect_stats, D.stream, &D.wf_scratch, &D.wf_scratch_bytes, &l));
         else if (P.variant == RZ_VARIANT_BVH) RZ_CUDA(rz_launch_bvh(&a, (int)p->collect_stats, D.sms, D.stream));
@@ -1112,20 +1146,22 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     RZ_CUDA(cudaEventRecord(D.ev[2], D.stream));
 
     RzResolveArgs r;
-    r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p; r.out_err = nullptr;
-    r.n_local_px = dp.n_local; r.width = p->width; r.spp = (uint32_t)P.next.samples;   // cumulative with RZ_RENDER_ACCUMULATE
+    r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p; r.out_err = nullptr; r.out_spp = nullptr;
+    r.n_px = adaptive ? D.n_px.p : nullptr;
+    r.n_local_px = trace ? dp.n_local : 0u; r.width = p->width; r.spp = (uint32_t)P.next.samples;   // cumulative with RZ_RENDER_ACCUMULATE
     r.dev_index = d; r.dev_count = ND; r.band_rows = P.sh.band;
     if (P.host_direct) {
         r.out_linear = D.loc_linear.p; r.out_rgb8 = D.loc_rgb8.p; r.dev_index = 0; r.dev_count = 1;
         D.loc_rows = dp.rows;
     }
     RZ_CUDA(rz_launch_resolve(&r, D.stream));
-    if (dp.n_local > 0) launches += 1;
+    if (trace) launches += 1;
     RZ_CUDA(cudaEventRecord(D.ev[3], D.stream));
     return RZ_OK;
 }
 
-static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, bool sync, bool host_direct = false) {
+static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, bool sync, bool host_direct = false,
+                       const uint32_t *n_list = nullptr) {
     if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "render: NULL argument");
     // Every render ends what the accumulators held unless it succeeds (the record is committed at the end) or it is an
     // RZ_RENDER_ACCUMULATE batch that is refused before anything was touched (the record is restored).
@@ -1133,7 +1169,7 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     const AccumRecord prev = ctx->acc;
     ctx->acc.valid = false;
     RenderPlan P;
-    if (const int rc = plan_render(ctx, cam, p, prev, P)) {
+    if (const int rc = plan_render(ctx, cam, p, prev, P, n_list)) {
         if (P.refused) ctx->acc = prev;
         return rc;
     }
@@ -1192,8 +1228,15 @@ extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     return RZ_OK;
 }
 
+// RZ_RENDER_ADAPTIVE needs the rounds of rayz_cuda_render_to_noise; a single render cannot honour it.
+static int refuse_adaptive(const RzRenderParams *p) {
+    if (p && (p->flags & RZ_RENDER_ADAPTIVE)) return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ADAPTIVE is honoured by rayz_cuda_render_to_noise only");
+    return RZ_OK;
+}
+
 extern "C" int rayz_cuda_render_device(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, void **d_linear_rgba,
                                        void **d_rgb8, uint64_t *out_paths, int sync) {
+    if (const int rc = refuse_adaptive(params)) return rc;
     const int rc = render_impl(ctx, cam, params, sync != 0);
     if (rc) return rc;
     if (d_linear_rgba) *d_linear_rgba = ctx->devs[0].out_linear.p;
@@ -1273,6 +1316,7 @@ static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams
 
 extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRenderParams *params, float *out_linear_rgba,
                                 uint8_t *out_rgb8, uint64_t *out_paths) {
+    if (const int rc = refuse_adaptive(params)) return rc;
     const int rc = render_host(ctx, cam, params, out_linear_rgba, out_rgb8, out_paths);
     if (ctx) {
         if (rc != RZ_OK && ctx->acc.pending) ctx->acc.valid = false;   // the paths ran but the call failed: the sums are not to be added to
@@ -1283,7 +1327,7 @@ extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRen
 
 // Noise of the accumulated frame: every device computes its pixels' errors from its own accumulators with the resolve kernel
 // (rows scattered into the gather root's buffer like the image) and reduces them in a fixed order; the host adds the partials
-// device by device, CTA by CTA.
+// device by device, CTA by CTA.  An adaptive frame takes each pixel's own sample count.
 extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzNoise *out) {
     if (!ctx) return rz_fail(RZ_ERR_INVALID_ARG, "noise: ctx is NULL");
     DeviceGuard guard;
@@ -1304,12 +1348,14 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
         if ((rc = D.noise_part.alloc(4 * (size_t)G))) return rc;
         if (out_err) {
             RzResolveArgs r;
-            r.accum = D.accum.p; r.out_linear = nullptr; r.out_rgb8 = nullptr; r.out_err = D0.out_err.p;
+            r.accum = D.accum.p; r.out_linear = nullptr; r.out_rgb8 = nullptr; r.out_err = D0.out_err.p; r.out_spp = nullptr;
+            r.n_px = A.adaptive ? D.n_px.p : nullptr;
             r.n_local_px = n_local; r.width = A.width; r.spp = (uint32_t)A.samples;
             r.dev_index = d; r.dev_count = ND; r.band_rows = A.band_rows;
             RZ_CUDA(rz_launch_resolve(&r, D.stream));
         }
-        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, n_local, (uint32_t)A.samples, (double)target, D.noise_part.p, D.stream));
+        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A.adaptive ? D.n_px.p : nullptr, n_local, (uint32_t)A.samples, (double)target, D.noise_part.p,
+                                       D.stream));
     }
     double sum = 0, sum2 = 0, mx = 0;
     uint64_t above = 0;
@@ -1341,8 +1387,64 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
     return RZ_OK;
 }
 
+// Per-pixel sample counts of the accumulated frame, laid out like rayz_cuda_noise's out_err: the resolve kernel scatters every
+// device's counts (an adaptive frame's own, else the uniform count) into the gather root's buffer.
+extern "C" int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp) {
+    if (!ctx || !out_spp) return rz_fail(RZ_ERR_INVALID_ARG, "pixel_samples: NULL argument");
+    DeviceGuard guard;
+    { const int rc = settle_accumulation(ctx); if (rc) return rc; }
+    const AccumRecord &A = ctx->acc;
+    if (!A.valid) return rz_fail(RZ_ERR_INVALID_ARG, "pixel_samples: no accumulated render (none, it failed, or a scene upload or reserve came in between)");
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    Dev &D0 = ctx->devs[0];
+    const uint32_t rows_ctx = rayz_cuda_context_rows(ctx, A.height, A.shard_index, A.shard_count, A.band_rows);
+    int rc;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if ((rc = D0.out_spp.alloc((size_t)rows_ctx * A.width))) return rc;
+    for (uint32_t d = 0; d < ND; d++) {
+        Dev &D = ctx->devs[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        RzResolveArgs r;
+        r.accum = D.accum.p; r.out_linear = nullptr; r.out_rgb8 = nullptr; r.out_err = nullptr; r.out_spp = D0.out_spp.p;
+        r.n_px = A.adaptive ? D.n_px.p : nullptr;
+        r.n_local_px = rayz_cuda_shard_rows(A.height, A.shard_index * ND + d, A.shard_count * ND, A.band_rows) * A.width;
+        r.width = A.width; r.spp = (uint32_t)A.samples;
+        r.dev_index = d; r.dev_count = ND; r.band_rows = A.band_rows;
+        RZ_CUDA(rz_launch_resolve(&r, D.stream));
+    }
+    for (Dev &D : ctx->devs) {   // every device's rows are in the gather root's buffer
+        RZ_CUDA(cudaSetDevice(D.id));
+        RZ_CUDA(cudaStreamSynchronize(D.stream));
+    }
+    RZ_CUDA(cudaSetDevice(D0.id));
+    RZ_CUDA(cudaMemcpyAsync(out_spp, D0.out_spp.p, (size_t)rows_ctx * A.width * sizeof(uint32_t), cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    return RZ_OK;
+}
+
+// Adaptive rounds: every device lists its active pixels (rz_adaptive.cu: count n_cur, error above the target) and adds `add`
+// to their counts; n_list[d] <- the length of device d's list, read behind its stream.
+static int build_pixel_lists(RzContext *ctx, uint32_t n_cur, uint32_t add, float target, uint32_t *n_list) {
+    const AccumRecord &A = ctx->acc;
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    for (uint32_t d = 0; d < ND; d++) {   // every device enqueues before the first wait
+        Dev &D = ctx->devs[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        const uint32_t n_local = rayz_cuda_shard_rows(A.height, A.shard_index * ND + d, A.shard_count * ND, A.band_rows) * A.width;
+        RZ_CUDA(rz_launch_pixel_list(D.accum.p, D.n_px.p, n_local, n_cur, add, target, D.px_list.p, D.list_scratch.p, D.stream));
+        RZ_CUDA(cudaMemcpyAsync(&n_list[d], D.list_scratch.p + rz_list_count_word(n_local), sizeof(uint32_t), cudaMemcpyDeviceToHost, D.stream));
+    }
+    for (Dev &D : ctx->devs) {
+        RZ_CUDA(cudaSetDevice(D.id));
+        RZ_CUDA(cudaStreamSynchronize(D.stream));
+    }
+    return RZ_OK;
+}
+
 // The stopping policy of progressive rendering, in one place for every host: batches that double the accumulated sample count
-// until the frame's rms error reaches the target or max_spp samples are in.
+// until the frame's rms error reaches the target or max_spp samples are in.  With RZ_RENDER_ADAPTIVE the same schedule runs
+// per pixel (DESIGN.md "Adaptive sampling"): after the first round, each round traces only the pixels that took part in every
+// earlier round and are still above the target.
 extern "C" int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float target, uint32_t max_spp,
                                          float *out_linear_rgba, uint8_t *out_rgb8, uint64_t *out_paths, RzNoise *out_noise) {
     const auto t0 = std::chrono::steady_clock::now();
@@ -1352,20 +1454,48 @@ extern "C" int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, co
     q.flags = (p->flags & ~RZ_RENDER_ACCUMULATE) | RZ_RENDER_MOMENTS;
     RzNoise nz;
     memset(&nz, 0, sizeof nz);
-    for (;;) {
+    const size_t npx = (size_t)rayz_cuda_context_rows(ctx, p->height, p->shard_index, p->shard_count, p->band_rows) * p->width;
+    uint64_t paths = 0;
+    if (!(p->flags & RZ_RENDER_ADAPTIVE)) {
+        for (;;) {
+            int rc = render_impl(ctx, cam, &q, true);
+            if (rc) return rc;
+            if ((rc = rayz_cuda_noise(ctx, target, nullptr, &nz))) return rc;
+            if (nz.rms_err <= (double)target || nz.samples >= max_spp) break;
+            q.sample_offset = p->sample_offset + (uint32_t)nz.samples;
+            q.spp = (uint32_t)std::min<uint64_t>(nz.samples, max_spp - nz.samples);
+            q.flags |= RZ_RENDER_ACCUMULATE;
+        }
+        paths = (uint64_t)npx * nz.samples;
+    } else {
+        // Round 0: every pixel, p->spp samples.  Round r + 1: the listed pixels, samples [n, n + b) past sample_offset; a pixel
+        // that drops out is never listed again, so every listed pixel holds exactly n samples and all share one sample range.
         int rc = render_impl(ctx, cam, &q, true);
         if (rc) return rc;
-        if ((rc = rayz_cuda_noise(ctx, target, nullptr, &nz))) return rc;
-        if (nz.rms_err <= (double)target || nz.samples >= max_spp) break;
-        q.sample_offset = p->sample_offset + (uint32_t)nz.samples;
-        q.spp = (uint32_t)std::min<uint64_t>(nz.samples, max_spp - nz.samples);
+        paths = (uint64_t)npx * q.spp;
         q.flags |= RZ_RENDER_ACCUMULATE;
+        uint32_t n_list[RZ_MAX_DEVICES] = {};
+        for (uint32_t n = p->spp; n < max_spp;) {
+            const uint32_t b = std::min(n, max_spp - n);
+            {
+                DeviceGuard g;
+                if ((rc = build_pixel_lists(ctx, n, b, target, n_list))) { ctx->acc.valid = false; return rc; }
+            }
+            uint64_t listed = 0;
+            for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) listed += n_list[d];
+            if (listed == 0) break;
+            q.sample_offset = p->sample_offset + n;
+            q.spp = b;
+            if ((rc = render_impl(ctx, cam, &q, true, false, n_list))) return rc;
+            paths += listed * b;
+            n += b;
+        }
+        if ((rc = rayz_cuda_noise(ctx, target, nullptr, &nz))) return rc;
     }
     DeviceGuard guard;
-    const size_t npx = (size_t)rayz_cuda_context_rows(ctx, p->height, p->shard_index, p->shard_count, p->band_rows) * p->width;
     { const int rc = copy_frame_to_host(ctx, npx, out_linear_rgba, out_rgb8); if (rc) return rc; }
     RZ_CUDA(cudaStreamSynchronize(ctx->devs[0].stream));
-    if (out_paths) *out_paths = (uint64_t)npx * nz.samples;
+    if (out_paths) *out_paths = paths;
     if (out_noise) *out_noise = nz;
     ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return RZ_OK;

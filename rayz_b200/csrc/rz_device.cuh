@@ -170,6 +170,10 @@ struct RzPathArgs {
     uint32_t bvh_descend_min;    // K3: a descend round ends once fewer lanes than this are still descending
     uint32_t tile_w;             // K3 camera stage: 0 = a work unit's 32 pixels are consecutive in a row; 8 = an 8 x 4 block (tile lists: the narrower cone)
     uint32_t moments;            // != 0 (RZ_RENDER_MOMENTS): a path that ends in the sky also adds its luminance squared to accum slot 3
+    // Adaptive rounds (RZ_RENDER_ADAPTIVE; the LIST instances of the unstaged K3 and of the single-form K1b only): work unit u
+    // covers list entries [tile * 32, tile * 32 + 32), and lane k's pixel is px_list[entry] instead of the entry itself.
+    const uint32_t *px_list;     // local pixel indices in increasing order (rz_adaptive.cu)
+    uint32_t n_list;             // entries in px_list
 };
 
 // ---------------------------------------------------------------------------------------------

@@ -11,7 +11,9 @@
 // Output rows may live on ANOTHER GPU (peer pointers): with out_row_stride/out_row_offset the
 // kernel scatters this device's compact band-interleaved rows straight into the gather root's
 // full-shard buffers over NVLink, i.e. resolve and gather are one kernel.
-// The same kernel writes the per-pixel noise estimate (out_err: rz_pixel_err of the four slots) when asked.
+// The same kernel writes the per-pixel noise estimate (out_err: rz_pixel_err of the four slots) and the pixels' sample counts
+// (out_spp) when asked.  An adaptive frame divides each pixel by its own count (n_px), in the same f64 arithmetic: a pixel
+// with c samples resolves exactly as the same pixel of a uniform c-spp render.
 // ---------------------------------------------------------------------------------------------
 #include "rz_device.cuh"   // rz_pixel_err
 
@@ -20,6 +22,8 @@ struct RzResolveArgs {
     float4 *out_linear;               // nullable
     uint8_t *out_rgb8;                // nullable
     float *out_err;                   // nullable: displayed-value standard error per pixel (needs slot 3, RZ_RENDER_MOMENTS)
+    uint32_t *out_spp;                // nullable: the pixel's sample count (rayz_cuda_pixel_samples)
+    const uint32_t *n_px;             // nullable: per-pixel sample counts of an adaptive frame (rz_adaptive.cu); null: spp
     uint32_t n_local_px, width;
     uint32_t spp;                     // samples summed in the accumulators (cumulative over RZ_RENDER_ACCUMULATE batches)
     // local row lr of this device -> destination row ((lr / band) * dev_count + dev_index) * band + lr % band
@@ -37,8 +41,10 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
         const uint32_t lb = lr / a.band_rows, within = lr - lb * a.band_rows;
         dst = (size_t)((lb * a.dev_count + a.dev_index) * a.band_rows + within) * a.width + i;
     }
-    if (a.out_err) a.out_err[dst] = (float)rz_pixel_err(q0.x, q0.y, q1, a.accum[(size_t)lp * 4 + 3], a.spp);
-    const double inv = 1.0 / (double)a.spp;
+    const uint32_t n = a.n_px ? a.n_px[lp] : a.spp;
+    if (a.out_spp) a.out_spp[dst] = n;
+    if (a.out_err) a.out_err[dst] = (float)rz_pixel_err(q0.x, q0.y, q1, a.accum[(size_t)lp * 4 + 3], n);
+    const double inv = 1.0 / (double)n;
     const double s = 2.3283064365386962890625e-10;  // 2^-32
     const double r = (double)q0.x * s * inv, g = (double)q0.y * s * inv, b = (double)q1 * s * inv;
     if (a.out_linear) a.out_linear[dst] = make_float4((float)r, (float)g, (float)b, 1.0f);
@@ -65,15 +71,16 @@ extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t st
 #define RZ_NOISE_GRID 256
 struct RzNoisePartial { double sum, sum2, max; unsigned long long above; };
 
-__global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned long long *__restrict__ accum, uint32_t n_local_px, uint32_t n,
-                                                              double target, RzNoisePartial *__restrict__ out) {
+// n_px (nullable): per-pixel sample counts of an adaptive frame, else every pixel has n samples.
+__global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned long long *__restrict__ accum, const uint32_t *__restrict__ n_px,
+                                                              uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *__restrict__ out) {
     __shared__ double s_sum[256], s_sum2[256], s_max[256];
     __shared__ unsigned long long s_above[256];
     double sum = 0, sum2 = 0, mx = 0;
     unsigned long long above = 0;
     for (uint32_t lp = blockIdx.x * 256u + threadIdx.x; lp < n_local_px; lp += RZ_NOISE_GRID * 256u) {
         const unsigned long long *q = accum + (size_t)lp * 4;
-        const double e = (double)(float)rz_pixel_err(q[0], q[1], q[2], q[3], n);   // the value out_err shows
+        const double e = (double)(float)rz_pixel_err(q[0], q[1], q[2], q[3], n_px ? n_px[lp] : n);   // the value out_err shows
         sum += e; sum2 += e * e; mx = fmax(mx, e); above += e > target ? 1u : 0u;
     }
     s_sum[threadIdx.x] = sum; s_sum2[threadIdx.x] = sum2; s_max[threadIdx.x] = mx; s_above[threadIdx.x] = above;
@@ -90,9 +97,9 @@ __global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned lon
 
 extern "C" uint32_t rz_noise_grid(void) { return RZ_NOISE_GRID; }
 // out: RZ_NOISE_GRID x 4 words (sum, sum2, max as doubles, then the count as an integer)
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, uint32_t n_local_px, uint32_t n, double target, void *out,
-                                              cudaStream_t stream) {
-    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_local_px, n, target, (RzNoisePartial *)out);
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, uint32_t n_local_px, uint32_t n,
+                                              double target, void *out, cudaStream_t stream) {
+    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, n_local_px, n, target, (RzNoisePartial *)out);
     return cudaGetLastError();
 }
 

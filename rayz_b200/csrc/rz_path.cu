@@ -62,7 +62,8 @@ struct RzStream {
 };
 
 // G = sphere PAIRS per search-loop iteration
-template <int R, int G, bool STATS, int MB, bool QUEUE>
+// LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list)
+template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false>
 __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -133,8 +134,9 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
                         st[r].alive = true;
                         need = false;
                     } else {
-                        const uint32_t lp = unit_lp0 + (k & 31u);
-                        if (lp < a.n_local_px) {
+                        uint32_t lp = unit_lp0 + (k & 31u);
+                        if (lp < (LIST ? a.n_list : a.n_local_px)) {
+                            if (LIST) lp = __ldg(a.px_list + lp);
                             uint32_t pi, pj;
                             rz_local_to_global(lp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
                             st[r].lp = lp;
@@ -615,9 +617,9 @@ __global__ void RZ_SECOND_BOUNDS rz_second_kernel(const RzPathArgs a) {
 }
 
 // ------------------------------------------------------------------------------ launchers
-template <int R, int G, bool STATS, int MB, bool QUEUE>
+template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false>
 static cudaError_t rz_launch_one(const RzPathArgs &a, int sm_count, size_t smem, cudaStream_t stream, int *grid_out) {
-    auto kern = rz_path_kernel<R, G, STATS, MB, QUEUE>;
+    auto kern = rz_path_kernel<R, G, STATS, MB, QUEUE, LIST>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int per_sm = 0;
@@ -712,7 +714,7 @@ extern "C" cudaError_t rz_launch_second(const RzPathArgs *a, int collect_stats, 
 }
 
 // Last stage (q_in != nullptr): the persistent megakernel started from a queue; or the single-stage form
-// (q_in == nullptr) that generates its own camera rays.  rays_per_thread in {1,2}.
+// (q_in == nullptr) that generates its own camera rays (of the pixels of px_list when it is set).  rays_per_thread in {1,2}.
 extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, int collect_stats, int sm_count, cudaStream_t stream,
                                       int *grid_out) {
     const bool stats = collect_stats != 0;
@@ -723,6 +725,13 @@ extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, 
                          : rz_launch_one<1, 2, false, 5, true>(*a, sm_count, smem, stream, grid_out);
         return stats ? rz_launch_one<2, 2, true, 5, true>(*a, sm_count, smem, stream, grid_out)
                      : rz_launch_one<2, 2, false, 8, true>(*a, sm_count, smem, stream, grid_out);
+    }
+    if (a->px_list) {   // an adaptive round: the same instances over the listed pixels
+        if (rays_per_thread == 1)
+            return stats ? rz_launch_one<1, 2, true, 5, false, true>(*a, sm_count, smem, stream, grid_out)
+                         : rz_launch_one<1, 2, false, 5, false, true>(*a, sm_count, smem, stream, grid_out);
+        return stats ? rz_launch_one<2, 2, true, 5, false, true>(*a, sm_count, smem, stream, grid_out)
+                     : rz_launch_one<2, 2, false, 8, false, true>(*a, sm_count, smem, stream, grid_out);
     }
     if (rays_per_thread == 1)
         return stats ? rz_launch_one<1, 2, true, 5, false>(*a, sm_count, smem, stream, grid_out)

@@ -334,9 +334,14 @@ class Backend:
         return err, nz.as_dict()
 
     def render_to_noise(self, cam: abi.RzCamera, p: abi.RzRenderParams, target: float, max_spp: int, want_linear=True,
-                        want_rgb8=True):
+                        want_rgb8=True, adaptive=False):
         """rayz_cuda_render_to_noise: p.spp samples, then batches doubling the count until rms_err <= target or max_spp.
-        Returns (linear [rows,w,4] f32, rgb8 [rows,w,3] u8, paths, summary dict as noise())."""
+        adaptive (RZ_RENDER_ADAPTIVE): the same schedule per pixel, until every pixel's error is <= target or max_spp; the
+        per-pixel counts are then pixel_samples().  Returns (linear [rows,w,4] f32, rgb8 [rows,w,3] u8, paths, summary dict
+        as noise())."""
+        if adaptive:
+            p = abi.RzRenderParams.from_buffer_copy(p)
+            p.flags |= abi.RENDER_ADAPTIVE
         rows = self.shard_rows(p)
         lin = np.empty((rows, p.width, 4), dtype=np.float32) if want_linear else None
         rgb8 = np.empty((rows, p.width, 3), dtype=np.uint8) if want_rgb8 else None
@@ -346,6 +351,16 @@ class Backend:
                                                      rgb8.ctypes.data if want_rgb8 else None, C.byref(n), C.byref(nz)))
         self._acc_shape = (p.height, p.width, p.shard_index, p.shard_count, p.band_rows)
         return lin, rgb8, n.value, nz.as_dict()
+
+    def pixel_samples(self) -> np.ndarray:
+        """rayz_cuda_pixel_samples: every pixel's sample count of the accumulated frame -> [rows,w] u32 (uniform after a
+        plain render or batches, each pixel's own after render_to_noise(adaptive=True))."""
+        if self._acc_shape is None:   # nothing rendered: the library says why
+            abi.check(self.lib.rayz_cuda_pixel_samples(self._h, None))
+        rows, w = int(self.lib.rayz_cuda_context_rows(self._h, self._acc_shape[0], *self._acc_shape[2:])), self._acc_shape[1]
+        out = np.empty((rows, w), dtype=np.uint32)
+        abi.check(self.lib.rayz_cuda_pixel_samples(self._h, out.ctypes.data))
+        return out
 
     def primary_ids(self, cam: abi.RzCamera, width: int, height: int, use_bvh=True) -> np.ndarray:
         out = np.empty((height, width), dtype=np.int32)
@@ -408,6 +423,7 @@ class Tracer:
         self.variant = "auto"
         self.devices = devices
         self.noise = None          # summary of the last render(noise_target=...) (rayz_cuda_render_to_noise)
+        self.pixel_samples = None  # [h, w] per-pixel sample counts of the last render(noise_target=..., adaptive=True)
         self._backend = None
 
     @property
@@ -416,17 +432,19 @@ class Tracer:
             self._backend = Backend(self.devices)
         return self._backend
 
-    def render(self, noise_target: float | None = None, max_spp: int = 4096) -> int:
+    def render(self, noise_target: float | None = None, max_spp: int = 4096, adaptive: bool = False) -> int:
         """noise_target (displayed-value rms error, 1/255 = one 8-bit step): start at samples_per_px and double the samples
         until the frame's rms error reaches it or max_spp samples are in (rayz_cuda_render_to_noise); `self.noise` then holds
-        the summary.  Without it, one render of samples_per_px, as the reference."""
+        the summary.  adaptive: the target bounds every pixel's error, and only the pixels still above it get more samples;
+        `self.pixel_samples` then holds the counts.  Without a target, one render of samples_per_px, as the reference."""
         b = self.backend
         b.upload_scene(self.pool.arrays())  # initHittables + bvh.build (renderer.zig:76-78)
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant)
         if noise_target is None:
             lin, rgb8, rays = b.render(self.camera.rz, p)
         else:
-            lin, rgb8, rays, self.noise = b.render_to_noise(self.camera.rz, p, noise_target, max_spp)
+            lin, rgb8, rays, self.noise = b.render_to_noise(self.camera.rz, p, noise_target, max_spp, adaptive=adaptive)
+            self.pixel_samples = b.pixel_samples() if adaptive else None
         self.img.pixels[:] = lin.reshape(-1, 4)[:, :3]
         self.img.rgb8 = rgb8
         return rays

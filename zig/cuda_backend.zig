@@ -73,6 +73,7 @@ pub const RzConfig = extern struct {
 
 pub const RZ_RENDER_MOMENTS: u32 = 2; // sum each path's luminance squared: rayz_cuda_noise
 pub const RZ_RENDER_ACCUMULATE: u32 = 4; // add this batch to the previous render's sums (progressive rendering)
+pub const RZ_RENDER_ADAPTIVE: u32 = 8; // rayz_cuda_render_to_noise: the target bounds every pixel, only pixels above it get more samples
 
 pub const RzNoise = extern struct {
     samples: u64,
@@ -93,6 +94,7 @@ pub extern fn rayz_cuda_render(ctx: *RzContext, cam: *const RzCamera, params: *c
 pub extern fn rayz_cuda_primary_ids(ctx: *RzContext, cam: *const RzCamera, width: u32, height: u32, use_bvh: c_int, out_ids: [*]i32) c_int;
 pub extern fn rayz_cuda_noise(ctx: *RzContext, target: f32, out_err: ?[*]f32, out: ?*RzNoise) c_int;
 pub extern fn rayz_cuda_render_to_noise(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, target: f32, max_spp: u32, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8, out_paths: ?*u64, out_noise: ?*RzNoise) c_int;
+pub extern fn rayz_cuda_pixel_samples(ctx: *RzContext, out_spp: [*]u32) c_int;
 pub extern fn rayz_cuda_last_error() [*:0]const u8;
 
 pub const Error = error{ CudaBackend, OutOfMemory };
