@@ -3,6 +3,7 @@
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
+//               [--guides PREFIX]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -11,7 +12,8 @@
 // step) starts at --spp samples and doubles them until the frame reaches X or --max-spp (default 4096); the samples reached
 // and the error go to stderr, the report line and the P3 output are unchanged.  With --adaptive, X bounds every pixel's error
 // and only the pixels still above it get more samples (RZ_RENDER_ADAPTIVE); stderr then also reports the paths traced and the
-// mean and max samples per pixel.
+// mean and max samples per pixel.  --guides PREFIX also writes the guide buffers of the render's camera samples for a denoiser
+// (rayz_cuda_render_guides) as PFM files: PREFIX_albedo.pfm and PREFIX_normal.pfm (3 channels), PREFIX_depth.pfm (1 channel).
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -36,7 +38,7 @@ int main(int argc, char **argv) {
     size_t spp = 10, depth = 50;
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
-    const char *dump_scene = nullptr, *dump_linear = nullptr;
+    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr;
     bool ppm_bench = false, penultimate = false, adaptive = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
@@ -55,6 +57,7 @@ int main(int argc, char **argv) {
         else if (a == "--noise-target") noise_target = std::strtof(val(), nullptr);
         else if (a == "--max-spp") max_spp = (uint32_t)std::strtoul(val(), nullptr, 10);
         else if (a == "--adaptive") adaptive = true;
+        else if (a == "--guides") guides = val();
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -94,6 +97,18 @@ int main(int argc, char **argv) {
             std::fprintf(stderr, "  [rayz_cuda] adaptive: %.0f paths, mean %.2f spp, max %llu spp, max error %.5f (%.2f 8-bit steps)\n", rays_traced,
                          rays_traced / std::max<double>(1.0, tracer.noise.n_pixels), (unsigned long long)tracer.noise.samples, tracer.noise.max_err,
                          tracer.noise.max_err * 255.0);
+        if (guides) {
+            tracer.renderGuides();
+            const struct { const char *name; const std::vector<float> &src; size_t first, channels; } files[3] = {
+                {"_albedo.pfm", tracer.albedo, 0, 3}, {"_normal.pfm", tracer.normal, 0, 3}, {"_depth.pfm", tracer.normal, 3, 1}};
+            for (const auto &o : files) {
+                const std::string path = std::string(guides) + o.name;
+                FILE *f = std::fopen(path.c_str(), "wb");
+                if (!f) { std::perror(path.c_str()); return 1; }
+                writePFM(f, o.src.data(), tracer.img.w, tracer.img.h, 4, o.first, o.channels);
+                std::fclose(f);
+            }
+        }
         if (dump_scene && !dumpScene(tracer, dump_scene)) { std::perror(dump_scene); return 1; }
         if (dump_linear) {
             FILE *f = std::fopen(dump_linear, "wb");

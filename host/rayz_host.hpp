@@ -221,6 +221,22 @@ struct Image {
     }
 };
 
+// PFM (portable float map) as OIDN's tools read it: "PF\n" (3 channels) or "Pf\n" (1 channel), "<w> <h>\n", "-1.0\n" (a negative
+// scale means little-endian), then f32 samples with the rows from the BOTTOM of the image to the top.  Takes `channels` floats
+// from each pixel of `src`, starting at float `first` of every `stride`; src rows are top to bottom.  Returns the bytes written.
+inline size_t writePFM(FILE *f, const float *src, size_t w, size_t h, size_t stride, size_t first, size_t channels) {
+    char head[64];
+    const int hn = std::snprintf(head, sizeof head, "%s\n%zu %zu\n-1.0\n", channels == 3 ? "PF" : "Pf", w, h);
+    size_t n = std::fwrite(head, 1, (size_t)hn, f);
+    std::vector<float> row(w * channels);
+    for (size_t j = h; j-- > 0;) {
+        for (size_t i = 0; i < w; i++)
+            for (size_t c = 0; c < channels; c++) row[i * channels + c] = src[(j * w + i) * stride + first + c];
+        n += std::fwrite(row.data(), sizeof(float), row.size(), f) * sizeof(float);
+    }
+    return n;
+}
+
 struct CudaBackendError : std::runtime_error {
     int code;
     CudaBackendError(int c, const char *msg) : std::runtime_error(msg), code(c) {}
@@ -245,6 +261,7 @@ struct Tracer {
     uint32_t max_spp = 4096;      // ... or this many samples are in
     RzNoise noise{};              // summary of the last render with a noise target
     bool adaptive = false;        // with noise_target: it bounds every pixel's error, and only pixels above it get more samples (RZ_RENDER_ADAPTIVE)
+    std::vector<float> albedo, normal;   // guide buffers of the last renderGuides(): rgb albedo + coverage, normal + hit distance (4 floats a pixel)
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
         : rng(seed) {
@@ -325,6 +342,16 @@ struct Tracer {
         for (size_t i = 0; i < img.w * img.h; i++) img.pixels[i] = {lin[4 * i], lin[4 * i + 1], lin[4 * i + 2]};
         rayz_cuda_timing(ctx, &timing);
         return (size_t)rays;
+    }
+
+    // Guide buffers for a denoiser over the camera samples render() traces (rayz_cuda_render_guides), after render().
+    void renderGuides() {
+        RzRenderParams p = renderParams();
+        p.flags = 0;
+        const RzCamera cam = camera.flat();
+        albedo.assign(img.w * img.h * 4, 0.f);
+        normal.assign(img.w * img.h * 4, 0.f);
+        check(rayz_cuda_render_guides(ctx, &cam, &p, albedo.data(), normal.data()));
     }
 };
 

@@ -289,6 +289,27 @@ int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, const RzRende
  */
 int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp);
 
+/*
+ * Guide buffers for a denoiser, of the camera samples [p->sample_offset, p->sample_offset + p->spp) of every pixel of the
+ * context's rows: the SAME camera rays (seed, global pixel, sample index -> jitter, lens point, time) a render with these
+ * parameters traces, each followed to its first hit only.  Host outputs, each nullable, laid out like out_linear_rgba:
+ *   out_albedo : rows * width * 4 floats: rgb = mean over all samples of the first hit's albedo,
+ *                a = coverage (fraction of samples that hit a sphere)
+ *   out_normal : rows * width * 4 floats: xyz = mean over all samples of the hit's unit normal (facing the ray, 0 for a miss),
+ *                w = mean hit distance over the samples that hit (0 if none did)
+ * Per sample: albedo = the texture colour at the f64-refined hit point for diffuse and metallic materials (the attenuation of
+ * their scatter, also where a metal's scatter would be absorbed), (1, 1, 1) for dielectrics, the sky colour of the ray's
+ * direction for a miss; normal = the unit normal of the hit in world space, flipped against the ray; distance = the hit's t
+ * along the unit camera ray from its lens-sampled origin.  Each pixel's samples are summed in f64 in sample order and the f32
+ * mean is written, so the buffers depend on (scene, camera, seed, pixel, sample range) only: not on shards, devices or launch
+ * shape.  The search is the BVH kernel's (RZ_VARIANT_BVH) whatever the variant; max_depth and collect_stats have no effect.
+ * Parameters a render refuses are refused with its codes and messages, prefixed "guides:"; RZ_RENDER_ACCUMULATE and
+ * RZ_RENDER_ADAPTIVE are refused with RZ_ERR_INVALID_ARG.  RZ_ERR_INTERNAL if the traversal stack overflowed (results withheld,
+ * the context stays usable).  Leaves the accumulated frame, its sample counts, RzStats and RzTiming untouched (a render
+ * enqueued by rayz_cuda_render_device(sync = 0) is waited for first, as rayz_cuda_noise does).
+ */
+int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float *out_albedo, float *out_normal);
+
 /* Number of image rows a shard owns under the banding rule above. */
 uint32_t rayz_cuda_shard_rows(uint32_t height, uint32_t shard_index, uint32_t shard_count,
                               uint32_t band_rows);

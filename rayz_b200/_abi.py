@@ -101,6 +101,7 @@ SYMBOLS = {
     "rayz_cuda_render_to_noise": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_float, C.c_uint32,
                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(RzNoise)]),
     "rayz_cuda_pixel_samples": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "rayz_cuda_render_guides": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_void_p, C.c_void_p]),
     "rayz_cuda_shard_rows": (C.c_uint32, [C.c_uint32] * 4),
     "rayz_cuda_context_rows": (C.c_uint32, [C.c_void_p] + [C.c_uint32] * 4),
     "rayz_cuda_primary_ids": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]),

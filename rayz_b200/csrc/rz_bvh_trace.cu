@@ -595,6 +595,80 @@ __global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_
     }
 }
 
+// First-hit albedo of a guide sample: the attenuation rz_scatter gives for the hit (rz_shade_segment's decode of the material
+// record, kept apart so that the path kernels stay as they are), whether or not a metal's scatter would be absorbed.
+__device__ __forceinline__ float3 rz_guide_albedo(const RzPathArgs &a, int k, const RzHit &h) {
+    const float4 *mr = a.mats.rec + 4u * a.set.mat[k];
+    const float4 m0 = __ldg(mr);
+    const uint32_t mbits = __float_as_uint(m0.x);
+    if ((mbits & 3u) >= 2u) return f3(1.f, 1.f, 1.f);   // dielectric (rz_scatter's third branch)
+    const float4 m1 = __ldg(mr + 1), m2 = __ldg(mr + 2), m3 = __ldg(mr + 3);
+    RzMatRec M;
+    M.kind = mbits & 3u; M.method = (mbits >> 2) & 3u; M.solid = ((mbits >> 4) & 1u) != 0u; M.checker2 = ((mbits >> 5) & 1u) != 0u;
+    M.fuzz = m0.y; M.ior = m0.z; M.tex = __float_as_uint(m0.w);
+    M.color = f3(m1.x, m1.y, m1.z); M.odd = f3(m2.x, m2.y, m2.z);
+    M.inv_scale = __hiloint2double(__float_as_int(m3.y), __float_as_int(m3.x));
+    return M.solid ? M.color : M.checker2 ? rz_checker2(M, h.px, h.py, h.pz) : rz_texture(a.texs, M.tex, h.px, h.py, h.pz);
+}
+
+// Guide buffers: the camera samples [sample_offset, sample_offset + spp) of every local pixel, each traced to its first hit by
+// the unstaged K3's walk (rz_bvh_round, the same tree and the same (t, k)), in this translation unit so that the camera ray
+// and the walk compile with the path kernels' flags.  One warp per 8 x 4 block of local rows, one lane per pixel, the warp's
+// samples in lockstep: a block's rays fan out over a third of the angle of 32 pixels of a row (the camera stage's reason for
+// the same blocks), so the lanes visit more of the same nodes.  Each lane sums its pixel's samples in f64, in sample order, and
+// divides once: the result depends on (scene, camera, seed, pixel, sample range) only.
+__global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGuideArgs g) {
+    const RzPathArgs &a = g.a;
+    const unsigned lane = threadIdx.x & 31u;
+    const float4 *__restrict__ nodes = reinterpret_cast<const float4 *>(a.bvh);
+    const uint32_t block = blockIdx.x * 4u + (threadIdx.x >> 5), tiles_x = (a.width + 7u) >> 3;
+    const uint32_t ty = block / tiles_x, tx = block - ty * tiles_x;
+    const uint32_t ti = tx * 8u + (lane & 7u), lp = (ty * 4u + (lane >> 3)) * a.width + ti;
+    const bool valid = ti < a.width && lp < a.n_local_px;
+    if (!__any_sync(0xffffffffu, valid)) return;   // the grid's last CTA: a warp past the last block
+    uint32_t pi = 0, pj = 0;
+    if (valid) rz_local_to_global(lp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
+    const uint32_t gpix = pj * a.width + pi;
+    const int descend_min = (int)a.bvh_descend_min;
+    int stack[RZ_STACK];
+    unsigned long long c_none = 0;   // rz_bvh_round's counters: untouched without STATS
+    double alb_r = 0, alb_g = 0, alb_b = 0, nx = 0, ny = 0, nz = 0, dist = 0;
+    uint32_t hits = 0;
+    for (uint32_t s = 0; s < a.spp; s++) {
+        RzRay ray;
+        if (valid) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi);
+        else { ray.o = f3(0.f, 0.f, 0.f); ray.d = f3(0.f, 1.f, 0.f); ray.time = 0.f; ray.self_k = -1; }
+        const float ix = 1.0f / ray.d.x, iy = 1.0f / ray.d.y, iz = 1.0f / ray.d.z;
+        float bt = 3.0e38f;
+        int bk = -1, sp = 0, cur = valid ? 0 : RZ_SENTINEL;
+        while (__any_sync(0xffffffffu, cur != RZ_SENTINEL))
+            rz_bvh_round<false>(a, nodes, ray, ix, iy, iz, cur, sp, stack, bt, bk, descend_min, c_none, c_none);
+        if (!valid) continue;
+        float3 alb;
+        if (bk < 0) {
+            alb = rz_sky(ray.d);   // a miss guides to its own radiance
+        } else {
+            const int k = bk & ~RZ_FAR_BIT;
+            const RzHit h = rz_refine_hit(a.set, ray, k, (bk & RZ_FAR_BIT) != 0);
+            alb = rz_guide_albedo(a, k, h);
+            nx += (double)h.n.x; ny += (double)h.n.y; nz += (double)h.n.z;
+            dist += (double)bt;
+            hits++;
+        }
+        alb_r += (double)alb.x; alb_g += (double)alb.y; alb_b += (double)alb.z;
+    }
+    if (!valid) return;
+    size_t dst = lp;
+    if (g.dev_count > 1u) {   // rz_resolve_kernel's band arithmetic
+        const uint32_t lr = lp / a.width, lb = lr / a.band_rows, within = lr - lb * a.band_rows;
+        dst = (size_t)((lb * g.dev_count + g.dev_index) * a.band_rows + within) * a.width + ti;
+    }
+    const double n = (double)a.spp;
+    if (g.out_albedo) g.out_albedo[dst] = make_float4((float)(alb_r / n), (float)(alb_g / n), (float)(alb_b / n), (float)((double)hits / n));
+    if (g.out_normal)
+        g.out_normal[dst] = make_float4((float)(nx / n), (float)(ny / n), (float)(nz / n), hits ? (float)(dist / (double)hits) : 0.f);
+}
+
 template <class K>
 cudaError_t launch_kernel(K kern, const RzPathArgs &a, int sm_count, cudaStream_t stream) {
     int per_sm = 0;
@@ -636,6 +710,17 @@ extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int
     if (b.px_list)
         return collect_stats ? launch_kernel(rz_bvh_kernel<true, false, 512, true>, b, sm_count, stream) : launch_kernel(rz_bvh_kernel<false, false, 512, true>, b, sm_count, stream);
     return collect_stats ? launch_kernel(rz_bvh_kernel<true, false>, b, sm_count, stream) : launch_kernel(rz_bvh_kernel<false, false>, b, sm_count, stream);
+}
+
+// Guide buffers of the device's local pixels: one warp per 8 x 4 block, four per CTA.
+extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t stream) {
+    RzGuideArgs b = *g;
+    rz_bvh_tuning(b.a);
+    const uint32_t rows = b.a.width ? b.a.n_local_px / b.a.width : 0u;
+    const uint32_t blocks = ((b.a.width + 7u) / 8u) * ((rows + 3u) / 4u);
+    if (blocks == 0u) return cudaSuccess;
+    rz_guides_kernel<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
+    return cudaGetLastError();
 }
 
 // One segment per launch: camera segments (q_in == nullptr) or the sorted entries of q_in; survivors -> q_out.

@@ -44,6 +44,7 @@ extern "C" cudaError_t rz_bvh_warm(void);
 extern "C" uint32_t rz_bvh_camera_tile_w(void);
 extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t stream);
 extern "C" size_t rz_lbvh_scratch_bytes(uint32_t n);
 extern "C" cudaError_t rz_bvh_finalize(RzBvhNode *nodes, uint32_t n_nodes, cudaStream_t stream);
 extern "C" cudaError_t rz_lbvh_build(uint32_t n, int leaf_max, const double4 *c64, const double4 *v64, const uint32_t *mat, void *scratch,
@@ -170,6 +171,7 @@ struct Dev {
     DBuf<float> out_err;              // rayz_cuda_noise: per-pixel error of the context's rows (gather root only)
     DBuf<double> noise_part;          // rayz_cuda_noise: the reduction's per-CTA partials of this device
     DBuf<uint32_t> out_spp;           // rayz_cuda_pixel_samples: per-pixel sample counts of the context's rows (gather root only)
+    DBuf<float4> out_guides;          // rayz_cuda_render_guides: albedo, then normal + depth, of the context's rows (gather root only)
     DBuf<uint32_t> n_px;              // RZ_RENDER_ADAPTIVE: every local pixel's sample count
     DBuf<uint32_t> px_list;           // RZ_RENDER_ADAPTIVE: the local pixels the next round traces, in increasing order
     DBuf<uint32_t> list_scratch;      // RZ_RENDER_ADAPTIVE: the list kernels' mask words, block offsets and list length (rz_adaptive.cu)
@@ -743,14 +745,14 @@ static int plan_and_alloc_queues(const RzTuning &tun, Dev &D, QueuePlan &qp, uin
 }
 
 // Every device's error word (RZ_DEV_ERR_*), read behind everything enqueued on its streams: RZ_ERR_INTERNAL if one is set, as
-// a device-side capacity was exceeded and work was dropped.
-static int read_error_words(RzContext *ctx) {
+// a device-side capacity was exceeded and work was dropped.  `who` prefixes the message.
+static int read_error_words(RzContext *ctx, const char *who = "render") {
     for (Dev &D : ctx->devs) {
         unsigned int ew = 0;
         RZ_CUDA(cudaSetDevice(D.id));
         RZ_CUDA(cudaMemcpyAsync(&ew, D.errword.p, sizeof ew, cudaMemcpyDeviceToHost, D.stream));
         RZ_CUDA(cudaStreamSynchronize(D.stream));
-        if (ew) return rz_fail(RZ_ERR_INTERNAL, "render: device %d reported%s%s (error word 0x%x): paths were dropped, result withheld", D.id,
+        if (ew) return rz_fail(RZ_ERR_INTERNAL, "%s: device %d reported%s%s (error word 0x%x): paths were dropped, result withheld", who, D.id,
                                (ew & RZ_DEV_ERR_QUEUE_OVERFLOW) ? " a queue overflow" : "", (ew & RZ_DEV_ERR_STACK_OVERFLOW) ? " a traversal-stack overflow" : "", ew);
     }
     return RZ_OK;
@@ -851,16 +853,16 @@ struct RenderPlan {
     bool list = false;                  // an adaptive round after the first: only the pixels of each device's list (Dev::px_list)
 };
 
-// Plans a render of these parameters, with the validations (and messages) of rayz_cuda_render.  cam == nullptr plans for
-// rayz_cuda_reserve: no scene is needed and no accumulation record is made.  n_list (rayz_cuda_render_to_noise's adaptive
-// rounds after the first, RZ_RENDER_ADAPTIVE | RZ_RENDER_ACCUMULATE): per device, the length of its pixel list.
+// Plans a render of these parameters, with the validations (and messages, prefixed `who`) of rayz_cuda_render.  cam == nullptr
+// plans for rayz_cuda_reserve: no scene is needed and no accumulation record is made.  n_list (rayz_cuda_render_to_noise's
+// adaptive rounds after the first, RZ_RENDER_ADAPTIVE | RZ_RENDER_ACCUMULATE): per device, the length of its pixel list.
+// rayz_cuda_render_guides validates its parameters here too and uses the rows of the plan.
 static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, const AccumRecord &prev, RenderPlan &P,
-                       const uint32_t *n_list = nullptr) {
+                       const char *who, const uint32_t *n_list = nullptr) {
     P.p = p;
     P.cam = cam;
     P.list = n_list != nullptr;
-    const char *who = cam ? "render" : "reserve";
-    if (cam && !ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "render: rayz_cuda_upload_scene has not been called");
+    if (cam && !ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "%s: rayz_cuda_upload_scene has not been called", who);
     if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "%s: width, height and spp must be > 0", who);
     if ((uint64_t)p->width * p->height >= (1ull << 31)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: image too large", who);
     P.sh = Shard(p->shard_index, p->shard_count, p->band_rows);
@@ -1169,7 +1171,7 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     const AccumRecord prev = ctx->acc;
     ctx->acc.valid = false;
     RenderPlan P;
-    if (const int rc = plan_render(ctx, cam, p, prev, P, n_list)) {
+    if (const int rc = plan_render(ctx, cam, p, prev, P, "render", n_list)) {
         if (P.refused) ctx->acc = prev;
         return rc;
     }
@@ -1215,7 +1217,7 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
 extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     if (!ctx || !p) return rz_fail(RZ_ERR_INVALID_ARG, "reserve: NULL argument");
     RenderPlan P;
-    int rc = plan_render(ctx, nullptr, p, ctx->acc, P);
+    int rc = plan_render(ctx, nullptr, p, ctx->acc, P, "reserve");
     if (rc) return rc;
     if (p->width != ctx->acc.width || p->height != ctx->acc.height || P.sh.s != ctx->acc.shard_index || P.sh.S != ctx->acc.shard_count || P.sh.band != ctx->acc.band_rows)
         ctx->acc.valid = false;   // another frame shape: a next batch may not add to the sums
@@ -1418,6 +1420,67 @@ extern "C" int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp) {
     }
     RZ_CUDA(cudaSetDevice(D0.id));
     RZ_CUDA(cudaMemcpyAsync(out_spp, D0.out_spp.p, (size_t)rows_ctx * A.width * sizeof(uint32_t), cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    return RZ_OK;
+}
+
+// Guide buffers (include/rayz_cuda.h): every device traces its rows' camera samples to their first hits with rz_guides_kernel,
+// which stores straight into the gather root's buffers like the resolve kernel; the error words are read behind every stream,
+// then the root's buffers are copied out.  The accumulators, their record, the per-pixel counts, stats and timing stay as
+// they are.
+extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float *out_albedo, float *out_normal) {
+    if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "guides: NULL argument");
+    if (p->flags & (RZ_RENDER_ACCUMULATE | RZ_RENDER_ADAPTIVE))
+        return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_ACCUMULATE and RZ_RENDER_ADAPTIVE do not apply to guide buffers");
+    RenderPlan P;
+    if (const int rc = plan_render(ctx, cam, p, ctx->acc, P, "guides")) return rc;
+    DeviceGuard guard;
+    // a render enqueued by rayz_cuda_render_device(sync = 0) reports through the error words this call clears: read them first
+    { const int rc = settle_accumulation(ctx); if (rc) return rc; }
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    const size_t npx = (size_t)P.rows_ctx * p->width;
+    Dev &D0 = ctx->devs[0];
+    int rc;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if ((rc = D0.out_guides.alloc(2 * npx))) return rc;
+    rc = for_each_device(ctx, [&](uint32_t d) -> int {
+        Dev &D = ctx->devs[d];
+        const DevPlan &dp = P.dev[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        int r;
+        if ((r = D.errword.alloc(4))) return r;
+        RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
+        RzGuideArgs g;
+        memset(&g, 0, sizeof g);
+        RzPathArgs &a = g.a;   // the fields enqueue_device sets for the K3 kernels
+        a.set = D.bvhset.view();
+        a.mats.kind = D.m_kind.p; a.mats.fuzz = D.m_fuzz.p; a.mats.ior = D.m_ior.p; a.mats.tex = D.m_tex.p; a.mats.method = D.m_method.p; a.mats.rec = D.m_rec.p;
+        a.texs.kind = D.t_kind.p; a.texs.color = D.t_color.p; a.texs.inv_scale = D.t_inv_scale.p; a.texs.even = D.t_even.p; a.texs.odd = D.t_odd.p;
+#ifdef RZ_BVH_WIDE
+        a.bvh = D.bvh4.p; a.bvh_nodes = D.bvh_nodes;
+#else
+        a.bvh = D.bvh.p; a.bvh_nodes = D.bvh_nodes;
+#endif
+        a.cam = cam_to_f32(cam);
+        a.width = p->width; a.height = p->height; a.n_local_px = dp.n_local;
+        a.spp = p->spp; a.sample_offset = p->sample_offset;
+        a.shard_index = P.sh.s * ND + d; a.shard_count = P.sh.S * ND; a.band_rows = P.sh.band;
+        a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
+        a.t_min = p->t_min > 0 ? p->t_min : 1e-4f;
+        a.err = D.errword.p;
+        a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
+        a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
+        g.out_albedo = D0.out_guides.p;
+        g.out_normal = D0.out_guides.p + npx;
+        g.dev_index = d; g.dev_count = ND;
+        RZ_CUDA(rz_launch_guides(&g, D.stream));
+        return RZ_OK;
+    });
+    if (rc) return rc;
+    if ((rc = read_error_words(ctx, "guides"))) return rc;   // behind every device's stream: the root's buffers are complete
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if (out_albedo) RZ_CUDA(cudaMemcpyAsync(out_albedo, D0.out_guides.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
+    if (out_normal) RZ_CUDA(cudaMemcpyAsync(out_normal, D0.out_guides.p + npx, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
     RZ_CUDA(cudaStreamSynchronize(D0.stream));
     return RZ_OK;
 }

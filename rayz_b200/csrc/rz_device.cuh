@@ -176,6 +176,17 @@ struct RzPathArgs {
     uint32_t n_list;             // entries in px_list
 };
 
+// Guide buffers (rayz_cuda_render_guides, rz_guides_kernel in rz_bvh_trace.cu): the camera segments of a render with these
+// RzPathArgs, each followed to its first hit only.  The outputs are the gather root's buffers at the context's rows (peer
+// pointers on the other devices), addressed as rz_resolve_kernel addresses its frame.
+struct RzGuideArgs {
+    RzPathArgs a;                 // set (the BVH-ordered one), mats, texs, bvh, cam, frame and shard fields, spp, sample_offset,
+                                  // seeds, t_min, err, stack_cap, bvh_descend_min; nothing else is read
+    float4 *out_albedo;           // nullable: rgb = mean first-hit albedo, a = fraction of samples that hit a sphere
+    float4 *out_normal;           // nullable: xyz = mean unit normal facing the ray (0 for a miss), w = mean hit distance of the hits
+    uint32_t dev_index, dev_count;   // local row lr -> context row ((lr / band_rows) * dev_count + dev_index) * band_rows + lr % band_rows
+};
+
 // ---------------------------------------------------------------------------------------------
 // Per-pixel noise (RZ_RENDER_MOMENTS, DESIGN.md "Progressive rendering").  Slot 3 of a pixel's accumulator sums Y^2 over its
 // paths in the 2^-32 fixed point of slots 0..2, Y = Rec. 709 luminance of the same clamped radiance the three colour atomics

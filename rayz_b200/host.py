@@ -362,6 +362,16 @@ class Backend:
         abi.check(self.lib.rayz_cuda_pixel_samples(self._h, out.ctypes.data))
         return out
 
+    def guides(self, cam: abi.RzCamera, p: abi.RzRenderParams):
+        """rayz_cuda_render_guides: the first hits of the camera samples a render with these parameters traces ->
+        (albedo [rows,w,4] f32: rgb mean albedo, a coverage; normal [rows,w,4] f32: xyz mean unit normal, w mean hit distance).
+        Leaves the accumulated frame, stats and timing as they were."""
+        rows = self.shard_rows(p)
+        albedo = np.empty((rows, p.width, 4), dtype=np.float32)
+        normal = np.empty((rows, p.width, 4), dtype=np.float32)
+        abi.check(self.lib.rayz_cuda_render_guides(self._h, C.byref(cam), C.byref(p), albedo.ctypes.data, normal.ctypes.data))
+        return albedo, normal
+
     def primary_ids(self, cam: abi.RzCamera, width: int, height: int, use_bvh=True) -> np.ndarray:
         out = np.empty((height, width), dtype=np.int32)
         abi.check(self.lib.rayz_cuda_primary_ids(self._h, C.byref(cam), width, height, 1 if use_bvh else 0, out.ctypes.data))
@@ -424,6 +434,8 @@ class Tracer:
         self.devices = devices
         self.noise = None          # summary of the last render(noise_target=...) (rayz_cuda_render_to_noise)
         self.pixel_samples = None  # [h, w] per-pixel sample counts of the last render(noise_target=..., adaptive=True)
+        self.albedo = None         # [h, w, 4] guide buffers of the last render_guides(): rgb albedo + coverage
+        self.normal = None         # [h, w, 4] ... unit normal + hit distance
         self._backend = None
 
     @property
@@ -448,6 +460,17 @@ class Tracer:
         self.img.pixels[:] = lin.reshape(-1, 4)[:, :3]
         self.img.rgb8 = rgb8
         return rays
+
+
+    def render_guides(self):
+        """Guide buffers for a denoiser over the camera samples render() traces (samples_per_px, seed): first-hit albedo with
+        coverage, and normal with hit distance (rayz_cuda_render_guides).  Returns (albedo, normal), also kept as
+        self.albedo and self.normal."""
+        b = self.backend
+        b.upload_scene(self.pool.arrays())
+        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant)
+        self.albedo, self.normal = b.guides(self.camera.rz, p)
+        return self.albedo, self.normal
 
 
 # ------------------------------------------------------------------------------- scenes (rayz.zig)

@@ -95,6 +95,8 @@ pub extern fn rayz_cuda_primary_ids(ctx: *RzContext, cam: *const RzCamera, width
 pub extern fn rayz_cuda_noise(ctx: *RzContext, target: f32, out_err: ?[*]f32, out: ?*RzNoise) c_int;
 pub extern fn rayz_cuda_render_to_noise(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, target: f32, max_spp: u32, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8, out_paths: ?*u64, out_noise: ?*RzNoise) c_int;
 pub extern fn rayz_cuda_pixel_samples(ctx: *RzContext, out_spp: [*]u32) c_int;
+// guide buffers for a denoiser: first-hit albedo + coverage, normal + hit distance (rows * width * 4 floats each)
+pub extern fn rayz_cuda_render_guides(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, out_albedo: ?[*]f32, out_normal: ?[*]f32) c_int;
 pub extern fn rayz_cuda_last_error() [*:0]const u8;
 
 pub const Error = error{ CudaBackend, OutOfMemory };
