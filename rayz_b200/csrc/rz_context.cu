@@ -177,7 +177,6 @@ struct Dev {
     DBuf<uint32_t> list_scratch;      // RZ_RENDER_ADAPTIVE: the list kernels' mask words, block offsets and list length (rz_adaptive.cu)
     DBuf<float4> loc_linear;          // multi-device render into HOST buffers: this device's own rows, copied out over its own PCIe link
     DBuf<uint8_t> loc_rgb8;
-    uint32_t loc_rows = 0;            // rows of the last such render
     DBuf<int32_t> ids;
     DBuf<float> sink;
     void *wf_scratch = nullptr;
@@ -205,12 +204,24 @@ struct Dev {
     }
 };
 
-// What the accumulators of the context's devices hold (RZ_RENDER_ACCUMULATE, include/rayz_cuda.h): the frame, shard and
-// sampling parameters a next batch must repeat, and the samples summed so far.  The device set is the context's own.
+// RzRenderParams' image size and shard fields as every render reads them: shard_count 0 or 1 is the whole frame (S = 1,
+// s = 0), band_rows 0 means 4.  Equal frames put the same pixels on every device (FrameSplit).
+struct Frame {
+    uint32_t width = 0, height = 0, S = 1, s = 0, band = 4;
+    Frame() = default;
+    Frame(uint32_t w, uint32_t h, uint32_t index, uint32_t count, uint32_t band_rows) : width(w), height(h), S(count <= 1 ? 1u : count), s(count <= 1 ? 0u : index), band(band_rows ? band_rows : 4u) {}
+    explicit Frame(const RzRenderParams *p) : Frame(p->width, p->height, p->shard_index, p->shard_count, p->band_rows) {}
+    bool operator==(const Frame &o) const { return width == o.width && height == o.height && S == o.S && s == o.s && band == o.band; }
+    bool operator!=(const Frame &o) const { return !(*this == o); }
+};
+
+// What the accumulators of the context's devices hold (RZ_RENDER_ACCUMULATE, include/rayz_cuda.h): the frame and sampling
+// parameters a next batch must repeat, and the samples summed so far.  The device set is the context's own.
 struct AccumRecord {
     bool valid = false;
     bool pending = false;   // enqueued by rayz_cuda_render_device(sync = 0): the device error words are not checked yet
-    uint32_t width = 0, height = 0, shard_index = 0, shard_count = 1, band_rows = 4, max_depth = 0, moments = 0;
+    Frame frame;
+    uint32_t max_depth = 0, moments = 0;
     uint64_t seed = 0;
     float t_min = 0;
     RzCamera cam{};
@@ -248,19 +259,27 @@ extern "C" uint32_t rayz_cuda_shard_rows(uint32_t height, uint32_t shard_index, 
     return rows;
 }
 
-// RzRenderParams' shard fields as every render reads them: shard_count 0 or 1 is the whole frame, band_rows 0 means 4.
-struct Shard {
-    uint32_t S, s, band;
-    Shard(uint32_t index, uint32_t count, uint32_t band_rows) : S(count <= 1 ? 1u : count), s(count <= 1 ? 0u : index), band(band_rows ? band_rows : 4u) {}
+// How a frame is dealt to the context's devices (ctx == nullptr: one device): device d renders shard s * ND + d of S * ND,
+// and the gather root's buffers hold the rows of all of them.
+struct FrameSplit {
+    uint32_t rows[RZ_MAX_DEVICES] = {}, n_local[RZ_MAX_DEVICES] = {};   // per device: rows and pixels
+    uint32_t rows_ctx = 0;                                              // of all the devices
+    size_t npx = 0;                                                     // pixels of those rows
+    FrameSplit() = default;
+    FrameSplit(const RzContext *ctx, const Frame &f) {
+        const uint32_t nd = ctx ? (uint32_t)ctx->devs.size() : 1u;
+        for (uint32_t d = 0; d < nd; d++) {
+            rows[d] = rayz_cuda_shard_rows(f.height, f.s * nd + d, f.S * nd, f.band);
+            n_local[d] = rows[d] * f.width;
+            rows_ctx += rows[d];
+        }
+        npx = (size_t)rows_ctx * f.width;
+    }
 };
 
 extern "C" uint32_t rayz_cuda_context_rows(const RzContext *ctx, uint32_t height, uint32_t shard_index, uint32_t shard_count,
                                            uint32_t band_rows) {
-    const Shard sh(shard_index, shard_count, band_rows);
-    const uint32_t nd = ctx ? (uint32_t)ctx->devs.size() : 1u;
-    uint32_t rows = 0;
-    for (uint32_t d = 0; d < nd; d++) rows += rayz_cuda_shard_rows(height, sh.s * nd + d, sh.S * nd, sh.band);
-    return rows;
+    return FrameSplit(ctx, Frame(0, height, shard_index, shard_count, band_rows)).rows_ctx;
 }
 
 // ------------------------------------------------------------------------------ host-side sphere sets (the tree builders: rz_host_bvh.hpp)
@@ -744,6 +763,14 @@ static int plan_and_alloc_queues(const RzTuning &tun, Dev &D, QueuePlan &qp, uin
     }
 }
 
+static int sync_devices(RzContext *ctx) {
+    for (Dev &D : ctx->devs) {
+        RZ_CUDA(cudaSetDevice(D.id));
+        RZ_CUDA(cudaStreamSynchronize(D.stream));
+    }
+    return RZ_OK;
+}
+
 // Every device's error word (RZ_DEV_ERR_*), read behind everything enqueued on its streams: RZ_ERR_INTERNAL if one is set, as
 // a device-side capacity was exceeded and work was dropped.  `who` prefixes the message.
 static int read_error_words(RzContext *ctx, const char *who = "render") {
@@ -758,8 +785,10 @@ static int read_error_words(RzContext *ctx, const char *who = "render") {
     return RZ_OK;
 }
 
-// Device timings (CUDA events) and, if asked for, the counters of the render that just finished on every stream.
-static int collect_timing_and_stats(RzContext *ctx, bool collect_stats) {
+// The end of a synchronous render: waits for every device, then reads the device timings (CUDA events), the error words and,
+// if asked for, the counters of the render; total_ms is the host time since the caller's t0.
+static int finish_render(RzContext *ctx, bool collect_stats, std::chrono::steady_clock::time_point t0) {
+    if (const int rc = sync_devices(ctx)) return rc;
     float kmax = 0, rmax = 0, pmax = 0, smax = 0, somax = 0;
     uint32_t passes = 0;
     for (Dev &D : ctx->devs) {
@@ -814,6 +843,7 @@ static int collect_timing_and_stats(RzContext *ctx, bool collect_stats) {
         for (int k = 0; k < 3; k++) ctx->stage_stats[k] = stage[k];
         ctx->stats_valid = true;
     }
+    ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return RZ_OK;
 }
 
@@ -829,9 +859,17 @@ static int settle_accumulation(RzContext *ctx) {
     return RZ_OK;
 }
 
+// The accumulated frame, settled, for the readouts of its sums; `who` prefixes the refusal when there is none.
+static int accumulated_frame(RzContext *ctx, const char *who, const AccumRecord *&A) {
+    if (const int rc = settle_accumulation(ctx)) return rc;
+    A = &ctx->acc;
+    if (!A->valid) return rz_fail(RZ_ERR_INVALID_ARG, "%s: no accumulated render (none, it failed, or a scene upload or reserve came in between)", who);
+    return RZ_OK;
+}
+
 // ------------------------------------------------------------------------------ render plan
 struct DevPlan {
-    uint32_t rows = 0, n_local = 0, n_tiles = 0, n_units = 0;   // n_units: work units of the first kernel
+    uint32_t n_tiles = 0, n_units = 0;                           // n_units: work units of the first kernel
     uint32_t n_list = 0;                                         // adaptive round: the pixels listed on this device
     QueuePlan qp;                                                // staged: the passes alloc_render could allocate
 };
@@ -842,8 +880,9 @@ struct RenderPlan {
     const RzRenderParams *p = nullptr;
     const RzCamera *cam = nullptr;   // nullptr: planned for rayz_cuda_reserve
     bool host_direct = false;        // every device resolves into its OWN compact buffers; rayz_cuda_render copies them out in parallel
-    Shard sh{0, 1, 0};
-    uint32_t variant = 0, rows_ctx = 0;   // variant: resolved to RZ_VARIANT_MEGA, _BVH or _WAVEFRONT; rows_ctx: of all the devices
+    Frame frame;
+    FrameSplit split;
+    uint32_t variant = 0;            // resolved to RZ_VARIANT_MEGA, _BVH or _WAVEFRONT
     bool mega_single = false, staged = false;   // staged: enqueue_staged; else one kernel, or the wavefront's own loop
     bool bvh_family = false, bvh_tail = false, enough_spheres = false, serial = false;   // the staged form's plan_queues inputs
     uint32_t chunk = 0, n_chunks = 0, tile_w = 0;   // the first kernel's work-unit size; tile_w: staged K3's camera-stage blocks
@@ -865,8 +904,8 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
     if (cam && !ctx->have_scene) return rz_fail(RZ_ERR_NO_SCENE, "%s: rayz_cuda_upload_scene has not been called", who);
     if (p->width == 0 || p->height == 0 || p->spp == 0) return rz_fail(RZ_ERR_INVALID_ARG, "%s: width, height and spp must be > 0", who);
     if ((uint64_t)p->width * p->height >= (1ull << 31)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: image too large", who);
-    P.sh = Shard(p->shard_index, p->shard_count, p->band_rows);
-    const uint32_t S = P.sh.S, s = P.sh.s, band = P.sh.band, ND = (uint32_t)ctx->devs.size();
+    P.frame = Frame(p);
+    const uint32_t S = P.frame.S, s = P.frame.s, ND = (uint32_t)ctx->devs.size();
     if (s >= S) return rz_fail(RZ_ERR_INVALID_ARG, "%s: shard_index %u >= shard_count %u", who, s, S);
     const Dev &D0 = ctx->devs[0];
     const uint32_t brute_smem = (D0.brute.n_pad * 2 - D0.brute.n_static_pad) * 16u;
@@ -895,7 +934,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
 
     if (cam) {
         AccumRecord &next = P.next;
-        next.width = p->width; next.height = p->height; next.shard_index = s; next.shard_count = S; next.band_rows = band;
+        next.frame = P.frame;
         next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
@@ -905,8 +944,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
             if (!prev.valid) return refuse("no previous render to add to (none, it failed, or a scene upload or reserve came in between)");
             if (prev.adaptive != next.adaptive)
                 return refuse("the accumulated frame was rendered adaptively: its pixels hold different sample counts, so no sample_offset continues it");
-            if (prev.width != next.width || prev.height != next.height || prev.shard_index != s || prev.shard_count != S || prev.band_rows != band)
-                return refuse("frame size, shard or band_rows differ from the accumulated render");
+            if (prev.frame != next.frame) return refuse("frame size, shard or band_rows differ from the accumulated render");
             if (prev.seed != next.seed || prev.max_depth != next.max_depth || memcmp(&prev.t_min, &next.t_min, sizeof(float)) != 0)
                 return refuse("seed, max_depth or t_min differ from the accumulated render");
             if (memcmp(&prev.cam, cam, sizeof(RzCamera)) != 0) return refuse("the camera differs from the accumulated render");
@@ -947,19 +985,17 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
     const uint32_t chunk = std::min(ctx->tun.chunk, p->spp), n_chunks = (p->spp + chunk - 1) / chunk;
     P.chunk = P.staged ? std::min(ctx->tun.chunk_primary, p->spp) : chunk;   // the camera-stage kernels build a culled sphere list per unit: their own, larger work-unit size
     P.n_chunks = (p->spp + P.chunk - 1) / P.chunk;
+    P.split = FrameSplit(ctx, P.frame);
     for (uint32_t d = 0; d < ND; d++) {
         DevPlan &dp = P.dev[d];
-        dp.rows = rayz_cuda_shard_rows(p->height, s * ND + d, S * ND, band);
-        dp.n_local = dp.rows * p->width;
-        dp.n_tiles = (dp.n_local + 31u) / 32u;
-        P.rows_ctx += dp.rows;
+        dp.n_tiles = (P.split.n_local[d] + 31u) / 32u;
         if ((uint64_t)dp.n_tiles * n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: too many work units", who);
         uint64_t tiles = dp.n_tiles;
         if (P.list) {   // work unit u: list entries [tile * 32, tile * 32 + 32) x one chunk of samples
             dp.n_list = n_list[d];
             tiles = (dp.n_list + 31u) / 32u;
         }
-        const uint64_t blocks = (uint64_t)((p->width + 7u) / 8u) * ((dp.rows + 3u) / 4u);   // K3's camera stage works on 8 x 4 pixel blocks
+        const uint64_t blocks = (uint64_t)((p->width + 7u) / 8u) * ((P.split.rows[d] + 3u) / 4u);   // K3's camera stage works on 8 x 4 pixel blocks
         if (P.tile_w) tiles = blocks;
         else if (P.staged && !ctx->have_scene) tiles = std::max(tiles, blocks);
         if (tiles * P.n_chunks >= (1ull << 32)) return rz_fail(RZ_ERR_INVALID_ARG, "%s: too many work units", who);
@@ -971,30 +1007,30 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
 // Everything the plan needs on every device, so that enqueueing it allocates nothing.  The one exception is the wavefront
 // form's scratch, which rz_wavefront_render sizes itself.
 static int alloc_render(RzContext *ctx, RenderPlan &P) {
-    const uint32_t width = P.p->width;
     int rc;
     if (!P.host_direct) {   // the gather root's frame, into which every device's resolve scatters its rows
         Dev &D0 = ctx->devs[0];
         RZ_CUDA(cudaSetDevice(D0.id));
-        if ((rc = D0.out_linear.alloc((size_t)P.rows_ctx * width)) || (rc = D0.out_rgb8.alloc((size_t)P.rows_ctx * width * 3))) return rc;
+        if ((rc = D0.out_linear.alloc(P.split.npx)) || (rc = D0.out_rgb8.alloc(P.split.npx * 3))) return rc;
     }
     for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {
         Dev &D = ctx->devs[d];
         DevPlan &dp = P.dev[d];
+        const uint32_t n_local = P.split.n_local[d];
         RZ_CUDA(cudaSetDevice(D.id));
         if ((rc = D.accum.alloc((size_t)dp.n_tiles * 32u * 4u))) return rc;
         if ((rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4))) return rc;
         if ((rc = D.stats.alloc(3))) return rc;   // [0] whole render / primary kernel, [1] sorted stages, [2] persistent tail kernel
-        if (P.staged && dp.n_local > 0) {
+        if (P.staged && n_local > 0) {
             if ((rc = plan_and_alloc_queues(ctx->tun, D, dp.qp, dp.n_units, P.chunk, P.serial, P.enough_spheres, P.bvh_family, P.bvh_tail))) return rc;
             // the sorted-segment kernel's pair lists, one row per sort group
             if (dp.qp.second_stage && !P.bvh_family && ctx->have_scene && (rc = D.bin_lists.alloc((size_t)RZ_SORT_BINS * rz_bin_row_bytes(D.brute.n_pad)))) return rc;
             for (cudaEvent_t e = nullptr; D.pass_ev.size() < 3 * (size_t)dp.qp.n_pass; D.pass_ev.push_back(e)) RZ_CUDA(cudaEventCreate(&e));
             for (cudaEvent_t e = nullptr; D.stage_ev.size() < 2 * (size_t)dp.qp.n_pass * dp.qp.n_second; D.stage_ev.push_back(e)) RZ_CUDA(cudaEventCreate(&e));
         }
-        if (P.host_direct && ((rc = D.loc_linear.alloc((size_t)dp.n_local)) || (rc = D.loc_rgb8.alloc((size_t)dp.n_local * 3)))) return rc;
+        if (P.host_direct && ((rc = D.loc_linear.alloc((size_t)n_local)) || (rc = D.loc_rgb8.alloc((size_t)n_local * 3)))) return rc;
         if ((P.p->flags & RZ_RENDER_ADAPTIVE) &&
-            ((rc = D.n_px.alloc(dp.n_local)) || (rc = D.px_list.alloc(dp.n_local)) || (rc = D.list_scratch.alloc(rz_list_scratch_words(dp.n_local)))))
+            ((rc = D.n_px.alloc(n_local)) || (rc = D.px_list.alloc(n_local)) || (rc = D.list_scratch.alloc(rz_list_scratch_words(n_local)))))
             return rc;
     }
     return RZ_OK;
@@ -1003,7 +1039,7 @@ static int alloc_render(RzContext *ctx, RenderPlan &P) {
 // The staged form on one device: primary kernel (tile-culled camera segments; K3: the block-culled camera stage) -> queue ->
 // [sort -> sorted-segment kernel (culled per unit) -> queue] x n_second -> persistent tail kernel (BVH, or brute force).
 // Passes are sized by the queues (RzTuning::queue_log2, default 2^27 entries per buffer; two buffers per side, two sides).
-// collect_timing_and_stats reads pass_ev and stage_ev by index: their records belong to the streams and places they have here.
+// finish_render reads pass_ev and stage_ev by index: their records belong to the streams and places they have here.
 static int enqueue_staged(RzContext *ctx, Dev &D, RzPathArgs a, const RenderPlan &P, const QueuePlan &qp, uint32_t &launches) {
     const RzCamera *cam = P.cam;
     const RzRenderParams *p = P.p;
@@ -1090,25 +1126,16 @@ static int enqueue_staged(RzContext *ctx, Dev &D, RzPathArgs a, const RenderPlan
     return RZ_OK;
 }
 
-// Everything device d does for this render, enqueued on its streams into what alloc_render allocated.
-static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint32_t &launches) {
+// The path-kernel arguments of device d's share of the planned frame that do not depend on the kernel form: the BVH-ordered
+// set, scene, camera, frame and shard, sampling, t_min, error word and traversal tuning.  rayz_cuda_render_guides launches
+// rz_guides_kernel with them as they are (RzGuideArgs); enqueue_device adds the render's buffers and work units.
+static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t d) {
     const RzRenderParams *p = P.p;
     const uint32_t ND = (uint32_t)ctx->devs.size();
-    Dev &D = ctx->devs[d], &D0 = ctx->devs[0];
-    const DevPlan &dp = P.dev[d];
-    const bool adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
-    const bool trace = dp.n_local > 0 && (!P.list || dp.n_list > 0);   // a device with an empty list launches nothing
-    RZ_CUDA(cudaSetDevice(D.id));
-    RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
-    if (!(p->flags & RZ_RENDER_ACCUMULATE)) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
-    if (adaptive && !P.list) RZ_CUDA(rz_launch_fill_u32(D.n_px.p, dp.n_local, p->spp, D.stream));   // first round: every pixel
-    RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
-    RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
-    if (p->collect_stats) RZ_CUDA(cudaMemsetAsync(D.stats.p, 0, 3 * sizeof(RzStatsDev), D.stream));
-
+    const Dev &D = ctx->devs[d];
     RzPathArgs a;
     memset(&a, 0, sizeof a);
-    a.set = (P.variant == RZ_VARIANT_BVH) ? D.bvhset.view() : D.brute.view();
+    a.set = D.bvhset.view();
     a.mats.kind = D.m_kind.p; a.mats.fuzz = D.m_fuzz.p; a.mats.ior = D.m_ior.p; a.mats.tex = D.m_tex.p; a.mats.method = D.m_method.p; a.mats.rec = D.m_rec.p;
     a.texs.kind = D.t_kind.p; a.texs.color = D.t_color.p; a.texs.inv_scale = D.t_inv_scale.p; a.texs.even = D.t_even.p; a.texs.odd = D.t_odd.p;
 #ifdef RZ_BVH_WIDE
@@ -1117,17 +1144,50 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     a.bvh = D.bvh.p; a.bvh_nodes = D.bvh_nodes;
 #endif
     a.cam = cam_to_f32(P.cam);
-    a.accum = D.accum.p; a.unit_counter = D.counter.p; a.stats = D.stats.p;
-    a.width = p->width; a.height = p->height; a.n_local_px = dp.n_local;
+    a.width = p->width; a.height = p->height; a.n_local_px = P.split.n_local[d];
     a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;
-    a.chunk = P.chunk; a.n_chunks = P.n_chunks; a.n_units = dp.n_units; a.tile_w = P.tile_w;
-    a.shard_index = P.sh.s * ND + d; a.shard_count = P.sh.S * ND; a.band_rows = P.sh.band;
+    a.shard_index = P.frame.s * ND + d; a.shard_count = P.frame.S * ND; a.band_rows = P.frame.band;
     a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
-    a.t_min = p->t_min > 0 ? p->t_min : 1e-4f;
+    a.t_min = P.next.t_min;   // plan_render applied the default
     a.err = D.errword.p;
     a.unit_entries = ctx->tun.unit_entries;
     a.bvh_active_min = (uint32_t)ctx->tun.bvh_active_min; a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
     a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
+    return a;
+}
+
+// The resolve kernel's arguments for device d's n_local pixels of the accumulated frame A: its sums, over each pixel's own
+// count when A is adaptive, scattered band by band into the gather root's rows.  Every output starts null.
+static RzResolveArgs resolve_args(const RzContext *ctx, uint32_t d, const AccumRecord &A, uint32_t n_local) {
+    const Dev &D = ctx->devs[d];
+    RzResolveArgs r{};
+    r.accum = D.accum.p;
+    r.n_px = A.adaptive ? D.n_px.p : nullptr;
+    r.n_local_px = n_local; r.width = A.frame.width; r.spp = (uint32_t)A.samples;
+    r.dev_index = d; r.dev_count = (uint32_t)ctx->devs.size(); r.band_rows = A.frame.band;
+    return r;
+}
+
+// Everything device d does for this render, enqueued on its streams into what alloc_render allocated.
+static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint32_t &launches) {
+    const RzRenderParams *p = P.p;
+    Dev &D = ctx->devs[d], &D0 = ctx->devs[0];
+    const DevPlan &dp = P.dev[d];
+    const uint32_t n_local = P.split.n_local[d];
+    const bool adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
+    const bool trace = n_local > 0 && (!P.list || dp.n_list > 0);   // a device with an empty list launches nothing
+    RZ_CUDA(cudaSetDevice(D.id));
+    RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
+    if (!(p->flags & RZ_RENDER_ACCUMULATE)) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
+    if (adaptive && !P.list) RZ_CUDA(rz_launch_fill_u32(D.n_px.p, n_local, p->spp, D.stream));   // first round: every pixel
+    RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
+    RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
+    if (p->collect_stats) RZ_CUDA(cudaMemsetAsync(D.stats.p, 0, 3 * sizeof(RzStatsDev), D.stream));
+
+    RzPathArgs a = path_args(ctx, P, d);
+    if (P.variant != RZ_VARIANT_BVH) a.set = D.brute.view();
+    a.accum = D.accum.p; a.unit_counter = D.counter.p; a.stats = D.stats.p;
+    a.chunk = P.chunk; a.n_chunks = P.n_chunks; a.n_units = dp.n_units; a.tile_w = P.tile_w;
     a.moments = P.next.moments;
     if (P.list) { a.px_list = D.px_list.p; a.n_list = dp.n_list; }
 
@@ -1147,14 +1207,10 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     }
     RZ_CUDA(cudaEventRecord(D.ev[2], D.stream));
 
-    RzResolveArgs r;
-    r.accum = D.accum.p; r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p; r.out_err = nullptr; r.out_spp = nullptr;
-    r.n_px = adaptive ? D.n_px.p : nullptr;
-    r.n_local_px = trace ? dp.n_local : 0u; r.width = p->width; r.spp = (uint32_t)P.next.samples;   // cumulative with RZ_RENDER_ACCUMULATE
-    r.dev_index = d; r.dev_count = ND; r.band_rows = P.sh.band;
+    RzResolveArgs r = resolve_args(ctx, d, P.next, trace ? n_local : 0u);   // the samples are cumulative with RZ_RENDER_ACCUMULATE
+    r.out_linear = D0.out_linear.p; r.out_rgb8 = D0.out_rgb8.p;
     if (P.host_direct) {
         r.out_linear = D.loc_linear.p; r.out_rgb8 = D.loc_rgb8.p; r.dev_index = 0; r.dev_count = 1;
-        D.loc_rows = dp.rows;
     }
     RZ_CUDA(rz_launch_resolve(&r, D.stream));
     if (trace) launches += 1;
@@ -1195,14 +1251,7 @@ static int render_impl(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     ctx->timing.launches = launches;
     ctx->timing.variant = P.mega_single ? (uint32_t)RZ_VARIANT_MEGA_SINGLE : P.variant;
     ctx->stats_valid = false;
-    if (sync) {
-        for (uint32_t d = 0; d < ND; d++) {
-            RZ_CUDA(cudaSetDevice(ctx->devs[d].id));
-            RZ_CUDA(cudaStreamSynchronize(ctx->devs[d].stream));
-        }
-        if ((rc = collect_timing_and_stats(ctx, p->collect_stats != 0))) return rc;
-        ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host0).count();
-    }
+    if (sync && (rc = finish_render(ctx, p->collect_stats != 0, t_host0))) return rc;
     ctx->acc = P.next;
     ctx->acc.valid = true;
     ctx->acc.pending = !sync;
@@ -1219,15 +1268,10 @@ extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     RenderPlan P;
     int rc = plan_render(ctx, nullptr, p, ctx->acc, P, "reserve");
     if (rc) return rc;
-    if (p->width != ctx->acc.width || p->height != ctx->acc.height || P.sh.s != ctx->acc.shard_index || P.sh.S != ctx->acc.shard_count || P.sh.band != ctx->acc.band_rows)
-        ctx->acc.valid = false;   // another frame shape: a next batch may not add to the sums
+    if (P.frame != ctx->acc.frame) ctx->acc.valid = false;   // another frame shape: a next batch may not add to the sums
     DeviceGuard guard;
     if ((rc = alloc_render(ctx, P))) return rc;
-    for (Dev &D : ctx->devs) {
-        RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaStreamSynchronize(D.stream));
-    }
-    return RZ_OK;
+    return sync_devices(ctx);
 }
 
 // RZ_RENDER_ADAPTIVE needs the rounds of rayz_cuda_render_to_noise; a single render cannot honour it.
@@ -1243,10 +1287,7 @@ extern "C" int rayz_cuda_render_device(RzContext *ctx, const RzCamera *cam, cons
     if (rc) return rc;
     if (d_linear_rgba) *d_linear_rgba = ctx->devs[0].out_linear.p;
     if (d_rgb8) *d_rgb8 = ctx->devs[0].out_rgb8.p;
-    if (out_paths) {
-        const uint32_t rows = rayz_cuda_context_rows(ctx, params->height, params->shard_index, params->shard_count, params->band_rows);
-        *out_paths = (uint64_t)rows * params->width * params->spp;
-    }
+    if (out_paths) *out_paths = (uint64_t)FrameSplit(ctx, Frame(params)).npx * params->spp;
     return RZ_OK;
 }
 
@@ -1281,14 +1322,14 @@ static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams
     const int rc = render_impl(ctx, cam, params, false, direct);
     if (rc) return rc;
     DeviceGuard guard;
-    const uint32_t rows = rayz_cuda_context_rows(ctx, params->height, params->shard_index, params->shard_count, params->band_rows);
-    const size_t npx = (size_t)rows * params->width;
+    const Frame f(params);
+    const FrameSplit sp(ctx, f);
     if (direct) {
-        const uint32_t band = Shard(params->shard_index, params->shard_count, params->band_rows).band, W = params->width;
+        const uint32_t band = f.band, W = f.width;
         for (uint32_t d = 0; d < ND; d++) {
             Dev &D = ctx->devs[d];
             RZ_CUDA(cudaSetDevice(D.id));
-            const uint32_t full = D.loc_rows / band, tail = D.loc_rows - full * band;   // whole bands + a partial last one
+            const uint32_t full = sp.rows[d] / band, tail = sp.rows[d] - full * band;   // whole bands + a partial last one
             auto copy = [&](void *dst0, const void *src0, size_t px_bytes) -> cudaError_t {
                 const size_t band_bytes = (size_t)band * W * px_bytes;
                 unsigned char *dst = (unsigned char *)dst0 + (size_t)d * band_bytes;
@@ -1303,16 +1344,11 @@ static int render_host(RzContext *ctx, const RzCamera *cam, const RzRenderParams
             if (out_rgb8) RZ_CUDA(copy(out_rgb8, D.loc_rgb8.p, 3));
         }
     } else {
-        const int rc2 = copy_frame_to_host(ctx, npx, out_linear_rgba, out_rgb8);
+        const int rc2 = copy_frame_to_host(ctx, sp.npx, out_linear_rgba, out_rgb8);
         if (rc2) return rc2;
     }
-    for (Dev &D : ctx->devs) {
-        RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaStreamSynchronize(D.stream));
-    }
-    { const int rc2 = collect_timing_and_stats(ctx, params->collect_stats != 0); if (rc2) return rc2; }
-    ctx->timing.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (out_paths) *out_paths = (uint64_t)npx * params->spp;
+    { const int rc2 = finish_render(ctx, params->collect_stats != 0, t0); if (rc2) return rc2; }
+    if (out_paths) *out_paths = (uint64_t)sp.npx * params->spp;
     return RZ_OK;
 }
 
@@ -1333,31 +1369,26 @@ extern "C" int rayz_cuda_render(RzContext *ctx, const RzCamera *cam, const RzRen
 extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzNoise *out) {
     if (!ctx) return rz_fail(RZ_ERR_INVALID_ARG, "noise: ctx is NULL");
     DeviceGuard guard;
-    { const int rc = settle_accumulation(ctx); if (rc) return rc; }
-    const AccumRecord &A = ctx->acc;
-    if (!A.valid) return rz_fail(RZ_ERR_INVALID_ARG, "noise: no accumulated render (none, it failed, or a scene upload or reserve came in between)");
-    if (!A.moments) return rz_fail(RZ_ERR_INVALID_ARG, "noise: the accumulated render(s) ran without RZ_RENDER_MOMENTS");
+    const AccumRecord *A = nullptr;
+    if (const int rc = accumulated_frame(ctx, "noise", A)) return rc;
+    if (!A->moments) return rz_fail(RZ_ERR_INVALID_ARG, "noise: the accumulated render(s) ran without RZ_RENDER_MOMENTS");
     const uint32_t ND = (uint32_t)ctx->devs.size(), G = rz_noise_grid();
     Dev &D0 = ctx->devs[0];
-    const uint32_t rows_ctx = rayz_cuda_context_rows(ctx, A.height, A.shard_index, A.shard_count, A.band_rows);
+    const FrameSplit sp(ctx, A->frame);
     int rc;
     RZ_CUDA(cudaSetDevice(D0.id));
-    if (out_err && (rc = D0.out_err.alloc((size_t)rows_ctx * A.width))) return rc;
+    if (out_err && (rc = D0.out_err.alloc(sp.npx))) return rc;
     for (uint32_t d = 0; d < ND; d++) {   // every device enqueues before the first wait
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        const uint32_t n_local = rayz_cuda_shard_rows(A.height, A.shard_index * ND + d, A.shard_count * ND, A.band_rows) * A.width;
         if ((rc = D.noise_part.alloc(4 * (size_t)G))) return rc;
         if (out_err) {
-            RzResolveArgs r;
-            r.accum = D.accum.p; r.out_linear = nullptr; r.out_rgb8 = nullptr; r.out_err = D0.out_err.p; r.out_spp = nullptr;
-            r.n_px = A.adaptive ? D.n_px.p : nullptr;
-            r.n_local_px = n_local; r.width = A.width; r.spp = (uint32_t)A.samples;
-            r.dev_index = d; r.dev_count = ND; r.band_rows = A.band_rows;
+            RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
+            r.out_err = D0.out_err.p;
             RZ_CUDA(rz_launch_resolve(&r, D.stream));
         }
-        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A.adaptive ? D.n_px.p : nullptr, n_local, (uint32_t)A.samples, (double)target, D.noise_part.p,
-                                       D.stream));
+        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A->adaptive ? D.n_px.p : nullptr, sp.n_local[d], (uint32_t)A->samples, (double)target,
+                                       D.noise_part.p, D.stream));
     }
     double sum = 0, sum2 = 0, mx = 0;
     uint64_t above = 0;
@@ -1374,13 +1405,13 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
     }
     if (out_err) {
         RZ_CUDA(cudaSetDevice(D0.id));
-        RZ_CUDA(cudaMemcpyAsync(out_err, D0.out_err.p, (size_t)rows_ctx * A.width * sizeof(float), cudaMemcpyDeviceToHost, D0.stream));
+        RZ_CUDA(cudaMemcpyAsync(out_err, D0.out_err.p, sp.npx * sizeof(float), cudaMemcpyDeviceToHost, D0.stream));
         RZ_CUDA(cudaStreamSynchronize(D0.stream));
     }
     if (out) {
-        const double npx = (double)rows_ctx * A.width;
-        out->samples = A.samples;
-        out->n_pixels = rows_ctx * A.width;
+        const double npx = (double)sp.npx;
+        out->samples = A->samples;
+        out->n_pixels = (uint32_t)sp.npx;
         out->n_above = (uint32_t)above;
         out->mean_err = npx > 0 ? sum / npx : 0.0;
         out->rms_err = npx > 0 ? std::sqrt(sum2 / npx) : 0.0;
@@ -1394,32 +1425,23 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
 extern "C" int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp) {
     if (!ctx || !out_spp) return rz_fail(RZ_ERR_INVALID_ARG, "pixel_samples: NULL argument");
     DeviceGuard guard;
-    { const int rc = settle_accumulation(ctx); if (rc) return rc; }
-    const AccumRecord &A = ctx->acc;
-    if (!A.valid) return rz_fail(RZ_ERR_INVALID_ARG, "pixel_samples: no accumulated render (none, it failed, or a scene upload or reserve came in between)");
-    const uint32_t ND = (uint32_t)ctx->devs.size();
+    const AccumRecord *A = nullptr;
+    if (const int rc = accumulated_frame(ctx, "pixel_samples", A)) return rc;
     Dev &D0 = ctx->devs[0];
-    const uint32_t rows_ctx = rayz_cuda_context_rows(ctx, A.height, A.shard_index, A.shard_count, A.band_rows);
+    const FrameSplit sp(ctx, A->frame);
     int rc;
     RZ_CUDA(cudaSetDevice(D0.id));
-    if ((rc = D0.out_spp.alloc((size_t)rows_ctx * A.width))) return rc;
-    for (uint32_t d = 0; d < ND; d++) {
+    if ((rc = D0.out_spp.alloc(sp.npx))) return rc;
+    for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        RzResolveArgs r;
-        r.accum = D.accum.p; r.out_linear = nullptr; r.out_rgb8 = nullptr; r.out_err = nullptr; r.out_spp = D0.out_spp.p;
-        r.n_px = A.adaptive ? D.n_px.p : nullptr;
-        r.n_local_px = rayz_cuda_shard_rows(A.height, A.shard_index * ND + d, A.shard_count * ND, A.band_rows) * A.width;
-        r.width = A.width; r.spp = (uint32_t)A.samples;
-        r.dev_index = d; r.dev_count = ND; r.band_rows = A.band_rows;
+        RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
+        r.out_spp = D0.out_spp.p;
         RZ_CUDA(rz_launch_resolve(&r, D.stream));
     }
-    for (Dev &D : ctx->devs) {   // every device's rows are in the gather root's buffer
-        RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaStreamSynchronize(D.stream));
-    }
+    if ((rc = sync_devices(ctx))) return rc;   // every device's rows are in the gather root's buffer
     RZ_CUDA(cudaSetDevice(D0.id));
-    RZ_CUDA(cudaMemcpyAsync(out_spp, D0.out_spp.p, (size_t)rows_ctx * A.width * sizeof(uint32_t), cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaMemcpyAsync(out_spp, D0.out_spp.p, sp.npx * sizeof(uint32_t), cudaMemcpyDeviceToHost, D0.stream));
     RZ_CUDA(cudaStreamSynchronize(D0.stream));
     return RZ_OK;
 }
@@ -1438,38 +1460,20 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
     // a render enqueued by rayz_cuda_render_device(sync = 0) reports through the error words this call clears: read them first
     { const int rc = settle_accumulation(ctx); if (rc) return rc; }
     const uint32_t ND = (uint32_t)ctx->devs.size();
-    const size_t npx = (size_t)P.rows_ctx * p->width;
+    const size_t npx = P.split.npx;
     Dev &D0 = ctx->devs[0];
     int rc;
     RZ_CUDA(cudaSetDevice(D0.id));
     if ((rc = D0.out_guides.alloc(2 * npx))) return rc;
     rc = for_each_device(ctx, [&](uint32_t d) -> int {
         Dev &D = ctx->devs[d];
-        const DevPlan &dp = P.dev[d];
         RZ_CUDA(cudaSetDevice(D.id));
         int r;
         if ((r = D.errword.alloc(4))) return r;
         RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
         RzGuideArgs g;
         memset(&g, 0, sizeof g);
-        RzPathArgs &a = g.a;   // the fields enqueue_device sets for the K3 kernels
-        a.set = D.bvhset.view();
-        a.mats.kind = D.m_kind.p; a.mats.fuzz = D.m_fuzz.p; a.mats.ior = D.m_ior.p; a.mats.tex = D.m_tex.p; a.mats.method = D.m_method.p; a.mats.rec = D.m_rec.p;
-        a.texs.kind = D.t_kind.p; a.texs.color = D.t_color.p; a.texs.inv_scale = D.t_inv_scale.p; a.texs.even = D.t_even.p; a.texs.odd = D.t_odd.p;
-#ifdef RZ_BVH_WIDE
-        a.bvh = D.bvh4.p; a.bvh_nodes = D.bvh_nodes;
-#else
-        a.bvh = D.bvh.p; a.bvh_nodes = D.bvh_nodes;
-#endif
-        a.cam = cam_to_f32(cam);
-        a.width = p->width; a.height = p->height; a.n_local_px = dp.n_local;
-        a.spp = p->spp; a.sample_offset = p->sample_offset;
-        a.shard_index = P.sh.s * ND + d; a.shard_count = P.sh.S * ND; a.band_rows = P.sh.band;
-        a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
-        a.t_min = p->t_min > 0 ? p->t_min : 1e-4f;
-        a.err = D.errword.p;
-        a.bvh_descend_min = (uint32_t)ctx->tun.bvh_descend_min;
-        a.stack_cap = ctx->tun.debug_stack_cap;   // 0 = the kernel's own RZ_STACK
+        g.a = path_args(ctx, P, d);
         g.out_albedo = D0.out_guides.p;
         g.out_normal = D0.out_guides.p + npx;
         g.dev_index = d; g.dev_count = ND;
@@ -1488,20 +1492,14 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
 // Adaptive rounds: every device lists its active pixels (rz_adaptive.cu: count n_cur, error above the target) and adds `add`
 // to their counts; n_list[d] <- the length of device d's list, read behind its stream.
 static int build_pixel_lists(RzContext *ctx, uint32_t n_cur, uint32_t add, float target, uint32_t *n_list) {
-    const AccumRecord &A = ctx->acc;
-    const uint32_t ND = (uint32_t)ctx->devs.size();
-    for (uint32_t d = 0; d < ND; d++) {   // every device enqueues before the first wait
+    const FrameSplit sp(ctx, ctx->acc.frame);
+    for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {   // every device enqueues before the first wait
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        const uint32_t n_local = rayz_cuda_shard_rows(A.height, A.shard_index * ND + d, A.shard_count * ND, A.band_rows) * A.width;
-        RZ_CUDA(rz_launch_pixel_list(D.accum.p, D.n_px.p, n_local, n_cur, add, target, D.px_list.p, D.list_scratch.p, D.stream));
-        RZ_CUDA(cudaMemcpyAsync(&n_list[d], D.list_scratch.p + rz_list_count_word(n_local), sizeof(uint32_t), cudaMemcpyDeviceToHost, D.stream));
+        RZ_CUDA(rz_launch_pixel_list(D.accum.p, D.n_px.p, sp.n_local[d], n_cur, add, target, D.px_list.p, D.list_scratch.p, D.stream));
+        RZ_CUDA(cudaMemcpyAsync(&n_list[d], D.list_scratch.p + rz_list_count_word(sp.n_local[d]), sizeof(uint32_t), cudaMemcpyDeviceToHost, D.stream));
     }
-    for (Dev &D : ctx->devs) {
-        RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaStreamSynchronize(D.stream));
-    }
-    return RZ_OK;
+    return sync_devices(ctx);
 }
 
 // The stopping policy of progressive rendering, in one place for every host: batches that double the accumulated sample count
@@ -1517,7 +1515,7 @@ extern "C" int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, co
     q.flags = (p->flags & ~RZ_RENDER_ACCUMULATE) | RZ_RENDER_MOMENTS;
     RzNoise nz;
     memset(&nz, 0, sizeof nz);
-    const size_t npx = (size_t)rayz_cuda_context_rows(ctx, p->height, p->shard_index, p->shard_count, p->band_rows) * p->width;
+    const size_t npx = FrameSplit(ctx, Frame(p)).npx;
     uint64_t paths = 0;
     if (!(p->flags & RZ_RENDER_ADAPTIVE)) {
         for (;;) {
