@@ -28,7 +28,6 @@ UNITS = {
     "rz_adaptive.cu": [],
     "rz_ids.cu": ["--fmad=false"],
     "rz_bvh_build.cu": [],
-    "rz_bvh_wide.cu": [],
     "rz_sort.cu": [],
     "rz_bvh_trace.cu": ["--use_fast_math"],
     "rz_context.cu": [],

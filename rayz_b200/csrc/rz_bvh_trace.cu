@@ -5,7 +5,7 @@
 // loop of renderer.zig:85-126.  The reference recurses per ray, left child first; here every lane of
 // a persistent warp walks its own ray through a flattened BVH2 (both child boxes in the parent, 64 B,
 // read through ld.global.nc), near child first, with an explicit per-lane stack.  (A 4-wide tree was measured and
-// rejected: rz_bvh_round under RZ_BVH_WIDE below.)
+// rejected: DESIGN.md section 3, "K3 and the wide BVH".)
 //
 // What shapes the kernel is SIMT divergence, not arithmetic: the first version (per-lane
 // `while (stack)` with the leaf tests nested inside, rays replaced only between segments) ran with
@@ -46,15 +46,6 @@ constexpr int RZ_SENTINEL = 0x7fffffff;
 #ifndef RZ_BVH_MINB
 #define RZ_BVH_MINB 8
 #endif
-// Camera stage of a large scene: per 32-pixel tile, the tree is culled against the tile's cone of camera rays and the rays search the
-// surviving spheres as a list (rz_bvh_stage_kernel, CAMERA).  0 = every camera ray walks the tree on its own.
-#ifndef RZ_BVH_CAMERA_LISTS
-#define RZ_BVH_CAMERA_LISTS 1
-#endif
-#ifdef RZ_BVH_WIDE
-#undef RZ_BVH_CAMERA_LISTS
-#define RZ_BVH_CAMERA_LISTS 0
-#endif
 #ifndef RZ_BVH_CAMERA_MINB
 #define RZ_BVH_CAMERA_MINB 6   // resident CTAs of the camera stage with tile lists: cull + packed search + shading + the per-ray walk in one kernel
 #endif
@@ -64,79 +55,8 @@ constexpr int RZ_SENTINEL = 0x7fffffff;
 #ifndef RZ_CL_WL
 #define RZ_CL_WL 256           // nodes in flight during the cull (ring buffer; power of two)
 #endif
-#ifdef RZ_BVH_WIDE
-constexpr int RZ_STACK = 144;  // binary LBVH depth <= 96 = 48 wide levels x 3 pushes
-#else
 constexpr int RZ_STACK = 96;   // LBVH depth bound: 63 Morton bits + 32 index tie-break bits
-#endif
 
-
-#ifdef RZ_BVH_WIDE
-// EXPERIMENT (build with -DRZ_BVH_WIDE, scripts/exp_build.sh): the 4-wide tree of rz_bvh_wide.cu.  Measured on B200 and NOT
-// adopted: config-2 scene 3158 vs 3584 Mpaths/s, 99,856 spheres 1556 vs 1716 — the same number of box tests per segment
-// (27.6 vs 25 / 48.7 vs 47) in half as many, twice as long node visits, plus a sorting network per visit; the tree is L1/L2
-// resident, so the traversal is issue-bound, not latency-bound, and wider nodes buy nothing (DESIGN.md section 3).
-// One while-while round for this lane's ray through the 4-wide tree: descend through internal nodes to the next leaf (or
-// until the warp's round is cut short), then test that leaf.  Shared by the persistent kernel and the staged (sorted) kernels.
-template <bool STATS>
-__device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *__restrict__ nodes, const RzRay &ray, float ix, float iy,
-                                             float iz, int &cur, int &sp, int (&stack)[RZ_STACK], float &bt, int &bk, int descend_min,
-                                             unsigned long long &c_nodes, unsigned long long &c_sph) {
-    // (1) descend through internal nodes until this lane holds a leaf or runs dry; the round ends early
-    //     once fewer than `descend_min` lanes are still descending, so that lanes holding a leaf do not idle
-    //     behind a few long descents (those lanes simply resume in the next round)
-    while ((unsigned)cur < (unsigned)RZ_SENTINEL) {
-        // slab test of AABB.hit (hit.zig:70-98) with multiply-by-inverse on the FOUR child boxes of the node (128 B, eight
-        // 16-byte loads through the read-only path); boxes are padded outward at build time
-        if (STATS) c_nodes += 4;
-        const float4 *n = nodes + (size_t)cur * 8u;
-        const float4 lx = __ldg(n + 0), hx = __ldg(n + 1), ly = __ldg(n + 2), hy = __ldg(n + 3), lz = __ldg(n + 4), hz = __ldg(n + 5);
-        const int4 ch = __ldg(reinterpret_cast<const int4 *>(n + 6));
-        const uint4 cn = __ldg(reinterpret_cast<const uint4 *>(n + 7));
-        const float ox = ray.o.x, oy = ray.o.y, oz = ray.o.z;
-        float tn[4];
-        int ref[4];
-#define RZ_BOX4(c, LX, HX, LY, HY, LZ, HZ, CH, CN)                                                                          \
-        {                                                                                                                   \
-            const float a0 = ((LX) - ox) * ix, b0 = ((HX) - ox) * ix, a1 = ((LY) - oy) * iy, b1 = ((HY) - oy) * iy;          \
-            const float a2 = ((LZ) - oz) * iz, b2 = ((HZ) - oz) * iz;                                                       \
-            const float t0 = fmaxf(fmaxf(fminf(a0, b0), fminf(a1, b1)), fmaxf(fminf(a2, b2), a.t_min));                     \
-            const float t1 = fminf(fminf(fmaxf(a0, b0), fmaxf(a1, b1)), fminf(fmaxf(a2, b2), bt));                          \
-            const bool h = (t0 <= t1 * 1.0000004f) && ((CH) >= 0 || (CN) != 0u);   /* an unused slot is a leaf of 0 spheres */ \
-            tn[c] = h ? t0 : 3.0e38f;                                                                                       \
-            ref[c] = (CH) >= 0 ? (CH) : rz_leaf_ref((CH), (CN));   /* internal index >= 0, or a leaf (negative, with its count) */ \
-        }
-        RZ_BOX4(0, lx.x, hx.x, ly.x, hy.x, lz.x, hz.x, ch.x, cn.x)
-        RZ_BOX4(1, lx.y, hx.y, ly.y, hy.y, lz.y, hz.y, ch.y, cn.y)
-        RZ_BOX4(2, lx.z, hx.z, ly.z, hy.z, lz.z, hz.z, ch.z, cn.z)
-        RZ_BOX4(3, lx.w, hx.w, ly.w, hy.w, lz.w, hz.w, ch.w, cn.w)
-#undef RZ_BOX4
-        // sort the four (entry distance, child) pairs, nearest first: a 5-comparator network; misses (3e38) sink to the end
-#define RZ_CSWAP(i, j)                                                                           \
-        {                                                                                        \
-            const bool sw = tn[j] < tn[i];                                                       \
-            const float tf = sw ? tn[j] : tn[i], tg = sw ? tn[i] : tn[j];                        \
-            const int rf = sw ? ref[j] : ref[i], rg = sw ? ref[i] : ref[j];                      \
-            tn[i] = tf; tn[j] = tg; ref[i] = rf; ref[j] = rg;                                    \
-        }
-        RZ_CSWAP(0, 1) RZ_CSWAP(2, 3) RZ_CSWAP(0, 2) RZ_CSWAP(1, 3) RZ_CSWAP(1, 2)
-#undef RZ_CSWAP
-        if (tn[0] < 3.0e38f) {
-            // the nearest child next; the others go on the stack, farthest first
-#pragma unroll
-            for (int c = 3; c >= 1; c--) {
-                if (tn[c] < 3.0e38f) {
-                    if (sp < (int)a.stack_cap) stack[sp++] = ref[c];
-                    else atomicOr(a.err, (unsigned)RZ_DEV_ERR_STACK_OVERFLOW);   // a dropped subtree would darken the image silently
-                }
-            }
-            cur = ref[0];
-        } else {
-            cur = sp > 0 ? stack[--sp] : RZ_SENTINEL;
-        }
-        if (__popc(__activemask()) < descend_min) break;
-    }
-#else
 // One while-while round for this lane's ray: descend through internal nodes to the next leaf (or until the warp's round
 // is cut short), then test that leaf.  Shared by the persistent kernel and the staged (sorted) kernels.
 template <bool STATS>
@@ -157,11 +77,6 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
             const float4 q1 = __ldg(nodes + cur * 4 + 1);  // loy0 loy1 hiy0 hiy1
             const float4 q2 = __ldg(nodes + cur * 4 + 2);  // loz0 loz1 hiz0 hiz1
             q3 = __ldg(reinterpret_cast<const int4 *>(nodes + cur * 4 + 3));
-#ifdef RZ_BVH_SCALAR_SLABS   // experiment (scripts/exp_build.sh): the 24 scalar FADD / FMUL of round 2's first form
-            const float ax0 = (q0.x - ox) * ix, bx0 = (q0.z - ox) * ix, ax1 = (q0.y - ox) * ix, bx1 = (q0.w - ox) * ix;
-            const float ay0 = (q1.x - oy) * iy, by0 = (q1.z - oy) * iy, ay1 = (q1.y - oy) * iy, by1 = (q1.w - oy) * iy;
-            const float az0 = (q2.x - oz) * iz, bz0 = (q2.z - oz) * iz, az1 = (q2.y - oz) * iz, bz1 = (q2.w - oz) * iz;
-#else
             // the two children's planes sit side by side in the node, so (plane - o) * inv_d is one FADD2 + one FMUL2 for both
             // (packed FP32x2, the ray's operands as broadcasts): 12 issue slots instead of 24, the same IEEE operations per half
             float ax0, ax1, bx0, bx1, ay0, ay1, by0, by1, az0, az1, bz0, bz1;
@@ -173,7 +88,6 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
             rz_unpack(rz_mul2(rz_add2(rz_pack(q1.z, q1.w), noy), iy2), by0, by1);
             rz_unpack(rz_mul2(rz_add2(rz_pack(q2.x, q2.y), noz), iz2), az0, az1);
             rz_unpack(rz_mul2(rz_add2(rz_pack(q2.z, q2.w), noz), iz2), bz0, bz1);
-#endif
             tn0 = fmaxf(fmaxf(fminf(ax0, bx0), fminf(ay0, by0)), fmaxf(fminf(az0, bz0), a.t_min));
             tf0 = fminf(fminf(fmaxf(ax0, bx0), fmaxf(ay0, by0)), fminf(fmaxf(az0, bz0), bt));
             tn1 = fmaxf(fmaxf(fminf(ax1, bx1), fminf(ay1, by1)), fmaxf(fminf(az1, bz1), a.t_min));
@@ -197,7 +111,6 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
         }
         if (__popc(__activemask()) < descend_min) break;
     }
-#endif
     // (2) leaf phase
     if (cur < 0) {
         const int code = ~cur;
@@ -355,11 +268,10 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
 // rays tile by tile and scattered rays in SORTED order (key of rz_sort_key: origin cell, octant, reach), 32 rays per warp at
 // a time.  Rays that start together and head the same way walk the same nodes, so the warp stays converged and the nodes stay
 // in L1; survivors go to the next queue, and the tail of the paths to the persistent kernel above (QUEUE).
-// CAMERA with RZ_BVH_CAMERA_LISTS (the default): the camera rays of a work unit — an 8 x 4-pixel block x `chunk` samples — do
-// not walk the tree one by one; the warp culls the tree once against the block's cone and the rays search the surviving
-// spheres as a list (below).  The sorted stages (CAMERA = false) are off by default (RzTuning::bvh_stages = 0: measured as a loss).
+// CAMERA: the camera rays of a work unit — an 8 x 4-pixel block x `chunk` samples — do not walk the tree one by one; the warp
+// culls the tree once against the block's cone and the rays search the surviving spheres as a list (below).  The sorted stages (CAMERA = false) are off by default (RzTuning::bvh_stages = 0: measured as a loss).
 template <bool STATS, bool CAMERA>
-__global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB) rz_bvh_stage_kernel(const RzPathArgs a) {
+__global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB) rz_bvh_stage_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
     const float4 *__restrict__ nodes = reinterpret_cast<const float4 *>(a.bvh);
@@ -369,7 +281,6 @@ __global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_
     const int descend_min = (int)a.bvh_descend_min;
     int stack[RZ_STACK];
     unsigned long long c_paths = 0, c_segs = 0, c_nodes = 0, c_sph = 0, c_hit[3] = {0, 0, 0}, c_sky = 0, c_abs = 0, c_depth = 0;
-#if RZ_BVH_CAMERA_LISTS
     // per-warp scratch of the camera stage's tile lists: candidate spheres (stationary ones from the front, moving ones from the
     // back), their positions in the set, the cull's ring buffer of nodes; idl = 0, 1, 2, ... (the lists the packed search walks)
     __shared__ float4 s_cl_cr[CAMERA ? 4 : 1][CAMERA ? RZ_CL_CAP : 1], s_cl_vel[CAMERA ? 4 : 1][CAMERA ? RZ_CL_CAP : 1];
@@ -379,7 +290,6 @@ __global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_
         for (unsigned i = threadIdx.x; i < (unsigned)RZ_CL_CAP; i += blockDim.x) s_cl_idl[i] = (unsigned short)i;
         __syncthreads();
     }
-#endif
 
     while (true) {
         unsigned u = 0;
@@ -391,7 +301,7 @@ __global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_
         if (CAMERA) {
             u += a.unit_base;
             const uint32_t tile = u / a.n_chunks, chunk = u - tile * a.n_chunks;
-            if (a.tile_w) {   // 8 x 4 pixel blocks (rz_bvh_camera_tile_w: the host counts the units accordingly)
+            if (a.tile_w) {   // 8 x 4 pixel blocks (the host sets tile_w = 8 for the BVH family and counts the units accordingly)
                 const uint32_t tiles_x = (a.width + 7u) >> 3;
                 const uint32_t ty = tile / tiles_x, tx = tile - ty * tiles_x;
                 const uint32_t ti = tx * 8u + (lane & 7u), tr = ty * 4u + (lane >> 3);
@@ -409,7 +319,6 @@ __global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_
             e0 = u * ue; ne = min(ue, n_in - e0);
             n_batches = (ne + 31u) / 32u;
         }
-#if RZ_BVH_CAMERA_LISTS
         if (CAMERA) {
             // ---- Camera rays of a 32-pixel tile are coherent: instead of 32 x chunk separate walks, the warp culls the TREE once
             // against the tile's cone (rz_tile_cone / rz_tile_keep of the primary kernel; a child box enters as its bounding
@@ -538,7 +447,6 @@ __global__ void __launch_bounds__(128, (CAMERA && RZ_BVH_CAMERA_LISTS) ? RZ_BVH_
                 continue;   // next unit
             }
         }
-#endif
         for (uint32_t b = 0; b < n_batches; b++) {
             RzRay ray;
             float3 thr = f3(1.f, 1.f, 1.f);
@@ -680,10 +588,6 @@ cudaError_t launch_kernel(K kern, const RzPathArgs &a, int sm_count, cudaStream_
 }
 
 }  // namespace
-
-// Pixel layout of the camera stage's work units the host has to count with (RzPathArgs::tile_w): 8 x 4 blocks when the stage
-// builds tile lists — the cone around a compact block is a third as wide as around 32 pixels of a row —, else 0 (rows).
-extern "C" uint32_t rz_bvh_camera_tile_w(void) { return RZ_BVH_CAMERA_LISTS ? 8u : 0u; }
 
 extern "C" cudaError_t rz_bvh_warm(void) {
     cudaFuncAttributes fa;

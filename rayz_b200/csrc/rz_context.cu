@@ -41,7 +41,6 @@ extern "C" cudaError_t rz_bin_sort(const unsigned short *keys_in, const unsigned
 extern "C" cudaError_t rz_sort_warm(void);
 extern "C" cudaError_t rz_launch_primary(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_bvh_warm(void);
-extern "C" uint32_t rz_bvh_camera_tile_w(void);
 extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t stream);
@@ -50,8 +49,6 @@ extern "C" cudaError_t rz_bvh_finalize(RzBvhNode *nodes, uint32_t n_nodes, cudaS
 extern "C" cudaError_t rz_lbvh_build(uint32_t n, int leaf_max, const double4 *c64, const double4 *v64, const uint32_t *mat, void *scratch,
                                      size_t scratch_bytes, RzBvhNode *nodes, float4 *o_cr, float4 *o_vel, double4 *o_c64,
                                      double4 *o_v64, uint32_t *o_mat, int32_t *o_orig, cudaStream_t stream);
-extern "C" size_t rz_bvh_wide_scratch_bytes(uint32_t n_nodes);
-extern "C" cudaError_t rz_bvh_wide_collapse(const RzBvhNode *n2, uint32_t n_nodes, void *scratch, RzBvh4Node *out, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_ids(const RzIdsArgs *a, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
 extern "C" uint32_t rz_noise_grid(void);
@@ -140,9 +137,7 @@ struct Dev {
     cudaEvent_t ev_s2 = nullptr, ev_tab = nullptr;
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // start, path0, path1, resolve1, done
     SetBufs brute, bvhset;
-    DBuf<RzBvhNode> bvh;              // the builders' binary tree (host SAH or device LBVH): input of the collapse
-    DBuf<RzBvh4Node> bvh4;            // what K3 walks: every second level collapsed (rz_bvh_wide.cu)
-    DBuf<int> wide_scratch;
+    DBuf<RzBvhNode> bvh;              // what K3 walks: the builders' binary tree (host SAH or device LBVH), finalized at upload
     uint32_t bvh_nodes = 0;
     DBuf<int32_t> brute_to_bvh;       // staged K1 with a BVH tail: position in `brute` -> position in `bvhset` (empty: no such tail)
     DBuf<RzRefNode> refnodes;
@@ -652,12 +647,7 @@ extern "C" int rayz_cuda_upload_scene(RzContext *ctx, const RzScene *sc) {
             RZ_CUDA(rz_lbvh_build(n, ctx->tun.lbvh_leaf, D.c64_orig.p, D.v64_orig.p, D.mat_orig.p, D.lbvh_scratch.p, D.lbvh_scratch.n, D.bvh.p, V.cr.p, V.vel.p,
                                   V.c64.p, V.v64.p, V.mat.p, V.orig.p, D.stream));
         }
-#ifdef RZ_BVH_WIDE   // experiment: K3 walks the 4-wide collapse of the builders' binary tree (three small kernels, no host round trip)
-        if ((rc = D.bvh4.alloc(D.bvh_nodes)) || (rc = D.wide_scratch.alloc(rz_bvh_wide_scratch_bytes(D.bvh_nodes) / sizeof(int)))) return rc;
-        RZ_CUDA(rz_bvh_wide_collapse(D.bvh.p, D.bvh_nodes, D.wide_scratch.p, D.bvh4.p, D.stream));
-#else
         RZ_CUDA(rz_bvh_finalize(D.bvh.p, D.bvh_nodes, D.stream));   // leaves -> the references K3 follows; no unused slots
-#endif
         if (device_build) RZ_CUDA(cudaEventRecord(D.ev[1], D.stream));
         if ((rc = D.m_rec.upload(mrec, D.stream)) || (rc = D.m_kind.upload(mk, D.stream)) || (rc = D.m_tex.upload(mt, D.stream)) || (rc = D.m_method.upload(mm, D.stream)) ||
             (rc = D.m_fuzz.upload(mf, D.stream)) || (rc = D.m_ior.upload(mi, D.stream)) || (rc = D.t_kind.upload(tk, D.stream)) ||
@@ -728,9 +718,9 @@ static QueuePlan plan_queues(const RzTuning &tun, uint32_t n_units, uint32_t chu
     q.units_per_pass = (uint32_t)std::max<uint64_t>(1, q.cap / q.unit_paths);
     q.n_pass = (n_units + q.units_per_pass - 1) / q.units_per_pass;
     // Passes alternate between two streams so that the next pass's first kernel fills the tail of the persistent one — except for
-    // K3 with tile lists: its camera stage holds 41 KB of shared memory per CTA, and running beside the traversal kernel of the
-    // previous pass it takes the L1 that kernel's node loads live in (config 4: 247.6 ms overlapped against 212.6 ms in series).
-    const bool overlap = !(bvh_family && rz_bvh_camera_tile_w() != 0u);
+    // K3: the tile lists of its camera stage hold 41 KB of shared memory per CTA, and running beside the traversal kernel of the
+    // previous pass that stage takes the L1 the kernel's node loads live in (config 4: 247.6 ms overlapped against 212.6 ms in series).
+    const bool overlap = !bvh_family;
     q.n_sides = (q.n_pass > 1 && !serial && overlap) ? 2 : 1;
     return q;
 }
@@ -980,7 +970,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         // It plans the largest staged form (brute force with sorted stages and a BVH tail, both tilings' units); the first
         // render still sizes the sorted stages' pair lists (a function of the set) and, if it runs more passes, their events.
         if (!ctx->have_scene) { P.bvh_family = false; P.bvh_tail = true; P.enough_spheres = true; }
-        P.tile_w = P.bvh_family ? rz_bvh_camera_tile_w() : 0u;
+        P.tile_w = P.bvh_family ? 8u : 0u;
     }
     const uint32_t chunk = std::min(ctx->tun.chunk, p->spp), n_chunks = (p->spp + chunk - 1) / chunk;
     P.chunk = P.staged ? std::min(ctx->tun.chunk_primary, p->spp) : chunk;   // the camera-stage kernels build a culled sphere list per unit: their own, larger work-unit size
@@ -1138,11 +1128,7 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
     a.set = D.bvhset.view();
     a.mats.kind = D.m_kind.p; a.mats.fuzz = D.m_fuzz.p; a.mats.ior = D.m_ior.p; a.mats.tex = D.m_tex.p; a.mats.method = D.m_method.p; a.mats.rec = D.m_rec.p;
     a.texs.kind = D.t_kind.p; a.texs.color = D.t_color.p; a.texs.inv_scale = D.t_inv_scale.p; a.texs.even = D.t_even.p; a.texs.odd = D.t_odd.p;
-#ifdef RZ_BVH_WIDE
-    a.bvh = D.bvh4.p; a.bvh_nodes = D.bvh_nodes;
-#else
     a.bvh = D.bvh.p; a.bvh_nodes = D.bvh_nodes;
-#endif
     a.cam = cam_to_f32(P.cam);
     a.width = p->width; a.height = p->height; a.n_local_px = P.split.n_local[d];
     a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;

@@ -98,14 +98,6 @@ struct __align__(16) RzBvhNode {
 // its sibling, so that the node visit neither decodes nor checks anything.
 RZ_HD int rz_leaf_ref(int child, uint32_t cnt) { return ~((int)((cnt - 1u) << 28) | ~child); }
 
-// BVH4 node (RZ_BVH_WIDE experiment, measured and not adopted): the four child boxes of a node in one 128-byte record, built by
-// collapsing every second level of the binary tree (rz_bvh_wide.cu).  Unused slots: empty box, child = ~0, cnt = 0.
-struct __align__(16) RzBvh4Node {
-    float lox[4], hix[4], loy[4], hiy[4], loz[4], hiz[4];
-    int32_t child[4];
-    uint32_t cnt[4];
-};
-
 struct RzCamF32 {
     float3 look_from, px_du, px_dv, px_origin, defocus_u, defocus_v;
     int defocus;
@@ -123,7 +115,7 @@ struct RzPathArgs {
     RzSphereSet set;
     RzMaterials mats;
     RzTextures texs;
-    const void *bvh;             // K3 only: RzBvhNode[] (or RzBvh4Node[] in the RZ_BVH_WIDE experiment)
+    const RzBvhNode *bvh;        // K3 only
     uint32_t bvh_nodes;
     RzCamF32 cam;
     unsigned long long *accum;   // [n_local_px_pad][4] u64 fixed point (2^-32), rgb + sum of Y^2 (only with `moments`)

@@ -231,15 +231,9 @@ struct RzSegCounters {
 // Shade the two rays of a lane after the search and append the survivors (with their sort keys) to the next queue.
 template <bool STATS>
 __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRay (&L)[2], unsigned lane, unsigned lt_mask, RzSegCounters &C) {
-#ifdef RZ_SHADE_UNROLL   // experiment (scripts/exp_build.sh): two copies of the shading code, the two rays' dependency chains interleave
-#pragma unroll
-    for (int trip = 0; trip < 2; trip++) {
-        RzLaneRay &Q = L[trip];
-#else
 #pragma unroll 1
     for (int trip = 0; trip < 2; trip++) {
         RzLaneRay &Q = L[0];
-#endif
         Q.cont = false;
         if (Q.live) {
             if (STATS) C.segs++;
@@ -253,9 +247,7 @@ __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRa
             }
             Q.cont = res == RZ_CONT;
         }
-#ifndef RZ_SHADE_UNROLL
         if (trip == 0) rz_swap_lane_rays(L[0], L[1]);   // ONE exchange per loop: the slots stay swapped afterwards, and nothing below cares which is which
-#endif
     }
     // ballot-compacted append: one atomic per warp for both rays
     const unsigned m0 = __ballot_sync(0xffffffffu, L[0].cont), m1 = __ballot_sync(0xffffffffu, L[1].cont);

@@ -65,13 +65,8 @@ __device__ __forceinline__ void rz_test2_static(const float4 A, const float4 B, 
     const float2 ocy = __fadd2_rn(rz_f2(A.z, A.w), rz_f2(q.noy, q.noy));
     const float2 ocz = __fadd2_rn(rz_f2(B.x, B.y), rz_f2(q.noz, q.noz));
     nb = __ffma2_rn(ocz, rz_f2(q.ndz, q.ndz), __ffma2_rn(ocy, rz_f2(q.ndy, q.ndy), __fmul2_rn(ocx, rz_f2(q.ndx, q.ndx))));
-#ifdef RZ_NAIVE_DISC   // experiment (scripts/exp_build.sh): round 1's textbook discriminant, to price the cancellation-free form
-    const float2 c = __ffma2_rn(ocz, ocz, __ffma2_rn(ocy, ocy, __ffma2_rn(ocx, ocx, rz_f2(B.z, B.w))));
-    nd = rz_f2(fmaf(-nb.x, nb.x, c.x), fmaf(-nb.y, nb.y, c.y));
-#else
     const float2 lx = __ffma2_rn(nb, rz_f2(q.dx, q.dx), ocx), ly = __ffma2_rn(nb, rz_f2(q.dy, q.dy), ocy), lz = __ffma2_rn(nb, rz_f2(q.dz, q.dz), ocz);
     nd = __ffma2_rn(lz, lz, __ffma2_rn(ly, ly, __ffma2_rn(lx, lx, rz_f2(B.z, B.w))));
-#endif
 }
 
 // two moving spheres (+ VA = vx0 vx1 vy0 vy1, VB = vz0 vz1 . .).  oc = (c0 - o) + v * time: each instruction reads ONE register
@@ -83,35 +78,17 @@ __device__ __forceinline__ void rz_test2_moving(const float4 A, const float4 B, 
     const float2 ocy = __ffma2_rn(rz_f2(VA.z, VA.w), tm, __fadd2_rn(rz_f2(A.z, A.w), rz_f2(q.noy, q.noy)));
     const float2 ocz = __ffma2_rn(rz_f2(VB.x, VB.y), tm, __fadd2_rn(rz_f2(B.x, B.y), rz_f2(q.noz, q.noz)));
     nb = __ffma2_rn(ocz, rz_f2(q.ndz, q.ndz), __ffma2_rn(ocy, rz_f2(q.ndy, q.ndy), __fmul2_rn(ocx, rz_f2(q.ndx, q.ndx))));
-#ifdef RZ_NAIVE_DISC   // experiment (scripts/exp_build.sh): round 1's textbook discriminant, to price the cancellation-free form
-    const float2 c = __ffma2_rn(ocz, ocz, __ffma2_rn(ocy, ocy, __ffma2_rn(ocx, ocx, rz_f2(B.z, B.w))));
-    nd = rz_f2(fmaf(-nb.x, nb.x, c.x), fmaf(-nb.y, nb.y, c.y));
-#else
     const float2 lx = __ffma2_rn(nb, rz_f2(q.dx, q.dx), ocx), ly = __ffma2_rn(nb, rz_f2(q.dy, q.dy), ocy), lz = __ffma2_rn(nb, rz_f2(q.dz, q.dz), ocz);
     nd = __ffma2_rn(lz, lz, __ffma2_rn(ly, ly, __ffma2_rn(lx, lx, rz_f2(B.z, B.w))));
-#endif
 }
 
-// Where the packed search reads the sphere operands from: shared memory (production).  A constant-bank source that feeds
-// them through the uniform datapath was measured and rejected (scripts/rz_search_variants.cuh).
-struct RzSrcShared {
-    const float4 *p;
-    __device__ __forceinline__ float4 operator[](int i) const { return p[i]; }
-};
-// Two knobs kept for scripts/searchbench.cu, both measured and left at their defaults: unrolling the moving loop by 2
-// (1475 vs 1519 Mpaths/s in the production kernel) and a warp-uniform entry into the rare path, __any_sync(c), which
-// needs no BSSY/BSYNC pair per iteration (53.2 % vs 53.1 % of FP32 peak: no difference).
-#ifndef RZ_MOVING_UNROLL
-#define RZ_MOVING_UNROLL 1
-#endif
-#ifndef RZ_TRIGGER
-#define RZ_TRIGGER(c) (c)
-#endif
 // Brute force over the whole set (RZ_VARIANT_MEGA_SINGLE, the wavefront's intersect stage, the brute-force tail).
 // G2 = sphere pairs per loop iteration (2 => 8 tests of 2 rays share one min tree + branch).  Sphere operands are warp-uniform
 // LDS.128 broadcasts; only when some lane has nd < 0 does the warp enter the rare path (rz_consider: square root, root rule).
-template <int R, int G2, class SRC>
-__device__ __forceinline__ void rz_search_brute2(const SRC src, int n_static_pad, int n_pad,
+// Measured and not adopted: operands from the constant bank through the uniform datapath, the moving loop unrolled by 2
+// (1475 vs 1519 Mpaths/s) and a warp-uniform entry into the rare path, __any_sync (no difference).
+template <int R, int G2>
+__device__ __forceinline__ void rz_search_brute2(const float4 *__restrict__ src, int n_static_pad, int n_pad,
                                                  const RzRay (&ray)[R], float t_min, float (&bt)[R], int (&bk)[R]) {
     RzRayOps q[R];
 #pragma unroll
@@ -133,7 +110,7 @@ __device__ __forceinline__ void rz_search_brute2(const SRC src, int n_static_pad
                 m = fminf(m, fminf(nd[r][j].x, nd[r][j].y));
             }
         }
-        if (RZ_TRIGGER(m < 0.0f)) {
+        if (m < 0.0f) {
 #pragma unroll
             for (int r = 0; r < R; r++)
 #pragma unroll
@@ -143,8 +120,7 @@ __device__ __forceinline__ void rz_search_brute2(const SRC src, int n_static_pad
                 }
         }
     }
-    constexpr int kMovingUnroll = RZ_MOVING_UNROLL;
-#pragma unroll kMovingUnroll
+#pragma unroll 1
     for (; k < n_pad; k += 2 * G2, f += 4 * G2) {
         float4 A[G2], B[G2], VA[G2], VB[G2];
 #pragma unroll
@@ -159,7 +135,7 @@ __device__ __forceinline__ void rz_search_brute2(const SRC src, int n_static_pad
                 m = fminf(m, fminf(nd[r][j].x, nd[r][j].y));
             }
         }
-        if (RZ_TRIGGER(m < 0.0f)) {
+        if (m < 0.0f) {
 #pragma unroll
             for (int r = 0; r < R; r++)
 #pragma unroll
@@ -169,12 +145,6 @@ __device__ __forceinline__ void rz_search_brute2(const SRC src, int n_static_pad
                 }
         }
     }
-}
-
-template <int R, int G2>
-__device__ __forceinline__ void rz_search_brute2(const float4 *__restrict__ s_pk, int n_static_pad, int n_pad,
-                                                 const RzRay (&ray)[R], float t_min, float (&bt)[R], int (&bk)[R]) {
-    rz_search_brute2<R, G2, RzSrcShared>(RzSrcShared{s_pk}, n_static_pad, n_pad, ray, t_min, bt, bk);
 }
 
 // ------------------------------------------------------------------------------ K1 search over a culled list
@@ -371,17 +341,10 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
     const RzHit h = rz_refine_hit(a.set, ray, k, (bk & RZ_FAR_BIT) != 0);
     const uint32_t mat = a.set.mat[k];
     const float4 *mr = a.mats.rec + 4u * mat;
-#ifdef RZ_NO_CHECKER2   // experiment (scripts/exp_build.sh): checkers always through the texture walk
-    const float4 m0 = __ldg(mr), m1 = __ldg(mr + 1), m2 = make_float4(0.f, 0.f, 0.f, 0.f), m3 = m2;
-#else
     const float4 m0 = __ldg(mr), m1 = __ldg(mr + 1), m2 = __ldg(mr + 2), m3 = __ldg(mr + 3);
-#endif
     const uint32_t mbits = __float_as_uint(m0.x);
     RzMatRec M;
     M.kind = mbits & 3u; M.method = (mbits >> 2) & 3u; M.solid = ((mbits >> 4) & 1u) != 0u; M.checker2 = ((mbits >> 5) & 1u) != 0u;
-#ifdef RZ_NO_CHECKER2
-    M.checker2 = false;
-#endif
     M.fuzz = m0.y; M.ior = m0.z; M.tex = __float_as_uint(m0.w);
     M.color = f3(m1.x, m1.y, m1.z); M.odd = f3(m2.x, m2.y, m2.z);
     M.inv_scale = __hiloint2double(__float_as_int(m3.y), __float_as_int(m3.x));

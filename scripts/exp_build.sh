@@ -1,7 +1,7 @@
 #!/bin/bash
-# Builds experimental variants of librayz_cuda.so that differ in compile-time knobs of ONE source file, rz_path.cu unless
-# SRC names another (SRC=rz_bvh_trace.cu), as scripts/_build/exp/<name>.so; scripts/exp_probe.py / exp_bvh.py --so load one of
-# them instead of the product library.
+# Builds occupancy/capacity variants of librayz_cuda.so that differ in the numeric compile-time constants of ONE source file
+# (RZ_PRIMARY_MINB, RZ_SECOND_MINB of rz_path.cu; RZ_BVH_MINB, RZ_BVH_CAMERA_MINB, RZ_CL_CAP, RZ_CL_WL with SRC=rz_bvh_trace.cu),
+# as scripts/_build/exp/<name>.so; scripts/exp_probe.py / exp_bvh.py --so load one of them instead of the product library.
 #   [SRC=rz_bvh_trace.cu] scripts/exp_build.sh name1 "-DFLAG=1 ..." [name2 "flags" ...]
 set -e
 cd "$(dirname "$0")/.."
