@@ -3,7 +3,7 @@
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
-//               [--guides PREFIX]
+//               [--guides PREFIX] [--denoise FILE]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -14,6 +14,8 @@
 // and only the pixels still above it get more samples (RZ_RENDER_ADAPTIVE); stderr then also reports the paths traced and the
 // mean and max samples per pixel.  --guides PREFIX also writes the guide buffers of the render's camera samples for a denoiser
 // (rayz_cuda_render_guides) as PFM files: PREFIX_albedo.pfm and PREFIX_normal.pfm (3 channels), PREFIX_depth.pfm (1 channel).
+// --denoise FILE renders with RZ_RENDER_MOMENTS (no pixel changes), computes guides over the render's own samples and writes the
+// frame denoised by rayz_cuda_denoise (default parameters) to FILE as P3; the normal output and the report line are unchanged.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -38,7 +40,7 @@ int main(int argc, char **argv) {
     size_t spp = 10, depth = 50;
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
-    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr;
+    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr;
     bool ppm_bench = false, penultimate = false, adaptive = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
@@ -58,6 +60,7 @@ int main(int argc, char **argv) {
         else if (a == "--max-spp") max_spp = (uint32_t)std::strtoul(val(), nullptr, 10);
         else if (a == "--adaptive") adaptive = true;
         else if (a == "--guides") guides = val();
+        else if (a == "--denoise") denoise = val();
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -77,6 +80,7 @@ int main(int argc, char **argv) {
         tracer.noise_target = noise_target;
         tracer.max_spp = max_spp;
         tracer.adaptive = adaptive;
+        tracer.moments = denoise != nullptr;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);
@@ -97,8 +101,8 @@ int main(int argc, char **argv) {
             std::fprintf(stderr, "  [rayz_cuda] adaptive: %.0f paths, mean %.2f spp, max %llu spp, max error %.5f (%.2f 8-bit steps)\n", rays_traced,
                          rays_traced / std::max<double>(1.0, tracer.noise.n_pixels), (unsigned long long)tracer.noise.samples, tracer.noise.max_err,
                          tracer.noise.max_err * 255.0);
+        if (guides || denoise) tracer.renderGuides();
         if (guides) {
-            tracer.renderGuides();
             const struct { const char *name; const std::vector<float> &src; size_t first, channels; } files[3] = {
                 {"_albedo.pfm", tracer.albedo, 0, 3}, {"_normal.pfm", tracer.normal, 0, 3}, {"_depth.pfm", tracer.normal, 3, 1}};
             for (const auto &o : files) {
@@ -108,6 +112,13 @@ int main(int argc, char **argv) {
                 writePFM(f, o.src.data(), tracer.img.w, tracer.img.h, 4, o.first, o.channels);
                 std::fclose(f);
             }
+        }
+        if (denoise) {
+            tracer.denoise();
+            FILE *f = std::fopen(denoise, "wb");
+            if (!f) { std::perror(denoise); return 1; }
+            tracer.denoised.writePPM(f);
+            std::fclose(f);
         }
         if (dump_scene && !dumpScene(tracer, dump_scene)) { std::perror(dump_scene); return 1; }
         if (dump_linear) {

@@ -262,6 +262,8 @@ struct Tracer {
     RzNoise noise{};              // summary of the last render with a noise target
     bool adaptive = false;        // with noise_target: it bounds every pixel's error, and only pixels above it get more samples (RZ_RENDER_ADAPTIVE)
     std::vector<float> albedo, normal;   // guide buffers of the last renderGuides(): rgb albedo + coverage, normal + hit distance (4 floats a pixel)
+    bool moments = false;         // render with RZ_RENDER_MOMENTS (no pixel changes), so that denoise() can follow
+    Image denoised;               // rgb8 of the last denoise()
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
         : rng(seed) {
@@ -295,6 +297,7 @@ struct Tracer {
         p.width = (uint32_t)img.w; p.height = (uint32_t)img.h; p.spp = (uint32_t)samples_per_px; p.max_depth = (uint32_t)max_bounces;
         p.seed = render_seed; p.variant = variant;
         if (adaptive && noise_target > 0) p.flags |= RZ_RENDER_ADAPTIVE;
+        if (moments) p.flags |= RZ_RENDER_MOMENTS;
         return p;
     }
 
@@ -352,6 +355,14 @@ struct Tracer {
         albedo.assign(img.w * img.h * 4, 0.f);
         normal.assign(img.w * img.h * 4, 0.f);
         check(rayz_cuda_render_guides(ctx, &cam, &p, albedo.data(), normal.data()));
+    }
+
+    // The frame of the last render() (with moments, or a noise target) denoised with the guides of renderGuides(), after it
+    // (rayz_cuda_denoise, default parameters).
+    void denoise() {
+        denoised = Image::initEmpty(img.h, img.w);
+        denoised.rgb8.resize(img.w * img.h * 3);
+        check(rayz_cuda_denoise(ctx, nullptr, nullptr, denoised.rgb8.data()));
     }
 };
 

@@ -310,6 +310,48 @@ int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp);
  */
 int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float *out_albedo, float *out_normal);
 
+/*
+ * Denoiser parameters (rayz_cuda_denoise).  A zero sigma takes its default.
+ */
+typedef struct RzDenoiseParams {
+    uint32_t struct_size;  /* sizeof(RzDenoiseParams) of the caller (checked, like RzTuning)                       */
+    uint32_t iterations;   /* à-trous levels, step 2^k for k = 0..iterations-1; 0..10; 0 = the input unchanged     */
+    float sigma_luminance; /* 0 => 4    */
+    float sigma_normal;    /* 0 => 128  */
+    float sigma_depth;     /* 0 => 1    */
+    uint32_t reserved0;
+} RzDenoiseParams;
+
+/*
+ * Denoised accumulated frame of the last render(s): an edge-avoiding à-trous filter (SVGF's spatial filter, Schied et al. 2017;
+ * Dammertz et al. 2010) steered by the per-pixel noise estimate and the guide buffers of the last successful
+ * rayz_cuda_render_guides call.  dp == NULL: 5 iterations and the default sigmas.  Host outputs, each nullable, laid out like
+ * rayz_cuda_render's: out_linear_rgba (a = 1) and out_rgb8 = trunc(255 clamp(sqrt(x), 0, 1)) of that f32 linear value in f64.
+ * Per pixel p, with Y(x) = 0.2126 x.r + 0.7152 x.g + 0.0722 x.b, c_p the resolved linear rgb (each pixel's own count after an
+ * adaptive render), e_p rayz_cuda_noise's error and a_p, n_p, z_p the guide albedo, normal and depth:
+ *   v_p = 4 e_p^2 max(Y(c_p), 1e-4)                         (variance of the pixel mean's luminance; e = +inf gives +inf)
+ *   i_p = c_p / max(a_p, 1e-3) per channel,  v_p /= max(Y(a_p), 1e-3)^2                             (demodulation)
+ *   g_p = ((z[x+1] - z[x-1]) / 2, (z[y+1] - z[y-1]) / 2), indices clamped at the frame edges (once per call)
+ *   level k, step s = 2^k, taps q = p + s (dx, dy), dx, dy in -2..2 (taps outside the frame skipped), h = (1, 4, 6, 4, 1) / 16:
+ *     gv_p = the 3 x 3 (1, 2, 1) binomial blur of the current v around p (taps outside the frame skipped, renormalised)
+ *     w_l  = exp(-|Y(i_p) - Y(i_q)| / (sigma_luminance sqrt(gv_p) + 1e-4))                     (1 when gv_p = +inf)
+ *     w_n  = clamp(n_p.n_q / (|n_p| |n_q|), 0, 1)^sigma_normal if both normals are nonzero, 1 if both are zero (sky), else 0
+ *     w_z  = exp(-|z_p - z_q| / (sigma_depth |g_p . (q - p)| + 1e-2))
+ *     w    = h[dx] h[dy] w_l w_n w_z,   i'_p = sum w i_q / sum w,   v'_p = sum w^2 v_q / (sum w)^2 (a tap whose f32 w^2 is 0
+ *            adds nothing to the variance)
+ *   out_p = i_p max(a_p, 1e-3)                                                                        (remodulation)
+ * iterations = 0 returns the resolved frame exactly (rayz_cuda_render's linear and rgb8 of the accumulated frame).  The filter
+ * runs in f32 on the gather root (device_ids[0]) over the whole frame, so every device count gives the same bytes.  The guides'
+ * sample range need not match the render's (cheap 16-spp guides under a 500-spp render are the intended use).
+ * Refused, nothing touched, with messages prefixed "denoise:": RZ_ERR_INVALID_ARG for a bad struct_size, iterations > 10 or a
+ * negative or non-finite sigma, no accumulated frame, one rendered without RZ_RENDER_MOMENTS, no guide buffers (none, the last
+ * guides call failed, or a scene upload or a reserve of another frame came in between) or guides whose frame, camera or seed
+ * differ from the accumulated frame's; RZ_ERR_UNSUPPORTED for a shard (shard_count > 1: its rows are not image neighbours).
+ * Leaves the accumulated frame, its sample counts, RzStats, RzTiming and rayz_cuda_render_device's buffers untouched (a render
+ * enqueued by rayz_cuda_render_device(sync = 0) is waited for first, as rayz_cuda_noise does).
+ */
+int rayz_cuda_denoise(RzContext *ctx, const RzDenoiseParams *dp, float *out_linear_rgba, uint8_t *out_rgb8);
+
 /* Number of image rows a shard owns under the banding rule above. */
 uint32_t rayz_cuda_shard_rows(uint32_t height, uint32_t shard_index, uint32_t shard_count,
                               uint32_t band_rows);

@@ -85,6 +85,11 @@ class RzTuning(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class RzDenoiseParams(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("iterations", C.c_uint32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float),
+                ("sigma_depth", C.c_float), ("reserved0", C.c_uint32)]
+
+
 # every symbol include/rayz_cuda.h declares: (restype, argtypes)
 SYMBOLS = {
     "rayz_cuda_abi_version": (C.c_uint32, []),
@@ -102,6 +107,7 @@ SYMBOLS = {
                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(RzNoise)]),
     "rayz_cuda_pixel_samples": (C.c_int, [C.c_void_p, C.c_void_p]),
     "rayz_cuda_render_guides": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_void_p, C.c_void_p]),
+    "rayz_cuda_denoise": (C.c_int, [C.c_void_p, C.POINTER(RzDenoiseParams), C.c_void_p, C.c_void_p]),
     "rayz_cuda_shard_rows": (C.c_uint32, [C.c_uint32] * 4),
     "rayz_cuda_context_rows": (C.c_uint32, [C.c_void_p] + [C.c_uint32] * 4),
     "rayz_cuda_primary_ids": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]),

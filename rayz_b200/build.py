@@ -25,6 +25,7 @@ UNITS = {
     "rz_path.cu": ["--use_fast_math"],
     "rz_wavefront.cu": ["--use_fast_math"],
     "rz_misc.cu": [],
+    "rz_denoise.cu": [],
     "rz_adaptive.cu": [],
     "rz_ids.cu": ["--fmad=false"],
     "rz_bvh_build.cu": [],
@@ -32,7 +33,7 @@ UNITS = {
     "rz_bvh_trace.cu": ["--use_fast_math"],
     "rz_context.cu": [],
 }
-HEADERS = ["rz_device.cuh", "rz_search.cuh", os.path.join("..", "..", "include", "rayz_cuda.h")]
+HEADERS = ["rz_device.cuh", "rz_search.cuh", "rz_denoise.cuh", os.path.join("..", "..", "include", "rayz_cuda.h")]
 
 
 def _nvcc() -> str:

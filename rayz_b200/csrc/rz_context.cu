@@ -16,6 +16,7 @@
 
 #include "../../include/rayz_cuda.h"
 #include "rz_device.cuh"
+#include "rz_denoise.cuh"   // RzDenoiseArgs
 #include "rz_host_bvh.hpp"   // Box, sphere_box, RefBuilder (K0's reference-shaped BVH), SahBuilder (K3's tree for small scenes); RzRefNode
 
 // from rz_path.cu / rz_ids.cu / rz_misc.cu / rz_wavefront.cu
@@ -44,6 +45,7 @@ extern "C" cudaError_t rz_bvh_warm(void);
 extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_denoise(const RzDenoiseArgs *a, cudaStream_t stream);
 extern "C" size_t rz_lbvh_scratch_bytes(uint32_t n);
 extern "C" cudaError_t rz_bvh_finalize(RzBvhNode *nodes, uint32_t n_nodes, cudaStream_t stream);
 extern "C" cudaError_t rz_lbvh_build(uint32_t n, int leaf_max, const double4 *c64, const double4 *v64, const uint32_t *mat, void *scratch,
@@ -167,6 +169,13 @@ struct Dev {
     DBuf<double> noise_part;          // rayz_cuda_noise: the reduction's per-CTA partials of this device
     DBuf<uint32_t> out_spp;           // rayz_cuda_pixel_samples: per-pixel sample counts of the context's rows (gather root only)
     DBuf<float4> out_guides;          // rayz_cuda_render_guides: albedo, then normal + depth, of the context's rows (gather root only)
+    // rayz_cuda_denoise (gather root only): the resolved frame, then the denoised one; the per-pixel error; the ping-pong pair of
+    // (demodulated rgb, variance); the depth gradient; the denoised rgb8.  Never Dev::out_linear / out_rgb8, which a
+    // rayz_cuda_render_device caller may still hold.
+    DBuf<float4> dn_linear, dn_work;
+    DBuf<float> dn_err;
+    DBuf<float2> dn_grad;
+    DBuf<uint8_t> dn_rgb8;
     DBuf<uint32_t> n_px;              // RZ_RENDER_ADAPTIVE: every local pixel's sample count
     DBuf<uint32_t> px_list;           // RZ_RENDER_ADAPTIVE: the local pixels the next round traces, in increasing order
     DBuf<uint32_t> list_scratch;      // RZ_RENDER_ADAPTIVE: the list kernels' mask words, block offsets and list length (rz_adaptive.cu)
@@ -225,10 +234,22 @@ struct AccumRecord {
     bool adaptive = false;     // RZ_RENDER_ADAPTIVE: the pixels' counts differ (Dev::n_px), no RZ_RENDER_ACCUMULATE batch continues them
 };
 
+// What the gather root's guide buffers (Dev::out_guides) hold after a successful rayz_cuda_render_guides: rayz_cuda_denoise
+// takes them for an accumulated frame of the same frame, camera and seed.  A failed guides call, a scene upload or a reserve of
+// another frame ends the record, as it ends the accumulation's.
+struct GuideRecord {
+    bool valid = false;
+    Frame frame;
+    RzCamera cam{};
+    uint64_t seed = 0;
+    uint32_t first_offset = 0, samples = 0;
+};
+
 struct RzContext {
     explicit RzContext(int n_devices) : devs(n_devices) {}
     std::vector<Dev> devs;
     AccumRecord acc;
+    GuideRecord guides;
     bool have_scene = false;
     uint32_t n_spheres = 0;
     RzStats stats{};
@@ -475,6 +496,7 @@ static int for_each_device(RzContext *ctx, F &&fn) {
 extern "C" int rayz_cuda_upload_scene(RzContext *ctx, const RzScene *sc) {
     if (!ctx || !sc) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: NULL argument");
     ctx->acc.valid = false;   // sums of the old scene: a next batch may not add to them
+    ctx->guides.valid = false;
     const uint32_t n = sc->n_spheres, nm = sc->n_materials, nt = sc->n_textures;
     if (n == 0) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: empty scene (BVH.build asserts nobjs > 0, hit.zig:132)");
     if (n >= (1u << 28)) return rz_fail(RZ_ERR_INVALID_ARG, "rayz_cuda_upload_scene: too many spheres (K3 leaf references hold 28 bits)");
@@ -1255,6 +1277,7 @@ extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     int rc = plan_render(ctx, nullptr, p, ctx->acc, P, "reserve");
     if (rc) return rc;
     if (P.frame != ctx->acc.frame) ctx->acc.valid = false;   // another frame shape: a next batch may not add to the sums
+    if (P.frame != ctx->guides.frame) ctx->guides.valid = false;
     DeviceGuard guard;
     if ((rc = alloc_render(ctx, P))) return rc;
     return sync_devices(ctx);
@@ -1437,7 +1460,9 @@ extern "C" int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp) {
 // then the root's buffers are copied out.  The accumulators, their record, the per-pixel counts, stats and timing stay as
 // they are.
 extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float *out_albedo, float *out_normal) {
-    if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "guides: NULL argument");
+    if (!ctx) return rz_fail(RZ_ERR_INVALID_ARG, "guides: NULL argument");
+    ctx->guides.valid = false;   // until this call succeeds
+    if (!cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "guides: NULL argument");
     if (p->flags & (RZ_RENDER_ACCUMULATE | RZ_RENDER_ADAPTIVE))
         return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_ACCUMULATE and RZ_RENDER_ADAPTIVE do not apply to guide buffers");
     RenderPlan P;
@@ -1471,6 +1496,77 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
     RZ_CUDA(cudaSetDevice(D0.id));
     if (out_albedo) RZ_CUDA(cudaMemcpyAsync(out_albedo, D0.out_guides.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
     if (out_normal) RZ_CUDA(cudaMemcpyAsync(out_normal, D0.out_guides.p + npx, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    GuideRecord &G = ctx->guides;
+    G.frame = P.frame; G.cam = *cam; G.seed = p->seed; G.first_offset = p->sample_offset; G.samples = p->spp;
+    G.valid = true;
+    return RZ_OK;
+}
+
+// Denoiser (include/rayz_cuda.h): every device resolves its rows of the accumulated frame (linear and error, or for 0
+// iterations linear and rgb8) into the gather root's denoiser buffers, as rayz_cuda_noise does for the error; behind every
+// device's stream the root runs rz_denoise.cu alone over the whole frame, so the device count changes no byte.  The
+// accumulators, their record, the per-pixel counts, stats, timing and the render's output buffers stay as they are.
+extern "C" int rayz_cuda_denoise(RzContext *ctx, const RzDenoiseParams *dp, float *out_linear_rgba, uint8_t *out_rgb8) {
+    if (!ctx) return rz_fail(RZ_ERR_INVALID_ARG, "denoise: ctx is NULL");
+    RzDenoiseParams q;
+    memset(&q, 0, sizeof q);
+    q.struct_size = sizeof q;
+    q.iterations = 5;
+    if (dp) {
+        if (dp->struct_size != sizeof(RzDenoiseParams))
+            return rz_fail(RZ_ERR_INVALID_ARG, "denoise: struct_size %u != sizeof(RzDenoiseParams) %zu", dp->struct_size, sizeof(RzDenoiseParams));
+        if (dp->iterations > 10) return rz_fail(RZ_ERR_INVALID_ARG, "denoise: iterations %u > 10", dp->iterations);
+        for (const float s : {dp->sigma_luminance, dp->sigma_normal, dp->sigma_depth})
+            if (!(s >= 0.f) || !std::isfinite(s)) return rz_fail(RZ_ERR_INVALID_ARG, "denoise: sigmas must be finite and >= 0 (got %g)", (double)s);
+        q = *dp;
+    }
+    if (q.sigma_luminance == 0.f) q.sigma_luminance = 4.f;
+    if (q.sigma_normal == 0.f) q.sigma_normal = 128.f;
+    if (q.sigma_depth == 0.f) q.sigma_depth = 1.f;
+    DeviceGuard guard;
+    const AccumRecord *A = nullptr;
+    if (const int rc = accumulated_frame(ctx, "denoise", A)) return rc;
+    if (!A->moments) return rz_fail(RZ_ERR_INVALID_ARG, "denoise: the accumulated render(s) ran without RZ_RENDER_MOMENTS: no noise estimate to steer the filter");
+    if (A->frame.S > 1)
+        return rz_fail(RZ_ERR_UNSUPPORTED, "denoise: the accumulated frame is shard %u of %u: its rows are not image neighbours", A->frame.s, A->frame.S);
+    const GuideRecord &G = ctx->guides;
+    if (!G.valid)
+        return rz_fail(RZ_ERR_INVALID_ARG, "denoise: no guide buffers (none, the last rayz_cuda_render_guides failed, or a scene upload or reserve came in between)");
+    if (G.frame != A->frame || memcmp(&G.cam, &A->cam, sizeof(RzCamera)) != 0 || G.seed != A->seed)
+        return rz_fail(RZ_ERR_INVALID_ARG, "denoise: the guide buffers' frame, camera or seed differ from the accumulated frame's");
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    Dev &D0 = ctx->devs[0];
+    const FrameSplit sp(ctx, A->frame);
+    const size_t npx = sp.npx;
+    const bool filter = q.iterations > 0;
+    int rc;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if ((rc = D0.dn_linear.alloc(npx)) || (rc = D0.dn_rgb8.alloc(npx * 3))) return rc;
+    if (filter && ((rc = D0.dn_err.alloc(npx)) || (rc = D0.dn_work.alloc(2 * npx)) || (rc = D0.dn_grad.alloc(npx)))) return rc;
+    for (uint32_t d = 0; d < ND; d++) {
+        Dev &D = ctx->devs[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
+        r.out_linear = D0.dn_linear.p;
+        if (filter) r.out_err = D0.dn_err.p;
+        else r.out_rgb8 = D0.dn_rgb8.p;
+        RZ_CUDA(rz_launch_resolve(&r, D.stream));
+    }
+    if ((rc = sync_devices(ctx))) return rc;   // every device's rows are in the gather root's buffers
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if (filter) {
+        RzDenoiseArgs a;
+        memset(&a, 0, sizeof a);
+        a.linear = D0.dn_linear.p; a.rgb8 = D0.dn_rgb8.p; a.err = D0.dn_err.p;
+        a.albedo = D0.out_guides.p; a.normal = D0.out_guides.p + npx;
+        a.work = D0.dn_work.p; a.grad = D0.dn_grad.p;
+        a.width = A->frame.width; a.height = A->frame.height; a.iterations = q.iterations;
+        a.sigma_l = q.sigma_luminance; a.sigma_n = q.sigma_normal; a.sigma_z = q.sigma_depth;
+        RZ_CUDA(rz_launch_denoise(&a, D0.stream));
+    }
+    if (out_linear_rgba) RZ_CUDA(cudaMemcpyAsync(out_linear_rgba, D0.dn_linear.p, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
+    if (out_rgb8) RZ_CUDA(cudaMemcpyAsync(out_rgb8, D0.dn_rgb8.p, npx * 3, cudaMemcpyDeviceToHost, D0.stream));
     RZ_CUDA(cudaStreamSynchronize(D0.stream));
     return RZ_OK;
 }

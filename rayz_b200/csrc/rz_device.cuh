@@ -215,6 +215,16 @@ RZ_HD double rz_pixel_err(unsigned long long q0, unsigned long long q1, unsigned
     return sqrt(s2 * inv) / (2.0 * sqrt(fmax(y, RZ_NOISE_Y_FLOOR)));
 }
 
+// writePPM's per-pixel transform (image.zig:35-38) in f64, as the resolve and the denoiser's finish kernel apply it:
+// V3.sqrt (x > 0 ? sqrt(x) : 0, vec.zig:87-93) -> clamp(0, 1) -> u8 = trunc(x * 255), into the three bytes of pixel i of out.
+RZ_HD void rz_quantise_rgb8(double r, double g, double b, uint8_t *out, size_t i) {
+    const double sr = r > 0 ? sqrt(r) : 0, sg = g > 0 ? sqrt(g) : 0, sb = b > 0 ? sqrt(b) : 0;
+    const double cr = fmin(fmax(sr, 0.0), 1.0), cg = fmin(fmax(sg, 0.0), 1.0), cb = fmin(fmax(sb, 0.0), 1.0);
+    out[i * 3 + 0] = (uint8_t)(cr * 255.0);
+    out[i * 3 + 1] = (uint8_t)(cg * 255.0);
+    out[i * 3 + 2] = (uint8_t)(cb * 255.0);
+}
+
 // ---------------------------------------------------------------------------------------------
 // Philox4x32 (Salmon et al., SC'11), seven rounds.  key = 64-bit seed; counter = (global pixel, sample,
 // bounce, lane) so the stream is a pure function of WHAT is sampled, never of where it runs:

@@ -15,7 +15,7 @@
 // (out_spp) when asked.  An adaptive frame divides each pixel by its own count (n_px), in the same f64 arithmetic: a pixel
 // with c samples resolves exactly as the same pixel of a uniform c-spp render.
 // ---------------------------------------------------------------------------------------------
-#include "rz_device.cuh"   // rz_pixel_err
+#include "rz_device.cuh"   // rz_pixel_err, rz_quantise_rgb8
 
 struct RzResolveArgs {
     const unsigned long long *accum;  // [n_local_px][4]
@@ -48,13 +48,7 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
     const double s = 2.3283064365386962890625e-10;  // 2^-32
     const double r = (double)q0.x * s * inv, g = (double)q0.y * s * inv, b = (double)q1 * s * inv;
     if (a.out_linear) a.out_linear[dst] = make_float4((float)r, (float)g, (float)b, 1.0f);
-    if (a.out_rgb8) {
-        const double sr = r > 0 ? sqrt(r) : 0, sg = g > 0 ? sqrt(g) : 0, sb = b > 0 ? sqrt(b) : 0;
-        const double cr = fmin(fmax(sr, 0.0), 1.0), cg = fmin(fmax(sg, 0.0), 1.0), cb = fmin(fmax(sb, 0.0), 1.0);
-        a.out_rgb8[dst * 3 + 0] = (uint8_t)(cr * 255.0);
-        a.out_rgb8[dst * 3 + 1] = (uint8_t)(cg * 255.0);
-        a.out_rgb8[dst * 3 + 2] = (uint8_t)(cb * 255.0);
-    }
+    if (a.out_rgb8) rz_quantise_rgb8(r, g, b, a.out_rgb8, dst);
 }
 
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream) {

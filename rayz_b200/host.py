@@ -372,6 +372,23 @@ class Backend:
         abi.check(self.lib.rayz_cuda_render_guides(self._h, C.byref(cam), C.byref(p), albedo.ctypes.data, normal.ctypes.data))
         return albedo, normal
 
+    def denoise(self, iterations: int = 5, sigma_luminance: float = 4.0, sigma_normal: float = 128.0, sigma_depth: float = 1.0):
+        """rayz_cuda_denoise: the accumulated frame (needs moments=True) filtered by the edge-avoiding à-trous filter, steered by
+        its noise estimate and the guides of the last guides() call of the same frame, camera and seed ->
+        (linear [rows,w,4] f32, rgb8 [rows,w,3] u8).  iterations=0 returns the resolved frame.  Leaves the accumulated frame,
+        stats and timing as they were."""
+        dp = abi.RzDenoiseParams()
+        dp.struct_size = C.sizeof(abi.RzDenoiseParams)
+        dp.iterations = iterations
+        dp.sigma_luminance, dp.sigma_normal, dp.sigma_depth = sigma_luminance, sigma_normal, sigma_depth
+        if self._acc_shape is None:   # nothing rendered: the library says why
+            abi.check(self.lib.rayz_cuda_denoise(self._h, C.byref(dp), None, None))
+        rows, w = int(self.lib.rayz_cuda_context_rows(self._h, self._acc_shape[0], *self._acc_shape[2:])), self._acc_shape[1]
+        lin = np.empty((rows, w, 4), dtype=np.float32)
+        rgb8 = np.empty((rows, w, 3), dtype=np.uint8)
+        abi.check(self.lib.rayz_cuda_denoise(self._h, C.byref(dp), lin.ctypes.data, rgb8.ctypes.data))
+        return lin, rgb8
+
     def primary_ids(self, cam: abi.RzCamera, width: int, height: int, use_bvh=True) -> np.ndarray:
         out = np.empty((height, width), dtype=np.int32)
         abi.check(self.lib.rayz_cuda_primary_ids(self._h, C.byref(cam), width, height, 1 if use_bvh else 0, out.ctypes.data))
@@ -436,7 +453,9 @@ class Tracer:
         self.pixel_samples = None  # [h, w] per-pixel sample counts of the last render(noise_target=..., adaptive=True)
         self.albedo = None         # [h, w, 4] guide buffers of the last render_guides(): rgb albedo + coverage
         self.normal = None         # [h, w, 4] ... unit normal + hit distance
+        self.denoised = None       # (linear [h, w, 4], rgb8 [h, w, 3]) of the last denoise()
         self._backend = None
+        self._uploaded = None      # the pool arrays of the backend's last scene upload
 
     @property
     def backend(self) -> Backend:
@@ -444,14 +463,19 @@ class Tracer:
             self._backend = Backend(self.devices)
         return self._backend
 
-    def render(self, noise_target: float | None = None, max_spp: int = 4096, adaptive: bool = False) -> int:
+    def render(self, noise_target: float | None = None, max_spp: int = 4096, adaptive: bool = False, moments: bool = False) -> int:
         """noise_target (displayed-value rms error, 1/255 = one 8-bit step): start at samples_per_px and double the samples
         until the frame's rms error reaches it or max_spp samples are in (rayz_cuda_render_to_noise); `self.noise` then holds
         the summary.  adaptive: the target bounds every pixel's error, and only the pixels still above it get more samples;
-        `self.pixel_samples` then holds the counts.  Without a target, one render of samples_per_px, as the reference."""
+        `self.pixel_samples` then holds the counts.  Without a target, one render of samples_per_px, as the reference; moments:
+        also sum what the per-pixel noise estimate needs (RZ_RENDER_MOMENTS, no pixel changes), so that denoise() can follow."""
         b = self.backend
-        b.upload_scene(self.pool.arrays())  # initHittables + bvh.build (renderer.zig:76-78)
-        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant)
+        arrays = self.pool.arrays()
+        self._uploaded = None
+        b.upload_scene(arrays)  # initHittables + bvh.build (renderer.zig:76-78)
+        self._uploaded = arrays
+        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
+                           moments=moments)
         if noise_target is None:
             lin, rgb8, rays = b.render(self.camera.rz, p)
         else:
@@ -465,12 +489,26 @@ class Tracer:
     def render_guides(self):
         """Guide buffers for a denoiser over the camera samples render() traces (samples_per_px, seed): first-hit albedo with
         coverage, and normal with hit distance (rayz_cuda_render_guides).  Returns (albedo, normal), also kept as
-        self.albedo and self.normal."""
+        self.albedo and self.normal.  The scene is uploaded only when the pool differs from the one this tracer last uploaded,
+        so that the frame of a previous render() stays accumulated for denoise() (it used to be uploaded on every call, which
+        ended that frame).  An upload made directly through self.backend is not seen: call render() after one."""
         b = self.backend
-        b.upload_scene(self.pool.arrays())
+        arrays = self.pool.arrays()
+        # the scene render() uploaded stays: uploading it again would end the accumulated frame that denoise() filters
+        if self._uploaded is None or arrays.keys() != self._uploaded.keys() or \
+                not all(np.array_equal(arrays[k], self._uploaded[k]) for k in arrays):
+            self._uploaded = None
+            b.upload_scene(arrays)
+            self._uploaded = arrays
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant)
         self.albedo, self.normal = b.guides(self.camera.rz, p)
         return self.albedo, self.normal
+
+    def denoise(self, iterations: int = 5, sigma_luminance: float = 4.0, sigma_normal: float = 128.0, sigma_depth: float = 1.0):
+        """The frame of the last render() (with moments=True, or a noise target) denoised with the guides of render_guides(),
+        called after it (rayz_cuda_denoise).  Returns (linear [h,w,4] f32, rgb8 [h,w,3] u8), also kept as self.denoised."""
+        self.denoised = self.backend.denoise(iterations, sigma_luminance, sigma_normal, sigma_depth)
+        return self.denoised
 
 
 # ------------------------------------------------------------------------------- scenes (rayz.zig)

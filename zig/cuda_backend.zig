@@ -84,6 +84,15 @@ pub const RzNoise = extern struct {
     max_err: f64,
 };
 
+pub const RzDenoiseParams = extern struct {
+    struct_size: u32 = @sizeOf(RzDenoiseParams),
+    iterations: u32 = 5, // à-trous levels, 0..10 (0 = the resolved frame unchanged)
+    sigma_luminance: f32 = 0, // 0 => 4
+    sigma_normal: f32 = 0, // 0 => 128
+    sigma_depth: f32 = 0, // 0 => 1
+    reserved0: u32 = 0,
+};
+
 pub const RzContext = opaque {};
 
 pub extern fn rayz_cuda_create(cfg: ?*const RzConfig, out: *?*RzContext) c_int;
@@ -97,6 +106,8 @@ pub extern fn rayz_cuda_render_to_noise(ctx: *RzContext, cam: *const RzCamera, p
 pub extern fn rayz_cuda_pixel_samples(ctx: *RzContext, out_spp: [*]u32) c_int;
 // guide buffers for a denoiser: first-hit albedo + coverage, normal + hit distance (rows * width * 4 floats each)
 pub extern fn rayz_cuda_render_guides(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, out_albedo: ?[*]f32, out_normal: ?[*]f32) c_int;
+// the accumulated frame (RZ_RENDER_MOMENTS) denoised with the guides of the last rayz_cuda_render_guides call (rows * width * 4 floats, * 3 bytes)
+pub extern fn rayz_cuda_denoise(ctx: *RzContext, dp: ?*const RzDenoiseParams, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8) c_int;
 pub extern fn rayz_cuda_last_error() [*:0]const u8;
 
 pub const Error = error{ CudaBackend, OutOfMemory };
