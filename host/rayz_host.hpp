@@ -263,6 +263,7 @@ struct Tracer {
     bool adaptive = false;        // with noise_target: it bounds every pixel's error, and only pixels above it get more samples (RZ_RENDER_ADAPTIVE)
     std::vector<float> albedo, normal;   // guide buffers of the last renderGuides(): rgb albedo + coverage, normal + hit distance (4 floats a pixel)
     bool moments = false;         // render with RZ_RENDER_MOMENTS (no pixel changes), so that denoise() can follow
+    bool sobol = false;           // RZ_RENDER_SOBOL: Owen-scrambled Sobol camera and scatter samples, in render() and renderGuides()
     Image denoised;               // rgb8 of the last denoise()
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
@@ -298,6 +299,7 @@ struct Tracer {
         p.seed = render_seed; p.variant = variant;
         if (adaptive && noise_target > 0) p.flags |= RZ_RENDER_ADAPTIVE;
         if (moments) p.flags |= RZ_RENDER_MOMENTS;
+        if (sobol) p.flags |= RZ_RENDER_SOBOL;
         return p;
     }
 
@@ -350,7 +352,7 @@ struct Tracer {
     // Guide buffers for a denoiser over the camera samples render() traces (rayz_cuda_render_guides), after render().
     void renderGuides() {
         RzRenderParams p = renderParams();
-        p.flags = 0;
+        p.flags &= RZ_RENDER_SOBOL;   // the render's own camera rays
         const RzCamera cam = camera.flat();
         albedo.assign(img.w * img.h * 4, 0.f);
         normal.assign(img.w * img.h * 4, 0.f);

@@ -146,7 +146,7 @@ typedef struct RzRenderParams {
                                     * two families agree up to a pixel or two (see RZ_VARIANT_AUTO): pin the variant where
                                     * bit equality matters.  Refused with RZ_ERR_INVALID_ARG, the sums untouched, unless the
                                     * previous render succeeded with the same width, height, shard_index/count, band_rows,
-                                    * seed, max_depth, t_min, camera and RZ_RENDER_MOMENTS bit on this context, no scene
+                                    * seed, max_depth, t_min, camera, RZ_RENDER_MOMENTS and RZ_RENDER_SOBOL bits on this context, no scene
                                     * upload or differently shaped reserve came in between, sample_offset equals the previous
                                     * batch's sample_offset + spp, and the cumulative count stays below 2^32.  A render that
                                     * fails ends the accumulation.  *out_paths counts this call's paths only.  With
@@ -164,6 +164,26 @@ typedef struct RzRenderParams {
                                     * Whether a pixel is active depends on its own sums only, so sharding changes no count.
                                     * rayz_cuda_noise and rayz_cuda_pixel_samples read the frame with each pixel's own count; an
                                     * RZ_RENDER_ACCUMULATE batch after it is refused, the sums untouched. */
+#define RZ_RENDER_SOBOL 0x10u      /* low-discrepancy sampling (DESIGN.md "Low-discrepancy sampling"): the camera's and each
+                                    * scatter's uniforms come from 2-D pairs of an Owen-scrambled Sobol sequence instead of
+                                    * independent Philox draws.  Pairs: camera A = jitter (x, y); camera B = lens (radius, angle,
+                                    * area-preserving polar map); camera C = shutter time (first coordinate); bounce s = 1..max_depth
+                                    * = the scatter's u.x, u.y (the sphere direction; u.x is also the dielectric's Fresnel choice).
+                                    * u.z and u.w of a bounce stay Philox.  Construction (Burley 2020, "Practical Hash-based Owen
+                                    * Scrambling", with padding): point i of a pair is (Sobol dimension 0, dimension 1) of the
+                                    * shuffled index i' = S(i, s_shuffle), each coordinate then scrambled x = S(x, s_dim), with S a
+                                    * nested-uniform (Owen) scramble (bit reversal, Laine-Karras-style hash keyed by s, bit
+                                    * reversal); dimension 0 = the bit-reversed index, dimension 1 = Joe-Kuo d = 2 (s = 1, a = 0,
+                                    * m = {1}); the top 24 bits become the uniform.  The seeds s are an integer hash of (seed, global
+                                    * pixel, pair) only, so every uniform is still a pure function of (seed, global pixel, sample
+                                    * index, bounce) and every guarantee above holds as written: sharding, batches, adaptive pixels,
+                                    * guides.  Stratification: for each pixel and pair, the 2^k points of an aligned sample block
+                                    * [m 2^k, (m + 1) 2^k) form a (0,k,2)-net: for every a + b = k each box of 2^-a x 2^-b holds
+                                    * exactly one point (the doubling schedule of rayz_cuda_render_to_noise hands out such blocks from
+                                    * a power-of-two start).  The noise estimate (rayz_cuda_noise) keeps its formula, which assumes
+                                    * independent samples: with this flag the error of the mean is expected to be smaller than it
+                                    * says (conservative), so rayz_cuda_render_to_noise stops about where it would without the flag;
+                                    * the gain shows in fixed-spp frames and in the denoiser's input. */
 
 /* Noise summary of the accumulated frame (rayz_cuda_noise).  Errors are standard errors of the DISPLAYED value
  * (gamma 2, as writePPM shows it) in units of [0, 1]: one 8-bit step is 1/255.  +inf while samples < 2. */

@@ -225,7 +225,7 @@ struct AccumRecord {
     bool valid = false;
     bool pending = false;   // enqueued by rayz_cuda_render_device(sync = 0): the device error words are not checked yet
     Frame frame;
-    uint32_t max_depth = 0, moments = 0;
+    uint32_t max_depth = 0, moments = 0, sobol = 0;
     uint64_t seed = 0;
     float t_min = 0;
     RzCamera cam{};
@@ -948,6 +948,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         AccumRecord &next = P.next;
         next.frame = P.frame;
         next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
+        next.sobol = (p->flags & RZ_RENDER_SOBOL) ? 1u : 0u;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
         next.adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
@@ -961,6 +962,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
                 return refuse("seed, max_depth or t_min differ from the accumulated render");
             if (memcmp(&prev.cam, cam, sizeof(RzCamera)) != 0) return refuse("the camera differs from the accumulated render");
             if (prev.moments != next.moments) return refuse("the RZ_RENDER_MOMENTS bit differs from the accumulated render");
+            if (prev.sobol != next.sobol) return refuse("the RZ_RENDER_SOBOL bit differs from the accumulated render");
             if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
                 return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
             if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
@@ -1139,7 +1141,7 @@ static int enqueue_staged(RzContext *ctx, Dev &D, RzPathArgs a, const RenderPlan
 }
 
 // The path-kernel arguments of device d's share of the planned frame that do not depend on the kernel form: the BVH-ordered
-// set, scene, camera, frame and shard, sampling, t_min, error word and traversal tuning.  rayz_cuda_render_guides launches
+// set, scene, camera, frame and shard, sampling (seed, sample range, sampler), t_min, error word and traversal tuning.  rayz_cuda_render_guides launches
 // rz_guides_kernel with them as they are (RzGuideArgs); enqueue_device adds the render's buffers and work units.
 static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t d) {
     const RzRenderParams *p = P.p;
@@ -1156,6 +1158,7 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
     a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;
     a.shard_index = P.frame.s * ND + d; a.shard_count = P.frame.S * ND; a.band_rows = P.frame.band;
     a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
+    a.sobol = (p->flags & RZ_RENDER_SOBOL) ? 1u : 0u;
     a.t_min = P.next.t_min;   // plan_render applied the default
     a.err = D.errword.p;
     a.unit_entries = ctx->tun.unit_entries;

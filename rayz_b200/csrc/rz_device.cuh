@@ -166,6 +166,7 @@ struct RzPathArgs {
     // covers list entries [tile * 32, tile * 32 + 32), and lane k's pixel is px_list[entry] instead of the entry itself.
     const uint32_t *px_list;     // local pixel indices in increasing order (rz_adaptive.cu)
     uint32_t n_list;             // entries in px_list
+    uint32_t sobol;              // != 0 (RZ_RENDER_SOBOL): the launchers run each kernel's SOBOL instance (rz_sampler.cuh's pairs)
 };
 
 // Guide buffers (rayz_cuda_render_guides, rz_guides_kernel in rz_bvh_trace.cu): the camera segments of a render with these
@@ -262,6 +263,8 @@ RZ_HD uint4 rz_philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32
 
 // 24 random bits -> [0,1)
 RZ_HD float rz_u01(uint32_t bits24) { return (float)bits24 * 5.9604644775390625e-8f; }
+
+#include "rz_sampler.cuh"   // RZ_RENDER_SOBOL's pairs
 
 // ---------------------------------------------------------------------------------------------
 // small float3 algebra
@@ -378,14 +381,10 @@ RZ_HD void rz_consider(int k, float nb, float nd, int self_k, float t_min, float
     }
 }
 
-// Camera.getRay with rng (camera.zig:59-77): jittered pixel position, thin-lens origin on the
-// defocus disk, time in [0,1).  Disk sample is polar instead of rejection (same distribution).
-// One Philox block gives the five uniforms: 4 x 24 high bits + 3 x 8 low bits.
-RZ_HD RzRay rz_camera_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, uint32_t gpix, uint32_t sample,
-                          uint32_t k0, uint32_t k1) {
-    const uint4 r = rz_philox(gpix, sample, 0u, 0u, k0, k1);
-    const float ux = rz_u01(r.x >> 8), uy = rz_u01(r.y >> 8), ut = rz_u01(r.z >> 8), ur = rz_u01(r.w >> 8);
-    const float ua = rz_u01(((r.x & 0xffu) << 16) | ((r.y & 0xffu) << 8) | (r.z & 0xffu));
+// Camera.getRay with rng (camera.zig:59-77) from its five uniforms: jittered pixel position, thin-lens origin on the defocus
+// disk, time in [0,1).  Disk sample is polar instead of rejection (same distribution, and area-preserving: strata of (ur, ua)
+// stay strata of the disk).
+RZ_HD RzRay rz_lens_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, float ux, float uy, float ut, float ur, float ua) {
     const float x = (float)px + (ux - 0.5f);
     const float y = (float)py + (uy - 0.5f);
     RzRay ray;
@@ -401,6 +400,23 @@ RZ_HD RzRay rz_camera_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, uint32_
     ray.time = ut;
     ray.self_k = -1;
     return ray;
+}
+
+// One Philox block gives the five uniforms: 4 x 24 high bits + 3 x 8 low bits.  With `sobol` (RZ_RENDER_SOBOL; the kernels pass
+// their SOBOL template argument) three Sobol pairs give them instead (rz_sampler.cuh): jitter, lens (radius, angle) and the
+// shutter time (first coordinate of the third pair).
+RZ_HD RzRay rz_camera_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, uint32_t gpix, uint32_t sample,
+                          uint32_t k0, uint32_t k1, bool sobol = false) {
+    if (sobol) {
+        const float2 j = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_JITTER, sample);
+        const float2 l = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_LENS, sample);
+        const float t = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_TIME, sample).x;
+        return rz_lens_ray(cam, px, py, j.x, j.y, t, l.x, l.y);
+    }
+    const uint4 r = rz_philox(gpix, sample, 0u, 0u, k0, k1);
+    const float ux = rz_u01(r.x >> 8), uy = rz_u01(r.y >> 8), ut = rz_u01(r.z >> 8), ur = rz_u01(r.w >> 8);
+    const float ua = rz_u01(((r.x & 0xffu) << 16) | ((r.y & 0xffu) << 8) | (r.z & 0xffu));
+    return rz_lens_ray(cam, px, py, ux, uy, ut, ur, ua);
 }
 
 // Sky of bounceRay's miss branch (renderer.zig:124-125): ((1-t)*1 + (0.5,0.7,1.0)) * t — not a lerp.

@@ -319,12 +319,19 @@ __device__ __forceinline__ const float4 *rz_stage_scene_cv(const RzSphereSet &se
 }
 
 // ------------------------------------------------------------------------------ shade
+// Every path kernel has a SOBOL template parameter (RZ_RENDER_SOBOL): the launchers pick the instance from RzPathArgs::sobol.
+// A runtime branch on the field instead raised the registers or spills of the Philox instances (DESIGN.md "Low-discrepancy
+// sampling"), which are the default and the benchmark.
+template <class K>
+static inline K rz_pick_sampler(const RzPathArgs &a, K philox, K sobol) { return a.sobol ? sobol : philox; }
+
 enum { RZ_CONT = 0, RZ_END_SKY = 1, RZ_END_ABSORBED = 2, RZ_END_DEPTH = 3 };
 
 // One step of bounceRay (renderer.zig:103-126) after the closest-hit query: miss -> sky and
-// accumulate; hit -> refine in f64, scatter, attenuate.  `kind_out` = material kind of the hit.
+// accumulate; hit -> refine in f64, scatter, attenuate.  `kind_out` = material kind of the hit.  `sobol`: the kernel's SOBOL
+// template argument (RZ_RENDER_SOBOL), a compile-time constant, so that the Philox instances carry no trace of the other sampler.
 __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray, float3 &thr, uint32_t &seg, uint32_t lp,
-                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out) {
+                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, bool sobol) {
     kind_out = 3u;
     if (bk < 0) {
         // miss: background (renderer.zig:124-125), path ends
@@ -352,7 +359,9 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
     kind_out = kind < 3u ? kind : 0u;
     seg++;
     const uint4 rb = rz_philox(gpix, sample, seg, 0u, a.seed_lo, a.seed_hi);
-    const float4 u = make_float4(rz_u01(rb.x >> 8), rz_u01(rb.y >> 8), rz_u01(rb.z >> 8), rz_u01(rb.w >> 8));
+    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(seg), sample)   // u.z, u.w stay Philox
+                           : make_float2(rz_u01(rb.x >> 8), rz_u01(rb.y >> 8));
+    const float4 u = make_float4(q.x, q.y, rz_u01(rb.z >> 8), rz_u01(rb.w >> 8));
     float3 att;
     if (!rz_scatter(M, a.texs, h, k, u, ray, att)) return RZ_END_ABSORBED;  // black (renderer.zig:109,120)
     thr = thr * att;

@@ -278,9 +278,10 @@ class Backend:
     @staticmethod
     def params(width, height, spp, max_depth=50, seed=1, sample_offset=0, variant="auto", t_min=0.0, shard_index=0,
                shard_count=1, band_rows=0, collect_stats=False, serial_passes=False, accumulate=False,
-               moments=False) -> abi.RzRenderParams:
+               moments=False, sobol=False) -> abi.RzRenderParams:
         """RzRenderParams.  accumulate: add this batch to the previous render's sums (RZ_RENDER_ACCUMULATE; sample_offset must
-        continue where they end); moments: also sum each path's luminance squared, so that noise() can estimate the error."""
+        continue where they end); moments: also sum each path's luminance squared, so that noise() can estimate the error;
+        sobol: draw the camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox (RZ_RENDER_SOBOL)."""
         p = abi.RzRenderParams()
         p.width, p.height, p.spp, p.max_depth = width, height, spp, max_depth
         p.seed, p.sample_offset = seed, sample_offset
@@ -289,7 +290,7 @@ class Backend:
         p.shard_index, p.shard_count, p.band_rows = shard_index, shard_count, band_rows
         p.collect_stats = 1 if collect_stats else 0
         p.flags = ((abi.RENDER_SERIAL_PASSES if serial_passes else 0) | (abi.RENDER_ACCUMULATE if accumulate else 0)
-                   | (abi.RENDER_MOMENTS if moments else 0))
+                   | (abi.RENDER_MOMENTS if moments else 0) | (abi.RENDER_SOBOL if sobol else 0))
         return p
 
     def reserve(self, p: abi.RzRenderParams):
@@ -448,6 +449,8 @@ class Tracer:
         self.pool = MemPool()
         self.seed = seed           # the reference seeds from the OS (renderer.zig:55-59)
         self.variant = "auto"
+        self.sampler = "philox"    # or "sobol": low-discrepancy camera and scatter samples (RZ_RENDER_SOBOL) in render(),
+                                   # render_guides() and so the denoised frame
         self.devices = devices
         self.noise = None          # summary of the last render(noise_target=...) (rayz_cuda_render_to_noise)
         self.pixel_samples = None  # [h, w] per-pixel sample counts of the last render(noise_target=..., adaptive=True)
@@ -456,6 +459,11 @@ class Tracer:
         self.denoised = None       # (linear [h, w, 4], rgb8 [h, w, 3]) of the last denoise()
         self._backend = None
         self._uploaded = None      # the pool arrays of the backend's last scene upload
+
+    def _sobol(self) -> bool:
+        if self.sampler not in ("philox", "sobol"):
+            raise ValueError(f"Tracer.sampler must be 'philox' or 'sobol', not {self.sampler!r}")
+        return self.sampler == "sobol"
 
     @property
     def backend(self) -> Backend:
@@ -475,7 +483,7 @@ class Tracer:
         b.upload_scene(arrays)  # initHittables + bvh.build (renderer.zig:76-78)
         self._uploaded = arrays
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
-                           moments=moments)
+                           moments=moments, sobol=self._sobol())
         if noise_target is None:
             lin, rgb8, rays = b.render(self.camera.rz, p)
         else:
@@ -500,7 +508,8 @@ class Tracer:
             self._uploaded = None
             b.upload_scene(arrays)
             self._uploaded = arrays
-        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant)
+        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
+                           sobol=self._sobol())
         self.albedo, self.normal = b.guides(self.camera.rz, p)
         return self.albedo, self.normal
 
