@@ -3,7 +3,7 @@
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
-//               [--guides PREFIX] [--denoise FILE] [--sobol]
+//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -17,7 +17,8 @@
 // --denoise FILE renders with RZ_RENDER_MOMENTS (no pixel changes), computes guides over the render's own samples and writes the
 // frame denoised by rayz_cuda_denoise (default parameters) to FILE as P3; the normal output and the report line are unchanged.
 // --sobol draws the camera and scatter samples from Owen-scrambled Sobol pairs (RZ_RENDER_SOBOL) in every one of these runs,
-// guides included.
+// guides included.  --rqmc does the same with two independently scrambled replicates per pixel and the noise estimate they
+// allow (RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS): --noise-target then stops on it; --spp and --max-spp must be even.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -43,7 +44,7 @@ int main(int argc, char **argv) {
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
     const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr;
-    bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false;
+    bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false, rqmc = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
     for (int i = 2; i < argc; i++) {
@@ -62,6 +63,7 @@ int main(int argc, char **argv) {
         else if (a == "--max-spp") max_spp = (uint32_t)std::strtoul(val(), nullptr, 10);
         else if (a == "--adaptive") adaptive = true;
         else if (a == "--sobol") sobol = true;
+        else if (a == "--rqmc") rqmc = true;
         else if (a == "--guides") guides = val();
         else if (a == "--denoise") denoise = val();
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
@@ -85,6 +87,7 @@ int main(int argc, char **argv) {
         tracer.adaptive = adaptive;
         tracer.moments = denoise != nullptr;
         tracer.sobol = sobol;
+        tracer.rqmc = rqmc;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);

@@ -264,6 +264,7 @@ struct Tracer {
     std::vector<float> albedo, normal;   // guide buffers of the last renderGuides(): rgb albedo + coverage, normal + hit distance (4 floats a pixel)
     bool moments = false;         // render with RZ_RENDER_MOMENTS (no pixel changes), so that denoise() can follow
     bool sobol = false;           // RZ_RENDER_SOBOL: Owen-scrambled Sobol camera and scatter samples, in render() and renderGuides()
+    bool rqmc = false;            // RZ_RENDER_RQMC (with SOBOL and MOMENTS): two Sobol replicates per pixel, a noise estimate that sees them
     Image denoised;               // rgb8 of the last denoise()
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
@@ -300,6 +301,7 @@ struct Tracer {
         if (adaptive && noise_target > 0) p.flags |= RZ_RENDER_ADAPTIVE;
         if (moments) p.flags |= RZ_RENDER_MOMENTS;
         if (sobol) p.flags |= RZ_RENDER_SOBOL;
+        if (rqmc) p.flags |= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;
         return p;
     }
 
@@ -352,7 +354,7 @@ struct Tracer {
     // Guide buffers for a denoiser over the camera samples render() traces (rayz_cuda_render_guides), after render().
     void renderGuides() {
         RzRenderParams p = renderParams();
-        p.flags &= RZ_RENDER_SOBOL;   // the render's own camera rays
+        p.flags &= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;   // the render's own camera rays (RQMC needs MOMENTS beside it)
         const RzCamera cam = camera.flat();
         albedo.assign(img.w * img.h * 4, 0.f);
         normal.assign(img.w * img.h * 4, 0.f);

@@ -146,8 +146,9 @@ typedef struct RzRenderParams {
                                     * two families agree up to a pixel or two (see RZ_VARIANT_AUTO): pin the variant where
                                     * bit equality matters.  Refused with RZ_ERR_INVALID_ARG, the sums untouched, unless the
                                     * previous render succeeded with the same width, height, shard_index/count, band_rows,
-                                    * seed, max_depth, t_min, camera, RZ_RENDER_MOMENTS and RZ_RENDER_SOBOL bits on this context, no scene
-                                    * upload or differently shaped reserve came in between, sample_offset equals the previous
+                                    * seed, max_depth, t_min, camera, RZ_RENDER_MOMENTS, RZ_RENDER_SOBOL and RZ_RENDER_RQMC bits on this context, no scene
+                                    * upload or differently shaped reserve (or an RZ_RENDER_RQMC reserve after a render without
+                                    * the flag, which grows the accumulators) came in between, sample_offset equals the previous
                                     * batch's sample_offset + spp, and the cumulative count stays below 2^32.  A render that
                                     * fails ends the accumulation.  *out_paths counts this call's paths only.  With
                                     * rayz_cuda_render_device(sync = 0), the next batch checks the previous one's device
@@ -161,7 +162,8 @@ typedef struct RzRenderParams {
                                     * rgb8, error), as every path is a function of (seed, pixel, sample index).  AUTO runs the BVH
                                     * family; a pinned MEGA, MEGA_SINGLE or WAVEFRONT runs its first round as pinned and the
                                     * others with the single-form brute-force kernel (the same family: for exactness, not speed).
-                                    * Whether a pixel is active depends on its own sums only, so sharding changes no count.
+                                    * Whether a pixel is active depends on its own sums only (under RZ_RENDER_RQMC, on them and on
+                                    * its row segment's gain, which no shard splits), so sharding changes no count.
                                     * rayz_cuda_noise and rayz_cuda_pixel_samples read the frame with each pixel's own count; an
                                     * RZ_RENDER_ACCUMULATE batch after it is refused, the sums untouched. */
 #define RZ_RENDER_SOBOL 0x10u      /* low-discrepancy sampling (DESIGN.md "Low-discrepancy sampling"): the camera's and each
@@ -183,7 +185,39 @@ typedef struct RzRenderParams {
                                     * a power-of-two start).  The noise estimate (rayz_cuda_noise) keeps its formula, which assumes
                                     * independent samples: with this flag the error of the mean is expected to be smaller than it
                                     * says (conservative), so rayz_cuda_render_to_noise stops about where it would without the flag;
-                                    * the gain shows in fixed-spp frames and in the denoiser's input. */
+                                    * the gain shows in fixed-spp frames and in the denoiser's input.  RZ_RENDER_RQMC makes the
+                                    * estimate see the gain. */
+#define RZ_RENDER_RQMC 0x20u       /* randomised-QMC noise estimate over RZ_RENDER_SOBOL (DESIGN.md "Low-discrepancy sampling",
+                                    * "The RQMC estimate").  Requires RZ_RENDER_SOBOL and RZ_RENDER_MOMENTS (rayz_cuda_render_to_noise
+                                    * implies MOMENTS, so there it needs SOBOL only), an even spp and sample_offset, and in
+                                    * rayz_cuda_render_to_noise an even max_spp; anything else is refused with RZ_ERR_INVALID_ARG,
+                                    * the message naming the rule, nothing touched.  An RZ_RENDER_ACCUMULATE batch whose RQMC bit
+                                    * differs from the accumulated render's is refused, the sums untouched.
+                                    * Replicates (R = 2): sample index i belongs to replicate r = i & 1 and is that replicate's sample
+                                    * j = i >> 1.  Each replicate is an Owen-scrambled Sobol sequence as above with its own seeds: the
+                                    * pair's base seed b = rz_sobol_pair_seed(seed, global pixel, pair) becomes
+                                    * b_r = rz_hash32(b ^ (0x9e3779b9 + r)), and point i is point j of the pair under b_r.  Every
+                                    * uniform is still a pure function of (seed, global pixel, sample index, bounce): sharding,
+                                    * batches, adaptive pixels and guides keep their guarantees.  Within each replicate the aligned
+                                    * blocks of j are (0,k,2)-nets.  The image and rayz_cuda_pixel_samples do not change meaning:
+                                    * a pixel is the mean of all n samples.
+                                    * The estimate.  A sky path adds its clamped luminance Y (rz_luma_sq's Y) in 2^-32 fixed point to
+                                    * its replicate's sum Q_r (16 bytes a pixel).  For a pixel with n samples, m = n / 2:
+                                    *   mu_r = Q_r 2^-32 / m,  V_rep = (mu_0 - mu_1)^2 / 4  (sum_r (mu_r - mu)^2 / (R (R - 1)), R = 2),
+                                    *   V_iid = s^2 / n  (the s^2 of the error formula of RzNoise / rayz_cuda_noise).
+                                    * A segment is the pixels of one global row with x in [64k, 64k + 64) (the last one of a row may be
+                                    * shorter); G = sum_seg V_rep / sum_seg V_iid, 1 when the denominator is 0, not clamped; and the
+                                    * pixel's error is e = e_iid sqrt(G), with the G of its segment when the pixel's count was last
+                                    * the frame's largest: in a uniform frame, the current G of every pixel; under RZ_RENDER_ADAPTIVE,
+                                    * the G its last stopping test read, so that a pixel that stopped keeps the error it stopped at
+                                    * while its segment's other pixels take more samples, and max_err <= target unless capped holds
+                                    * as without the flag.  One pixel's V_rep has one degree of freedom; a segment pools
+                                    * about 64, so sqrt(G) is good to about +-9 %, while the per-pixel shape comes from the iid term.
+                                    * Segments lie inside a global row, which no shard or device splits: e and every adaptive count
+                                    * are shard- and device-invariant.  This e is what out_err, the summary and n_above of
+                                    * rayz_cuda_noise, both tests of rayz_cuda_render_to_noise and the denoiser's v_p use.
+                                    * Trade-off: two replicates of n / 2 points carry more variance than one sequence of n points, so
+                                    * the frame itself is somewhat noisier than under RZ_RENDER_SOBOL alone; hence a separate flag. */
 
 /* Noise summary of the accumulated frame (rayz_cuda_noise).  Errors are standard errors of the DISPLAYED value
  * (gamma 2, as writePPM shows it) in units of [0, 1]: one 8-bit step is 1/255.  +inf while samples < 2. */

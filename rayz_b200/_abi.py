@@ -19,7 +19,7 @@ TEX_CHECKER, TEX_SOLID = 0, 1
 DIFFUSE_UNIT_SPHERE, DIFFUSE_UNIT_SPHERE_SURFACE, DIFFUSE_HEMISPHERE = 0, 1, 2
 VARIANT_AUTO, VARIANT_MEGA, VARIANT_WAVEFRONT, VARIANT_BVH = 0, 1, 2, 3
 VARIANTS = {"auto": 0, "mega": 1, "wavefront": 2, "bvh": 3, "mega_single": 4}
-RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE, RENDER_ADAPTIVE, RENDER_SOBOL = 1, 2, 4, 8, 0x10   # RzRenderParams.flags (RZ_RENDER_*)
+RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE, RENDER_ADAPTIVE, RENDER_SOBOL, RENDER_RQMC = 1, 2, 4, 8, 0x10, 0x20   # RzRenderParams.flags (RZ_RENDER_*)
 
 _dp, _up = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 

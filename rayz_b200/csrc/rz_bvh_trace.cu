@@ -131,7 +131,7 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
 }
 
 // LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list).
-template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false, bool SOBOL = false>
+template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false, int SOBOL = 0>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -173,7 +173,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
         if (alive && cur == RZ_SENTINEL) {
             if (STATS) c_segs++;
             uint32_t kind;
-            const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, sample, bk, kind, SOBOL);
+            const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, sample, bk, kind, SOBOL != 0, SOBOL == 2);
             if (STATS) {
                 if (kind < 3u) c_hit[kind]++;
                 if (res == RZ_END_SKY) c_sky++;
@@ -230,7 +230,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
                             lp = nlp;
                             gpix = pj * a.width + pi;
                             sample = a.sample_offset + unit_s0 + (k >> 5);
-                            ray = rz_camera_ray(a.cam, pi, pj, gpix, sample, a.seed_lo, a.seed_hi, SOBOL);
+                            ray = rz_camera_ray(a.cam, pi, pj, gpix, sample, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
                             thr = f3(1.f, 1.f, 1.f);
                             seg = 0;
                             alive = a.max_depth > 0u;
@@ -270,7 +270,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
 // in L1; survivors go to the next queue, and the tail of the paths to the persistent kernel above (QUEUE).
 // CAMERA: the camera rays of a work unit — an 8 x 4-pixel block x `chunk` samples — do not walk the tree one by one; the warp
 // culls the tree once against the block's cone and the rays search the surviving spheres as a list (below).  The sorted stages (CAMERA = false) are off by default (RzTuning::bvh_stages = 0: measured as a loss).
-template <bool STATS, bool CAMERA, bool SOBOL = false>
+template <bool STATS, bool CAMERA, int SOBOL = 0>
 __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB) rz_bvh_stage_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -407,7 +407,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                         const bool have = valid && (b + (uint32_t)r < n_batches);
                         live[r] = have && a.max_depth > 0u;
                         if (STATS && have) { c_paths++; if (!live[r]) c_depth++; }
-                        if (live[r]) rays[r] = rz_camera_ray(a.cam, pi, pj, gpix0, smp[r], a.seed_lo, a.seed_hi, SOBOL);
+                        if (live[r]) rays[r] = rz_camera_ray(a.cam, pi, pj, gpix0, smp[r], a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
                         else { rays[r].o = f3(0.f, 0.f, 0.f); rays[r].d = f3(0.f, 1.f, 0.f); rays[r].time = 0.f; rays[r].self_k = -1; }
                     }
                     float bt[2] = {3.0e38f, 3.0e38f};
@@ -424,7 +424,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                             const int hit = bk[0] < 0 ? -1 : (w_gid[bk[0] & ~RZ_FAR_BIT] | (bk[0] & RZ_FAR_BIT));   // list slot -> position in the set
                             if (STATS) c_segs++;
                             uint32_t kind;
-                            const int res = rz_shade_segment(a, rays[0], thr[0], seg[0], lp0, gpix0, smp[0], hit, kind, SOBOL);
+                            const int res = rz_shade_segment(a, rays[0], thr[0], seg[0], lp0, gpix0, smp[0], hit, kind, SOBOL != 0, SOBOL == 2);
                             if (STATS) {
                                 if (kind < 3u) c_hit[kind]++;
                                 if (res == RZ_END_SKY) c_sky++;
@@ -456,7 +456,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                 smp = a.sample_offset + s0 + b;
                 live = valid && a.max_depth > 0u;
                 if (STATS && valid) { c_paths++; if (!live) c_depth++; }
-                if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, smp, a.seed_lo, a.seed_hi, SOBOL);
+                if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, smp, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
             } else {
                 const uint32_t i = b * 32u + lane;
                 live = i < ne;
@@ -479,7 +479,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
             if (live) {
                 if (STATS) c_segs++;
                 uint32_t kind;
-                const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, smp, bk, kind, SOBOL);
+                const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, smp, bk, kind, SOBOL != 0, SOBOL == 2);
                 if (STATS) {
                     if (kind < 3u) c_hit[kind]++;
                     if (res == RZ_END_SKY) c_sky++;
@@ -525,7 +525,7 @@ __device__ __forceinline__ float3 rz_guide_albedo(const RzPathArgs &a, int k, co
 // samples in lockstep: a block's rays fan out over a third of the angle of 32 pixels of a row (the camera stage's reason for
 // the same blocks), so the lanes visit more of the same nodes.  Each lane sums its pixel's samples in f64, in sample order, and
 // divides once: the result depends on (scene, camera, seed, pixel, sample range) only.
-template <bool SOBOL>
+template <int SOBOL>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGuideArgs g) {
     const RzPathArgs &a = g.a;
     const unsigned lane = threadIdx.x & 31u;
@@ -545,7 +545,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGui
     uint32_t hits = 0;
     for (uint32_t s = 0; s < a.spp; s++) {
         RzRay ray;
-        if (valid) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL);
+        if (valid) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
         else { ray.o = f3(0.f, 0.f, 0.f); ray.d = f3(0.f, 1.f, 0.f); ray.time = 0.f; ray.self_k = -1; }
         const float ix = 1.0f / ray.d.x, iy = 1.0f / ray.d.y, iz = 1.0f / ray.d.z;
         float bt = 3.0e38f;
@@ -578,10 +578,10 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGui
         g.out_normal[dst] = make_float4((float)(nx / n), (float)(ny / n), (float)(nz / n), hits ? (float)(dist / (double)hits) : 0.f);
 }
 
-// kern_sobol: the same kernel's SOBOL instance, launched instead for RZ_RENDER_SOBOL
+// kern_sobol, kern_rqmc: the same kernel's SOBOL = 1 and SOBOL = 2 instances, launched instead for RZ_RENDER_SOBOL (and RZ_RENDER_RQMC)
 template <class K>
-cudaError_t launch_kernel(K kern, K kern_sobol, const RzPathArgs &a, int sm_count, cudaStream_t stream) {
-    kern = rz_pick_sampler(a, kern, kern_sobol);
+cudaError_t launch_kernel(K kern, K kern_sobol, K kern_rqmc, const RzPathArgs &a, int sm_count, cudaStream_t stream) {
+    kern = rz_pick_sampler(a, kern, kern_sobol, kern_rqmc);
     int per_sm = 0;
     cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, 0);
     if (e != cudaSuccess) return e;
@@ -612,16 +612,16 @@ extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int
     RzPathArgs b = *a;
     rz_bvh_tuning(b);
     if (b.q_in && b.self_map)   // the tail of the staged K1 (entries written by a brute-force stage): a short queue, small units
-        return collect_stats ? launch_kernel(rz_bvh_kernel<true, true, 64>, rz_bvh_kernel<true, true, 64, false, true>, b, sm_count, stream)
-                             : launch_kernel(rz_bvh_kernel<false, true, 64>, rz_bvh_kernel<false, true, 64, false, true>, b, sm_count, stream);
+        return collect_stats ? launch_kernel(rz_bvh_kernel<true, true, 64>, rz_bvh_kernel<true, true, 64, false, 1>, rz_bvh_kernel<true, true, 64, false, 2>, b, sm_count, stream)
+                             : launch_kernel(rz_bvh_kernel<false, true, 64>, rz_bvh_kernel<false, true, 64, false, 1>, rz_bvh_kernel<false, true, 64, false, 2>, b, sm_count, stream);
     if (b.q_in)
-        return collect_stats ? launch_kernel(rz_bvh_kernel<true, true>, rz_bvh_kernel<true, true, 512, false, true>, b, sm_count, stream)
-                             : launch_kernel(rz_bvh_kernel<false, true>, rz_bvh_kernel<false, true, 512, false, true>, b, sm_count, stream);
+        return collect_stats ? launch_kernel(rz_bvh_kernel<true, true>, rz_bvh_kernel<true, true, 512, false, 1>, rz_bvh_kernel<true, true, 512, false, 2>, b, sm_count, stream)
+                             : launch_kernel(rz_bvh_kernel<false, true>, rz_bvh_kernel<false, true, 512, false, 1>, rz_bvh_kernel<false, true, 512, false, 2>, b, sm_count, stream);
     if (b.px_list)
-        return collect_stats ? launch_kernel(rz_bvh_kernel<true, false, 512, true>, rz_bvh_kernel<true, false, 512, true, true>, b, sm_count, stream)
-                             : launch_kernel(rz_bvh_kernel<false, false, 512, true>, rz_bvh_kernel<false, false, 512, true, true>, b, sm_count, stream);
-    return collect_stats ? launch_kernel(rz_bvh_kernel<true, false>, rz_bvh_kernel<true, false, 512, false, true>, b, sm_count, stream)
-                         : launch_kernel(rz_bvh_kernel<false, false>, rz_bvh_kernel<false, false, 512, false, true>, b, sm_count, stream);
+        return collect_stats ? launch_kernel(rz_bvh_kernel<true, false, 512, true>, rz_bvh_kernel<true, false, 512, true, 1>, rz_bvh_kernel<true, false, 512, true, 2>, b, sm_count, stream)
+                             : launch_kernel(rz_bvh_kernel<false, false, 512, true>, rz_bvh_kernel<false, false, 512, true, 1>, rz_bvh_kernel<false, false, 512, true, 2>, b, sm_count, stream);
+    return collect_stats ? launch_kernel(rz_bvh_kernel<true, false>, rz_bvh_kernel<true, false, 512, false, 1>, rz_bvh_kernel<true, false, 512, false, 2>, b, sm_count, stream)
+                         : launch_kernel(rz_bvh_kernel<false, false>, rz_bvh_kernel<false, false, 512, false, 1>, rz_bvh_kernel<false, false, 512, false, 2>, b, sm_count, stream);
 }
 
 // Guide buffers of the device's local pixels: one warp per 8 x 4 block, four per CTA.
@@ -631,7 +631,7 @@ extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t strea
     const uint32_t rows = b.a.width ? b.a.n_local_px / b.a.width : 0u;
     const uint32_t blocks = ((b.a.width + 7u) / 8u) * ((rows + 3u) / 4u);
     if (blocks == 0u) return cudaSuccess;
-    rz_pick_sampler(b.a, rz_guides_kernel<false>, rz_guides_kernel<true>)<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
+    rz_pick_sampler(b.a, rz_guides_kernel<0>, rz_guides_kernel<1>, rz_guides_kernel<2>)<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
     return cudaGetLastError();
 }
 
@@ -640,8 +640,8 @@ extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stat
     RzPathArgs b = *a;
     rz_bvh_tuning(b);
     if (!b.q_in)
-        return collect_stats ? launch_kernel(rz_bvh_stage_kernel<true, true>, rz_bvh_stage_kernel<true, true, true>, b, sm_count, stream)
-                             : launch_kernel(rz_bvh_stage_kernel<false, true>, rz_bvh_stage_kernel<false, true, true>, b, sm_count, stream);
-    return collect_stats ? launch_kernel(rz_bvh_stage_kernel<true, false>, rz_bvh_stage_kernel<true, false, true>, b, sm_count, stream)
-                         : launch_kernel(rz_bvh_stage_kernel<false, false>, rz_bvh_stage_kernel<false, false, true>, b, sm_count, stream);
+        return collect_stats ? launch_kernel(rz_bvh_stage_kernel<true, true>, rz_bvh_stage_kernel<true, true, 1>, rz_bvh_stage_kernel<true, true, 2>, b, sm_count, stream)
+                             : launch_kernel(rz_bvh_stage_kernel<false, true>, rz_bvh_stage_kernel<false, true, 1>, rz_bvh_stage_kernel<false, true, 2>, b, sm_count, stream);
+    return collect_stats ? launch_kernel(rz_bvh_stage_kernel<true, false>, rz_bvh_stage_kernel<true, false, 1>, rz_bvh_stage_kernel<true, false, 2>, b, sm_count, stream)
+                         : launch_kernel(rz_bvh_stage_kernel<false, false>, rz_bvh_stage_kernel<false, false, 1>, rz_bvh_stage_kernel<false, false, 2>, b, sm_count, stream);
 }

@@ -27,7 +27,7 @@ struct RzIdsArgs {
 };
 struct RzResolveArgs {
     const unsigned long long *accum; float4 *out_linear; uint8_t *out_rgb8; float *out_err; uint32_t *out_spp; const uint32_t *n_px;
-    uint32_t n_local_px, width; uint32_t spp; uint32_t dev_index, dev_count, band_rows;
+    const double *gain; uint32_t n_local_px, width; uint32_t spp; uint32_t dev_index, dev_count, band_rows;
 };
 extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, int collect_stats, int sm_count,
                                       cudaStream_t stream, int *grid_out);
@@ -54,11 +54,15 @@ extern "C" cudaError_t rz_lbvh_build(uint32_t n, int leaf_max, const double4 *c6
 extern "C" cudaError_t rz_launch_ids(const RzIdsArgs *a, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
 extern "C" uint32_t rz_noise_grid(void);
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, uint32_t n_local_px, uint32_t n,
-                                              double target, void *out, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain,
+                                              uint32_t n_local_px, uint32_t n, double target, void *out, cudaStream_t stream);
+extern "C" size_t rz_rqmc_gain_words(uint32_t n_local_px, uint32_t width);
+extern "C" cudaError_t rz_launch_rqmc_gain(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
+                                           uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, cudaStream_t stream);
 extern "C" size_t rz_list_scratch_words(uint32_t n_local_px);
 extern "C" size_t rz_list_count_word(uint32_t n_local_px);
-extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, uint32_t *n_px, uint32_t n_local_px, uint32_t n_cur, uint32_t add,
+extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, const double *gain, uint32_t *n_px,
+                                            uint32_t n_local_px, uint32_t n_cur, uint32_t add,
                                             float target, uint32_t *list, uint32_t *scratch, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_fill_u32(uint32_t *p, uint32_t n, uint32_t v, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_ffma_peak(float *sink, int grid, int iters, int mode, cudaStream_t stream);
@@ -153,7 +157,9 @@ struct Dev {
     DBuf<float4> m_rec;
     DBuf<float4> t_color;
     DBuf<double> t_inv_scale;
-    DBuf<unsigned long long> accum;
+    DBuf<unsigned long long> accum;   // + RZ_RENDER_RQMC's replicate sums behind the accumulators (rz_rep_offset)
+    DBuf<double> gain;                // RZ_RENDER_RQMC: the segment gains of the local rows (rz_rqmc_gain_kernel)
+    DBuf<double> px_gain;             // RZ_RENDER_RQMC: every local pixel's gain, frozen when an adaptive pixel stops (rz_rqmc_gain_kernel)
     // staged K1, one set per side (passes alternate between two streams): q1 = after the camera segment, q2 = after the second
     DBuf<float4> q1[2], q2[2];
     DBuf<unsigned short> keys[2];
@@ -225,7 +231,7 @@ struct AccumRecord {
     bool valid = false;
     bool pending = false;   // enqueued by rayz_cuda_render_device(sync = 0): the device error words are not checked yet
     Frame frame;
-    uint32_t max_depth = 0, moments = 0, sobol = 0;
+    uint32_t max_depth = 0, moments = 0, sobol = 0, rqmc = 0;
     uint64_t seed = 0;
     float t_min = 0;
     RzCamera cam{};
@@ -943,12 +949,20 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         return rz_fail(RZ_ERR_INVALID_ARG, "%s: unknown variant %u", who, p->variant);
     if (P.variant == RZ_VARIANT_MEGA && brute_smem > RZ_SMEM_BUDGET)
         return rz_fail(RZ_ERR_UNSUPPORTED, "%s: scene needs %u B of shared memory for the brute-force kernel (budget %u); use RZ_VARIANT_BVH", who, brute_smem, RZ_SMEM_BUDGET);
+    if (p->flags & RZ_RENDER_RQMC) {   // refused before anything is touched: the accumulated render stays as it was
+        const char *rule = !(p->flags & RZ_RENDER_SOBOL) ? "RZ_RENDER_RQMC requires RZ_RENDER_SOBOL"
+                           : !(p->flags & RZ_RENDER_MOMENTS) ? "RZ_RENDER_RQMC requires RZ_RENDER_MOMENTS"
+                           : (p->spp & 1u) ? "RZ_RENDER_RQMC requires an even spp (two replicates)"
+                           : (p->sample_offset & 1u) ? "RZ_RENDER_RQMC requires an even sample_offset (two replicates)" : nullptr;
+        if (rule) { P.refused = true; return rz_fail(RZ_ERR_INVALID_ARG, "%s: %s", who, rule); }
+    }
 
     if (cam) {
         AccumRecord &next = P.next;
         next.frame = P.frame;
         next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
         next.sobol = (p->flags & RZ_RENDER_SOBOL) ? 1u : 0u;
+        next.rqmc = (p->flags & RZ_RENDER_RQMC) ? 1u : 0u;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
         next.adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
@@ -963,6 +977,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
             if (memcmp(&prev.cam, cam, sizeof(RzCamera)) != 0) return refuse("the camera differs from the accumulated render");
             if (prev.moments != next.moments) return refuse("the RZ_RENDER_MOMENTS bit differs from the accumulated render");
             if (prev.sobol != next.sobol) return refuse("the RZ_RENDER_SOBOL bit differs from the accumulated render");
+            if (prev.rqmc != next.rqmc) return refuse("the RZ_RENDER_RQMC bit differs from the accumulated render");
             if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
                 return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
             if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
@@ -1032,7 +1047,11 @@ static int alloc_render(RzContext *ctx, RenderPlan &P) {
         DevPlan &dp = P.dev[d];
         const uint32_t n_local = P.split.n_local[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        if ((rc = D.accum.alloc((size_t)dp.n_tiles * 32u * 4u))) return rc;
+        const bool rqmc = (P.p->flags & RZ_RENDER_RQMC) != 0;
+        const unsigned long long *held = D.accum.p;
+        if ((rc = D.accum.alloc((size_t)dp.n_tiles * 32u * (rqmc ? 6u : 4u)))) return rc;
+        if (D.accum.p != held) ctx->acc.valid = false;   // grown (a reserve for RZ_RENDER_RQMC of the same frame): the sums are gone
+        if (rqmc && ((rc = D.gain.alloc(rz_rqmc_gain_words(n_local, P.frame.width))) || (rc = D.px_gain.alloc(n_local)))) return rc;
         if ((rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4))) return rc;
         if ((rc = D.stats.alloc(3))) return rc;   // [0] whole render / primary kernel, [1] sorted stages, [2] persistent tail kernel
         if (P.staged && n_local > 0) {
@@ -1158,7 +1177,7 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
     a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;
     a.shard_index = P.frame.s * ND + d; a.shard_count = P.frame.S * ND; a.band_rows = P.frame.band;
     a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
-    a.sobol = (p->flags & RZ_RENDER_SOBOL) ? 1u : 0u;
+    a.sobol = ((p->flags & RZ_RENDER_SOBOL) ? RZ_SAMPLER_SOBOL : 0u) | ((p->flags & RZ_RENDER_RQMC) ? RZ_SAMPLER_RQMC : 0u);
     a.t_min = P.next.t_min;   // plan_render applied the default
     a.err = D.errword.p;
     a.unit_entries = ctx->tun.unit_entries;
@@ -1168,15 +1187,29 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
 }
 
 // The resolve kernel's arguments for device d's n_local pixels of the accumulated frame A: its sums, over each pixel's own
-// count when A is adaptive, scattered band by band into the gather root's rows.  Every output starts null.
+// count when A is adaptive, scattered band by band into the gather root's rows.  Every output starts null.  Under RZ_RENDER_RQMC
+// out_err reads the segment gains, which rqmc_gain must have enqueued before.
 static RzResolveArgs resolve_args(const RzContext *ctx, uint32_t d, const AccumRecord &A, uint32_t n_local) {
     const Dev &D = ctx->devs[d];
     RzResolveArgs r{};
     r.accum = D.accum.p;
     r.n_px = A.adaptive ? D.n_px.p : nullptr;
+    r.gain = A.rqmc ? D.px_gain.p : nullptr;
     r.n_local_px = n_local; r.width = A.frame.width; r.spp = (uint32_t)A.samples;
     r.dev_index = d; r.dev_count = (uint32_t)ctx->devs.size(); r.band_rows = A.frame.band;
     return r;
+}
+
+// RZ_RENDER_RQMC: device d's gains of the accumulated frame A, on its stream, before any consumer of the error (the resolve's
+// out_err, the noise reduction, the adaptive flags): the segment gains, copied to the pixels whose count is A's largest (every
+// pixel of a uniform frame; the pixels still sampled of an adaptive one).  The per-pixel gains those consumers take, or null.
+static int rqmc_gain(RzContext *ctx, uint32_t d, const AccumRecord &A, uint32_t n_local, const double **gain = nullptr) {
+    Dev &D = ctx->devs[d];
+    if (gain) *gain = A.rqmc ? D.px_gain.p : nullptr;
+    if (!A.rqmc) return RZ_OK;
+    RZ_CUDA(rz_launch_rqmc_gain(D.accum.p, D.accum.p + rz_rep_offset(n_local), A.adaptive ? D.n_px.p : nullptr, (uint32_t)A.samples,
+                                n_local, A.frame.width, D.gain.p, D.px_gain.p, D.stream));
+    return RZ_OK;
 }
 
 // Everything device d does for this render, enqueued on its streams into what alloc_render allocated.
@@ -1189,7 +1222,8 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     const bool trace = n_local > 0 && (!P.list || dp.n_list > 0);   // a device with an empty list launches nothing
     RZ_CUDA(cudaSetDevice(D.id));
     RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
-    if (!(p->flags & RZ_RENDER_ACCUMULATE)) RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * 4u * sizeof(unsigned long long), D.stream));
+    if (!(p->flags & RZ_RENDER_ACCUMULATE))   // with the replicate sums behind them under RZ_RENDER_RQMC
+        RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * (P.next.rqmc ? 6u : 4u) * sizeof(unsigned long long), D.stream));
     if (adaptive && !P.list) RZ_CUDA(rz_launch_fill_u32(D.n_px.p, n_local, p->spp, D.stream));   // first round: every pixel
     RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
     RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
@@ -1394,13 +1428,15 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
         if ((rc = D.noise_part.alloc(4 * (size_t)G))) return rc;
+        const double *gain;
+        if ((rc = rqmc_gain(ctx, d, *A, sp.n_local[d], &gain))) return rc;
         if (out_err) {
             RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
             r.out_err = D0.out_err.p;
             RZ_CUDA(rz_launch_resolve(&r, D.stream));
         }
-        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A->adaptive ? D.n_px.p : nullptr, sp.n_local[d], (uint32_t)A->samples, (double)target,
-                                       D.noise_part.p, D.stream));
+        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A->adaptive ? D.n_px.p : nullptr, gain, sp.n_local[d], (uint32_t)A->samples,
+                                       (double)target, D.noise_part.p, D.stream));
     }
     double sum = 0, sum2 = 0, mx = 0;
     uint64_t above = 0;
@@ -1550,6 +1586,7 @@ extern "C" int rayz_cuda_denoise(RzContext *ctx, const RzDenoiseParams *dp, floa
     for (uint32_t d = 0; d < ND; d++) {
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
+        if (filter && (rc = rqmc_gain(ctx, d, *A, sp.n_local[d]))) return rc;
         RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
         r.out_linear = D0.dn_linear.p;
         if (filter) r.out_err = D0.dn_err.p;
@@ -1581,7 +1618,10 @@ static int build_pixel_lists(RzContext *ctx, uint32_t n_cur, uint32_t add, float
     for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {   // every device enqueues before the first wait
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(rz_launch_pixel_list(D.accum.p, D.n_px.p, sp.n_local[d], n_cur, add, target, D.px_list.p, D.list_scratch.p, D.stream));
+        const double *gain;
+        if (const int rc = rqmc_gain(ctx, d, ctx->acc, sp.n_local[d], &gain)) return rc;
+        RZ_CUDA(rz_launch_pixel_list(D.accum.p, gain, D.n_px.p, sp.n_local[d], n_cur, add, target, D.px_list.p,
+                                     D.list_scratch.p, D.stream));
         RZ_CUDA(cudaMemcpyAsync(&n_list[d], D.list_scratch.p + rz_list_count_word(sp.n_local[d]), sizeof(uint32_t), cudaMemcpyDeviceToHost, D.stream));
     }
     return sync_devices(ctx);
@@ -1596,6 +1636,8 @@ extern "C" int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, co
     const auto t0 = std::chrono::steady_clock::now();
     if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "render_to_noise: NULL argument");
     if (p->spp == 0 || max_spp < p->spp) return rz_fail(RZ_ERR_INVALID_ARG, "render_to_noise: need 0 < spp <= max_spp (spp %u, max_spp %u)", p->spp, max_spp);
+    if ((p->flags & RZ_RENDER_RQMC) && (max_spp & 1u))
+        return rz_fail(RZ_ERR_INVALID_ARG, "render_to_noise: RZ_RENDER_RQMC requires an even max_spp (two replicates)");
     RzRenderParams q = *p;
     q.flags = (p->flags & ~RZ_RENDER_ACCUMULATE) | RZ_RENDER_MOMENTS;
     RzNoise nz;

@@ -166,8 +166,18 @@ struct RzPathArgs {
     // covers list entries [tile * 32, tile * 32 + 32), and lane k's pixel is px_list[entry] instead of the entry itself.
     const uint32_t *px_list;     // local pixel indices in increasing order (rz_adaptive.cu)
     uint32_t n_list;             // entries in px_list
-    uint32_t sobol;              // != 0 (RZ_RENDER_SOBOL): the launchers run each kernel's SOBOL instance (rz_sampler.cuh's pairs)
+    uint32_t sobol;              // RZ_SAMPLER_* bits.  != 0 (RZ_RENDER_SOBOL): the launchers run each kernel's SOBOL instance
+                                 // (rz_sampler.cuh's pairs), with RZ_SAMPLER_RQMC its SOBOL = 2 instance
 };
+
+// RzPathArgs::sobol.  RZ_SAMPLER_RQMC (RZ_RENDER_RQMC) rides in the same word, so that the Philox instances see the very
+// arguments they saw before the flag existed; the launchers run the SOBOL = 2 instances for it (rz_pick_sampler): the replicate
+// mapping of rz_sobol_pair, and a sky path also adds its clamped luminance to its replicate's sum (rz_rep_offset).
+enum { RZ_SAMPLER_SOBOL = 1u, RZ_SAMPLER_RQMC = 2u };
+// RZ_RENDER_RQMC's replicate sums share the accumulators' allocation: [n_pad][4] accumulators, then [n_pad][2] replicate sums
+// (2^-32 fixed point, slot lp * 2 + (sample & 1)), n_pad = n_local_px rounded up to whole warps.  This is the offset, in words,
+// of the replicate sums.
+RZ_HD size_t rz_rep_offset(uint32_t n_local_px) { return (size_t)((n_local_px + 31u) / 32u) * 32u * 4u; }
 
 // Guide buffers (rayz_cuda_render_guides, rz_guides_kernel in rz_bvh_trace.cu): the camera segments of a render with these
 // RzPathArgs, each followed to its first hit only.  The outputs are the gather root's buffers at the context's rows (peer
@@ -198,9 +208,11 @@ RZ_HD unsigned long long rz_fixed32(float v) {
     return (unsigned long long)nearbyint((double)(v * 4294967296.f));
 #endif
 }
-// Y^2 of a path's clamped radiance, clamped like the colour channels; the FMAs are explicit so host and device agree bit for bit
+// Y of a path's clamped radiance; the FMAs are explicit so host and device agree bit for bit
+RZ_HD float rz_luma(float r, float g, float b) { return fmaf(0.0722f, b, fmaf(0.7152f, g, 0.2126f * r)); }
+// Y^2 of a path's clamped radiance, clamped like the colour channels
 RZ_HD float rz_luma_sq(float r, float g, float b) {
-    const float y = fmaf(0.0722f, b, fmaf(0.7152f, g, 0.2126f * r));
+    const float y = rz_luma(r, g, b);
     return rz_clamp_radiance(y * y);
 }
 
@@ -214,6 +226,45 @@ RZ_HD double rz_pixel_err(unsigned long long q0, unsigned long long q1, unsigned
     const double y = (0.2126 * (double)q0 + 0.7152 * (double)q1 + 0.0722 * (double)q2) * s * inv;
     const double s2 = fmax(0.0, (double)q3 * s * inv - y * y) * ((double)n / (double)(n - 1u));
     return sqrt(s2 * inv) / (2.0 * sqrt(fmax(y, RZ_NOISE_Y_FLOOR)));
+}
+
+// RZ_RENDER_RQMC (include/rayz_cuda.h, DESIGN.md "The RQMC estimate"): the error of the iid formula above, scaled by the
+// segment's pooled ratio of the two replicates' spread to the iid variance, as it was when the pixel's count was last the frame's
+// largest (an adaptive pixel keeps the gain its stopping test read).  A segment is RZ_RQMC_SEGMENT pixels of one row (the
+// last of a row may be shorter); local rows are whole global rows, so local pixel lp's segment is a function of (row, x).
+#define RZ_RQMC_SEGMENT 64u
+RZ_HD uint32_t rz_rqmc_segments(uint32_t width) { return (width + RZ_RQMC_SEGMENT - 1u) / RZ_RQMC_SEGMENT; }
+// index of local pixel lp's segment in a [local rows][rz_rqmc_segments(width)] buffer
+RZ_HD size_t rz_rqmc_segment_of(uint32_t lp, uint32_t width) {
+    const uint32_t lr = lp / width;
+    return (size_t)lr * rz_rqmc_segments(width) + (lp - lr * width) / RZ_RQMC_SEGMENT;
+}
+// V_iid = s^2 / n with rz_pixel_err's s^2; 0 while n < 2
+RZ_HD double rz_pixel_var_iid(unsigned long long q0, unsigned long long q1, unsigned long long q2, unsigned long long q3, uint32_t n) {
+    if (n < 2u) return 0.0;
+    const double s = 2.3283064365386962890625e-10, inv = 1.0 / (double)n;   // 2^-32
+    const double y = (0.2126 * (double)q0 + 0.7152 * (double)q1 + 0.0722 * (double)q2) * s * inv;
+    return fmax(0.0, (double)q3 * s * inv - y * y) * ((double)n / (double)(n - 1u)) * inv;
+}
+// V_rep = (mu_0 - mu_1)^2 / 4, mu_r = r_r 2^-32 / (n / 2): the R = 2 replicate variance of the pixel mean; 0 while n < 2
+RZ_HD double rz_pixel_var_rep(unsigned long long r0, unsigned long long r1, uint32_t n) {
+    if (n < 2u) return 0.0;
+    const double inv_m = 2.3283064365386962890625e-10 / (double)(n / 2u);
+    const double d = (double)r0 * inv_m - (double)r1 * inv_m;
+    return 0.25 * d * d;
+}
+// G of a segment from its sums of V_rep and V_iid: not clamped; 1 when there is no iid variance to scale
+RZ_HD double rz_rqmc_gain(double sum_rep, double sum_iid) { return sum_iid > 0.0 ? sum_rep / sum_iid : 1.0; }
+// e = rz_pixel_err * sqrt(G); +inf while n < 2, as rz_pixel_err
+RZ_HD double rz_pixel_err_rqmc(unsigned long long q0, unsigned long long q1, unsigned long long q2, unsigned long long q3, uint32_t n,
+                               double gain) {
+    if (n < 2u) return INFINITY;
+    return rz_pixel_err(q0, q1, q2, q3, n) * sqrt(gain);
+}
+// the error a consumer shows: rz_pixel_err, or under RZ_RENDER_RQMC (gain != null: one gain per local pixel, rz_rqmc_gain_kernel)
+// rz_pixel_err_rqmc with local pixel lp's gain
+RZ_HD double rz_pixel_err_of(const unsigned long long *q, uint32_t n, const double *gain, uint32_t lp) {
+    return gain ? rz_pixel_err_rqmc(q[0], q[1], q[2], q[3], n, gain[lp]) : rz_pixel_err(q[0], q[1], q[2], q[3], n);
 }
 
 // writePPM's per-pixel transform (image.zig:35-38) in f64, as the resolve and the denoiser's finish kernel apply it:
@@ -404,13 +455,13 @@ RZ_HD RzRay rz_lens_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, float ux,
 
 // One Philox block gives the five uniforms: 4 x 24 high bits + 3 x 8 low bits.  With `sobol` (RZ_RENDER_SOBOL; the kernels pass
 // their SOBOL template argument) three Sobol pairs give them instead (rz_sampler.cuh): jitter, lens (radius, angle) and the
-// shutter time (first coordinate of the third pair).
+// shutter time (first coordinate of the third pair); `rqmc` (the SOBOL = 2 instances) draws them from the sample's replicate.
 RZ_HD RzRay rz_camera_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, uint32_t gpix, uint32_t sample,
-                          uint32_t k0, uint32_t k1, bool sobol = false) {
+                          uint32_t k0, uint32_t k1, bool sobol = false, bool rqmc = false) {
     if (sobol) {
-        const float2 j = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_JITTER, sample);
-        const float2 l = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_LENS, sample);
-        const float t = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_TIME, sample).x;
+        const float2 j = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_JITTER, sample, rqmc);
+        const float2 l = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_LENS, sample, rqmc);
+        const float t = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_TIME, sample, rqmc).x;
         return rz_lens_ray(cam, px, py, j.x, j.y, t, l.x, l.y);
     }
     const uint4 r = rz_philox(gpix, sample, 0u, 0u, k0, k1);

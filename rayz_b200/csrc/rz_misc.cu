@@ -24,6 +24,7 @@ struct RzResolveArgs {
     float *out_err;                   // nullable: displayed-value standard error per pixel (needs slot 3, RZ_RENDER_MOMENTS)
     uint32_t *out_spp;                // nullable: the pixel's sample count (rayz_cuda_pixel_samples)
     const uint32_t *n_px;             // nullable: per-pixel sample counts of an adaptive frame (rz_adaptive.cu); null: spp
+    const double *gain;               // nullable: RZ_RENDER_RQMC's per-pixel gains (rz_rqmc_gain_kernel); out_err is then rz_pixel_err_rqmc
     uint32_t n_local_px, width;
     uint32_t spp;                     // samples summed in the accumulators (cumulative over RZ_RENDER_ACCUMULATE batches)
     // local row lr of this device -> destination row ((lr / band) * dev_count + dev_index) * band + lr % band
@@ -43,7 +44,10 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
     }
     const uint32_t n = a.n_px ? a.n_px[lp] : a.spp;
     if (a.out_spp) a.out_spp[dst] = n;
-    if (a.out_err) a.out_err[dst] = (float)rz_pixel_err(q0.x, q0.y, q1, a.accum[(size_t)lp * 4 + 3], n);
+    if (a.out_err) {
+        const unsigned long long q3 = a.accum[(size_t)lp * 4 + 3];
+        a.out_err[dst] = (float)(a.gain ? rz_pixel_err_rqmc(q0.x, q0.y, q1, q3, n, a.gain[lp]) : rz_pixel_err(q0.x, q0.y, q1, q3, n));
+    }
     const double inv = 1.0 / (double)n;
     const double s = 2.3283064365386962890625e-10;  // 2^-32
     const double r = (double)q0.x * s * inv, g = (double)q0.y * s * inv, b = (double)q1 * s * inv;
@@ -65,16 +69,17 @@ extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t st
 #define RZ_NOISE_GRID 256
 struct RzNoisePartial { double sum, sum2, max; unsigned long long above; };
 
-// n_px (nullable): per-pixel sample counts of an adaptive frame, else every pixel has n samples.
+// n_px (nullable): per-pixel sample counts of an adaptive frame, else every pixel has n samples.  gain (nullable): RZ_RENDER_RQMC's
+// per-pixel gains.
 __global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned long long *__restrict__ accum, const uint32_t *__restrict__ n_px,
-                                                              uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *__restrict__ out) {
+                                                              const double *__restrict__ gain, uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *__restrict__ out) {
     __shared__ double s_sum[256], s_sum2[256], s_max[256];
     __shared__ unsigned long long s_above[256];
     double sum = 0, sum2 = 0, mx = 0;
     unsigned long long above = 0;
     for (uint32_t lp = blockIdx.x * 256u + threadIdx.x; lp < n_local_px; lp += RZ_NOISE_GRID * 256u) {
         const unsigned long long *q = accum + (size_t)lp * 4;
-        const double e = (double)(float)rz_pixel_err(q[0], q[1], q[2], q[3], n_px ? n_px[lp] : n);   // the value out_err shows
+        const double e = (double)(float)rz_pixel_err_of(q, n_px ? n_px[lp] : n, gain, lp);   // the value out_err shows
         sum += e; sum2 += e * e; mx = fmax(mx, e); above += e > target ? 1u : 0u;
     }
     s_sum[threadIdx.x] = sum; s_sum2[threadIdx.x] = sum2; s_max[threadIdx.x] = mx; s_above[threadIdx.x] = above;
@@ -91,9 +96,53 @@ __global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned lon
 
 extern "C" uint32_t rz_noise_grid(void) { return RZ_NOISE_GRID; }
 // out: RZ_NOISE_GRID x 4 words (sum, sum2, max as doubles, then the count as an integer)
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, uint32_t n_local_px, uint32_t n,
-                                              double target, void *out, cudaStream_t stream) {
-    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, n_local_px, n, target, (RzNoisePartial *)out);
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain,
+                                              uint32_t n_local_px, uint32_t n, double target, void *out, cudaStream_t stream) {
+    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, gain, n_local_px, n, target, (RzNoisePartial *)out);
+    return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------
+// RZ_RENDER_RQMC: the gain G of every segment of the device's local rows (rz_rqmc_gain of the segment's sums of V_rep and V_iid),
+// into seg_gain[row][rz_rqmc_segments(width)], and into px_gain[lp] for every pixel whose count is n, the frame's largest: every
+// pixel of a uniform frame; of an adaptive one, the pixels the next stopping test reads.  A pixel that stopped keeps the gain its
+// test read, so its error stays what the test saw while its segment's other pixels take more samples.  One warp per segment:
+// lane k adds its pixels x0 + k, x0 + k + 32 in that order, then a fixed xor tree that leaves the sums in every lane; no
+// floating-point atomics, so the gain is a function of the segment's sums only, wherever the row renders.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(128) rz_rqmc_gain_kernel(const unsigned long long *__restrict__ accum, const unsigned long long *__restrict__ rep,
+                                                           const uint32_t *__restrict__ n_px, uint32_t n, uint32_t n_local_px, uint32_t width,
+                                                           double *__restrict__ seg_gain, double *__restrict__ px_gain) {
+    const uint32_t nseg = rz_rqmc_segments(width), rows = n_local_px / width;
+    const uint32_t seg = blockIdx.x * 4u + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
+    if (seg >= rows * nseg) return;   // the whole warp
+    const uint32_t lr = seg / nseg, x0 = (seg - lr * nseg) * RZ_RQMC_SEGMENT, x1 = min(x0 + RZ_RQMC_SEGMENT, width);
+    double v_rep = 0.0, v_iid = 0.0;
+    for (uint32_t x = x0 + lane; x < x1; x += 32u) {
+        const uint32_t lp = lr * width + x, c = n_px ? n_px[lp] : n;
+        const unsigned long long *q = accum + (size_t)lp * 4;
+        v_rep += rz_pixel_var_rep(rep[(size_t)lp * 2], rep[(size_t)lp * 2 + 1], c);
+        v_iid += rz_pixel_var_iid(q[0], q[1], q[2], q[3], c);
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        v_rep += __shfl_xor_sync(0xffffffffu, v_rep, o);
+        v_iid += __shfl_xor_sync(0xffffffffu, v_iid, o);
+    }
+    const double g = rz_rqmc_gain(v_rep, v_iid);
+    if (lane == 0) seg_gain[seg] = g;
+    for (uint32_t x = x0 + lane; x < x1; x += 32u) {
+        const uint32_t lp = lr * width + x;
+        if (!n_px || n_px[lp] == n) px_gain[lp] = g;
+    }
+}
+
+// Doubles of the segment-gain buffer for n_local_px pixels in rows of `width` (px_gain: n_local_px doubles).
+extern "C" size_t rz_rqmc_gain_words(uint32_t n_local_px, uint32_t width) { return width ? (size_t)(n_local_px / width) * rz_rqmc_segments(width) : 0; }
+extern "C" cudaError_t rz_launch_rqmc_gain(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
+                                           uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, cudaStream_t stream) {
+    const size_t segs = rz_rqmc_gain_words(n_local_px, width);
+    if (segs == 0) return cudaSuccess;
+    rz_rqmc_gain_kernel<<<(unsigned)((segs + 3) / 4), 128, 0, stream>>>(accum, rep, n_px, n, n_local_px, width, seg_gain, px_gain);
     return cudaGetLastError();
 }
 

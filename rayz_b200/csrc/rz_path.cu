@@ -63,7 +63,7 @@ struct RzStream {
 
 // G = sphere PAIRS per search-loop iteration
 // LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list)
-template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false, bool SOBOL = false>
+template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false, int SOBOL = 0>
 __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -142,7 +142,7 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
                             st[r].lp = lp;
                             st[r].gpix = pj * a.width + pi;
                             st[r].sample = a.sample_offset + unit_s0 + (k >> 5);
-                            st[r].ray = rz_camera_ray(a.cam, pi, pj, st[r].gpix, st[r].sample, a.seed_lo, a.seed_hi, SOBOL);
+                            st[r].ray = rz_camera_ray(a.cam, pi, pj, st[r].gpix, st[r].sample, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
                             st[r].thr = f3(1.f, 1.f, 1.f);
                             st[r].seg = 0;
                             st[r].alive = a.max_depth > 0u;
@@ -177,7 +177,7 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
             if (!st[r].alive) continue;
             if (STATS) { c_segs++; c_sph += a.set.n; }   // brute force: every sphere of the set
             uint32_t kind;
-            const int res = rz_shade_segment(a, st[r].ray, st[r].thr, st[r].seg, st[r].lp, st[r].gpix, st[r].sample, bk[r], kind, SOBOL);
+            const int res = rz_shade_segment(a, st[r].ray, st[r].thr, st[r].seg, st[r].lp, st[r].gpix, st[r].sample, bk[r], kind, SOBOL != 0, SOBOL == 2);
             if (STATS) {
                 if (kind < 3u) c_hit[kind]++;
                 if (res == RZ_END_SKY) c_sky++;
@@ -229,7 +229,7 @@ struct RzSegCounters {
 };
 
 // Shade the two rays of a lane after the search and append the survivors (with their sort keys) to the next queue.
-template <bool STATS, bool SOBOL>
+template <bool STATS, int SOBOL>
 __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRay (&L)[2], unsigned lane, unsigned lt_mask, RzSegCounters &C) {
 #pragma unroll 1
     for (int trip = 0; trip < 2; trip++) {
@@ -238,7 +238,7 @@ __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRa
         if (Q.live) {
             if (STATS) C.segs++;
             uint32_t kind;
-            const int res = rz_shade_segment(a, Q.ray, Q.thr, Q.seg, Q.lp, Q.gpix, Q.smp, Q.bk, kind, SOBOL);
+            const int res = rz_shade_segment(a, Q.ray, Q.thr, Q.seg, Q.lp, Q.gpix, Q.smp, Q.bk, kind, SOBOL != 0, SOBOL == 2);
             if (STATS) {
                 if (kind < 3u) C.hit[kind]++;
                 if (res == RZ_END_SKY) C.sky++;
@@ -302,7 +302,7 @@ __device__ __forceinline__ void rz_flush_counters(const RzPathArgs &a, const RzS
 // Paths that scatter are appended, ballot-compacted, to the HBM queue the sorted stages start from; paths
 // that leave the scene or are absorbed accumulate here.  36 % of all segments are camera segments.  The cull
 // (rz_tile_cone / rz_tile_keep, rz_device.cuh) is host + device and property-tested on the CPU.
-template <bool STATS, bool SOBOL = false>
+template <bool STATS, int SOBOL = 0>
 __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -369,7 +369,7 @@ __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
                 const bool have = valid && (s + (uint32_t)trip < ns);
                 Q.live = have && a.max_depth > 0u;
                 if (STATS && have) { C.paths++; if (!Q.live) C.depth++; }
-                if (Q.live) Q.ray = rz_camera_ray(a.cam, pi, pj, gpix, Q.smp, a.seed_lo, a.seed_hi, SOBOL);
+                if (Q.live) Q.ray = rz_camera_ray(a.cam, pi, pj, gpix, Q.smp, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
                 else { Q.ray.o = f3(0.f, 0.f, 0.f); Q.ray.d = f3(0.f, 1.f, 0.f); Q.ray.time = 0.f; Q.ray.self_k = -1; }
                 Q.thr = f3(1.f, 1.f, 1.f); Q.seg = 0u; Q.lp = lp; Q.gpix = gpix; Q.bk = -1; Q.cont = false; Q.key = 0u;
                 if (trip == 0) L[1] = L[0];   // slot 0 is rewritten by the second trip
@@ -474,7 +474,7 @@ __global__ void __launch_bounds__(128) rz_bin_lists_kernel(const RzPathArgs a) {
 // Round 1 sorted on all 16 key bits (two radix passes) and culled each unit with its largest reach; ordering by reach
 // inside the unit costs one global pass less and culls every batch with its OWN reach.  The cull functions are host +
 // device and property-tested on the CPU (tests/test_hostsim_cpu.py).
-template <bool STATS, bool SOBOL = false>
+template <bool STATS, int SOBOL = 0>
 __global__ void RZ_SECOND_BOUNDS rz_second_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -611,7 +611,7 @@ __global__ void RZ_SECOND_BOUNDS rz_second_kernel(const RzPathArgs a) {
 // ------------------------------------------------------------------------------ launchers
 template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false>
 static cudaError_t rz_launch_one(const RzPathArgs &a, int sm_count, size_t smem, cudaStream_t stream, int *grid_out) {
-    auto kern = rz_pick_sampler(a, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, false>, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, true>);
+    auto kern = rz_pick_sampler(a, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, 0>, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, 1>, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, 2>);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int per_sm = 0;
@@ -661,8 +661,8 @@ extern "C" cudaError_t rz_launch_primary(const RzPathArgs *a, int collect_stats,
         kern<<<grid, 128, smem, stream>>>(*a);
         return cudaGetLastError();
     };
-    return collect_stats ? launch(rz_pick_sampler(*a, rz_primary_kernel<true, false>, rz_primary_kernel<true, true>))
-                         : launch(rz_pick_sampler(*a, rz_primary_kernel<false, false>, rz_primary_kernel<false, true>));
+    return collect_stats ? launch(rz_pick_sampler(*a, rz_primary_kernel<true, 0>, rz_primary_kernel<true, 1>, rz_primary_kernel<true, 2>))
+                         : launch(rz_pick_sampler(*a, rz_primary_kernel<false, 0>, rz_primary_kernel<false, 1>, rz_primary_kernel<false, 2>));
 }
 
 // Per-group pair lists of the sorted-segment kernel (a->bin_lists: RZ_SORT_BINS rows of a->bin_row bytes).
@@ -687,8 +687,8 @@ extern "C" cudaError_t rz_second_grid(const RzPathArgs *a, int collect_stats, in
         *grid = sm_count * per_sm;
         return cudaSuccess;
     };
-    return collect_stats ? query(rz_pick_sampler(*a, rz_second_kernel<true, false>, rz_second_kernel<true, true>))
-                         : query(rz_pick_sampler(*a, rz_second_kernel<false, false>, rz_second_kernel<false, true>));
+    return collect_stats ? query(rz_pick_sampler(*a, rz_second_kernel<true, 0>, rz_second_kernel<true, 1>, rz_second_kernel<true, 2>))
+                         : query(rz_pick_sampler(*a, rz_second_kernel<false, 0>, rz_second_kernel<false, 1>, rz_second_kernel<false, 2>));
 }
 
 // Stage 2: second segments of the sorted queue (q_in through q_in_idx) -> q_out.
@@ -704,8 +704,8 @@ extern "C" cudaError_t rz_launch_second(const RzPathArgs *a, int collect_stats, 
         kern<<<sm_count * per_sm, 128, smem, stream>>>(*a);
         return cudaGetLastError();
     };
-    return collect_stats ? launch(rz_pick_sampler(*a, rz_second_kernel<true, false>, rz_second_kernel<true, true>))
-                         : launch(rz_pick_sampler(*a, rz_second_kernel<false, false>, rz_second_kernel<false, true>));
+    return collect_stats ? launch(rz_pick_sampler(*a, rz_second_kernel<true, 0>, rz_second_kernel<true, 1>, rz_second_kernel<true, 2>))
+                         : launch(rz_pick_sampler(*a, rz_second_kernel<false, 0>, rz_second_kernel<false, 1>, rz_second_kernel<false, 2>));
 }
 
 // Last stage (q_in != nullptr): the persistent megakernel started from a queue; or the single-stage form

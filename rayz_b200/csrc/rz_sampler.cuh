@@ -75,15 +75,23 @@ RZ_HD uint32_t rz_sobol_pair_seed(uint32_t k0, uint32_t k1, uint32_t gpix, uint3
     return rz_hash32(h ^ pair);
 }
 
+// RZ_RENDER_RQMC: the base seed of replicate r (0 or 1) of a pair, from the pair's own base seed
+RZ_HD uint32_t rz_rqmc_replicate_seed(uint32_t base, uint32_t r) { return rz_hash32(base ^ (0x9e3779b9u + r)); }
+
 // The 32-bit coordinates of sample `sample` of `pair` for pixel gpix (callers keep the top 24 bits: rz_u01(x >> 8)).
-RZ_HD uint2 rz_sobol_pair(uint32_t k0, uint32_t k1, uint32_t gpix, uint32_t pair, uint32_t sample) {
-    const uint32_t base = rz_sobol_pair_seed(k0, k1, gpix, pair);
+// `rqmc` (RZ_RENDER_RQMC): sample i is sample i >> 1 of replicate i & 1, a sequence of its own (rz_rqmc_replicate_seed).
+RZ_HD uint2 rz_sobol_pair(uint32_t k0, uint32_t k1, uint32_t gpix, uint32_t pair, uint32_t sample, bool rqmc = false) {
+    uint32_t base = rz_sobol_pair_seed(k0, k1, gpix, pair);
+    if (rqmc) {
+        base = rz_rqmc_replicate_seed(base, sample & 1u);
+        sample >>= 1;
+    }
     const uint32_t i = rz_owen_scramble(sample, rz_hash32(base));
     return make_uint2(rz_owen_scramble(rz_sobol_d0(i), rz_hash32(base ^ 1u)), rz_owen_scramble(rz_sobol_d1(i), rz_hash32(base ^ 2u)));
 }
 
 // The pair's two uniforms: rz_u01 of the top 24 bits of each coordinate.
-RZ_HD float2 rz_sobol_u01(uint32_t k0, uint32_t k1, uint32_t gpix, uint32_t pair, uint32_t sample) {
-    const uint2 q = rz_sobol_pair(k0, k1, gpix, pair, sample);
+RZ_HD float2 rz_sobol_u01(uint32_t k0, uint32_t k1, uint32_t gpix, uint32_t pair, uint32_t sample, bool rqmc = false) {
+    const uint2 q = rz_sobol_pair(k0, k1, gpix, pair, sample, rqmc);
     return make_float2(rz_u01(q.x >> 8), rz_u01(q.y >> 8));
 }

@@ -319,19 +319,25 @@ __device__ __forceinline__ const float4 *rz_stage_scene_cv(const RzSphereSet &se
 }
 
 // ------------------------------------------------------------------------------ shade
-// Every path kernel has a SOBOL template parameter (RZ_RENDER_SOBOL): the launchers pick the instance from RzPathArgs::sobol.
+// Every path kernel has a SOBOL template parameter (RZ_RENDER_SOBOL, RZ_RENDER_RQMC): the launchers pick the instance from
+// RzPathArgs::sobol.
 // A runtime branch on the field instead raised the registers or spills of the Philox instances (DESIGN.md "Low-discrepancy
 // sampling"), which are the default and the benchmark.
+// SOBOL = 0 is Philox, 1 Sobol, 2 Sobol with RZ_RENDER_RQMC's replicates and sums: a third instance, because the RQMC code read
+// as a uniform bit inside the Sobol instances cost plain Sobol 2 to 4 % of its Mpaths/s.
 template <class K>
-static inline K rz_pick_sampler(const RzPathArgs &a, K philox, K sobol) { return a.sobol ? sobol : philox; }
+static inline K rz_pick_sampler(const RzPathArgs &a, K philox, K sobol, K rqmc) {
+    return (a.sobol & RZ_SAMPLER_RQMC) ? rqmc : a.sobol ? sobol : philox;
+}
 
 enum { RZ_CONT = 0, RZ_END_SKY = 1, RZ_END_ABSORBED = 2, RZ_END_DEPTH = 3 };
 
 // One step of bounceRay (renderer.zig:103-126) after the closest-hit query: miss -> sky and
 // accumulate; hit -> refine in f64, scatter, attenuate.  `kind_out` = material kind of the hit.  `sobol`: the kernel's SOBOL
-// template argument (RZ_RENDER_SOBOL), a compile-time constant, so that the Philox instances carry no trace of the other sampler.
+// template argument (RZ_RENDER_SOBOL), a compile-time constant, so that the Philox instances carry no trace of the other sampler;
+// `rqmc`: the SOBOL = 2 instances' (RZ_RENDER_RQMC), compile-time as well.
 __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray, float3 &thr, uint32_t &seg, uint32_t lp,
-                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, bool sobol) {
+                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, bool sobol, bool rqmc) {
     kind_out = 3u;
     if (bk < 0) {
         // miss: background (renderer.zig:124-125), path ends
@@ -342,6 +348,10 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
         atomicAdd(acc + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.f), 1048576.f) * 4294967296.f));
         // the noise estimate's second moment (the only accumulation site besides the three above: every kernel shades here)
         if (a.moments) atomicAdd(acc + 3, rz_fixed32(rz_luma_sq(rz_clamp_radiance(L.x), rz_clamp_radiance(L.y), rz_clamp_radiance(L.z))));
+        // RZ_RENDER_RQMC: the replicate's luminance sum (rz_pixel_err_rqmc)
+        if (rqmc)
+            atomicAdd(a.accum + rz_rep_offset(a.n_local_px) + (size_t)lp * 2u + (sample & 1u),
+                      rz_fixed32(rz_clamp_radiance(rz_luma(rz_clamp_radiance(L.x), rz_clamp_radiance(L.y), rz_clamp_radiance(L.z)))));
         return RZ_END_SKY;
     }
     const int k = bk & ~RZ_FAR_BIT;
@@ -359,7 +369,7 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
     kind_out = kind < 3u ? kind : 0u;
     seg++;
     const uint4 rb = rz_philox(gpix, sample, seg, 0u, a.seed_lo, a.seed_hi);
-    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(seg), sample)   // u.z, u.w stay Philox
+    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(seg), sample, rqmc)   // u.z, u.w stay Philox
                            : make_float2(rz_u01(rb.x >> 8), rz_u01(rb.y >> 8));
     const float4 u = make_float4(q.x, q.y, rz_u01(rb.z >> 8), rz_u01(rb.w >> 8));
     float3 att;

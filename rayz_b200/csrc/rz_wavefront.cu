@@ -72,7 +72,7 @@ __device__ __forceinline__ void wf_decode(const RzPathArgs &a, unsigned long lon
     sample = r >> 5;
 }
 
-template <bool STATS, bool SOBOL>
+template <bool STATS, int SOBOL>
 __global__ void __launch_bounds__(256) wf_generate(const RzPathArgs a, WfState s) {
     const WfCounters c = *s.ctr;
     const unsigned long long remaining = c.total_paths - c.next_path;
@@ -90,7 +90,7 @@ __global__ void __launch_bounds__(256) wf_generate(const RzPathArgs a, WfState s
             uint32_t pi, pj;
             rz_local_to_global(lp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
             d.y = pj * a.width + pi;
-            const RzRay ray = rz_camera_ray(a.cam, pi, pj, d.y, d.z, a.seed_lo, a.seed_hi, SOBOL);
+            const RzRay ray = rz_camera_ray(a.cam, pi, pj, d.y, d.z, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
             A = make_float4(ray.o.x, ray.o.y, ray.o.z, ray.time);
             B = make_float4(ray.d.x, ray.d.y, ray.d.z, __int_as_float(ray.self_k));
             C = make_float4(1.f, 1.f, 1.f, __uint_as_float(0u));
@@ -195,7 +195,7 @@ __global__ void wf_after_intersect(WfState s) {
     c->q_total = off;
 }
 
-template <bool STATS, bool SOBOL>
+template <bool STATS, int SOBOL>
 __global__ void __launch_bounds__(256) wf_shade(const RzPathArgs a, WfState s) {
     const WfCounters c = *s.ctr;
     const unsigned int M = s.M;
@@ -223,7 +223,7 @@ __global__ void __launch_bounds__(256) wf_shade(const RzPathArgs a, WfState s) {
             if (doa) { res = RZ_END_DEPTH; kind = 3u; }
             else {
                 if (STATS) c_segs++;
-                res = rz_shade_segment(a, ray, thr, seg, D.x, D.y, D.z, (int)D.w, kind, SOBOL);
+                res = rz_shade_segment(a, ray, thr, seg, D.x, D.y, D.z, (int)D.w, kind, SOBOL != 0, SOBOL == 2);
                 if (STATS) {
                     if (kind < 3u) c_hit[kind]++;
                     if (res == RZ_END_SKY) c_sky++;
@@ -327,11 +327,11 @@ extern "C" cudaError_t rz_wavefront_render(const RzPathArgs *a, int sm_count, in
         cudaGraph_t g;
         if ((e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal)) != cudaSuccess) return e;
         for (int it = 0; it < ITERS; it++) {
-            (st ? rz_pick_sampler(*a, wf_generate<true, false>, wf_generate<true, true>) : rz_pick_sampler(*a, wf_generate<false, false>, wf_generate<false, true>))<<<grid_s, 256, 0, cap>>>(*a, ws->st);
+            (st ? rz_pick_sampler(*a, wf_generate<true, 0>, wf_generate<true, 1>, wf_generate<true, 2>) : rz_pick_sampler(*a, wf_generate<false, 0>, wf_generate<false, 1>, wf_generate<false, 2>))<<<grid_s, 256, 0, cap>>>(*a, ws->st);
             wf_after_generate<<<1, 1, 0, cap>>>(ws->st);
             wf_intersect<2><<<grid_i, 128, smem, cap>>>(*a, ws->st);
             wf_after_intersect<<<1, 1, 0, cap>>>(ws->st);
-            (st ? rz_pick_sampler(*a, wf_shade<true, false>, wf_shade<true, true>) : rz_pick_sampler(*a, wf_shade<false, false>, wf_shade<false, true>))<<<grid_s, 256, 0, cap>>>(*a, ws->st);
+            (st ? rz_pick_sampler(*a, wf_shade<true, 0>, wf_shade<true, 1>, wf_shade<true, 2>) : rz_pick_sampler(*a, wf_shade<false, 0>, wf_shade<false, 1>, wf_shade<false, 2>))<<<grid_s, 256, 0, cap>>>(*a, ws->st);
             wf_advance<<<1, 1, 0, cap>>>(ws->st);
         }
         cudaMemcpyAsync(ws->h_done, &ws->st.ctr->done, sizeof(unsigned int), cudaMemcpyDeviceToHost, cap);

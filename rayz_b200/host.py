@@ -278,10 +278,13 @@ class Backend:
     @staticmethod
     def params(width, height, spp, max_depth=50, seed=1, sample_offset=0, variant="auto", t_min=0.0, shard_index=0,
                shard_count=1, band_rows=0, collect_stats=False, serial_passes=False, accumulate=False,
-               moments=False, sobol=False) -> abi.RzRenderParams:
+               moments=False, sobol=False, rqmc=False) -> abi.RzRenderParams:
         """RzRenderParams.  accumulate: add this batch to the previous render's sums (RZ_RENDER_ACCUMULATE; sample_offset must
         continue where they end); moments: also sum each path's luminance squared, so that noise() can estimate the error;
-        sobol: draw the camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox (RZ_RENDER_SOBOL)."""
+        sobol: draw the camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox (RZ_RENDER_SOBOL);
+        rqmc: two independently scrambled Sobol replicates per pixel, so that the noise estimate sees the stratification
+        (RZ_RENDER_RQMC).  rqmc does not imply sobol or moments: the library refuses it without both, and with an odd spp or
+        sample_offset."""
         p = abi.RzRenderParams()
         p.width, p.height, p.spp, p.max_depth = width, height, spp, max_depth
         p.seed, p.sample_offset = seed, sample_offset
@@ -290,7 +293,7 @@ class Backend:
         p.shard_index, p.shard_count, p.band_rows = shard_index, shard_count, band_rows
         p.collect_stats = 1 if collect_stats else 0
         p.flags = ((abi.RENDER_SERIAL_PASSES if serial_passes else 0) | (abi.RENDER_ACCUMULATE if accumulate else 0)
-                   | (abi.RENDER_MOMENTS if moments else 0) | (abi.RENDER_SOBOL if sobol else 0))
+                   | (abi.RENDER_MOMENTS if moments else 0) | (abi.RENDER_SOBOL if sobol else 0) | (abi.RENDER_RQMC if rqmc else 0))
         return p
 
     def reserve(self, p: abi.RzRenderParams):
@@ -450,7 +453,8 @@ class Tracer:
         self.seed = seed           # the reference seeds from the OS (renderer.zig:55-59)
         self.variant = "auto"
         self.sampler = "philox"    # or "sobol": low-discrepancy camera and scatter samples (RZ_RENDER_SOBOL) in render(),
-                                   # render_guides() and so the denoised frame
+                                   # render_guides() and so the denoised frame; or "sobol-rqmc": the same with two replicates
+                                   # per pixel and the noise estimate they allow (RZ_RENDER_RQMC, with moments)
         self.devices = devices
         self.noise = None          # summary of the last render(noise_target=...) (rayz_cuda_render_to_noise)
         self.pixel_samples = None  # [h, w] per-pixel sample counts of the last render(noise_target=..., adaptive=True)
@@ -460,10 +464,13 @@ class Tracer:
         self._backend = None
         self._uploaded = None      # the pool arrays of the backend's last scene upload
 
-    def _sobol(self) -> bool:
-        if self.sampler not in ("philox", "sobol"):
-            raise ValueError(f"Tracer.sampler must be 'philox' or 'sobol', not {self.sampler!r}")
-        return self.sampler == "sobol"
+    SAMPLERS = {"philox": {}, "sobol": {"sobol": True}, "sobol-rqmc": {"sobol": True, "rqmc": True, "moments": True}}
+
+    def _sampler(self) -> dict:
+        """Backend.params keywords of self.sampler."""
+        if self.sampler not in self.SAMPLERS:
+            raise ValueError(f"Tracer.sampler must be 'philox', 'sobol' or 'sobol-rqmc', not {self.sampler!r}")
+        return dict(self.SAMPLERS[self.sampler])
 
     @property
     def backend(self) -> Backend:
@@ -482,8 +489,9 @@ class Tracer:
         self._uploaded = None
         b.upload_scene(arrays)  # initHittables + bvh.build (renderer.zig:76-78)
         self._uploaded = arrays
-        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
-                           moments=moments, sobol=self._sobol())
+        kw = self._sampler()
+        kw["moments"] = moments or kw.get("moments", False)
+        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant, **kw)
         if noise_target is None:
             lin, rgb8, rays = b.render(self.camera.rz, p)
         else:
@@ -509,7 +517,7 @@ class Tracer:
             b.upload_scene(arrays)
             self._uploaded = arrays
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
-                           sobol=self._sobol())
+                           **self._sampler())
         self.albedo, self.normal = b.guides(self.camera.rz, p)
         return self.albedo, self.normal
 

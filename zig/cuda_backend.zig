@@ -75,6 +75,7 @@ pub const RZ_RENDER_MOMENTS: u32 = 2; // sum each path's luminance squared: rayz
 pub const RZ_RENDER_ACCUMULATE: u32 = 4; // add this batch to the previous render's sums (progressive rendering)
 pub const RZ_RENDER_ADAPTIVE: u32 = 8; // rayz_cuda_render_to_noise: the target bounds every pixel, only pixels above it get more samples
 pub const RZ_RENDER_SOBOL: u32 = 0x10; // camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox
+pub const RZ_RENDER_RQMC: u32 = 0x20; // with SOBOL and MOMENTS: two scrambled replicates per pixel, a noise estimate that sees the stratification
 
 pub const RzNoise = extern struct {
     samples: u64,
