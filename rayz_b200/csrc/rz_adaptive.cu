@@ -8,6 +8,7 @@
 //   scan    : one CTA turns the block counts into block offsets and writes the list length;
 //   scatter : every active pixel goes to its place in the list, and its count grows by the round's batch.
 #include "rz_device.cuh"   // rz_pixel_err_of
+#include "rz_launch.h"
 
 #define RZ_LIST_BLOCK 1024u   // pixels (one per thread) per block of the flag and scatter kernels
 

@@ -25,6 +25,7 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "rz_device.cuh"
+#include "rz_launch.h"
 
 namespace {
 

@@ -17,58 +17,8 @@
 #include "../../include/rayz_cuda.h"
 #include "rz_device.cuh"
 #include "rz_denoise.cuh"   // RzDenoiseArgs
-#include "rz_host_bvh.hpp"   // Box, sphere_box, RefBuilder (K0's reference-shaped BVH), SahBuilder (K3's tree for small scenes); RzRefNode
-
-// from rz_path.cu / rz_ids.cu / rz_misc.cu / rz_wavefront.cu
-struct RzIdsArgs {
-    const RzRefNode *nodes; const uint32_t *order; const double4 *c64; const double4 *v64;
-    uint32_t n_spheres, n_nodes; double look_from[3], px_du[3], px_dv[3], px_origin[3];
-    uint32_t width, height; int use_bvh; int32_t *out; unsigned int *err;
-};
-struct RzResolveArgs {
-    const unsigned long long *accum; float4 *out_linear; uint8_t *out_rgb8; float *out_err; uint32_t *out_spp; const uint32_t *n_px;
-    const double *gain; uint32_t n_local_px, width; uint32_t spp; uint32_t dev_index, dev_count, band_rows;
-};
-extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, int collect_stats, int sm_count,
-                                      cudaStream_t stream, int *grid_out);
-extern "C" cudaError_t rz_path_warm(void);
-extern "C" size_t rz_primary_smem_bytes(const RzPathArgs *a);
-extern "C" cudaError_t rz_launch_second(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
-extern "C" size_t rz_bin_scratch_bytes(void);
-extern "C" cudaError_t rz_launch_bin_lists(const RzPathArgs *a, int sm_count, cudaStream_t stream);
-extern "C" cudaError_t rz_second_grid(const RzPathArgs *a, int collect_stats, int sm_count, int *grid);
-extern "C" cudaError_t rz_bin_sort(const unsigned short *keys_in, const unsigned int *count, uint32_t cap, unsigned int *bins,
-                                   unsigned short *keys_out, uint32_t *idx_out, uint32_t ue_max, uint32_t ue_div, int sm_count, cudaStream_t stream);
-extern "C" cudaError_t rz_sort_warm(void);
-extern "C" cudaError_t rz_launch_primary(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
-extern "C" cudaError_t rz_bvh_warm(void);
-extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_denoise(const RzDenoiseArgs *a, cudaStream_t stream);
-extern "C" size_t rz_lbvh_scratch_bytes(uint32_t n);
-extern "C" cudaError_t rz_bvh_finalize(RzBvhNode *nodes, uint32_t n_nodes, cudaStream_t stream);
-extern "C" cudaError_t rz_lbvh_build(uint32_t n, int leaf_max, const double4 *c64, const double4 *v64, const uint32_t *mat, void *scratch,
-                                     size_t scratch_bytes, RzBvhNode *nodes, float4 *o_cr, float4 *o_vel, double4 *o_c64,
-                                     double4 *o_v64, uint32_t *o_mat, int32_t *o_orig, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_ids(const RzIdsArgs *a, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
-extern "C" uint32_t rz_noise_grid(void);
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain,
-                                              uint32_t n_local_px, uint32_t n, double target, void *out, cudaStream_t stream);
-extern "C" size_t rz_rqmc_gain_words(uint32_t n_local_px, uint32_t width);
-extern "C" cudaError_t rz_launch_rqmc_gain(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
-                                           uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, cudaStream_t stream);
-extern "C" size_t rz_list_scratch_words(uint32_t n_local_px);
-extern "C" size_t rz_list_count_word(uint32_t n_local_px);
-extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, const double *gain, uint32_t *n_px,
-                                            uint32_t n_local_px, uint32_t n_cur, uint32_t add,
-                                            float target, uint32_t *list, uint32_t *scratch, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_fill_u32(uint32_t *p, uint32_t n, uint32_t v, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_ffma_peak(float *sink, int grid, int iters, int mode, cudaStream_t stream);
-extern "C" cudaError_t rz_wavefront_render(const RzPathArgs *a, int sm_count, int collect_stats, cudaStream_t stream,
-                                           void **scratch, size_t *scratch_bytes, uint32_t *launches);
-extern "C" void rz_wavefront_free(void *scratch);
+#include "rz_host_bvh.hpp"   // Box, sphere_box, RefBuilder (K0's reference-shaped BVH), SahBuilder (K3's tree for small scenes)
+#include "rz_launch.h"       // the kernel units' launchers and their argument records
 
 // ------------------------------------------------------------------------------ errors
 static thread_local char g_err[512] = "";
@@ -172,7 +122,7 @@ struct Dev {
     DBuf<float4> out_linear;
     DBuf<uint8_t> out_rgb8;
     DBuf<float> out_err;              // rayz_cuda_noise: per-pixel error of the context's rows (gather root only)
-    DBuf<double> noise_part;          // rayz_cuda_noise: the reduction's per-CTA partials of this device
+    DBuf<RzNoisePartial> noise_part;  // rayz_cuda_noise: the reduction's per-CTA partials of this device
     DBuf<uint32_t> out_spp;           // rayz_cuda_pixel_samples: per-pixel sample counts of the context's rows (gather root only)
     DBuf<float4> out_guides;          // rayz_cuda_render_guides: albedo, then normal + depth, of the context's rows (gather root only)
     // rayz_cuda_denoise (gather root only): the resolved frame, then the denoised one; the per-pixel error; the ping-pong pair of
@@ -1418,7 +1368,7 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
     const AccumRecord *A = nullptr;
     if (const int rc = accumulated_frame(ctx, "noise", A)) return rc;
     if (!A->moments) return rz_fail(RZ_ERR_INVALID_ARG, "noise: the accumulated render(s) ran without RZ_RENDER_MOMENTS");
-    const uint32_t ND = (uint32_t)ctx->devs.size(), G = rz_noise_grid();
+    const uint32_t ND = (uint32_t)ctx->devs.size();
     Dev &D0 = ctx->devs[0];
     const FrameSplit sp(ctx, A->frame);
     int rc;
@@ -1427,7 +1377,7 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
     for (uint32_t d = 0; d < ND; d++) {   // every device enqueues before the first wait
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        if ((rc = D.noise_part.alloc(4 * (size_t)G))) return rc;
+        if ((rc = D.noise_part.alloc(RZ_NOISE_GRID))) return rc;
         const double *gain;
         if ((rc = rqmc_gain(ctx, d, *A, sp.n_local[d], &gain))) return rc;
         if (out_err) {
@@ -1440,16 +1390,12 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
     }
     double sum = 0, sum2 = 0, mx = 0;
     uint64_t above = 0;
-    std::vector<double> part(4 * (size_t)G);
+    std::vector<RzNoisePartial> part(RZ_NOISE_GRID);
     for (Dev &D : ctx->devs) {
         RZ_CUDA(cudaSetDevice(D.id));
-        RZ_CUDA(cudaMemcpyAsync(part.data(), D.noise_part.p, part.size() * sizeof(double), cudaMemcpyDeviceToHost, D.stream));
+        RZ_CUDA(cudaMemcpyAsync(part.data(), D.noise_part.p, part.size() * sizeof(RzNoisePartial), cudaMemcpyDeviceToHost, D.stream));
         RZ_CUDA(cudaStreamSynchronize(D.stream));
-        for (uint32_t g = 0; g < G; g++) {
-            uint64_t cnt;
-            memcpy(&cnt, &part[4 * (size_t)g + 3], sizeof cnt);
-            sum += part[4 * (size_t)g]; sum2 += part[4 * (size_t)g + 1]; mx = std::max(mx, part[4 * (size_t)g + 2]); above += cnt;
-        }
+        for (const RzNoisePartial &g : part) { sum += g.sum; sum2 += g.sum2; mx = std::max(mx, g.max); above += g.above; }
     }
     if (out_err) {
         RZ_CUDA(cudaSetDevice(D0.id));

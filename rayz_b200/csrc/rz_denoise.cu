@@ -10,6 +10,7 @@
 #include <stdint.h>
 
 #include "rz_denoise.cuh"   // RzDenoiseArgs and the arithmetic
+#include "rz_launch.h"
 
 
 #define RZ_DN_BX 32

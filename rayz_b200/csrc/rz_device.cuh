@@ -453,12 +453,13 @@ RZ_HD RzRay rz_lens_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, float ux,
     return ray;
 }
 
-// One Philox block gives the five uniforms: 4 x 24 high bits + 3 x 8 low bits.  With `sobol` (RZ_RENDER_SOBOL; the kernels pass
-// their SOBOL template argument) three Sobol pairs give them instead (rz_sampler.cuh): jitter, lens (radius, angle) and the
-// shutter time (first coordinate of the third pair); `rqmc` (the SOBOL = 2 instances) draws them from the sample's replicate.
+// One Philox block gives the five uniforms: 4 x 24 high bits + 3 x 8 low bits.  With `sobol` != 0 (RZ_RENDER_SOBOL; the kernels
+// pass their SOBOL template argument) three Sobol pairs give them instead (rz_sampler.cuh): jitter, lens (radius, angle) and the
+// shutter time (first coordinate of the third pair); `sobol` = 2 (RZ_RENDER_RQMC) draws them from the sample's replicate.
 RZ_HD RzRay rz_camera_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, uint32_t gpix, uint32_t sample,
-                          uint32_t k0, uint32_t k1, bool sobol = false, bool rqmc = false) {
+                          uint32_t k0, uint32_t k1, int sobol = 0) {
     if (sobol) {
+        const bool rqmc = sobol == 2;
         const float2 j = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_JITTER, sample, rqmc);
         const float2 l = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_LENS, sample, rqmc);
         const float t = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_TIME, sample, rqmc).x;

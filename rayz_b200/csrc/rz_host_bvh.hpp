@@ -1,7 +1,7 @@
 // rz_host_bvh.hpp — host-side tree builders of the C ABI's rayz_cuda_upload_scene (rz_context.cu): the reference-shaped BVH
 // K0 walks for the bit-exact primary ids (BVH.build, reference src/hit.zig:130-161) and the binned-SAH BVH2 of the FP32
 // traversal kernel K3 for scenes below 8192 spheres (larger ones: rz_bvh_build.cu on the device).  Plain host C++ over
-// include/rayz_cuda.h's RzScene and the node records of rz_device.cuh / rz_ids.cu; compiled into the library by rz_context.cu and,
+// include/rayz_cuda.h's RzScene and the node records of rz_device.cuh / rz_launch.h; compiled into the library by rz_context.cu and,
 // on its own, by tests/hostsim/hostbvh.cu (tree invariants and the rounding helpers on the CPU).  Builds trees only: nothing
 // here intersects a ray.
 #pragma once
@@ -14,11 +14,7 @@
 
 #include "../../include/rayz_cuda.h"
 #include "rz_device.cuh"
-
-#ifndef RZ_REF_NODE_DEFINED
-#define RZ_REF_NODE_DEFINED
-struct RzRefNode { double low[3], high[3]; int32_t left, right, start, end; };   // rz_ids.cu's node: BVH of hit.zig:101-108, children by index
-#endif
+#include "rz_launch.h"   // RzRefNode
 
 namespace {
 

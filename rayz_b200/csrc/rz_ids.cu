@@ -12,26 +12,7 @@
 // The recursion of findHit is an explicit stack here: every accepted hit has t <= the tmax in
 // force, so "tmax passed down" always equals the running closest t and a depth-first,
 // left-first walk with one running `best` visits and accepts exactly what the recursion does.
-#include <cuda_runtime.h>
-#include <stdint.h>
-
-struct RzRefNode {  // BVH of hit.zig:101-108, children by index
-    double low[3], high[3];
-    int32_t left, right, start, end;
-};
-
-struct RzIdsArgs {
-    const RzRefNode *nodes;     // reference-shaped tree (host build restating hit.zig:130-161)
-    const uint32_t *order;      // hittables order after the build's sorts
-    const double4 *c64;         // [n] (cx,cy,cz,r)   caller's sphere order
-    const double4 *v64;         // [n] (vx,vy,vz,0)
-    uint32_t n_spheres, n_nodes;
-    double look_from[3], px_du[3], px_dv[3], px_origin[3];
-    uint32_t width, height;
-    int use_bvh;
-    int32_t *out;
-    unsigned int *err;          // device error word: bit 2 = traversal stack overflow (never silently dropped)
-};
+#include "rz_launch.h"   // RzRefNode, RzIdsArgs
 
 struct D3 { double x, y, z; };
 __device__ __forceinline__ D3 d3(double x, double y, double z) { D3 r; r.x = x; r.y = y; r.z = z; return r; }

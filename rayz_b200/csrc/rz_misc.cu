@@ -1,6 +1,4 @@
 // rz_misc.cu — K5 resolve/quantise and K6 FP32 peak microbenchmark.
-#include <cuda_runtime.h>
-#include <stdint.h>
 
 // ---------------------------------------------------------------------------------------------
 // K5.  Fixed-point accumulators -> linear float4 + gamma-2 RGB8.
@@ -16,20 +14,7 @@
 // with c samples resolves exactly as the same pixel of a uniform c-spp render.
 // ---------------------------------------------------------------------------------------------
 #include "rz_device.cuh"   // rz_pixel_err, rz_quantise_rgb8
-
-struct RzResolveArgs {
-    const unsigned long long *accum;  // [n_local_px][4]
-    float4 *out_linear;               // nullable
-    uint8_t *out_rgb8;                // nullable
-    float *out_err;                   // nullable: displayed-value standard error per pixel (needs slot 3, RZ_RENDER_MOMENTS)
-    uint32_t *out_spp;                // nullable: the pixel's sample count (rayz_cuda_pixel_samples)
-    const uint32_t *n_px;             // nullable: per-pixel sample counts of an adaptive frame (rz_adaptive.cu); null: spp
-    const double *gain;               // nullable: RZ_RENDER_RQMC's per-pixel gains (rz_rqmc_gain_kernel); out_err is then rz_pixel_err_rqmc
-    uint32_t n_local_px, width;
-    uint32_t spp;                     // samples summed in the accumulators (cumulative over RZ_RENDER_ACCUMULATE batches)
-    // local row lr of this device -> destination row ((lr / band) * dev_count + dev_index) * band + lr % band
-    uint32_t dev_index, dev_count, band_rows;
-};
+#include "rz_launch.h"     // RzResolveArgs, RzNoisePartial
 
 __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) {
     const uint32_t lp = blockIdx.x * blockDim.x + threadIdx.x;
@@ -66,8 +51,6 @@ extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t st
 // count of pixels with e > target over the pixels lp = cta * 256 + tid + k * grid * 256, reduced in a fixed tree.  The host
 // adds the CTAs' partials in order: no floating-point atomics, so two identical calls give identical summaries.
 // ---------------------------------------------------------------------------------------------
-#define RZ_NOISE_GRID 256
-struct RzNoisePartial { double sum, sum2, max; unsigned long long above; };
 
 // n_px (nullable): per-pixel sample counts of an adaptive frame, else every pixel has n samples.  gain (nullable): RZ_RENDER_RQMC's
 // per-pixel gains.
@@ -94,11 +77,9 @@ __global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned lon
     if (threadIdx.x == 0) out[blockIdx.x] = RzNoisePartial{s_sum[0], s_sum2[0], s_max[0], s_above[0]};
 }
 
-extern "C" uint32_t rz_noise_grid(void) { return RZ_NOISE_GRID; }
-// out: RZ_NOISE_GRID x 4 words (sum, sum2, max as doubles, then the count as an integer)
 extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain,
-                                              uint32_t n_local_px, uint32_t n, double target, void *out, cudaStream_t stream) {
-    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, gain, n_local_px, n, target, (RzNoisePartial *)out);
+                                              uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *out, cudaStream_t stream) {
+    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, gain, n_local_px, n, target, out);
     return cudaGetLastError();
 }
 

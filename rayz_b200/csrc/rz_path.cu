@@ -33,6 +33,7 @@
 //   * large scenes use the BVH kernels of rz_bvh_trace.cu (K3) instead.
 #include <algorithm>
 
+#include "rz_launch.h"
 #include "rz_search.cuh"
 
 // Resident CTAs per SM the staged kernels are compiled for (register cap = 65536 / (128 * N)); undefined = ptxas decides.
@@ -142,7 +143,7 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
                             st[r].lp = lp;
                             st[r].gpix = pj * a.width + pi;
                             st[r].sample = a.sample_offset + unit_s0 + (k >> 5);
-                            st[r].ray = rz_camera_ray(a.cam, pi, pj, st[r].gpix, st[r].sample, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
+                            st[r].ray = rz_camera_ray(a.cam, pi, pj, st[r].gpix, st[r].sample, a.seed_lo, a.seed_hi, SOBOL);
                             st[r].thr = f3(1.f, 1.f, 1.f);
                             st[r].seg = 0;
                             st[r].alive = a.max_depth > 0u;
@@ -177,7 +178,7 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
             if (!st[r].alive) continue;
             if (STATS) { c_segs++; c_sph += a.set.n; }   // brute force: every sphere of the set
             uint32_t kind;
-            const int res = rz_shade_segment(a, st[r].ray, st[r].thr, st[r].seg, st[r].lp, st[r].gpix, st[r].sample, bk[r], kind, SOBOL != 0, SOBOL == 2);
+            const int res = rz_shade_segment(a, st[r].ray, st[r].thr, st[r].seg, st[r].lp, st[r].gpix, st[r].sample, bk[r], kind, SOBOL);
             if (STATS) {
                 if (kind < 3u) c_hit[kind]++;
                 if (res == RZ_END_SKY) c_sky++;
@@ -238,7 +239,7 @@ __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRa
         if (Q.live) {
             if (STATS) C.segs++;
             uint32_t kind;
-            const int res = rz_shade_segment(a, Q.ray, Q.thr, Q.seg, Q.lp, Q.gpix, Q.smp, Q.bk, kind, SOBOL != 0, SOBOL == 2);
+            const int res = rz_shade_segment(a, Q.ray, Q.thr, Q.seg, Q.lp, Q.gpix, Q.smp, Q.bk, kind, SOBOL);
             if (STATS) {
                 if (kind < 3u) C.hit[kind]++;
                 if (res == RZ_END_SKY) C.sky++;
@@ -369,7 +370,7 @@ __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
                 const bool have = valid && (s + (uint32_t)trip < ns);
                 Q.live = have && a.max_depth > 0u;
                 if (STATS && have) { C.paths++; if (!Q.live) C.depth++; }
-                if (Q.live) Q.ray = rz_camera_ray(a.cam, pi, pj, gpix, Q.smp, a.seed_lo, a.seed_hi, SOBOL != 0, SOBOL == 2);
+                if (Q.live) Q.ray = rz_camera_ray(a.cam, pi, pj, gpix, Q.smp, a.seed_lo, a.seed_hi, SOBOL);
                 else { Q.ray.o = f3(0.f, 0.f, 0.f); Q.ray.d = f3(0.f, 1.f, 0.f); Q.ray.time = 0.f; Q.ray.self_k = -1; }
                 Q.thr = f3(1.f, 1.f, 1.f); Q.seg = 0u; Q.lp = lp; Q.gpix = gpix; Q.bk = -1; Q.cont = false; Q.key = 0u;
                 if (trip == 0) L[1] = L[0];   // slot 0 is rewritten by the second trip
@@ -609,22 +610,36 @@ __global__ void RZ_SECOND_BOUNDS rz_second_kernel(const RzPathArgs a) {
 }
 
 // ------------------------------------------------------------------------------ launchers
-template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false>
-static cudaError_t rz_launch_one(const RzPathArgs &a, int sm_count, size_t smem, cudaStream_t stream, int *grid_out) {
-    auto kern = rz_pick_sampler(a, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, 0>, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, 1>, rz_path_kernel<R, G, STATS, MB, QUEUE, LIST, 2>);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+static size_t rz_pk_bytes(const RzPathArgs &a) { return (size_t)(a.set.n_pad + (a.set.n_pad - a.set.n_static_pad)) * 16u; }
+
+// Shared memory the sorted-stage kernel needs: the set + per-warp scratch (rz_second_warp_bytes).
+static size_t rz_second_smem_bytes(const RzPathArgs &a) {
+    return rz_pk_bytes(a) + 4u * (size_t)rz_second_warp_bytes(a.set.n_pad, a.unit_entries);
+}
+
+static auto rz_second_instance(const RzPathArgs &a, int collect_stats) {
+    return rz_pick_instance(a, collect_stats, [](auto S, auto M) { return rz_second_kernel<decltype(S)::value, decltype(M)::value>; });
+}
+
+// One form of rz_path_kernel on the persistent grid; rays_per_thread in {1,2}.
+template <bool QUEUE, bool LIST>
+static cudaError_t rz_launch_one(const RzPathArgs &a, int rays_per_thread, int collect_stats, int sm_count, cudaStream_t stream,
+                                 int *grid_out) {
+    const auto one = rz_pick_instance(a, collect_stats, [](auto S, auto M) { return rz_path_kernel<1, 2, decltype(S)::value, 5, QUEUE, LIST, decltype(M)::value>; });
+    // 8 resident CTAs per SM (64 registers, 232 B of spills outside the search loop) measured 3 % faster than the 5 CTAs the
+    // unconstrained 88-register build gets: 1522 vs 1472 Mpaths/s at config 2 / 100 spp.  (The STATS instances keep 5.)
+    const auto two = rz_pick_instance(a, collect_stats, [](auto S, auto M) {
+        return rz_path_kernel<2, 2, decltype(S)::value, decltype(S)::value ? 5 : 8, QUEUE, LIST, decltype(M)::value>;
+    });
+    const auto kern = rays_per_thread == 1 ? one : two;
+    const size_t smem = rz_pk_bytes(a);
+    int grid = 0;
+    const cudaError_t e = rz_persistent_grid(kern, smem, sm_count, &grid);
     if (e != cudaSuccess) return e;
-    int per_sm = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorInvalidConfiguration;
-    const int grid = sm_count * per_sm;
     if (grid_out) *grid_out = grid;
     kern<<<grid, 128, smem, stream>>>(a);
     return cudaGetLastError();
 }
-
-static size_t rz_pk_bytes(const RzPathArgs &a) { return (size_t)(a.set.n_pad + (a.set.n_pad - a.set.n_static_pad)) * 16u; }
 
 // Forces the lazily loaded path kernels into the context (called once from rayz_cuda_create so that
 // the first render does not pay module loading).
@@ -636,11 +651,6 @@ extern "C" cudaError_t rz_path_warm(void) {
     return e;
 }
 
-// Shared memory the sorted-stage kernel needs: the set + per-warp scratch (rz_second_warp_bytes).
-extern "C" size_t rz_second_smem_bytes(const RzPathArgs *a) {
-    return rz_pk_bytes(*a) + 4u * (size_t)rz_second_warp_bytes(a->set.n_pad, a->unit_entries);
-}
-
 // Shared memory the primary kernel needs: the pair-interleaved set + one pair list per warp.
 extern "C" size_t rz_primary_smem_bytes(const RzPathArgs *a) {
     return rz_pk_bytes(*a) + ((4u * (size_t)a->set.n_pad * sizeof(unsigned short) + 15u) & ~size_t(15));
@@ -648,21 +658,14 @@ extern "C" size_t rz_primary_smem_bytes(const RzPathArgs *a) {
 
 // Stage 1: camera segments of the work units [unit_base, unit_base + n_units) -> queue.
 extern "C" cudaError_t rz_launch_primary(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream) {
+    const auto kern = rz_pick_instance(*a, collect_stats, [](auto S, auto M) { return rz_primary_kernel<decltype(S)::value, decltype(M)::value>; });
     const size_t smem = rz_primary_smem_bytes(a);
-    auto launch = [&](auto kern) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int per_sm = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorInvalidConfiguration;
-        const unsigned want = (a->n_units + 3u) / 4u;   // 4 warps per CTA, one unit per warp at a time
-        const unsigned grid = (unsigned)std::max(1u, std::min((unsigned)(sm_count * per_sm), want));
-        kern<<<grid, 128, smem, stream>>>(*a);
-        return cudaGetLastError();
-    };
-    return collect_stats ? launch(rz_pick_sampler(*a, rz_primary_kernel<true, 0>, rz_primary_kernel<true, 1>, rz_primary_kernel<true, 2>))
-                         : launch(rz_pick_sampler(*a, rz_primary_kernel<false, 0>, rz_primary_kernel<false, 1>, rz_primary_kernel<false, 2>));
+    int grid = 0;
+    const cudaError_t e = rz_persistent_grid(kern, smem, sm_count, &grid);
+    if (e != cudaSuccess) return e;
+    const unsigned want = (a->n_units + 3u) / 4u;   // 4 warps per CTA, one unit per warp at a time
+    kern<<<std::max(1u, std::min((unsigned)grid, want)), 128, smem, stream>>>(*a);
+    return cudaGetLastError();
 }
 
 // Per-group pair lists of the sorted-segment kernel (a->bin_lists: RZ_SORT_BINS rows of a->bin_row bytes).
@@ -676,63 +679,24 @@ extern "C" cudaError_t rz_launch_bin_lists(const RzPathArgs *a, int sm_count, cu
 
 // Grid size of the sorted-segment kernel (the sort sizes the work units with it).
 extern "C" cudaError_t rz_second_grid(const RzPathArgs *a, int collect_stats, int sm_count, int *grid) {
-    const size_t smem = rz_second_smem_bytes(a);
-    auto query = [&](auto kern) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int per_sm = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorInvalidConfiguration;
-        *grid = sm_count * per_sm;
-        return cudaSuccess;
-    };
-    return collect_stats ? query(rz_pick_sampler(*a, rz_second_kernel<true, 0>, rz_second_kernel<true, 1>, rz_second_kernel<true, 2>))
-                         : query(rz_pick_sampler(*a, rz_second_kernel<false, 0>, rz_second_kernel<false, 1>, rz_second_kernel<false, 2>));
+    return rz_persistent_grid(rz_second_instance(*a, collect_stats), rz_second_smem_bytes(*a), sm_count, grid);
 }
 
 // Stage 2: second segments of the sorted queue (q_in through q_in_idx) -> q_out.
 extern "C" cudaError_t rz_launch_second(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream) {
-    const size_t smem = rz_second_smem_bytes(a);
-    auto launch = [&](auto kern) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int per_sm = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorInvalidConfiguration;
-        kern<<<sm_count * per_sm, 128, smem, stream>>>(*a);
-        return cudaGetLastError();
-    };
-    return collect_stats ? launch(rz_pick_sampler(*a, rz_second_kernel<true, 0>, rz_second_kernel<true, 1>, rz_second_kernel<true, 2>))
-                         : launch(rz_pick_sampler(*a, rz_second_kernel<false, 0>, rz_second_kernel<false, 1>, rz_second_kernel<false, 2>));
+    int grid = 0;
+    const cudaError_t e = rz_second_grid(a, collect_stats, sm_count, &grid);
+    if (e != cudaSuccess) return e;
+    rz_second_instance(*a, collect_stats)<<<grid, 128, rz_second_smem_bytes(*a), stream>>>(*a);
+    return cudaGetLastError();
 }
 
 // Last stage (q_in != nullptr): the persistent megakernel started from a queue; or the single-stage form
 // (q_in == nullptr) that generates its own camera rays (of the pixels of px_list when it is set).  rays_per_thread in {1,2}.
 extern "C" cudaError_t rz_launch_path(const RzPathArgs *a, int rays_per_thread, int collect_stats, int sm_count, cudaStream_t stream,
                                       int *grid_out) {
-    const bool stats = collect_stats != 0;
-    const size_t smem = rz_pk_bytes(*a);
-    if (a->q_in) {
-        if (rays_per_thread == 1)
-            return stats ? rz_launch_one<1, 2, true, 5, true>(*a, sm_count, smem, stream, grid_out)
-                         : rz_launch_one<1, 2, false, 5, true>(*a, sm_count, smem, stream, grid_out);
-        return stats ? rz_launch_one<2, 2, true, 5, true>(*a, sm_count, smem, stream, grid_out)
-                     : rz_launch_one<2, 2, false, 8, true>(*a, sm_count, smem, stream, grid_out);
-    }
-    if (a->px_list) {   // an adaptive round: the same instances over the listed pixels
-        if (rays_per_thread == 1)
-            return stats ? rz_launch_one<1, 2, true, 5, false, true>(*a, sm_count, smem, stream, grid_out)
-                         : rz_launch_one<1, 2, false, 5, false, true>(*a, sm_count, smem, stream, grid_out);
-        return stats ? rz_launch_one<2, 2, true, 5, false, true>(*a, sm_count, smem, stream, grid_out)
-                     : rz_launch_one<2, 2, false, 8, false, true>(*a, sm_count, smem, stream, grid_out);
-    }
-    if (rays_per_thread == 1)
-        return stats ? rz_launch_one<1, 2, true, 5, false>(*a, sm_count, smem, stream, grid_out)
-                     : rz_launch_one<1, 2, false, 5, false>(*a, sm_count, smem, stream, grid_out);
-    // 8 resident CTAs per SM (64 registers, 232 B of spills outside the search loop) measured 3 % faster than
-    // the 5 CTAs the unconstrained 88-register build gets: 1522 vs 1472 Mpaths/s at config 2 / 100 spp.
-    return stats ? rz_launch_one<2, 2, true, 5, false>(*a, sm_count, smem, stream, grid_out)
-                 : rz_launch_one<2, 2, false, 8, false>(*a, sm_count, smem, stream, grid_out);
+    if (a->q_in) return rz_launch_one<true, false>(*a, rays_per_thread, collect_stats, sm_count, stream, grid_out);
+    if (a->px_list)   // an adaptive round: the same instances over the listed pixels
+        return rz_launch_one<false, true>(*a, rays_per_thread, collect_stats, sm_count, stream, grid_out);
+    return rz_launch_one<false, false>(*a, rays_per_thread, collect_stats, sm_count, stream, grid_out);
 }

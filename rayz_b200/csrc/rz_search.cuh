@@ -3,6 +3,8 @@
 // per-segment shading step.  Both kernel families call the SAME functions, so for equal RNG keys
 // they produce bit-identical radiance.
 #pragma once
+#include <type_traits>
+
 #include "rz_device.cuh"
 
 
@@ -330,14 +332,39 @@ static inline K rz_pick_sampler(const RzPathArgs &a, K philox, K sobol, K rqmc) 
     return (a.sobol & RZ_SAMPLER_RQMC) ? rqmc : a.sobol ? sobol : philox;
 }
 
+// The instance a launcher runs for (collect_stats, a.sobol).  `inst` names the kernel's instances once, as a generic lambda of
+// (std::integral_constant<bool, STATS>, std::integral_constant<int, SOBOL>), e.g.
+//   [](auto S, auto M) { return rz_second_kernel<decltype(S)::value, decltype(M)::value>; }
+template <int V> using rz_int_c = std::integral_constant<int, V>;
+template <class F>
+static inline auto rz_pick_instance(const RzPathArgs &a, int collect_stats, F inst) {
+    const std::true_type T{};
+    const std::false_type N{};
+    return collect_stats ? rz_pick_sampler(a, inst(T, rz_int_c<0>()), inst(T, rz_int_c<1>()), inst(T, rz_int_c<2>()))
+                         : rz_pick_sampler(a, inst(N, rz_int_c<0>()), inst(N, rz_int_c<1>()), inst(N, rz_int_c<2>()));
+}
+
+// Grid of a persistent kernel: as many 128-thread CTAs as fit on every SM with `smem` bytes of dynamic shared memory.  The
+// attribute that admits that much is set only when smem > 0 (the BVH kernels take none).
+template <class K>
+static inline cudaError_t rz_persistent_grid(K kern, size_t smem, int sm_count, int *grid) {
+    cudaError_t e;
+    if (smem > 0 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    int per_sm = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem)) != cudaSuccess) return e;
+    if (per_sm < 1) return cudaErrorInvalidConfiguration;
+    *grid = sm_count * per_sm;
+    return cudaSuccess;
+}
+
 enum { RZ_CONT = 0, RZ_END_SKY = 1, RZ_END_ABSORBED = 2, RZ_END_DEPTH = 3 };
 
 // One step of bounceRay (renderer.zig:103-126) after the closest-hit query: miss -> sky and
 // accumulate; hit -> refine in f64, scatter, attenuate.  `kind_out` = material kind of the hit.  `sobol`: the kernel's SOBOL
-// template argument (RZ_RENDER_SOBOL), a compile-time constant, so that the Philox instances carry no trace of the other sampler;
-// `rqmc`: the SOBOL = 2 instances' (RZ_RENDER_RQMC), compile-time as well.
+// template argument (0 Philox, 1 RZ_RENDER_SOBOL, 2 with RZ_RENDER_RQMC), a compile-time constant, so that the Philox instances
+// carry no trace of the other sampler.
 __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray, float3 &thr, uint32_t &seg, uint32_t lp,
-                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, bool sobol, bool rqmc) {
+                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, int sobol) {
     kind_out = 3u;
     if (bk < 0) {
         // miss: background (renderer.zig:124-125), path ends
@@ -349,7 +376,7 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
         // the noise estimate's second moment (the only accumulation site besides the three above: every kernel shades here)
         if (a.moments) atomicAdd(acc + 3, rz_fixed32(rz_luma_sq(rz_clamp_radiance(L.x), rz_clamp_radiance(L.y), rz_clamp_radiance(L.z))));
         // RZ_RENDER_RQMC: the replicate's luminance sum (rz_pixel_err_rqmc)
-        if (rqmc)
+        if (sobol == 2)
             atomicAdd(a.accum + rz_rep_offset(a.n_local_px) + (size_t)lp * 2u + (sample & 1u),
                       rz_fixed32(rz_clamp_radiance(rz_luma(rz_clamp_radiance(L.x), rz_clamp_radiance(L.y), rz_clamp_radiance(L.z)))));
         return RZ_END_SKY;
@@ -369,7 +396,7 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
     kind_out = kind < 3u ? kind : 0u;
     seg++;
     const uint4 rb = rz_philox(gpix, sample, seg, 0u, a.seed_lo, a.seed_hi);
-    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(seg), sample, rqmc)   // u.z, u.w stay Philox
+    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(seg), sample, sobol == 2)   // u.z, u.w stay Philox
                            : make_float2(rz_u01(rb.x >> 8), rz_u01(rb.y >> 8));
     const float4 u = make_float4(q.x, q.y, rz_u01(rb.z >> 8), rz_u01(rb.w >> 8));
     float3 att;

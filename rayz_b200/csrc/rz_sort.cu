@@ -26,6 +26,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "rz_device.cuh"
+#include "rz_launch.h"
 
 namespace {
 

@@ -4,6 +4,6 @@ set -e
 cd "$(dirname "$0")"
 mkdir -p ../_build
 SO=../_build/libhostbvh.so
-if [ ! -f $SO ] || [ hostbvh.cu -nt $SO ] || [ ../../rayz_b200/csrc/rz_host_bvh.hpp -nt $SO ] || [ ../../rayz_b200/csrc/rz_device.cuh -nt $SO ]; then
+if [ ! -f $SO ] || [ hostbvh.cu -nt $SO ] || [ ../../rayz_b200/csrc/rz_host_bvh.hpp -nt $SO ] || [ ../../rayz_b200/csrc/rz_launch.h -nt $SO ] || [ ../../rayz_b200/csrc/rz_device.cuh -nt $SO ]; then
   nvcc -x cu -O2 -std=c++17 -shared -Xcompiler -fPIC -Wno-deprecated-gpu-targets -o $SO hostbvh.cu
 fi
