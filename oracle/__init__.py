@@ -98,6 +98,9 @@ def lib():
         L.orc_rng_u64.argtypes = [C.c_uint64, C.c_uint32, C.c_void_p]
         L.orc_bvh_export.restype = C.c_uint32
         L.orc_bvh_export.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.orc_replay.argtypes = [C.c_void_p, C.POINTER(OrcCamera)] + [C.c_uint32] * 5 + [C.c_uint64, C.c_float, C.c_int32,
+                                                                                       C.c_double, C.c_uint32] + [C.c_void_p] * 9
+        L.orc_replay_uniforms.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, C.c_void_p]
     return _lib
 
 
@@ -177,12 +180,43 @@ class Scene:
         lib().orc_texture_value(self._h, tex, pp, o.ctypes.data_as(C.POINTER(C.c_double)))
         return o
 
+    def replay(self, cam, w: int, h: int, sample_offset: int, spp: int, depth: int = 50, seed: int = 1, t_min: float = 0.0,
+               sampler: str = "philox", perturb: float = 0.0, threads: int = 0) -> dict:
+        """The backend's path algorithm replayed in f64 with the uniforms its kernels draw (rayz_oracle.cpp, namespace replay):
+        one entry per path of samples [sample_offset, sample_offset + spp) of every pixel, arrays shaped [h, w, spp, ...].
+        cam: an OrcCamera or the backend's RzCamera (same layout).  sampler: "philox", "sobol" or "sobol-rqmc".  perturb: the
+        angle by which the perturbed replays turn every direction (0: the default, 1e-5 rad).
+        Keys: rgb (clamped radiance), y (its luminance), segs, end (END_*), hits ([diffuse, metallic, dielectric]), hash (event
+        sequence), reason / fseg (first fragile decision, REASONS; 0 = robust), robust, tol (radiance tolerance of a robust path)."""
+        cam = cam if isinstance(cam, OrcCamera) else OrcCamera.from_buffer_copy(cam)
+        n = (h, w, spp)
+        out = dict(rgb=np.zeros(n + (3,)), y=np.zeros(n), segs=np.zeros(n, np.uint32), end=np.zeros(n, np.uint8),
+                   hits=np.zeros(n + (3,), np.uint32), hash=np.zeros(n, np.uint64), reason=np.zeros(n, np.uint8),
+                   fseg=np.zeros(n, np.int32), tol=np.zeros(n))
+        lib().orc_replay(self._h, C.byref(cam), w, h, sample_offset, spp, depth, seed, t_min, SAMPLERS[sampler], perturb, threads,
+                         *[out[k].ctypes.data for k in ("rgb", "y", "segs", "end", "hits", "hash", "reason", "fseg", "tol")])
+        out["robust"] = out["reason"] == 0
+        return out
+
     def bvh(self):
         ns, _, _ = self.counts()
         mx = 2 * ns + 2
         boxes = np.zeros((mx, 6)); links = np.zeros((mx, 4), dtype=np.int32); order = np.zeros(ns, dtype=np.uint32)
         n = lib().orc_bvh_export(self._h, mx, boxes.ctypes.data, links.ctypes.data, order.ctypes.data)
         return boxes[:n], links[:n], order
+
+
+SAMPLERS = {"philox": 0, "sobol": 1, "sobol-rqmc": 2}
+END_SKY, END_ABSORBED, END_DEPTH = 0, 1, 2
+REASONS = ("robust", "tie", "graze", "t_min", "self_b", "diffuse_flip", "metal_rn", "tir", "fresnel", "self_out", "checker",
+           "degenerate", "perturbed")
+
+
+def replay_uniforms(seed: int, gpix: int, sample: int, depth: int, sampler: str = "philox") -> np.ndarray:
+    """The uniforms the replay draws for one path: camera ux, uy, ut, ur, ua, then u.x..u.w of bounces 1..depth."""
+    out = np.zeros(5 + 4 * depth)
+    lib().orc_replay_uniforms(seed, gpix, sample, depth, SAMPLERS[sampler], out.ctypes.data)
+    return out
 
 
 def camera(vfov, focus_dist, defocus_angle, look_from, look_at, vup, img_h, img_w) -> OrcCamera:

@@ -511,6 +511,347 @@ void renderRows(const Scene &sc, const Camera &cam, size_t w, size_t j0, size_t 
 
 struct OrcScene { Scene sc; };
 
+// =====================================================================================
+// Path replay: the CUDA backend's documented path algorithm restated in f64, drawing the same uniforms, so that every
+// GPU path (seed, pixel, sample) can be compared with its f64 counterpart one by one (tests/test_replay_*.py).  Restated from
+// the product's CONTRACT, not from its code: nothing here includes or links a product header.  Each step cites the contract
+// lines it follows (rayz_b200/csrc/rz_device.cuh, rz_search.cuh, rz_sampler.cuh, include/rayz_cuda.h).
+//
+// Where the algorithm deliberately differs from the reference above (the reference's sequential PRNG, its 1e-10 t_min and
+// epsilon-free self intersection, its rejection samplers) the replay follows the backend, because it checks the backend path
+// by path; tests/test_replay_cpu.py checks that the replay agrees with Scene.render in distribution.
+//
+// Robustness.  The GPU path runs in f32, so a path whose f64 decisions sit within f32 rounding of a boundary may take the
+// other branch there.  The replay marks a path fragile from the first decision within the margins below, and also replays
+// it with its camera and scatter directions perturbed by +-REPLAY_PERTURB: a changed event sequence marks it fragile too,
+// and the largest radiance change sets its tolerance.
+// =====================================================================================
+namespace replay {
+
+// ---- margins (the f32 error model each comes from)
+const double U32 = 5.9604644775390625e-08;   // 2^-24: unit roundoff of f32
+// Lengths (sphere-test operands, roots, hit points): every f32 operand carries its own rounding (|centre|, |origin|, r) and
+// the sphere test chains ~a dozen roundings of numbers of size |oc| (rz_sphere_test: fma chains of oc, nb, l): 16 u per scale.
+const double K_POS = 16.0 * U32;
+// Directions: the GPU's unit directions carry ~1e-6 rad of error (__sincosf of the scatter angles, rsqrtf normalisation,
+// the f32 normal); not measured, so the margin takes four times that.
+const double DIR_ERR = 4e-6;
+// Dot products of two such directions (diffuse flip s.n, metal r.n, the 1e-3 self-out margin): both operands' errors.
+const double DOT_TOL = 2.0 * DIR_ERR;
+// Schlick(cos, eta) against u.x and eta sin against 1: |dSchlick/dcos| = 5 (1 - r0) m^4 <= 5, and eta sin moves by
+// eta cos / sin dcos: a direction error of DIR_ERR moves both by at most ~5 DIR_ERR away from grazing.
+const double FRESNEL_TOL = 5.0 * DIR_ERR;
+// Perturbed replays: directions turned by this angle (ten times the GPU's ~1e-6 rad direction error: 4e-6 missed a path of
+// the all-materials scene whose f32 error grew through reflections between spheres in contact), in antithetic pairs
+// (the default of orc_replay's `perturb`).
+const double REPLAY_PERTURB = 1e-5;
+const int REPLAY_PAIRS = 2;
+// Tolerance of a robust path's radiance: SAFETY x the largest change among its perturbed replays, plus the f32 rounding of
+// the throughput product (two roundings per bounce: the f32 colour and the product) and of the sky, plus an absolute floor
+// (the 2^-32 fixed point of the accumulators and the f32 output).
+const double TOL_SAFETY = 4.0;
+const double TOL_REL_PER_SEG = 8.0 * U32;
+const double TOL_ABS = 1e-8;
+
+enum Reason { R_NONE = 0, R_TIE, R_GRAZE, R_TMIN, R_SELF_B, R_FLIP, R_METAL, R_TIR, R_FRESNEL, R_SELF_OUT, R_CHECKER,
+              R_DEGENERATE, R_PERTURB };
+enum End { E_SKY = 0, E_ABSORBED = 1, E_DEPTH = 2 };
+
+// ---- uniforms (rz_device.cuh:281-316 Philox4x32-7; rz_sampler.cuh Owen-scrambled Sobol, restated after the numpy model of
+// tests/test_sampler_cpu.py)
+void philox(uint32_t c[4], uint32_t k0, uint32_t k1) {
+    for (int i = 0; i < 7; i++) {
+        const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
+        const uint32_t h0 = (uint32_t)(p0 >> 32), l0 = (uint32_t)p0, h1 = (uint32_t)(p1 >> 32), l1 = (uint32_t)p1;
+        const uint32_t n0 = h1 ^ c[1] ^ k0, n2 = h0 ^ c[3] ^ k1;
+        c[0] = n0; c[1] = l1; c[2] = n2; c[3] = l0;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+}
+uint32_t brev(uint32_t x) { uint32_t r = 0; for (int b = 0; b < 32; b++) r |= ((x >> b) & 1u) << (31 - b); return r; }
+uint32_t hash32(uint32_t x) { x ^= x >> 16; x *= 0x7feb352du; x ^= x >> 15; x *= 0x846ca68bu; x ^= x >> 16; return x; }
+uint32_t owen(uint32_t x, uint32_t seed) {
+    x = brev(x) + seed;
+    for (uint32_t c : {0x6c50b47cu, 0xb82f1e52u, 0xc7afe638u, 0x8d22f6e6u}) x ^= x * c;
+    return brev(x);
+}
+uint32_t sobol_d1(uint32_t i) {   // Joe-Kuo d = 2: V_j = m_j << (31 - j), m_0 = 1, m_j = m_{j-1} ^ (m_{j-1} << 1)
+    uint32_t m = 1, r = 0;
+    for (int j = 0; j < 32; j++) {
+        if ((i >> j) & 1u) r ^= m << (31 - j);
+        m ^= m << 1;
+    }
+    return r;
+}
+// the pair's two uniforms, top 24 bits of each coordinate (include/rayz_cuda.h RZ_RENDER_SOBOL / RZ_RENDER_RQMC)
+void sobol_pair(uint32_t k0, uint32_t k1, uint32_t gpix, uint32_t pair, uint32_t sample, bool rqmc, double out[2]) {
+    uint32_t base = hash32(hash32(hash32(hash32(k0 ^ 0x6a09e667u) ^ k1) ^ gpix) ^ pair);
+    if (rqmc) { base = hash32(base ^ (0x9e3779b9u + (sample & 1u))); sample >>= 1; }
+    const uint32_t i = owen(sample, hash32(base));
+    out[0] = (double)(owen(brev(i), hash32(base ^ 1u)) >> 8) * U32;
+    out[1] = (double)(owen(sobol_d1(i), hash32(base ^ 2u)) >> 8) * U32;
+}
+struct Keys { uint32_t k0, k1, gpix, sample; int sampler; };   // sampler: 0 Philox, 1 Sobol, 2 Sobol-RQMC
+// camera: ux, uy (jitter), ut (time), ur, ua (lens radius, angle)   (rz_device.cuh:456-472)
+void camera_uniforms(const Keys &K, double u[5]) {
+    if (K.sampler) {
+        double j[2], l[2], t[2];
+        sobol_pair(K.k0, K.k1, K.gpix, 0, K.sample, K.sampler == 2, j);
+        sobol_pair(K.k0, K.k1, K.gpix, 1, K.sample, K.sampler == 2, l);
+        sobol_pair(K.k0, K.k1, K.gpix, 2, K.sample, K.sampler == 2, t);
+        u[0] = j[0]; u[1] = j[1]; u[2] = t[0]; u[3] = l[0]; u[4] = l[1];
+        return;
+    }
+    uint32_t c[4] = {K.gpix, K.sample, 0u, 0u};
+    philox(c, K.k0, K.k1);
+    u[0] = (double)(c[0] >> 8) * U32; u[1] = (double)(c[1] >> 8) * U32; u[2] = (double)(c[2] >> 8) * U32; u[3] = (double)(c[3] >> 8) * U32;
+    u[4] = (double)(((c[0] & 0xffu) << 16) | ((c[1] & 0xffu) << 8) | (c[2] & 0xffu)) * U32;
+}
+// bounce s (1-based): Philox counter (gpix, sample, s, 0); Sobol pair 2 + s replaces u.x, u.y   (rz_search.cuh:397-401)
+void bounce_uniforms(const Keys &K, uint32_t s, double u[4]) {
+    uint32_t c[4] = {K.gpix, K.sample, s, 0u};
+    philox(c, K.k0, K.k1);
+    for (int i = 0; i < 4; i++) u[i] = (double)(c[i] >> 8) * U32;
+    if (K.sampler) sobol_pair(K.k0, K.k1, K.gpix, 2u + s, K.sample, K.sampler == 2, u);
+}
+
+// ---- one path
+struct Params {
+    const Scene *sc;
+    Camera cam;
+    uint32_t depth;
+    double t_min;
+    double perturb;       // direction perturbation of this replay (0: the nominal path)
+    uint32_t pert_id;     // which perturbation (hash input)
+};
+struct Path {
+    double rgb[3] = {0, 0, 0};
+    uint32_t segs = 0, hits[3] = {0, 0, 0};
+    int end = E_DEPTH;
+    int reason = R_NONE, fseg = -1;        // first fragile decision and its segment (0 = camera segment)
+    std::vector<uint64_t> ev;              // one event word per segment, then the end kind
+};
+
+V3 perturbed(V3 d, const Keys &K, const Params &P, uint32_t seg) {
+    if (P.perturb == 0) return d;
+    // a direction perpendicular to d from a hash of (path, segment, perturbation); antithetic pairs share it with opposite signs
+    uint32_t h = hash32(hash32(hash32(K.gpix * 0x9e3779b9u ^ K.sample) ^ seg) ^ (P.pert_id >> 1));
+    V3 e;
+    e.x = (double)(h & 0xffff) / 65535.0 - 0.5; h = hash32(h);
+    e.y = (double)(h & 0xffff) / 65535.0 - 0.5; h = hash32(h);
+    e.z = (double)(h & 0xffff) / 65535.0 - 0.5;
+    e = e.sub(d.mul(e.dot(d)));
+    const double m = e.mag();
+    if (!(m > 1e-9)) return d;
+    const double s = (P.pert_id & 1u) ? -P.perturb : P.perturb;
+    return d.add(e.mul(s / m)).unit();
+}
+
+void fragile(Path &p, int reason, uint32_t seg) {
+    if (p.reason == R_NONE) { p.reason = reason; p.fseg = (int)seg; }
+}
+
+// Texture walk in f64 on the f64 hit point (rz_device.cuh:481-503): floor(p * (1 / scale)), floor-mod 2 of the sum.  Returns
+// the final texture; `near_edge` is set when a lattice coordinate lies within `dp` (hit-point error) of a cell boundary.
+uint32_t texture_at(const Scene &sc, uint32_t tex, V3 p, double dp, bool &near_edge) {
+    for (int level = 0; level < 8 && sc.textures[tex].kind == 0; level++) {
+        const Texture &t = sc.textures[tex];
+        const double inv = 1.0 / t.scale;
+        int64_t s = 0;
+        for (int ax = 0; ax < 3; ax++) {
+            const double x = p.at(ax) * inv, f = std::floor(x);
+            if (x - f < dp * inv || f + 1.0 - x < dp * inv) near_edge = true;
+            s += (int64_t)f;
+        }
+        tex = (s & 1) == 0 ? t.even : t.odd;
+    }
+    return tex;
+}
+
+// rz_uniform_sphere: z = 1 - 2 u1, angle (u2 - 0.5) 2 pi
+V3 uniform_sphere(double u1, double u2) {
+    const double z = 1.0 - 2.0 * u1, r = std::sqrt(std::fmax(0.0, 1.0 - z * z));
+    const double a = (u2 - 0.5) * 6.283185307179586476925286766559;
+    V3 v; v.x = r * std::cos(a); v.y = r * std::sin(a); v.z = z;
+    return v;
+}
+
+uint64_t fnv(uint64_t h, uint64_t w) { for (int i = 0; i < 8; i++) { h ^= (w >> (8 * i)) & 0xffu; h *= 0x100000001b3ull; } return h; }
+
+void trace(const Keys &K, uint32_t px, uint32_t py, const Params &P, Path &out) {
+    const Scene &sc = *P.sc;
+    const Camera &cam = P.cam;
+    const uint32_t n = (uint32_t)sc.spheres.size();
+    double cu[5];
+    camera_uniforms(K, cu);
+    // Camera (rz_lens_ray, rz_device.cuh:435-454): x = px + (ux - 0.5), y = py + (uy - 0.5); thin lens polar, radius sqrt(ur),
+    // angle (ua - 0.5) 2 pi; dir = px_du x + px_dv y + px_origin - o, normalised; time = ut
+    V3 o = cam.look_from;
+    double o_err = 0;   // f32 error of the origin beyond its own representation: the lens offset's arithmetic
+    if (cam.defocus) {
+        const double rad = std::sqrt(cu[3]), a = (cu[4] - 0.5) * 6.283185307179586476925286766559;
+        const V3 off = cam.defocus_u.mul(rad * std::cos(a)).add(cam.defocus_v.mul(rad * std::sin(a)));
+        o = o.add(off);
+        o_err = DIR_ERR * off.mag();
+    }
+    const double x = (double)px + (cu[0] - 0.5), y = (double)py + (cu[1] - 0.5);
+    const V3 dir = cam.px_du.mul(x).add(cam.px_dv.mul(y)).add(cam.px_origin).sub(o);
+    V3 d = dir.unit();
+    d = perturbed(d, K, P, 0);
+    // the f32 camera: its six vectors rounded, and the sum rounded at the size of its largest term
+    double d_err = DIR_ERR + K_POS * (cam.px_du.mag() * std::fabs(x) + cam.px_dv.mag() * std::fabs(y) + cam.px_origin.mag() + o.mag()) / dir.mag();
+    const double time = cu[2];
+    int self = -1;
+    bool self_out = false;
+    V3 thr = V3::of(1.0);
+    uint32_t seg = 0;
+    // rz_path.cu:149 / rz_search.cuh:405: a depth-0 path ends at once, black, counted as ended_depth (renderer.zig:104-105)
+    if (P.depth == 0) { out.end = E_DEPTH; out.ev.push_back(0xd0); return; }
+    while (true) {
+        // ---- closest hit over every sphere, centre moved to c + v time (rz_sphere_test, rz_consider: rz_device.cuh:404-433)
+        const double o_scale = o.mag();
+        double bt = INF, bt_err = 0, t2 = INF, t2_err = 0;
+        int bk = -1;
+        bool bfar = false;
+        for (uint32_t k = 0; k < n; k++) {
+            const Sphere &s = sc.spheres[k];
+            const V3 C = s.center.origin.add(s.center.dir.mul(time));
+            const V3 oc = C.sub(o);
+            const double b = oc.dot(d);
+            const V3 l = oc.sub(d.mul(b));
+            const double r = s.radius, ll = l.mag();
+            const double occ = oc.mag();
+            // f32 error of the line test and of b: operand roundings at the scale of the numbers involved (the origin, oc, r),
+            // plus the direction error over the distance b to the closest approach, plus the origin's own
+            const double dl = K_POS * (o_scale + std::fmax(occ, r)) + d_err * std::fabs(b) + o_err;
+            if (std::fabs(ll - r) < dl) fragile(out, R_GRAZE, seg);
+            const double nd = ll * ll - r * r;   // the line meets the sphere iff nd < 0
+            if (!(nd < 0)) continue;
+            const double sq = std::sqrt(-nd);
+            const double dt = dl * (1.0 + std::fmin(ll / std::fmax(sq, 1e-300), 1e6));   // roots: sq = sqrt(r^2 - |l|^2) amplifies
+            double t;
+            bool far = false;
+            if ((int)k == self) {
+                // the sphere the ray starts on: only the far root, only while b > 0, never after RZ_SELF_OUT
+                if (self_out) continue;
+                if (std::fabs(b) < dl) fragile(out, R_SELF_B, seg);
+                if (!(b > 0)) continue;
+                t = b + sq; far = true;
+            } else {
+                t = b - sq;
+                if (std::fabs(t - P.t_min) < dt) fragile(out, R_TMIN, seg);
+                if (!(t > P.t_min)) { t = b + sq; far = true; }
+            }
+            if (std::fabs(t - P.t_min) < dt) fragile(out, R_TMIN, seg);
+            if (!(t > P.t_min)) continue;
+            if (t < bt) { t2 = bt; t2_err = bt_err; bt = t; bt_err = dt; bk = (int)k; bfar = far; }
+            else if (t < t2) { t2 = t; t2_err = dt; }
+        }
+        if (bk >= 0 && t2 < INF && t2 - bt < bt_err + t2_err) fragile(out, R_TIE, seg);
+        if (bk < 0) {
+            // ---- sky (rz_sky, rz_device.cuh:474-479): ((1 - t) + (0.5, 0.7, 1.0)) t, t = 0.5 (d.y + 1); clamp [0, 2^20]
+            out.segs++;
+            const double t = 0.5 * (d.y + 1.0), a = 1.0 - t;
+            const double L[3] = {thr.x * (a + 0.5) * t, thr.y * (a + 0.7) * t, thr.z * (a + 1.0) * t};
+            for (int c = 0; c < 3; c++) out.rgb[c] = std::fmin(std::fmax(L[c], 0.0), 1048576.0);
+            out.end = E_SKY;
+            out.ev.push_back(0x5c);
+            return;
+        }
+        out.segs++;
+        // ---- the hit, in f64 (rz_refine_hit, rz_device.cuh:512-546): normal flipped against the ray
+        const Sphere &s = sc.spheres[bk];
+        const Material &m = sc.materials[s.material];
+        const V3 C = s.center.origin.add(s.center.dir.mul(time));
+        const V3 p = o.add(d.mul(bt));
+        V3 nrm = p.sub(C).mul(1.0 / s.radius);
+        const bool front = nrm.dot(d) < 0;
+        if (!front) nrm = nrm.mul(-1);
+        out.hits[m.kind < 3 ? m.kind : 0]++;
+        seg++;
+        double uu[4];
+        bounce_uniforms(K, seg, uu);
+        // hit-point error: the ray's origin and direction errors, along the surface (1 / cos of the incidence)
+        const double cosi = std::fmax(std::fabs(nrm.dot(d)), 1e-3);
+        const double dp = (K_POS * o_scale + d_err * bt + o_err) / cosi + K_POS * p.mag();
+        V3 nd;
+        int branch;
+        uint32_t tex_hit = 0xffffffffu;
+        bool edge = false;
+        // ---- scatter (rz_scatter, rz_device.cuh:566-613)
+        if (m.kind == 0) {
+            const V3 sdir = uniform_sphere(uu[0], uu[1]);
+            if (m.method == 2) {
+                const double sn = sdir.dot(nrm);
+                if (std::fabs(sn) < DOT_TOL) fragile(out, R_FLIP, seg - 1);
+                nd = sn > 0 ? sdir : sdir.mul(-1);
+            } else {
+                const double rad = m.method == 0 ? std::cbrt(uu[2]) : 1.0;
+                V3 t = nrm.add(sdir.mul(rad));
+                const double tt = t.dot(t);
+                if (tt < 1e-10) fragile(out, R_DEGENERATE, seg - 1);
+                if (tt < 1e-12) t = nrm;
+                nd = t.unit();
+            }
+            tex_hit = texture_at(sc, m.texture, p, dp, edge);
+            thr = thr.vmul(sc.textures[tex_hit].color);
+            branch = 0;
+        } else if (m.kind == 1) {
+            V3 r = d.sub(nrm.mul(2.0 * d.dot(nrm)));
+            if (m.fuzz > 0) r = r.add(uniform_sphere(uu[0], uu[1]).mul(std::fmin(m.fuzz, 1.0)));
+            const double rn = r.dot(nrm);
+            if (std::fabs(rn) < DOT_TOL * (1.0 + std::fmin(m.fuzz, 1.0))) fragile(out, R_METAL, seg - 1);
+            if (!(rn > 0)) {
+                out.end = E_ABSORBED;
+                out.ev.push_back(fnv(fnv(0xcbf29ce484222325ull, (uint64_t)bk * 2 + (bfar ? 1 : 0)), 0xab));
+                out.ev.push_back(0xab);
+                return;
+            }
+            nd = r.unit();
+            tex_hit = texture_at(sc, m.texture, p, dp, edge);
+            thr = thr.vmul(sc.textures[tex_hit].color);
+            branch = 1;
+        } else {
+            const double ior = m.ior;
+            const double eta = front ? 1.0 / ior : ior;
+            const double cos_t = std::fmin(-d.dot(nrm), 1.0);
+            const double sin_t = std::sqrt(std::fmax(0.0, 1.0 - cos_t * cos_t));
+            double r0 = (1.0 - eta) / (1.0 + eta);
+            r0 *= r0;
+            const double mm = 1.0 - cos_t;
+            const double schlick = r0 + (1.0 - r0) * (mm * mm * mm * mm * mm);
+            if (std::fabs(eta * sin_t - 1.0) < FRESNEL_TOL) fragile(out, R_TIR, seg - 1);
+            const bool tir = eta * sin_t > 1.0;
+            if (!tir && std::fabs(schlick - uu[0]) < FRESNEL_TOL) fragile(out, R_FRESNEL, seg - 1);
+            if (tir || schlick > uu[0]) {
+                nd = d.sub(nrm.mul(2.0 * d.dot(nrm)));
+                branch = tir ? 2 : 3;
+            } else {
+                const V3 perp = d.add(nrm.mul(cos_t)).mul(eta);
+                const double par = -std::sqrt(std::fmax(0.0, 1.0 - perp.dot(perp)));
+                nd = perp.add(nrm.mul(par));
+                branch = 4;
+            }
+            nd = nd.unit();
+        }
+        if (edge) fragile(out, R_CHECKER, seg - 1);
+        out.ev.push_back(fnv(fnv(fnv(0xcbf29ce484222325ull, (uint64_t)bk * 2 + (bfar ? 1 : 0)), (uint64_t)branch), tex_hit));
+        nd = perturbed(nd, K, P, seg);
+        // RZ_SELF_OUT: the ray leaves its sphere outward by more than 1e-3 (rz_device.cuh:609-611); time is kept
+        const double outd = nd.dot(nrm), so = front ? outd : -outd;
+        if (std::fabs(so - 1e-3) < DOT_TOL) fragile(out, R_SELF_OUT, seg - 1);
+        self_out = so > 1e-3;
+        self = bk;
+        o = p;
+        o_err = 0;
+        d_err = DIR_ERR;
+        d = nd;
+        if (seg >= P.depth) { out.end = E_DEPTH; out.ev.push_back(0xd0); return; }   // rz_search.cuh:405
+    }
+}
+
+}  // namespace replay
+
 }  // namespace
 
 // =====================================================================================
@@ -821,6 +1162,74 @@ uint32_t orc_bvh_export(OrcScene *s, uint32_t max_nodes, double *boxes6, int32_t
     }
     for (size_t i = 0; i < sc.hittables.size(); i++) order[i] = sc.hittables[i].sphere;
     return n;
+}
+
+// ---- path replay (namespace replay above).  The paths of samples [sample_offset, sample_offset + spp) of every pixel of a
+// w x h frame, pixel-major (index (j w + i) spp + s).  sampler: 0 Philox, 1 Sobol, 2 Sobol-RQMC.  t_min: the backend's f32
+// t_min (0 => 1e-4).  perturb: angle of the perturbed replays (0 => REPLAY_PERTURB).  Outputs per path: rgb[3] clamped radiance, y = its Rec. 709 luminance, segs (closest-hit queries),
+// end (0 sky, 1 absorbed, 2 depth), hits[3] per material kind, hash of the event sequence, reason / fseg of the first fragile
+// decision (reason 0: robust), tol = the radiance tolerance of a robust path.  threads == 0 => hardware_concurrency.
+void orc_replay(OrcScene *s, const OrcCamera *cam, uint32_t w, uint32_t h, uint32_t sample_offset, uint32_t spp, uint32_t depth,
+                uint64_t seed, float t_min, int32_t sampler, double perturb, uint32_t threads, double *rgb, double *y, uint32_t *segs, uint8_t *end,
+                uint32_t *hits, uint64_t *hash, uint8_t *reason, int32_t *fseg, double *tol) {
+    using namespace replay;
+    Params P;
+    P.sc = &s->sc;
+    P.cam = toCam(cam);
+    P.depth = depth;
+    P.t_min = t_min > 0 ? (double)t_min : (double)1e-4f;   // include/rayz_cuda.h RzRenderParams.t_min
+    P.perturb = 0; P.pert_id = 0;
+    if (threads == 0) threads = std::max(1u, std::thread::hardware_concurrency());
+    std::atomic<uint32_t> next(0);
+    auto work = [&]() {
+        while (true) {
+            const uint32_t j = next.fetch_add(1);
+            if (j >= h) break;
+            for (uint32_t i = 0; i < w; i++) {
+                for (uint32_t sl = 0; sl < spp; sl++) {
+                    const size_t q = ((size_t)j * w + i) * spp + sl;
+                    const Keys K{(uint32_t)seed, (uint32_t)(seed >> 32), j * w + i, sample_offset + sl, sampler};
+                    Path p;
+                    trace(K, i, j, P, p);
+                    double dev = 0;
+                    for (int pr = 0; pr < 2 * REPLAY_PAIRS; pr++) {
+                        Params Q = P;
+                        Q.perturb = perturb > 0 ? perturb : REPLAY_PERTURB; Q.pert_id = (uint32_t)pr;
+                        Path pp;
+                        trace(K, i, j, Q, pp);
+                        if (pp.ev != p.ev) {
+                            size_t e = 0;
+                            while (e < p.ev.size() && e < pp.ev.size() && p.ev[e] == pp.ev[e]) e++;
+                            fragile(p, R_PERTURB, (uint32_t)e);
+                        }
+                        for (int c = 0; c < 3; c++) dev = std::fmax(dev, std::fabs(pp.rgb[c] - p.rgb[c]));
+                    }
+                    uint64_t hh = 0xcbf29ce484222325ull;
+                    for (uint64_t e : p.ev) hh = fnv(hh, e);
+                    for (int c = 0; c < 3; c++) rgb[3 * q + c] = p.rgb[c];
+                    y[q] = 0.2126 * p.rgb[0] + 0.7152 * p.rgb[1] + 0.0722 * p.rgb[2];
+                    segs[q] = p.segs;
+                    end[q] = (uint8_t)p.end;
+                    for (int c = 0; c < 3; c++) hits[3 * q + c] = p.hits[c];
+                    hash[q] = hh;
+                    reason[q] = (uint8_t)p.reason;
+                    fseg[q] = p.fseg;
+                    const double mx = std::fmax(p.rgb[0], std::fmax(p.rgb[1], p.rgb[2]));
+                    tol[q] = TOL_SAFETY * dev + TOL_REL_PER_SEG * (2.0 * p.segs + 4.0) * mx + TOL_ABS;
+                }
+            }
+        }
+    };
+    std::vector<std::thread> pool;
+    for (uint32_t t = 0; t < threads; t++) pool.emplace_back(work);
+    for (auto &t : pool) t.join();
+}
+
+// The replay's uniforms of one path: camera ux, uy, ut, ur, ua, then u.x, u.y, u.z, u.w of bounces 1..depth (5 + 4 depth).
+void orc_replay_uniforms(uint64_t seed, uint32_t gpix, uint32_t sample, uint32_t depth, int32_t sampler, double *out) {
+    const replay::Keys K{(uint32_t)seed, (uint32_t)(seed >> 32), gpix, sample, sampler};
+    replay::camera_uniforms(K, out);
+    for (uint32_t s = 1; s <= depth; s++) replay::bounce_uniforms(K, s, out + 5 + 4 * (s - 1));
 }
 
 }  // extern "C"

@@ -121,6 +121,114 @@ extern "C" int hostsim_render(const RzScene *sc, const RzCamera *cam, uint32_t w
 }
 
 // ---------------------------------------------------------------------------------------------
+// Path by path, for the f64 replay (oracle Scene.replay, tests/test_replay_cpu.py): the paths of samples [sample_offset,
+// sample_offset + spp) of every pixel, pixel-major, each through the product's camera, sphere test, root rule, refinement,
+// scatter and sky, with the uniforms rz_shade_segment draws (rz_search.cuh:397-401) for sampler 0 (Philox), 1 (Sobol) or
+// 2 (Sobol-RQMC), and the material records as the library packs them (solid and checker-of-two-solids shortcuts,
+// rz_context.cu).  Outputs per path: rgb[3] clamped f32 radiance, segs, end (0 sky, 1 absorbed, 2 depth), hits[3].
+// ---------------------------------------------------------------------------------------------
+extern "C" int hostsim_paths(const RzScene *sc, const RzCamera *cam, uint32_t w, uint32_t h, uint32_t sample_offset, uint32_t spp,
+                             uint32_t max_depth, uint64_t seed, float t_min, int sampler, uint32_t threads, float *out_rgb,
+                             uint32_t *out_segs, uint8_t *out_end, uint32_t *out_hits) {
+    const uint32_t n = sc->n_spheres;
+    std::vector<float4> cr(n), vel(n);
+    std::vector<double4> c64(n), v64(n);
+    std::vector<uint32_t> smat(n);
+    std::vector<int32_t> orig(n);
+    for (uint32_t i = 0; i < n; i++) {
+        const double *c = sc->sphere_center + 3 * i, *v = sc->sphere_velocity + 3 * i; const double r = sc->sphere_radius[i];
+        cr[i] = make_float4((float)c[0], (float)c[1], (float)c[2], -(float)(r * r));
+        vel[i] = make_float4((float)v[0], (float)v[1], (float)v[2], (float)r);
+        c64[i] = make_double4(c[0], c[1], c[2], r); v64[i] = make_double4(v[0], v[1], v[2], 1.0 / r);
+        smat[i] = sc->sphere_material[i]; orig[i] = (int32_t)i;
+    }
+    const uint32_t nm = sc->n_materials, nt = sc->n_textures;
+    std::vector<uint32_t> tk(nt), te(nt), to(nt);
+    std::vector<float4> tc(nt); std::vector<double> ts(nt);
+    for (uint32_t i = 0; i < nt; i++) { tk[i] = sc->tex_kind[i]; te[i] = sc->tex_even[i]; to[i] = sc->tex_odd[i];
+        tc[i] = make_float4((float)sc->tex_color[3*i], (float)sc->tex_color[3*i+1], (float)sc->tex_color[3*i+2], 0); ts[i] = sc->tex_kind[i] == 0 ? 1.0 / sc->tex_scale[i] : 0; }
+    std::vector<RzMatRec> recs(nm);
+    for (uint32_t i = 0; i < nm; i++) {
+        RzMatRec &R = recs[i];
+        R.kind = sc->mat_kind[i]; R.method = sc->mat_method ? sc->mat_method[i] : 2u; R.tex = R.kind == 2u ? 0u : sc->mat_texture[i];
+        R.fuzz = (float)sc->mat_fuzz[i]; R.ior = (float)sc->mat_ior[i];
+        const bool textured = R.kind != 2u && nt > 0;
+        R.solid = textured && tk[R.tex] != 0u;
+        R.checker2 = textured && !R.solid && tk[te[R.tex]] != 0u && tk[to[R.tex]] != 0u;
+        const float4 even = R.solid ? tc[R.tex] : R.checker2 ? tc[te[R.tex]] : make_float4(0, 0, 0, 0), odd = R.checker2 ? tc[to[R.tex]] : make_float4(0, 0, 0, 0);
+        R.color = f3(even.x, even.y, even.z); R.odd = f3(odd.x, odd.y, odd.z);
+        R.inv_scale = R.checker2 ? ts[R.tex] : 0.0;
+    }
+    RzSphereSet S; S.cr = cr.data(); S.vel = vel.data(); S.c64 = c64.data(); S.v64 = v64.data(); S.mat = smat.data(); S.orig = orig.data(); S.n = n; S.n_static = 0; S.n_static_pad = 0; S.n_pad = n;
+    RzTextures T; T.kind = tk.data(); T.color = tc.data(); T.inv_scale = ts.data(); T.even = te.data(); T.odd = to.data();
+    RzCamF32 C;
+    C.look_from = make_float3((float)cam->look_from[0], (float)cam->look_from[1], (float)cam->look_from[2]);
+    C.px_du = make_float3((float)cam->px_du[0], (float)cam->px_du[1], (float)cam->px_du[2]);
+    C.px_dv = make_float3((float)cam->px_dv[0], (float)cam->px_dv[1], (float)cam->px_dv[2]);
+    C.px_origin = make_float3((float)cam->px_origin[0], (float)cam->px_origin[1], (float)cam->px_origin[2]);
+    C.defocus_u = make_float3((float)cam->defocus_u[0], (float)cam->defocus_u[1], (float)cam->defocus_u[2]);
+    C.defocus_v = make_float3((float)cam->defocus_v[0], (float)cam->defocus_v[1], (float)cam->defocus_v[2]);
+    C.defocus = cam->defocus;
+    const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+    if (!(t_min > 0)) t_min = 1e-4f;
+    if (threads == 0) threads = std::max(1u, std::thread::hardware_concurrency());
+    std::atomic<uint32_t> next(0);
+    auto work = [&]() {
+        while (true) {
+            const uint32_t j = next.fetch_add(1);
+            if (j >= h) break;
+            for (uint32_t i = 0; i < w; i++) {
+                const uint32_t gpix = j * w + i;
+                for (uint32_t sl = 0; sl < spp; sl++) {
+                    const size_t q = (size_t)gpix * spp + sl;
+                    const uint32_t sample = sample_offset + sl;
+                    RzRay ray = rz_camera_ray(C, i, j, gpix, sample, k0, k1, sampler);
+                    float3 thr = f3(1, 1, 1), L = f3(0, 0, 0);
+                    uint32_t seg = 0, segs = 0, hits[3] = {0, 0, 0};
+                    uint8_t end = 2;
+                    bool alive = max_depth > 0;
+                    while (alive) {
+                        float bt = 3.0e38f; int bk = -1;
+                        for (uint32_t k = 0; k < n; k++) {
+                            float nb, nd;
+                            rz_sphere_test(cr[k].x, cr[k].y, cr[k].z, vel[k].x, vel[k].y, vel[k].z, cr[k].w, ray.o.x, ray.o.y, ray.o.z, ray.d.x, ray.d.y, ray.d.z, ray.time, nb, nd);
+                            if (nd < 0.0f) consider((int)k, nb, nd, ray.self_k, t_min, bt, bk);
+                        }
+                        segs++;
+                        if (bk < 0) {   // rz_shade_segment's miss branch
+                            const float3 c = thr * rz_sky(ray.d);
+                            L = f3(rz_clamp_radiance(c.x), rz_clamp_radiance(c.y), rz_clamp_radiance(c.z));
+                            end = 0;
+                            break;
+                        }
+                        const int k = bk & ~RZ_FAR_BIT;
+                        const RzHit hit = rz_refine_hit(S, ray, k, (bk & RZ_FAR_BIT) != 0);
+                        const RzMatRec &M = recs[smat[k]];
+                        hits[M.kind < 3u ? M.kind : 0u]++;
+                        seg++;
+                        const uint4 rb = rz_philox(gpix, sample, seg, 0u, k0, k1);
+                        const float2 qq = sampler ? rz_sobol_u01(k0, k1, gpix, rz_pair_bounce(seg), sample, sampler == 2)
+                                                  : make_float2(rz_u01(rb.x >> 8), rz_u01(rb.y >> 8));
+                        const float4 u = make_float4(qq.x, qq.y, rz_u01(rb.z >> 8), rz_u01(rb.w >> 8));
+                        float3 att;
+                        if (!rz_scatter(M, T, hit, k, u, ray, att)) { end = 1; break; }
+                        thr = thr * att;
+                        if (seg >= max_depth) break;
+                    }
+                    out_rgb[3 * q] = L.x; out_rgb[3 * q + 1] = L.y; out_rgb[3 * q + 2] = L.z;
+                    out_segs[q] = segs; out_end[q] = end;
+                    for (int c = 0; c < 3; c++) out_hits[3 * q + c] = hits[c];
+                }
+            }
+        }
+    };
+    std::vector<std::thread> pool;
+    for (uint32_t t = 0; t < threads; t++) pool.emplace_back(work);
+    for (auto &t : pool) t.join();
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Property check of the staged K1's sort key (rz_device.cuh: rz_key_grid / rz_sort_key / rz_key_bounds): for random rays
 // in and around the sphere box, the bounds decoded from a ray's key must contain the ray — origin inside the key's cell
 // box, direction signs equal to the key's octant, exit time from the sphere box below the key's reach bound.  The

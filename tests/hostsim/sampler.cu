@@ -27,3 +27,19 @@ extern "C" void hostsampler_uniforms(uint64_t seed, uint32_t gpix, uint32_t samp
         u[3 + 2 * s] = b.x; u[4 + 2 * s] = b.y;
     }
 }
+
+// The Philox words of one block (rz_philox: counter (gpix, sample, seg, 0), key = seed), and the Sobol or Sobol-RQMC uniforms of
+// one pair (rz_sobol_u01 with pair numbers RZ_PAIR_CAMERA_* / rz_pair_bounce(s) passed by the caller).
+extern "C" void hostsampler_philox(uint64_t seed, uint32_t gpix, uint32_t sample, uint32_t seg, uint32_t *words) {
+    const uint4 r = rz_philox(gpix, sample, seg, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
+    words[0] = r.x; words[1] = r.y; words[2] = r.z; words[3] = r.w;
+}
+extern "C" void hostsampler_sobol_u01(uint64_t seed, uint32_t gpix, uint32_t pair, uint32_t sample, int rqmc, float *u) {
+    const float2 q = rz_sobol_u01((uint32_t)seed, (uint32_t)(seed >> 32), gpix, pair, sample, rqmc != 0);
+    u[0] = q.x; u[1] = q.y;
+}
+// the pair numbers the kernels use: camera jitter, lens, time, then bounce s = 1..n
+extern "C" void hostsampler_pair_numbers(uint32_t n, uint32_t *out) {
+    out[0] = RZ_PAIR_CAMERA_JITTER; out[1] = RZ_PAIR_CAMERA_LENS; out[2] = RZ_PAIR_CAMERA_TIME;
+    for (uint32_t s = 1; s <= n; s++) out[2 + s] = rz_pair_bounce(s);
+}
