@@ -3,7 +3,7 @@
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
-//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc]
+//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc] [--pooled]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -19,6 +19,8 @@
 // --sobol draws the camera and scatter samples from Owen-scrambled Sobol pairs (RZ_RENDER_SOBOL) in every one of these runs,
 // guides included.  --rqmc does the same with two independently scrambled replicates per pixel and the noise estimate they
 // allow (RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS): --noise-target then stops on it; --spp and --max-spp must be even.
+// --pooled (with --noise-target X --adaptive) stops each pixel on an error pooled over its row segment (RZ_RENDER_ADAPTIVE_POOLED),
+// so that X bounds the measured error too; without --adaptive the library refuses it.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -44,7 +46,7 @@ int main(int argc, char **argv) {
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
     const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr;
-    bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false, rqmc = false;
+    bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false, rqmc = false, pooled = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
     for (int i = 2; i < argc; i++) {
@@ -64,6 +66,7 @@ int main(int argc, char **argv) {
         else if (a == "--adaptive") adaptive = true;
         else if (a == "--sobol") sobol = true;
         else if (a == "--rqmc") rqmc = true;
+        else if (a == "--pooled") pooled = true;
         else if (a == "--guides") guides = val();
         else if (a == "--denoise") denoise = val();
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
@@ -88,6 +91,7 @@ int main(int argc, char **argv) {
         tracer.moments = denoise != nullptr;
         tracer.sobol = sobol;
         tracer.rqmc = rqmc;
+        tracer.pooled = pooled;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);

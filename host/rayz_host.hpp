@@ -265,6 +265,7 @@ struct Tracer {
     bool moments = false;         // render with RZ_RENDER_MOMENTS (no pixel changes), so that denoise() can follow
     bool sobol = false;           // RZ_RENDER_SOBOL: Owen-scrambled Sobol camera and scatter samples, in render() and renderGuides()
     bool rqmc = false;            // RZ_RENDER_RQMC (with SOBOL and MOMENTS): two Sobol replicates per pixel, a noise estimate that sees them
+    bool pooled = false;          // RZ_RENDER_ADAPTIVE_POOLED, passed through: with adaptive, each pixel stops on an error pooled over its row segment
     Image denoised;               // rgb8 of the last denoise()
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
@@ -302,6 +303,7 @@ struct Tracer {
         if (moments) p.flags |= RZ_RENDER_MOMENTS;
         if (sobol) p.flags |= RZ_RENDER_SOBOL;
         if (rqmc) p.flags |= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;
+        if (pooled) p.flags |= RZ_RENDER_ADAPTIVE_POOLED;   // the library refuses it without RZ_RENDER_ADAPTIVE
         return p;
     }
 

@@ -218,6 +218,33 @@ typedef struct RzRenderParams {
                                     * rayz_cuda_noise, both tests of rayz_cuda_render_to_noise and the denoiser's v_p use.
                                     * Trade-off: two replicates of n / 2 points carry more variance than one sequence of n points, so
                                     * the frame itself is somewhat noisier than under RZ_RENDER_SOBOL alone; hence a separate flag. */
+#define RZ_RENDER_ADAPTIVE_POOLED 0x40u /* pooled adaptive stopping (DESIGN.md "Adaptive sampling", "Pooled stopping"): honoured
+                                    * by rayz_cuda_render_to_noise together with RZ_RENDER_ADAPTIVE only; without ADAPTIVE, and in
+                                    * rayz_cuda_render, rayz_cuda_render_device and rayz_cuda_render_guides, it is refused with
+                                    * RZ_ERR_INVALID_ARG, the message naming the rule, nothing touched (rayz_cuda_reserve takes it
+                                    * with ADAPTIVE).  The plain rule stops a pixel on its own iid estimate, which after 4 or 16
+                                    * samples is itself very noisy: the pixels that stop early are those whose estimate came out
+                                    * low, and the measured error of the frame is several times the target.  Under this flag a
+                                    * pixel's per-sample variance is shrunk toward its row segment's (the segment of RZ_RENDER_RQMC:
+                                    * the pixels of one global row with x in [64k, 64k + 64), the last one of a row may be shorter).
+                                    * For a pixel with n samples, e its rz_pixel_err (the formula of rayz_cuda_noise), u = n e^2,
+                                    * d = n - 1:
+                                    *   U_S = sum d_i u_i / sum d_i over the segment's pixels with n_i >= 2 (0 if there are none),
+                                    *   e* = sqrt((NU0 U_S + d u) / (NU0 + d) / n)   (+inf while n < 2),  NU0 = 16,
+                                    * and under RZ_RENDER_RQMC e* sqrt(G).  NU0 is the prior's weight in degrees of freedom, chosen
+                                    * by measurement (DESIGN.md).  U_S is frozen like G: a pixel keeps the U_S its last stopping
+                                    * test read, so that a pixel that stopped keeps the error it stopped at while its segment's
+                                    * other pixels take more samples.  e* is what out_err, the summary and n_above of
+                                    * rayz_cuda_noise, the stopping test and the denoiser's v_p use, so max_err <= target unless
+                                    * samples == max_spp holds as written; rayz_cuda_noise, rayz_cuda_pixel_samples and
+                                    * rayz_cuda_denoise after the call read e*.  A pixel's activity now depends on its segment's
+                                    * sums as well as its own (a lucky pixel in a noisy segment cannot stop on a few agreeing
+                                    * samples; a pixel of a clean segment still stops early); segments lie inside a global row,
+                                    * which no shard or device splits, so every count, the image and e* stay shard- and
+                                    * device-invariant.  Costs: 8 bytes per pixel and one double per segment, and one warp per
+                                    * segment before each stopping test (the pass RZ_RENDER_RQMC's gain runs in); the path kernels
+                                    * are those of the plain rule, and more samples are spent where the plain rule stopped too
+                                    * early. */
 
 /* Noise summary of the accumulated frame (rayz_cuda_noise).  Errors are standard errors of the DISPLAYED value
  * (gamma 2, as writePPM shows it) in units of [0, 1]: one 8-bit step is 1/255.  +inf while samples < 2. */

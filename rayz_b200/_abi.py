@@ -20,6 +20,7 @@ DIFFUSE_UNIT_SPHERE, DIFFUSE_UNIT_SPHERE_SURFACE, DIFFUSE_HEMISPHERE = 0, 1, 2
 VARIANT_AUTO, VARIANT_MEGA, VARIANT_WAVEFRONT, VARIANT_BVH = 0, 1, 2, 3
 VARIANTS = {"auto": 0, "mega": 1, "wavefront": 2, "bvh": 3, "mega_single": 4}
 RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE, RENDER_ADAPTIVE, RENDER_SOBOL, RENDER_RQMC = 1, 2, 4, 8, 0x10, 0x20   # RzRenderParams.flags (RZ_RENDER_*)
+RENDER_ADAPTIVE_POOLED = 0x40   # with RENDER_ADAPTIVE in render_to_noise: stop each pixel on an error pooled over its row segment
 
 _dp, _up = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 

@@ -12,9 +12,9 @@
 
 #define RZ_LIST_BLOCK 1024u   // pixels (one per thread) per block of the flag and scatter kernels
 
-// gain (nullable): RZ_RENDER_RQMC's per-pixel gains, as rz_noise_reduce_kernel takes them.
+// gain, pool (nullable): RZ_RENDER_RQMC's per-pixel gains and RZ_RENDER_ADAPTIVE_POOLED's priors, as rz_noise_reduce_kernel takes them.
 __global__ void __launch_bounds__(RZ_LIST_BLOCK) rz_list_flag_kernel(const unsigned long long *__restrict__ accum,
-                                                                     const double *__restrict__ gain,
+                                                                     const double *__restrict__ gain, const double *__restrict__ pool,
                                                                      const uint32_t *__restrict__ n_px, uint32_t n_local_px,
                                                                      uint32_t n_cur, double target, uint32_t *__restrict__ mask,
                                                                      uint32_t *__restrict__ block_count) {
@@ -23,7 +23,7 @@ __global__ void __launch_bounds__(RZ_LIST_BLOCK) rz_list_flag_kernel(const unsig
     bool active = false;
     if (lp < n_local_px && n_px[lp] == n_cur) {
         const unsigned long long *q = accum + (size_t)lp * 4;
-        active = (double)(float)rz_pixel_err_of(q, n_cur, gain, lp) > target;
+        active = (double)(float)rz_pixel_err_of(q, n_cur, gain, pool, lp) > target;
     }
     const uint32_t m = __ballot_sync(0xffffffffu, active);
     if (lane == 0) {
@@ -107,14 +107,15 @@ extern "C" size_t rz_list_scratch_words(uint32_t n_local_px) { return (size_t)rz
 extern "C" size_t rz_list_count_word(uint32_t n_local_px) { return (size_t)rz_list_blocks(n_local_px) * 33u; }
 
 // The active pixels of this device before the next round: list <- every local pixel with n_px == n_cur and error > target,
-// in increasing order; their counts grow by `add`; scratch[rz_list_count_word(n_local_px)] <- the list length.  gain
-// (nullable): RZ_RENDER_RQMC's per-pixel gains, so that the error is the one rayz_cuda_noise shows.
-extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, const double *gain, uint32_t *n_px,
+// in increasing order; their counts grow by `add`; scratch[rz_list_count_word(n_local_px)] <- the list length.  gain, pool
+// (nullable): RZ_RENDER_RQMC's per-pixel gains and RZ_RENDER_ADAPTIVE_POOLED's priors, so that the error is the one
+// rayz_cuda_noise shows.
+extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, const double *gain, const double *pool, uint32_t *n_px,
                                             uint32_t n_local_px, uint32_t n_cur, uint32_t add,
                                             float target, uint32_t *list, uint32_t *scratch, cudaStream_t stream) {
     const uint32_t nb = rz_list_blocks(n_local_px);
     uint32_t *mask = scratch, *block = scratch + (size_t)nb * 32u, *total = scratch + rz_list_count_word(n_local_px);
-    if (nb) rz_list_flag_kernel<<<nb, RZ_LIST_BLOCK, 0, stream>>>(accum, gain, n_px, n_local_px, n_cur, (double)target, mask, block);
+    if (nb) rz_list_flag_kernel<<<nb, RZ_LIST_BLOCK, 0, stream>>>(accum, gain, pool, n_px, n_local_px, n_cur, (double)target, mask, block);
     rz_list_scan_kernel<<<1, 1024, 0, stream>>>(block, nb, total);
     if (nb) rz_list_scatter_kernel<<<nb, RZ_LIST_BLOCK, 0, stream>>>(mask, block, n_local_px, add, n_px, list);
     return cudaGetLastError();

@@ -108,8 +108,10 @@ struct Dev {
     DBuf<float4> t_color;
     DBuf<double> t_inv_scale;
     DBuf<unsigned long long> accum;   // + RZ_RENDER_RQMC's replicate sums behind the accumulators (rz_rep_offset)
-    DBuf<double> gain;                // RZ_RENDER_RQMC: the segment gains of the local rows (rz_rqmc_gain_kernel)
-    DBuf<double> px_gain;             // RZ_RENDER_RQMC: every local pixel's gain, frozen when an adaptive pixel stops (rz_rqmc_gain_kernel)
+    DBuf<double> gain;                // RZ_RENDER_RQMC: the segment gains of the local rows (rz_segment_kernel)
+    DBuf<double> px_gain;             // RZ_RENDER_RQMC: every local pixel's gain, frozen when an adaptive pixel stops (rz_segment_kernel)
+    DBuf<double> pool;                // RZ_RENDER_ADAPTIVE_POOLED: the segment priors U_S of the local rows (rz_segment_kernel)
+    DBuf<double> px_pool;             // RZ_RENDER_ADAPTIVE_POOLED: every local pixel's U_S, frozen when it stops (rz_segment_kernel)
     // staged K1, one set per side (passes alternate between two streams): q1 = after the camera segment, q2 = after the second
     DBuf<float4> q1[2], q2[2];
     DBuf<unsigned short> keys[2];
@@ -182,6 +184,7 @@ struct AccumRecord {
     bool pending = false;   // enqueued by rayz_cuda_render_device(sync = 0): the device error words are not checked yet
     Frame frame;
     uint32_t max_depth = 0, moments = 0, sobol = 0, rqmc = 0;
+    uint32_t pooled = 0;       // RZ_RENDER_ADAPTIVE_POOLED: every consumer of the error reads the pooled e* (Dev::px_pool)
     uint64_t seed = 0;
     float t_min = 0;
     RzCamera cam{};
@@ -906,6 +909,10 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
                            : (p->sample_offset & 1u) ? "RZ_RENDER_RQMC requires an even sample_offset (two replicates)" : nullptr;
         if (rule) { P.refused = true; return rz_fail(RZ_ERR_INVALID_ARG, "%s: %s", who, rule); }
     }
+    if ((p->flags & RZ_RENDER_ADAPTIVE_POOLED) && !(p->flags & RZ_RENDER_ADAPTIVE)) {
+        P.refused = true;
+        return rz_fail(RZ_ERR_INVALID_ARG, "%s: RZ_RENDER_ADAPTIVE_POOLED requires RZ_RENDER_ADAPTIVE (rayz_cuda_render_to_noise only)", who);
+    }
 
     if (cam) {
         AccumRecord &next = P.next;
@@ -913,6 +920,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         next.max_depth = p->max_depth; next.moments = (p->flags & RZ_RENDER_MOMENTS) ? 1u : 0u; next.seed = p->seed;
         next.sobol = (p->flags & RZ_RENDER_SOBOL) ? 1u : 0u;
         next.rqmc = (p->flags & RZ_RENDER_RQMC) ? 1u : 0u;
+        next.pooled = (p->flags & RZ_RENDER_ADAPTIVE_POOLED) ? 1u : 0u;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
         next.adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
@@ -1002,6 +1010,9 @@ static int alloc_render(RzContext *ctx, RenderPlan &P) {
         if ((rc = D.accum.alloc((size_t)dp.n_tiles * 32u * (rqmc ? 6u : 4u)))) return rc;
         if (D.accum.p != held) ctx->acc.valid = false;   // grown (a reserve for RZ_RENDER_RQMC of the same frame): the sums are gone
         if (rqmc && ((rc = D.gain.alloc(rz_rqmc_gain_words(n_local, P.frame.width))) || (rc = D.px_gain.alloc(n_local)))) return rc;
+        if ((P.p->flags & RZ_RENDER_ADAPTIVE_POOLED) &&
+            ((rc = D.pool.alloc(rz_rqmc_gain_words(n_local, P.frame.width))) || (rc = D.px_pool.alloc(n_local))))
+            return rc;
         if ((rc = D.counter.alloc(16)) || (rc = D.errword.alloc(4))) return rc;
         if ((rc = D.stats.alloc(3))) return rc;   // [0] whole render / primary kernel, [1] sorted stages, [2] persistent tail kernel
         if (P.staged && n_local > 0) {
@@ -1138,27 +1149,32 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
 
 // The resolve kernel's arguments for device d's n_local pixels of the accumulated frame A: its sums, over each pixel's own
 // count when A is adaptive, scattered band by band into the gather root's rows.  Every output starts null.  Under RZ_RENDER_RQMC
-// out_err reads the segment gains, which rqmc_gain must have enqueued before.
+// and RZ_RENDER_ADAPTIVE_POOLED out_err reads the segment gains and priors, which segment_pass must have enqueued before.
 static RzResolveArgs resolve_args(const RzContext *ctx, uint32_t d, const AccumRecord &A, uint32_t n_local) {
     const Dev &D = ctx->devs[d];
     RzResolveArgs r{};
     r.accum = D.accum.p;
     r.n_px = A.adaptive ? D.n_px.p : nullptr;
     r.gain = A.rqmc ? D.px_gain.p : nullptr;
+    r.pool = A.pooled ? D.px_pool.p : nullptr;
     r.n_local_px = n_local; r.width = A.frame.width; r.spp = (uint32_t)A.samples;
     r.dev_index = d; r.dev_count = (uint32_t)ctx->devs.size(); r.band_rows = A.frame.band;
     return r;
 }
 
-// RZ_RENDER_RQMC: device d's gains of the accumulated frame A, on its stream, before any consumer of the error (the resolve's
-// out_err, the noise reduction, the adaptive flags): the segment gains, copied to the pixels whose count is A's largest (every
-// pixel of a uniform frame; the pixels still sampled of an adaptive one).  The per-pixel gains those consumers take, or null.
-static int rqmc_gain(RzContext *ctx, uint32_t d, const AccumRecord &A, uint32_t n_local, const double **gain = nullptr) {
+// RZ_RENDER_RQMC and RZ_RENDER_ADAPTIVE_POOLED: device d's segment records of the accumulated frame A, in one launch on its
+// stream, before any consumer of the error (the resolve's out_err, the noise reduction, the adaptive flags): the segment gains
+// and priors U_S, copied to the pixels whose count is A's largest (every pixel of a uniform frame; the pixels still sampled of an
+// adaptive one).  The per-pixel gains and priors those consumers take, or null.
+static int segment_pass(RzContext *ctx, uint32_t d, const AccumRecord &A, uint32_t n_local, const double **gain = nullptr,
+                        const double **pool = nullptr) {
     Dev &D = ctx->devs[d];
     if (gain) *gain = A.rqmc ? D.px_gain.p : nullptr;
-    if (!A.rqmc) return RZ_OK;
-    RZ_CUDA(rz_launch_rqmc_gain(D.accum.p, D.accum.p + rz_rep_offset(n_local), A.adaptive ? D.n_px.p : nullptr, (uint32_t)A.samples,
-                                n_local, A.frame.width, D.gain.p, D.px_gain.p, D.stream));
+    if (pool) *pool = A.pooled ? D.px_pool.p : nullptr;
+    if (!A.rqmc && !A.pooled) return RZ_OK;
+    RZ_CUDA(rz_launch_segment_pass(D.accum.p, A.rqmc ? D.accum.p + rz_rep_offset(n_local) : nullptr, A.adaptive ? D.n_px.p : nullptr,
+                                   (uint32_t)A.samples, n_local, A.frame.width, A.rqmc ? D.gain.p : nullptr, A.rqmc ? D.px_gain.p : nullptr,
+                                   A.pooled ? D.pool.p : nullptr, A.pooled ? D.px_pool.p : nullptr, D.stream));
     return RZ_OK;
 }
 
@@ -1270,8 +1286,11 @@ extern "C" int rayz_cuda_reserve(RzContext *ctx, const RzRenderParams *p) {
     return sync_devices(ctx);
 }
 
-// RZ_RENDER_ADAPTIVE needs the rounds of rayz_cuda_render_to_noise; a single render cannot honour it.
+// RZ_RENDER_ADAPTIVE (and RZ_RENDER_ADAPTIVE_POOLED with it) needs the rounds of rayz_cuda_render_to_noise; a single render
+// cannot honour it.
 static int refuse_adaptive(const RzRenderParams *p) {
+    if (p && (p->flags & RZ_RENDER_ADAPTIVE_POOLED))
+        return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ADAPTIVE_POOLED is honoured by rayz_cuda_render_to_noise with RZ_RENDER_ADAPTIVE only");
     if (p && (p->flags & RZ_RENDER_ADAPTIVE)) return rz_fail(RZ_ERR_INVALID_ARG, "render: RZ_RENDER_ADAPTIVE is honoured by rayz_cuda_render_to_noise only");
     return RZ_OK;
 }
@@ -1378,14 +1397,14 @@ extern "C" int rayz_cuda_noise(RzContext *ctx, float target, float *out_err, RzN
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
         if ((rc = D.noise_part.alloc(RZ_NOISE_GRID))) return rc;
-        const double *gain;
-        if ((rc = rqmc_gain(ctx, d, *A, sp.n_local[d], &gain))) return rc;
+        const double *gain, *pool;
+        if ((rc = segment_pass(ctx, d, *A, sp.n_local[d], &gain, &pool))) return rc;
         if (out_err) {
             RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
             r.out_err = D0.out_err.p;
             RZ_CUDA(rz_launch_resolve(&r, D.stream));
         }
-        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A->adaptive ? D.n_px.p : nullptr, gain, sp.n_local[d], (uint32_t)A->samples,
+        RZ_CUDA(rz_launch_noise_reduce(D.accum.p, A->adaptive ? D.n_px.p : nullptr, gain, pool, sp.n_local[d], (uint32_t)A->samples,
                                        (double)target, D.noise_part.p, D.stream));
     }
     double sum = 0, sum2 = 0, mx = 0;
@@ -1448,6 +1467,8 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
     if (!ctx) return rz_fail(RZ_ERR_INVALID_ARG, "guides: NULL argument");
     ctx->guides.valid = false;   // until this call succeeds
     if (!cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "guides: NULL argument");
+    if (p->flags & RZ_RENDER_ADAPTIVE_POOLED)
+        return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_ADAPTIVE_POOLED is honoured by rayz_cuda_render_to_noise with RZ_RENDER_ADAPTIVE only");
     if (p->flags & (RZ_RENDER_ACCUMULATE | RZ_RENDER_ADAPTIVE))
         return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_ACCUMULATE and RZ_RENDER_ADAPTIVE do not apply to guide buffers");
     RenderPlan P;
@@ -1532,7 +1553,7 @@ extern "C" int rayz_cuda_denoise(RzContext *ctx, const RzDenoiseParams *dp, floa
     for (uint32_t d = 0; d < ND; d++) {
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        if (filter && (rc = rqmc_gain(ctx, d, *A, sp.n_local[d]))) return rc;
+        if (filter && (rc = segment_pass(ctx, d, *A, sp.n_local[d]))) return rc;
         RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
         r.out_linear = D0.dn_linear.p;
         if (filter) r.out_err = D0.dn_err.p;
@@ -1564,9 +1585,9 @@ static int build_pixel_lists(RzContext *ctx, uint32_t n_cur, uint32_t add, float
     for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {   // every device enqueues before the first wait
         Dev &D = ctx->devs[d];
         RZ_CUDA(cudaSetDevice(D.id));
-        const double *gain;
-        if (const int rc = rqmc_gain(ctx, d, ctx->acc, sp.n_local[d], &gain)) return rc;
-        RZ_CUDA(rz_launch_pixel_list(D.accum.p, gain, D.n_px.p, sp.n_local[d], n_cur, add, target, D.px_list.p,
+        const double *gain, *pool;
+        if (const int rc = segment_pass(ctx, d, ctx->acc, sp.n_local[d], &gain, &pool)) return rc;
+        RZ_CUDA(rz_launch_pixel_list(D.accum.p, gain, pool, D.n_px.p, sp.n_local[d], n_cur, add, target, D.px_list.p,
                                      D.list_scratch.p, D.stream));
         RZ_CUDA(cudaMemcpyAsync(&n_list[d], D.list_scratch.p + rz_list_count_word(sp.n_local[d]), sizeof(uint32_t), cudaMemcpyDeviceToHost, D.stream));
     }

@@ -261,9 +261,40 @@ RZ_HD double rz_pixel_err_rqmc(unsigned long long q0, unsigned long long q1, uns
     if (n < 2u) return INFINITY;
     return rz_pixel_err(q0, q1, q2, q3, n) * sqrt(gain);
 }
-// the error a consumer shows: rz_pixel_err, or under RZ_RENDER_RQMC (gain != null: one gain per local pixel, rz_rqmc_gain_kernel)
-// rz_pixel_err_rqmc with local pixel lp's gain
-RZ_HD double rz_pixel_err_of(const unsigned long long *q, uint32_t n, const double *gain, uint32_t lp) {
+// RZ_RENDER_ADAPTIVE_POOLED (include/rayz_cuda.h, DESIGN.md "Pooled stopping"): a pixel's per-sample displayed variance
+// u = n e^2 (e: rz_pixel_err) is shrunk toward its RQMC segment's, U_S = sum d_i u_i / sum d_i over the segment's pixels with
+// n_i >= 2, d = n - 1, with the weight of RZ_POOL_NU0 degrees of freedom:
+//   e* = sqrt((NU0 U_S + d u) / (NU0 + d) / n)   (+inf while n < 2),   under RZ_RENDER_RQMC e* sqrt(G).
+// U_S is the one a pixel's last stopping test read, as for G (rz_segment_kernel freezes it).
+#define RZ_POOL_NU0 16.0
+// u = s^2 / (4 max(Ybar, RZ_NOISE_Y_FLOOR)) = n e^2 with rz_pixel_err's s^2 and Ybar; 0 while n < 2
+RZ_HD double rz_pixel_u(unsigned long long q0, unsigned long long q1, unsigned long long q2, unsigned long long q3, uint32_t n) {
+    if (n < 2u) return 0.0;
+    const double s = 2.3283064365386962890625e-10, inv = 1.0 / (double)n;   // 2^-32
+    const double y = (0.2126 * (double)q0 + 0.7152 * (double)q1 + 0.0722 * (double)q2) * s * inv;
+    const double s2 = fmax(0.0, (double)q3 * s * inv - y * y) * ((double)n / (double)(n - 1u));
+    return s2 / (4.0 * fmax(y, RZ_NOISE_Y_FLOOR));
+}
+// U_S of a segment from its sums of d u and d: 0 when no pixel has two samples
+RZ_HD double rz_pool_u(double sum_du, double sum_d) { return sum_d > 0.0 ? sum_du / sum_d : 0.0; }
+// e* of a pixel whose segment's (frozen) prior is pool_u
+RZ_HD double rz_pixel_err_pooled(unsigned long long q0, unsigned long long q1, unsigned long long q2, unsigned long long q3, uint32_t n,
+                                 double pool_u) {
+    if (n < 2u) return INFINITY;
+    const double d = (double)(n - 1u);
+    return sqrt((RZ_POOL_NU0 * pool_u + d * rz_pixel_u(q0, q1, q2, q3, n)) / (RZ_POOL_NU0 + d) / (double)n);
+}
+// e* sqrt(G): RZ_RENDER_ADAPTIVE_POOLED over RZ_RENDER_RQMC; +inf while n < 2
+RZ_HD double rz_pixel_err_pooled_rqmc(unsigned long long q0, unsigned long long q1, unsigned long long q2, unsigned long long q3, uint32_t n,
+                                      double pool_u, double gain) {
+    if (n < 2u) return INFINITY;
+    return rz_pixel_err_pooled(q0, q1, q2, q3, n, pool_u) * sqrt(gain);
+}
+// the error a consumer shows: rz_pixel_err, or under RZ_RENDER_RQMC (gain != null: one gain per local pixel, rz_segment_kernel)
+// rz_pixel_err_rqmc with local pixel lp's gain; under RZ_RENDER_ADAPTIVE_POOLED (pool != null: one frozen U_S per local pixel)
+// the pooled forms
+RZ_HD double rz_pixel_err_of(const unsigned long long *q, uint32_t n, const double *gain, const double *pool, uint32_t lp) {
+    if (pool) return gain ? rz_pixel_err_pooled_rqmc(q[0], q[1], q[2], q[3], n, pool[lp], gain[lp]) : rz_pixel_err_pooled(q[0], q[1], q[2], q[3], n, pool[lp]);
     return gain ? rz_pixel_err_rqmc(q[0], q[1], q[2], q[3], n, gain[lp]) : rz_pixel_err(q[0], q[1], q[2], q[3], n);
 }
 

@@ -26,7 +26,7 @@ struct RzIdsArgs {
 
 extern "C" cudaError_t rz_launch_ids(const RzIdsArgs *a, cudaStream_t stream);
 
-// ------------------------------------------------------------------------------ K5 resolve, noise, RQMC gain, K6 (rz_misc.cu)
+// ------------------------------------------------------------------------------ K5 resolve, noise, segment pass, K6 (rz_misc.cu)
 struct RzResolveArgs {
     const unsigned long long *accum;  // [n_local_px][4]
     float4 *out_linear;               // nullable
@@ -34,7 +34,8 @@ struct RzResolveArgs {
     float *out_err;                   // nullable: displayed-value standard error per pixel (needs slot 3, RZ_RENDER_MOMENTS)
     uint32_t *out_spp;                // nullable: the pixel's sample count (rayz_cuda_pixel_samples)
     const uint32_t *n_px;             // nullable: per-pixel sample counts of an adaptive frame (rz_adaptive.cu); null: spp
-    const double *gain;               // nullable: RZ_RENDER_RQMC's per-pixel gains (rz_rqmc_gain_kernel); out_err is then rz_pixel_err_rqmc
+    const double *gain;               // nullable: RZ_RENDER_RQMC's per-pixel gains (rz_segment_kernel); out_err is then rz_pixel_err_rqmc
+    const double *pool;               // nullable: RZ_RENDER_ADAPTIVE_POOLED's per-pixel priors (rz_segment_kernel); out_err is then pooled
     uint32_t n_local_px, width;
     uint32_t spp;                     // samples summed in the accumulators (cumulative over RZ_RENDER_ACCUMULATE batches)
     // local row lr of this device -> destination row ((lr / band) * dev_count + dev_index) * band + lr % band
@@ -45,17 +46,20 @@ struct RzResolveArgs {
 struct RzNoisePartial { double sum, sum2, max; unsigned long long above; };
 
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain,
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain, const double *pool,
                                               uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *out, cudaStream_t stream);
 extern "C" size_t rz_rqmc_gain_words(uint32_t n_local_px, uint32_t width);
 extern "C" cudaError_t rz_launch_rqmc_gain(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
                                            uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_segment_pass(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
+                                              uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, double *seg_pool,
+                                              double *px_pool, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_ffma_peak(float *sink, int grid, int iters, int mode, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------ adaptive pixel lists (rz_adaptive.cu)
 extern "C" size_t rz_list_scratch_words(uint32_t n_local_px);
 extern "C" size_t rz_list_count_word(uint32_t n_local_px);
-extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, const double *gain, uint32_t *n_px,
+extern "C" cudaError_t rz_launch_pixel_list(const unsigned long long *accum, const double *gain, const double *pool, uint32_t *n_px,
                                             uint32_t n_local_px, uint32_t n_cur, uint32_t add,
                                             float target, uint32_t *list, uint32_t *scratch, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_fill_u32(uint32_t *p, uint32_t n, uint32_t v, cudaStream_t stream);

@@ -1,4 +1,4 @@
-// rz_misc.cu — K5 resolve/quantise and K6 FP32 peak microbenchmark.
+// rz_misc.cu — K5 resolve/quantise, the noise summary, the segment pass and K6 FP32 peak microbenchmark.
 
 // ---------------------------------------------------------------------------------------------
 // K5.  Fixed-point accumulators -> linear float4 + gamma-2 RGB8.
@@ -9,11 +9,11 @@
 // Output rows may live on ANOTHER GPU (peer pointers): with out_row_stride/out_row_offset the
 // kernel scatters this device's compact band-interleaved rows straight into the gather root's
 // full-shard buffers over NVLink, i.e. resolve and gather are one kernel.
-// The same kernel writes the per-pixel noise estimate (out_err: rz_pixel_err of the four slots) and the pixels' sample counts
+// The same kernel writes the per-pixel noise estimate (out_err: rz_pixel_err_of the four slots, with the gain and prior when given) and the pixels' sample counts
 // (out_spp) when asked.  An adaptive frame divides each pixel by its own count (n_px), in the same f64 arithmetic: a pixel
 // with c samples resolves exactly as the same pixel of a uniform c-spp render.
 // ---------------------------------------------------------------------------------------------
-#include "rz_device.cuh"   // rz_pixel_err, rz_quantise_rgb8
+#include "rz_device.cuh"   // rz_pixel_err_of, rz_quantise_rgb8
 #include "rz_launch.h"     // RzResolveArgs, RzNoisePartial
 
 __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) {
@@ -29,10 +29,7 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
     }
     const uint32_t n = a.n_px ? a.n_px[lp] : a.spp;
     if (a.out_spp) a.out_spp[dst] = n;
-    if (a.out_err) {
-        const unsigned long long q3 = a.accum[(size_t)lp * 4 + 3];
-        a.out_err[dst] = (float)(a.gain ? rz_pixel_err_rqmc(q0.x, q0.y, q1, q3, n, a.gain[lp]) : rz_pixel_err(q0.x, q0.y, q1, q3, n));
-    }
+    if (a.out_err) a.out_err[dst] = (float)rz_pixel_err_of(a.accum + (size_t)lp * 4, n, a.gain, a.pool, lp);
     const double inv = 1.0 / (double)n;
     const double s = 2.3283064365386962890625e-10;  // 2^-32
     const double r = (double)q0.x * s * inv, g = (double)q0.y * s * inv, b = (double)q1 * s * inv;
@@ -53,16 +50,17 @@ extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t st
 // ---------------------------------------------------------------------------------------------
 
 // n_px (nullable): per-pixel sample counts of an adaptive frame, else every pixel has n samples.  gain (nullable): RZ_RENDER_RQMC's
-// per-pixel gains.
+// per-pixel gains.  pool (nullable): RZ_RENDER_ADAPTIVE_POOLED's per-pixel frozen priors U_S.
 __global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned long long *__restrict__ accum, const uint32_t *__restrict__ n_px,
-                                                              const double *__restrict__ gain, uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *__restrict__ out) {
+                                                              const double *__restrict__ gain, const double *__restrict__ pool, uint32_t n_local_px,
+                                                              uint32_t n, double target, RzNoisePartial *__restrict__ out) {
     __shared__ double s_sum[256], s_sum2[256], s_max[256];
     __shared__ unsigned long long s_above[256];
     double sum = 0, sum2 = 0, mx = 0;
     unsigned long long above = 0;
     for (uint32_t lp = blockIdx.x * 256u + threadIdx.x; lp < n_local_px; lp += RZ_NOISE_GRID * 256u) {
         const unsigned long long *q = accum + (size_t)lp * 4;
-        const double e = (double)(float)rz_pixel_err_of(q, n_px ? n_px[lp] : n, gain, lp);   // the value out_err shows
+        const double e = (double)(float)rz_pixel_err_of(q, n_px ? n_px[lp] : n, gain, pool, lp);   // the value out_err shows
         sum += e; sum2 += e * e; mx = fmax(mx, e); above += e > target ? 1u : 0u;
     }
     s_sum[threadIdx.x] = sum; s_sum2[threadIdx.x] = sum2; s_max[threadIdx.x] = mx; s_above[threadIdx.x] = above;
@@ -77,54 +75,79 @@ __global__ void __launch_bounds__(256) rz_noise_reduce_kernel(const unsigned lon
     if (threadIdx.x == 0) out[blockIdx.x] = RzNoisePartial{s_sum[0], s_sum2[0], s_max[0], s_above[0]};
 }
 
-extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain,
+extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain, const double *pool,
                                               uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *out, cudaStream_t stream) {
-    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, gain, n_local_px, n, target, out);
+    rz_noise_reduce_kernel<<<RZ_NOISE_GRID, 256, 0, stream>>>(accum, n_px, gain, pool, n_local_px, n, target, out);
     return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------------------------------------
-// RZ_RENDER_RQMC: the gain G of every segment of the device's local rows (rz_rqmc_gain of the segment's sums of V_rep and V_iid),
-// into seg_gain[row][rz_rqmc_segments(width)], and into px_gain[lp] for every pixel whose count is n, the frame's largest: every
-// pixel of a uniform frame; of an adaptive one, the pixels the next stopping test reads.  A pixel that stopped keeps the gain its
-// test read, so its error stays what the test saw while its segment's other pixels take more samples.  One warp per segment:
-// lane k adds its pixels x0 + k, x0 + k + 32 in that order, then a fixed xor tree that leaves the sums in every lane; no
-// floating-point atomics, so the gain is a function of the segment's sums only, wherever the row renders.
+// The segment pass: per segment of the device's local rows (RZ_RQMC_SEGMENT pixels of one row, rz_rqmc_segment_of), whichever
+// of two records the frame needs, into [row][rz_rqmc_segments(width)] and per pixel:
+//   RZ_RENDER_RQMC (rep != null): the gain G (rz_rqmc_gain of the segment's sums of V_rep and V_iid) -> seg_gain, px_gain;
+//   RZ_RENDER_ADAPTIVE_POOLED (seg_pool != null): the prior U_S (rz_pool_u of the sums of d u and d over the pixels with
+//   n >= 2) -> seg_pool, px_pool.
+// The per-pixel copies go to every pixel whose count is n, the frame's largest: every pixel of a uniform frame; of an adaptive
+// one, the pixels the next stopping test reads.  A pixel that stopped keeps the gain and prior its test read, so its error stays
+// what the test saw while its segment's other pixels take more samples.  One warp per segment: lane k adds its pixels x0 + k,
+// x0 + k + 32 in that order, then a fixed xor tree that leaves the sums in every lane; no floating-point atomics, so both
+// records are functions of the segment's sums only, wherever the row renders.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) rz_rqmc_gain_kernel(const unsigned long long *__restrict__ accum, const unsigned long long *__restrict__ rep,
-                                                           const uint32_t *__restrict__ n_px, uint32_t n, uint32_t n_local_px, uint32_t width,
-                                                           double *__restrict__ seg_gain, double *__restrict__ px_gain) {
+__global__ void __launch_bounds__(128) rz_segment_kernel(const unsigned long long *__restrict__ accum, const unsigned long long *__restrict__ rep,
+                                                         const uint32_t *__restrict__ n_px, uint32_t n, uint32_t n_local_px, uint32_t width,
+                                                         double *__restrict__ seg_gain, double *__restrict__ px_gain,
+                                                         double *__restrict__ seg_pool, double *__restrict__ px_pool) {
     const uint32_t nseg = rz_rqmc_segments(width), rows = n_local_px / width;
     const uint32_t seg = blockIdx.x * 4u + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
     if (seg >= rows * nseg) return;   // the whole warp
     const uint32_t lr = seg / nseg, x0 = (seg - lr * nseg) * RZ_RQMC_SEGMENT, x1 = min(x0 + RZ_RQMC_SEGMENT, width);
-    double v_rep = 0.0, v_iid = 0.0;
+    double v_rep = 0.0, v_iid = 0.0, du = 0.0, dd = 0.0;
     for (uint32_t x = x0 + lane; x < x1; x += 32u) {
         const uint32_t lp = lr * width + x, c = n_px ? n_px[lp] : n;
         const unsigned long long *q = accum + (size_t)lp * 4;
-        v_rep += rz_pixel_var_rep(rep[(size_t)lp * 2], rep[(size_t)lp * 2 + 1], c);
-        v_iid += rz_pixel_var_iid(q[0], q[1], q[2], q[3], c);
+        if (rep) {
+            v_rep += rz_pixel_var_rep(rep[(size_t)lp * 2], rep[(size_t)lp * 2 + 1], c);
+            v_iid += rz_pixel_var_iid(q[0], q[1], q[2], q[3], c);
+        }
+        if (seg_pool && c >= 2u) {
+            const double d = (double)(c - 1u);
+            du += d * rz_pixel_u(q[0], q[1], q[2], q[3], c);
+            dd += d;
+        }
     }
     for (int o = 16; o > 0; o >>= 1) {
         v_rep += __shfl_xor_sync(0xffffffffu, v_rep, o);
         v_iid += __shfl_xor_sync(0xffffffffu, v_iid, o);
+        du += __shfl_xor_sync(0xffffffffu, du, o);
+        dd += __shfl_xor_sync(0xffffffffu, dd, o);
     }
-    const double g = rz_rqmc_gain(v_rep, v_iid);
-    if (lane == 0) seg_gain[seg] = g;
+    const double g = rz_rqmc_gain(v_rep, v_iid), u = rz_pool_u(du, dd);
+    if (lane == 0) {
+        if (rep) seg_gain[seg] = g;
+        if (seg_pool) seg_pool[seg] = u;
+    }
     for (uint32_t x = x0 + lane; x < x1; x += 32u) {
         const uint32_t lp = lr * width + x;
-        if (!n_px || n_px[lp] == n) px_gain[lp] = g;
+        if (n_px && n_px[lp] != n) continue;
+        if (rep) px_gain[lp] = g;
+        if (seg_pool) px_pool[lp] = u;
     }
 }
 
-// Doubles of the segment-gain buffer for n_local_px pixels in rows of `width` (px_gain: n_local_px doubles).
+// Doubles of a per-segment buffer for n_local_px pixels in rows of `width` (the per-pixel copies: n_local_px doubles).
 extern "C" size_t rz_rqmc_gain_words(uint32_t n_local_px, uint32_t width) { return width ? (size_t)(n_local_px / width) * rz_rqmc_segments(width) : 0; }
+extern "C" cudaError_t rz_launch_segment_pass(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
+                                              uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, double *seg_pool,
+                                              double *px_pool, cudaStream_t stream) {
+    const size_t segs = rz_rqmc_gain_words(n_local_px, width);
+    if (segs == 0 || (!rep && !seg_pool)) return cudaSuccess;
+    rz_segment_kernel<<<(unsigned)((segs + 3) / 4), 128, 0, stream>>>(accum, rep, n_px, n, n_local_px, width, seg_gain, px_gain, seg_pool, px_pool);
+    return cudaGetLastError();
+}
+// The gains alone (RZ_RENDER_RQMC without RZ_RENDER_ADAPTIVE_POOLED).
 extern "C" cudaError_t rz_launch_rqmc_gain(const unsigned long long *accum, const unsigned long long *rep, const uint32_t *n_px, uint32_t n,
                                            uint32_t n_local_px, uint32_t width, double *seg_gain, double *px_gain, cudaStream_t stream) {
-    const size_t segs = rz_rqmc_gain_words(n_local_px, width);
-    if (segs == 0) return cudaSuccess;
-    rz_rqmc_gain_kernel<<<(unsigned)((segs + 3) / 4), 128, 0, stream>>>(accum, rep, n_px, n, n_local_px, width, seg_gain, px_gain);
-    return cudaGetLastError();
+    return rz_launch_segment_pass(accum, rep, n_px, n, n_local_px, width, seg_gain, px_gain, nullptr, nullptr, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

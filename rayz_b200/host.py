@@ -338,14 +338,15 @@ class Backend:
         return err, nz.as_dict()
 
     def render_to_noise(self, cam: abi.RzCamera, p: abi.RzRenderParams, target: float, max_spp: int, want_linear=True,
-                        want_rgb8=True, adaptive=False):
+                        want_rgb8=True, adaptive=False, pooled=False):
         """rayz_cuda_render_to_noise: p.spp samples, then batches doubling the count until rms_err <= target or max_spp.
         adaptive (RZ_RENDER_ADAPTIVE): the same schedule per pixel, until every pixel's error is <= target or max_spp; the
-        per-pixel counts are then pixel_samples().  Returns (linear [rows,w,4] f32, rgb8 [rows,w,3] u8, paths, summary dict
-        as noise())."""
-        if adaptive:
+        per-pixel counts are then pixel_samples().  pooled (RZ_RENDER_ADAPTIVE_POOLED): each pixel's error is pooled with its
+        row segment's, so that the per-pixel bound holds for the measured error, not only for the estimate; the library
+        refuses it without adaptive.  Returns (linear [rows,w,4] f32, rgb8 [rows,w,3] u8, paths, summary dict as noise())."""
+        if adaptive or pooled:
             p = abi.RzRenderParams.from_buffer_copy(p)
-            p.flags |= abi.RENDER_ADAPTIVE
+            p.flags |= (abi.RENDER_ADAPTIVE if adaptive else 0) | (abi.RENDER_ADAPTIVE_POOLED if pooled else 0)
         rows = self.shard_rows(p)
         lin = np.empty((rows, p.width, 4), dtype=np.float32) if want_linear else None
         rgb8 = np.empty((rows, p.width, 3), dtype=np.uint8) if want_rgb8 else None
@@ -478,12 +479,15 @@ class Tracer:
             self._backend = Backend(self.devices)
         return self._backend
 
-    def render(self, noise_target: float | None = None, max_spp: int = 4096, adaptive: bool = False, moments: bool = False) -> int:
+    def render(self, noise_target: float | None = None, max_spp: int = 4096, adaptive: bool = False, moments: bool = False,
+               pooled: bool = False) -> int:
         """noise_target (displayed-value rms error, 1/255 = one 8-bit step): start at samples_per_px and double the samples
         until the frame's rms error reaches it or max_spp samples are in (rayz_cuda_render_to_noise); `self.noise` then holds
         the summary.  adaptive: the target bounds every pixel's error, and only the pixels still above it get more samples;
-        `self.pixel_samples` then holds the counts.  Without a target, one render of samples_per_px, as the reference; moments:
-        also sum what the per-pixel noise estimate needs (RZ_RENDER_MOMENTS, no pixel changes), so that denoise() can follow."""
+        `self.pixel_samples` then holds the counts; pooled (with adaptive): each pixel stops on an error pooled with its row
+        segment's (RZ_RENDER_ADAPTIVE_POOLED), so that the bound holds for the measured error; the library refuses it
+        elsewhere.  Without a target, one render of samples_per_px, as the reference; moments: also sum what the per-pixel
+        noise estimate needs (RZ_RENDER_MOMENTS, no pixel changes), so that denoise() can follow."""
         b = self.backend
         arrays = self.pool.arrays()
         self._uploaded = None
@@ -492,6 +496,8 @@ class Tracer:
         kw = self._sampler()
         kw["moments"] = moments or kw.get("moments", False)
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant, **kw)
+        if pooled:
+            p.flags |= abi.RENDER_ADAPTIVE_POOLED
         if noise_target is None:
             lin, rgb8, rays = b.render(self.camera.rz, p)
         else:

@@ -10,7 +10,7 @@ With the card's name and power limit read in the same call (depth 50):
   * stopping at 1200 x 675 on both scenes: rayz_cuda_render_to_noise, rms and adaptive, at 2/255 and 1/255 (start 4 spp, cap
     4096): paths, wall time, the estimate and the measured rms displayed error of the returned frame, per sampler;
   * speed: Mpaths/s of a 1200 x 675, 64-spp render with and without the flag over Sobol (AUTO and the BVH variant), alternated;
-  * the segment-gain kernel's device time (torch.profiler) at 1200 x 675 and 3840 x 2160.
+  * the segment pass's device time (rz_segment_kernel, which computes the gains) (torch.profiler) at 1200 x 675 and 3840 x 2160.
 """
 from __future__ import annotations
 
@@ -145,7 +145,7 @@ def main():
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
             for _ in range(20):
                 b.noise()
-        ev = [e for e in prof.events() if "rz_rqmc_gain_kernel" in e.name]
+        ev = [e for e in prof.events() if "rz_segment_kernel" in e.name]
         gk[f"{w}x{h}"] = {"calls": len(ev), "mean_us": float(np.mean([e.device_time for e in ev])) if ev else None}
         print("gain kernel", w, gk[f"{w}x{h}"], flush=True)
     res["gain_kernel"] = gk

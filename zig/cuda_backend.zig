@@ -76,6 +76,7 @@ pub const RZ_RENDER_ACCUMULATE: u32 = 4; // add this batch to the previous rende
 pub const RZ_RENDER_ADAPTIVE: u32 = 8; // rayz_cuda_render_to_noise: the target bounds every pixel, only pixels above it get more samples
 pub const RZ_RENDER_SOBOL: u32 = 0x10; // camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox
 pub const RZ_RENDER_RQMC: u32 = 0x20; // with SOBOL and MOMENTS: two scrambled replicates per pixel, a noise estimate that sees the stratification
+pub const RZ_RENDER_ADAPTIVE_POOLED: u32 = 0x40; // with ADAPTIVE, rayz_cuda_render_to_noise only: stop each pixel on an error pooled over its row segment
 
 pub const RzNoise = extern struct {
     samples: u64,
