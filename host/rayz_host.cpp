@@ -3,7 +3,7 @@
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
-//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc] [--pooled]
+//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc] [--pooled] [--passes PREFIX]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -21,6 +21,9 @@
 // allow (RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS): --noise-target then stops on it; --spp and --max-spp must be even.
 // --pooled (with --noise-target X --adaptive) stops each pixel on an error pooled over its row segment (RZ_RENDER_ADAPTIVE_POOLED),
 // so that X bounds the measured error too; without --adaptive the library refuses it.
+// --passes PREFIX renders with RZ_RENDER_PASSES (no pixel changes) and writes the frame's seven light-path passes
+// (rayz_cuda_passes) as 3-channel PFM files PREFIX_<name>.pfm, name = environment, diffuse_direct, diffuse_indirect,
+// glossy_direct, glossy_indirect, transmission_direct, transmission_indirect; they sum to the frame's linear values.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -45,7 +48,7 @@ int main(int argc, char **argv) {
     size_t spp = 10, depth = 50;
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
-    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr;
+    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr, *passes = nullptr;
     bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false, rqmc = false, pooled = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
@@ -69,6 +72,7 @@ int main(int argc, char **argv) {
         else if (a == "--pooled") pooled = true;
         else if (a == "--guides") guides = val();
         else if (a == "--denoise") denoise = val();
+        else if (a == "--passes") passes = val();
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -92,6 +96,7 @@ int main(int argc, char **argv) {
         tracer.sobol = sobol;
         tracer.rqmc = rqmc;
         tracer.pooled = pooled;
+        tracer.passes = passes != nullptr;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);
@@ -112,6 +117,19 @@ int main(int argc, char **argv) {
             std::fprintf(stderr, "  [rayz_cuda] adaptive: %.0f paths, mean %.2f spp, max %llu spp, max error %.5f (%.2f 8-bit steps)\n", rays_traced,
                          rays_traced / std::max<double>(1.0, tracer.noise.n_pixels), (unsigned long long)tracer.noise.samples, tracer.noise.max_err,
                          tracer.noise.max_err * 255.0);
+        if (passes) {
+            tracer.readPasses();
+            static const char *const names[RZ_PASS_COUNT] = {"environment", "diffuse_direct", "diffuse_indirect", "glossy_direct",
+                                                             "glossy_indirect", "transmission_direct", "transmission_indirect"};
+            const size_t plane = tracer.img.w * tracer.img.h * 4;
+            for (int i = 0; i < RZ_PASS_COUNT; i++) {
+                const std::string path = std::string(passes) + "_" + names[i] + ".pfm";
+                FILE *f = std::fopen(path.c_str(), "wb");
+                if (!f) { std::perror(path.c_str()); return 1; }
+                writePFM(f, tracer.pass_planes.data() + i * plane, tracer.img.w, tracer.img.h, 4, 0, 3);
+                std::fclose(f);
+            }
+        }
         if (guides || denoise) tracer.renderGuides();
         if (guides) {
             const struct { const char *name; const std::vector<float> &src; size_t first, channels; } files[3] = {

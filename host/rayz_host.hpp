@@ -266,6 +266,8 @@ struct Tracer {
     bool sobol = false;           // RZ_RENDER_SOBOL: Owen-scrambled Sobol camera and scatter samples, in render() and renderGuides()
     bool rqmc = false;            // RZ_RENDER_RQMC (with SOBOL and MOMENTS): two Sobol replicates per pixel, a noise estimate that sees them
     bool pooled = false;          // RZ_RENDER_ADAPTIVE_POOLED, passed through: with adaptive, each pixel stops on an error pooled over its row segment
+    bool passes = false;          // RZ_RENDER_PASSES (no pixel changes), so that readPasses() can follow
+    std::vector<float> pass_planes;   // light-path passes of the last readPasses(): RZ_PASS_COUNT planes of h x w x 4 floats
     Image denoised;               // rgb8 of the last denoise()
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
@@ -304,6 +306,7 @@ struct Tracer {
         if (sobol) p.flags |= RZ_RENDER_SOBOL;
         if (rqmc) p.flags |= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;
         if (pooled) p.flags |= RZ_RENDER_ADAPTIVE_POOLED;   // the library refuses it without RZ_RENDER_ADAPTIVE
+        if (passes) p.flags |= RZ_RENDER_PASSES;
         return p;
     }
 
@@ -351,6 +354,12 @@ struct Tracer {
         for (size_t i = 0; i < img.w * img.h; i++) img.pixels[i] = {lin[4 * i], lin[4 * i + 1], lin[4 * i + 2]};
         rayz_cuda_timing(ctx, &timing);
         return (size_t)rays;
+    }
+
+    // The light-path passes of the frame of the last render() (with passes), after it (rayz_cuda_passes).
+    void readPasses() {
+        pass_planes.assign((size_t)RZ_PASS_COUNT * img.w * img.h * 4, 0.f);
+        check(rayz_cuda_passes(ctx, pass_planes.data()));
     }
 
     // Guide buffers for a denoiser over the camera samples render() traces (rayz_cuda_render_guides), after render().

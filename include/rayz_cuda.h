@@ -146,7 +146,7 @@ typedef struct RzRenderParams {
                                     * two families agree up to a pixel or two (see RZ_VARIANT_AUTO): pin the variant where
                                     * bit equality matters.  Refused with RZ_ERR_INVALID_ARG, the sums untouched, unless the
                                     * previous render succeeded with the same width, height, shard_index/count, band_rows,
-                                    * seed, max_depth, t_min, camera, RZ_RENDER_MOMENTS, RZ_RENDER_SOBOL and RZ_RENDER_RQMC bits on this context, no scene
+                                    * seed, max_depth, t_min, camera, RZ_RENDER_MOMENTS, RZ_RENDER_SOBOL, RZ_RENDER_RQMC and RZ_RENDER_PASSES bits on this context, no scene
                                     * upload or differently shaped reserve (or an RZ_RENDER_RQMC reserve after a render without
                                     * the flag, which grows the accumulators) came in between, sample_offset equals the previous
                                     * batch's sample_offset + spp, and the cumulative count stays below 2^32.  A render that
@@ -245,6 +245,39 @@ typedef struct RzRenderParams {
                                     * segment before each stopping test (the pass RZ_RENDER_RQMC's gain runs in); the path kernels
                                     * are those of the plain rule, and more samples are spent where the plain rule stopped too
                                     * early. */
+#define RZ_RENDER_PASSES 0x80u     /* light-path passes (DESIGN.md "Light-path passes"): also sum each path's radiance into the
+                                    * one pass (RZ_PASS_*, below) its path belongs to, so that rayz_cuda_passes can split every
+                                    * pixel by how its light reached the sky.  Changes no pixel of the image and no noise estimate.
+                                    * Honoured by rayz_cuda_render, rayz_cuda_render_device and rayz_cuda_render_to_noise (plain,
+                                    * adaptive and pooled), by every variant and sampler; rayz_cuda_reserve also allocates the pass
+                                    * sums (RZ_PASS_COUNT x 3 x 8 = 168 bytes per pixel).  An RZ_RENDER_ACCUMULATE batch whose
+                                    * PASSES bit differs from the accumulated render's is refused, the sums untouched;
+                                    * rayz_cuda_render_guides refuses the flag; max_depth > 2^29 - 1 is refused with
+                                    * RZ_ERR_INVALID_ARG (the first hit's kind rides in the top bits of a path's hit count). */
+
+/*
+ * Light-path passes (RZ_RENDER_PASSES).  A path that ends in the sky with h scattering hits before it adds its clamped
+ * radiance, the same 2^-32 fixed-point values the three colour accumulators add, to exactly one pass:
+ *   RZ_PASS_ENVIRONMENT                                  h = 0 (the camera ray missed)
+ *   RZ_PASS_DIFFUSE_DIRECT / RZ_PASS_DIFFUSE_INDIRECT    first hit RZ_MAT_DIFFUSE;    h = 1 / h >= 2
+ *   RZ_PASS_GLOSSY_DIRECT / RZ_PASS_GLOSSY_INDIRECT      first hit RZ_MAT_METALLIC;   h = 1 / h >= 2
+ *   RZ_PASS_TRANSMISSION_DIRECT / _INDIRECT              first hit RZ_MAT_DIELECTRIC (whether it reflected or refracted);
+ *                                                        h = 1 / h >= 2
+ * The class is decided by the first hit's MATERIAL KIND, not by the lobe its scatter took: a dielectric hit that reflects
+ * still counts as transmission.  Paths that end absorbed or at the depth limit add nothing to any pass, as they add nothing
+ * to the image.  Since every path adds the same integers to its pass as to the image, for every pixel and channel the sum of
+ * the seven pass sums equals the image's sum bit for bit, through batches, shards, devices and adaptive rounds.
+ */
+enum {
+    RZ_PASS_ENVIRONMENT = 0,
+    RZ_PASS_DIFFUSE_DIRECT = 1,
+    RZ_PASS_DIFFUSE_INDIRECT = 2,
+    RZ_PASS_GLOSSY_DIRECT = 3,
+    RZ_PASS_GLOSSY_INDIRECT = 4,
+    RZ_PASS_TRANSMISSION_DIRECT = 5,
+    RZ_PASS_TRANSMISSION_INDIRECT = 6,
+    RZ_PASS_COUNT = 7
+};
 
 /* Noise summary of the accumulated frame (rayz_cuda_noise).  Errors are standard errors of the DISPLAYED value
  * (gamma 2, as writePPM shows it) in units of [0, 1]: one 8-bit step is 1/255.  +inf while samples < 2. */
@@ -371,6 +404,17 @@ int rayz_cuda_render_to_noise(RzContext *ctx, const RzCamera *cam, const RzRende
 int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp);
 
 /*
+ * Light-path passes of the accumulated frame (RZ_RENDER_PASSES).  out_passes holds RZ_PASS_COUNT planes of rows of the context
+ * * width * 4 floats, plane i at out_passes + i * rows * width * 4, each laid out like out_linear_rgba: rgb = the pass sum over
+ * the pixel's own sample count (n_px after an adaptive rayz_cuda_render_to_noise), in the resolve's f64 arithmetic, stored as
+ * f32; a = 1.  Their sum equals out_linear_rgba to f32 rounding.  RZ_ERR_INVALID_ARG, nothing touched, if out_passes is NULL,
+ * there is no accumulated frame or it was rendered without RZ_RENDER_PASSES.  Leaves the accumulated frame, its sample counts,
+ * RzStats, RzTiming and rayz_cuda_render_device's buffers untouched (a render enqueued by rayz_cuda_render_device(sync = 0) is
+ * waited for first, as rayz_cuda_noise does).
+ */
+int rayz_cuda_passes(RzContext *ctx, float *out_passes);
+
+/*
  * Guide buffers for a denoiser, of the camera samples [p->sample_offset, p->sample_offset + p->spp) of every pixel of the
  * context's rows: the SAME camera rays (seed, global pixel, sample index -> jitter, lens point, time) a render with these
  * parameters traces, each followed to its first hit only.  Host outputs, each nullable, laid out like out_linear_rgba:
@@ -384,8 +428,8 @@ int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp);
  * along the unit camera ray from its lens-sampled origin.  Each pixel's samples are summed in f64 in sample order and the f32
  * mean is written, so the buffers depend on (scene, camera, seed, pixel, sample range) only: not on shards, devices or launch
  * shape.  The search is the BVH kernel's (RZ_VARIANT_BVH) whatever the variant; max_depth and collect_stats have no effect.
- * Parameters a render refuses are refused with its codes and messages, prefixed "guides:"; RZ_RENDER_ACCUMULATE and
- * RZ_RENDER_ADAPTIVE are refused with RZ_ERR_INVALID_ARG.  RZ_ERR_INTERNAL if the traversal stack overflowed (results withheld,
+ * Parameters a render refuses are refused with its codes and messages, prefixed "guides:"; RZ_RENDER_ACCUMULATE,
+ * RZ_RENDER_ADAPTIVE and RZ_RENDER_PASSES are refused with RZ_ERR_INVALID_ARG.  RZ_ERR_INTERNAL if the traversal stack overflowed (results withheld,
  * the context stays usable).  Leaves the accumulated frame, its sample counts, RzStats and RzTiming untouched (a render
  * enqueued by rayz_cuda_render_device(sync = 0) is waited for first, as rayz_cuda_noise does).
  */

@@ -21,6 +21,11 @@ VARIANT_AUTO, VARIANT_MEGA, VARIANT_WAVEFRONT, VARIANT_BVH = 0, 1, 2, 3
 VARIANTS = {"auto": 0, "mega": 1, "wavefront": 2, "bvh": 3, "mega_single": 4}
 RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE, RENDER_ADAPTIVE, RENDER_SOBOL, RENDER_RQMC = 1, 2, 4, 8, 0x10, 0x20   # RzRenderParams.flags (RZ_RENDER_*)
 RENDER_ADAPTIVE_POOLED = 0x40   # with RENDER_ADAPTIVE in render_to_noise: stop each pixel on an error pooled over its row segment
+RENDER_PASSES = 0x80            # also sum each sky path's radiance into its light-path pass (rayz_cuda_passes)
+# RZ_PASS_*: index -> name of the light-path passes rayz_cuda_passes returns, in plane order
+PASS_NAMES = ("environment", "diffuse_direct", "diffuse_indirect", "glossy_direct", "glossy_indirect", "transmission_direct",
+              "transmission_indirect")
+PASS_COUNT = len(PASS_NAMES)
 
 _dp, _up = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 
@@ -107,6 +112,7 @@ SYMBOLS = {
     "rayz_cuda_render_to_noise": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_float, C.c_uint32,
                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(RzNoise)]),
     "rayz_cuda_pixel_samples": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "rayz_cuda_passes": (C.c_int, [C.c_void_p, C.c_void_p]),
     "rayz_cuda_render_guides": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_void_p, C.c_void_p]),
     "rayz_cuda_denoise": (C.c_int, [C.c_void_p, C.POINTER(RzDenoiseParams), C.c_void_p, C.c_void_p]),
     "rayz_cuda_shard_rows": (C.c_uint32, [C.c_uint32] * 4),

@@ -132,7 +132,7 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
 }
 
 // LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list).
-template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false, int SOBOL = 0>
+template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false, int SOBOL = 0, bool PASSES = false>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -174,7 +174,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
         if (alive && cur == RZ_SENTINEL) {
             if (STATS) c_segs++;
             uint32_t kind;
-            const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, sample, bk, kind, SOBOL);
+            const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, sample, bk, kind, SOBOL, PASSES);
             if (STATS) {
                 if (kind < 3u) c_hit[kind]++;
                 if (res == RZ_END_SKY) c_sky++;
@@ -271,7 +271,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
 // in L1; survivors go to the next queue, and the tail of the paths to the persistent kernel above (QUEUE).
 // CAMERA: the camera rays of a work unit — an 8 x 4-pixel block x `chunk` samples — do not walk the tree one by one; the warp
 // culls the tree once against the block's cone and the rays search the surviving spheres as a list (below).  The sorted stages (CAMERA = false) are off by default (RzTuning::bvh_stages = 0: measured as a loss).
-template <bool STATS, bool CAMERA, int SOBOL = 0>
+template <bool STATS, bool CAMERA, int SOBOL = 0, bool PASSES = false>
 __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB) rz_bvh_stage_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -425,7 +425,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                             const int hit = bk[0] < 0 ? -1 : (w_gid[bk[0] & ~RZ_FAR_BIT] | (bk[0] & RZ_FAR_BIT));   // list slot -> position in the set
                             if (STATS) c_segs++;
                             uint32_t kind;
-                            const int res = rz_shade_segment(a, rays[0], thr[0], seg[0], lp0, gpix0, smp[0], hit, kind, SOBOL);
+                            const int res = rz_shade_segment(a, rays[0], thr[0], seg[0], lp0, gpix0, smp[0], hit, kind, SOBOL, PASSES);
                             if (STATS) {
                                 if (kind < 3u) c_hit[kind]++;
                                 if (res == RZ_END_SKY) c_sky++;
@@ -480,7 +480,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
             if (live) {
                 if (STATS) c_segs++;
                 uint32_t kind;
-                const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, smp, bk, kind, SOBOL);
+                const int res = rz_shade_segment(a, ray, thr, seg, lp, gpix, smp, bk, kind, SOBOL, PASSES);
                 if (STATS) {
                     if (kind < 3u) c_hit[kind]++;
                     if (res == RZ_END_SKY) c_sky++;
@@ -612,12 +612,12 @@ extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int
     RzPathArgs b = *a;
     rz_bvh_tuning(b);
     if (b.q_in && b.self_map)   // the tail of the staged K1 (entries written by a brute-force stage): a short queue, small units
-        return launch_kernel([](auto S, auto M) { return rz_bvh_kernel<decltype(S)::value, true, 64, false, decltype(M)::value>; }, b, collect_stats, sm_count, stream);
+        return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, true, 64, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
     if (b.q_in)
-        return launch_kernel([](auto S, auto M) { return rz_bvh_kernel<decltype(S)::value, true, 512, false, decltype(M)::value>; }, b, collect_stats, sm_count, stream);
+        return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, true, 512, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
     if (b.px_list)
-        return launch_kernel([](auto S, auto M) { return rz_bvh_kernel<decltype(S)::value, false, 512, true, decltype(M)::value>; }, b, collect_stats, sm_count, stream);
-    return launch_kernel([](auto S, auto M) { return rz_bvh_kernel<decltype(S)::value, false, 512, false, decltype(M)::value>; }, b, collect_stats, sm_count, stream);
+        return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, false, 512, true, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
+    return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, false, 512, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
 }
 
 // Guide buffers of the device's local pixels: one warp per 8 x 4 block, four per CTA.
@@ -627,7 +627,7 @@ extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t strea
     const uint32_t rows = b.a.width ? b.a.n_local_px / b.a.width : 0u;
     const uint32_t blocks = ((b.a.width + 7u) / 8u) * ((rows + 3u) / 4u);
     if (blocks == 0u) return cudaSuccess;
-    rz_pick_instance(b.a, 0, [](auto, auto M) { return rz_guides_kernel<decltype(M)::value>; })<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
+    rz_pick_instance(b.a, 0, [](auto, auto M, auto) { return rz_guides_kernel<decltype(M)::value>; })<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
     return cudaGetLastError();
 }
 
@@ -636,6 +636,6 @@ extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stat
     RzPathArgs b = *a;
     rz_bvh_tuning(b);
     if (!b.q_in)
-        return launch_kernel([](auto S, auto M) { return rz_bvh_stage_kernel<decltype(S)::value, true, decltype(M)::value>; }, b, collect_stats, sm_count, stream);
-    return launch_kernel([](auto S, auto M) { return rz_bvh_stage_kernel<decltype(S)::value, false, decltype(M)::value>; }, b, collect_stats, sm_count, stream);
+        return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_stage_kernel<decltype(S)::value, true, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
+    return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_stage_kernel<decltype(S)::value, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
 }

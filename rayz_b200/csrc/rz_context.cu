@@ -107,7 +107,8 @@ struct Dev {
     DBuf<float4> m_rec;
     DBuf<float4> t_color;
     DBuf<double> t_inv_scale;
-    DBuf<unsigned long long> accum;   // + RZ_RENDER_RQMC's replicate sums behind the accumulators (rz_rep_offset)
+    DBuf<unsigned long long> accum;   // + RZ_RENDER_RQMC's replicate sums and RZ_RENDER_PASSES' pass sums behind the accumulators
+                                      // (rz_rep_offset, rz_pass_offset; rz_accum_words)
     DBuf<double> gain;                // RZ_RENDER_RQMC: the segment gains of the local rows (rz_segment_kernel)
     DBuf<double> px_gain;             // RZ_RENDER_RQMC: every local pixel's gain, frozen when an adaptive pixel stops (rz_segment_kernel)
     DBuf<double> pool;                // RZ_RENDER_ADAPTIVE_POOLED: the segment priors U_S of the local rows (rz_segment_kernel)
@@ -126,6 +127,7 @@ struct Dev {
     DBuf<float> out_err;              // rayz_cuda_noise: per-pixel error of the context's rows (gather root only)
     DBuf<RzNoisePartial> noise_part;  // rayz_cuda_noise: the reduction's per-CTA partials of this device
     DBuf<uint32_t> out_spp;           // rayz_cuda_pixel_samples: per-pixel sample counts of the context's rows (gather root only)
+    DBuf<float4> out_passes;          // rayz_cuda_passes: RZ_PASS_COUNT planes of the context's rows (gather root only)
     DBuf<float4> out_guides;          // rayz_cuda_render_guides: albedo, then normal + depth, of the context's rows (gather root only)
     // rayz_cuda_denoise (gather root only): the resolved frame, then the denoised one; the per-pixel error; the ping-pong pair of
     // (demodulated rgb, variance); the depth gradient; the denoised rgb8.  Never Dev::out_linear / out_rgb8, which a
@@ -185,6 +187,7 @@ struct AccumRecord {
     Frame frame;
     uint32_t max_depth = 0, moments = 0, sobol = 0, rqmc = 0;
     uint32_t pooled = 0;       // RZ_RENDER_ADAPTIVE_POOLED: every consumer of the error reads the pooled e* (Dev::px_pool)
+    uint32_t passes = 0;       // RZ_RENDER_PASSES: the pass sums behind the accumulators hold the frame's light-path passes
     uint64_t seed = 0;
     float t_min = 0;
     RzCamera cam{};
@@ -913,6 +916,11 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         P.refused = true;
         return rz_fail(RZ_ERR_INVALID_ARG, "%s: RZ_RENDER_ADAPTIVE_POOLED requires RZ_RENDER_ADAPTIVE (rayz_cuda_render_to_noise only)", who);
     }
+    if ((p->flags & RZ_RENDER_PASSES) && p->max_depth > RZ_PASS_MAX_DEPTH) {   // the count must stay out of the kind bits (rz_seg_after_hit)
+        P.refused = true;
+        return rz_fail(RZ_ERR_INVALID_ARG, "%s: RZ_RENDER_PASSES requires max_depth <= 2^29 - 1 (the first hit's kind rides in the top bits of a path's hit count; got %u)",
+                       who, p->max_depth);
+    }
 
     if (cam) {
         AccumRecord &next = P.next;
@@ -921,6 +929,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         next.sobol = (p->flags & RZ_RENDER_SOBOL) ? 1u : 0u;
         next.rqmc = (p->flags & RZ_RENDER_RQMC) ? 1u : 0u;
         next.pooled = (p->flags & RZ_RENDER_ADAPTIVE_POOLED) ? 1u : 0u;
+        next.passes = (p->flags & RZ_RENDER_PASSES) ? 1u : 0u;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
         next.adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
@@ -936,6 +945,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
             if (prev.moments != next.moments) return refuse("the RZ_RENDER_MOMENTS bit differs from the accumulated render");
             if (prev.sobol != next.sobol) return refuse("the RZ_RENDER_SOBOL bit differs from the accumulated render");
             if (prev.rqmc != next.rqmc) return refuse("the RZ_RENDER_RQMC bit differs from the accumulated render");
+            if (prev.passes != next.passes) return refuse("the RZ_RENDER_PASSES bit differs from the accumulated render");
             if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
                 return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
             if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
@@ -1007,8 +1017,8 @@ static int alloc_render(RzContext *ctx, RenderPlan &P) {
         RZ_CUDA(cudaSetDevice(D.id));
         const bool rqmc = (P.p->flags & RZ_RENDER_RQMC) != 0;
         const unsigned long long *held = D.accum.p;
-        if ((rc = D.accum.alloc((size_t)dp.n_tiles * 32u * (rqmc ? 6u : 4u)))) return rc;
-        if (D.accum.p != held) ctx->acc.valid = false;   // grown (a reserve for RZ_RENDER_RQMC of the same frame): the sums are gone
+        if ((rc = D.accum.alloc(rz_accum_words(dp.n_tiles, rqmc, (P.p->flags & RZ_RENDER_PASSES) != 0)))) return rc;
+        if (D.accum.p != held) ctx->acc.valid = false;   // grown (a reserve for RZ_RENDER_RQMC or RZ_RENDER_PASSES of the same frame): the sums are gone
         if (rqmc && ((rc = D.gain.alloc(rz_rqmc_gain_words(n_local, P.frame.width))) || (rc = D.px_gain.alloc(n_local)))) return rc;
         if ((P.p->flags & RZ_RENDER_ADAPTIVE_POOLED) &&
             ((rc = D.pool.alloc(rz_rqmc_gain_words(n_local, P.frame.width))) || (rc = D.px_pool.alloc(n_local))))
@@ -1138,7 +1148,8 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
     a.spp = p->spp; a.sample_offset = p->sample_offset; a.max_depth = p->max_depth;
     a.shard_index = P.frame.s * ND + d; a.shard_count = P.frame.S * ND; a.band_rows = P.frame.band;
     a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
-    a.sobol = ((p->flags & RZ_RENDER_SOBOL) ? RZ_SAMPLER_SOBOL : 0u) | ((p->flags & RZ_RENDER_RQMC) ? RZ_SAMPLER_RQMC : 0u);
+    a.sobol = ((p->flags & RZ_RENDER_SOBOL) ? RZ_SAMPLER_SOBOL : 0u) | ((p->flags & RZ_RENDER_RQMC) ? RZ_SAMPLER_RQMC : 0u) |
+              ((p->flags & RZ_RENDER_PASSES) ? RZ_PATH_PASSES : 0u);
     a.t_min = P.next.t_min;   // plan_render applied the default
     a.err = D.errword.p;
     a.unit_entries = ctx->tun.unit_entries;
@@ -1188,8 +1199,8 @@ static int enqueue_device(RzContext *ctx, const RenderPlan &P, uint32_t d, uint3
     const bool trace = n_local > 0 && (!P.list || dp.n_list > 0);   // a device with an empty list launches nothing
     RZ_CUDA(cudaSetDevice(D.id));
     RZ_CUDA(cudaEventRecord(D.ev[0], D.stream));
-    if (!(p->flags & RZ_RENDER_ACCUMULATE))   // with the replicate sums behind them under RZ_RENDER_RQMC
-        RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, (size_t)dp.n_tiles * 32u * (P.next.rqmc ? 6u : 4u) * sizeof(unsigned long long), D.stream));
+    if (!(p->flags & RZ_RENDER_ACCUMULATE))   // with the replicate sums and the pass sums behind them under RZ_RENDER_RQMC, RZ_RENDER_PASSES
+        RZ_CUDA(cudaMemsetAsync(D.accum.p, 0, rz_accum_words(dp.n_tiles, P.next.rqmc, P.next.passes) * sizeof(unsigned long long), D.stream));
     if (adaptive && !P.list) RZ_CUDA(rz_launch_fill_u32(D.n_px.p, n_local, p->spp, D.stream));   // first round: every pixel
     RZ_CUDA(cudaMemsetAsync(D.counter.p, 0, 16 * sizeof(unsigned int), D.stream));
     RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
@@ -1459,6 +1470,32 @@ extern "C" int rayz_cuda_pixel_samples(RzContext *ctx, uint32_t *out_spp) {
     return RZ_OK;
 }
 
+// Light-path passes of the accumulated frame, laid out like rayz_cuda_noise's out_err but RZ_PASS_COUNT planes deep: every
+// device's rz_passes_resolve_kernel scatters its rows into the gather root's planes as the resolve does the image.
+extern "C" int rayz_cuda_passes(RzContext *ctx, float *out_passes) {
+    if (!ctx || !out_passes) return rz_fail(RZ_ERR_INVALID_ARG, "passes: NULL argument");
+    DeviceGuard guard;
+    const AccumRecord *A = nullptr;
+    if (const int rc = accumulated_frame(ctx, "passes", A)) return rc;
+    if (!A->passes) return rz_fail(RZ_ERR_INVALID_ARG, "passes: the accumulated render(s) ran without RZ_RENDER_PASSES");
+    Dev &D0 = ctx->devs[0];
+    const FrameSplit sp(ctx, A->frame);
+    int rc;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if ((rc = D0.out_passes.alloc((size_t)RZ_PASS_COUNT * sp.npx))) return rc;
+    for (uint32_t d = 0; d < (uint32_t)ctx->devs.size(); d++) {
+        Dev &D = ctx->devs[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        const RzResolveArgs r = resolve_args(ctx, d, *A, sp.n_local[d]);
+        RZ_CUDA(rz_launch_passes_resolve(&r, D.accum.p + rz_pass_offset(sp.n_local[d], A->rqmc != 0), D0.out_passes.p, sp.npx, D.stream));
+    }
+    if ((rc = sync_devices(ctx))) return rc;   // every device's rows are in the gather root's planes
+    RZ_CUDA(cudaSetDevice(D0.id));
+    RZ_CUDA(cudaMemcpyAsync(out_passes, D0.out_passes.p, (size_t)RZ_PASS_COUNT * sp.npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaStreamSynchronize(D0.stream));
+    return RZ_OK;
+}
+
 // Guide buffers (include/rayz_cuda.h): every device traces its rows' camera samples to their first hits with rz_guides_kernel,
 // which stores straight into the gather root's buffers like the resolve kernel; the error words are read behind every stream,
 // then the root's buffers are copied out.  The accumulators, their record, the per-pixel counts, stats and timing stay as
@@ -1471,6 +1508,7 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
         return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_ADAPTIVE_POOLED is honoured by rayz_cuda_render_to_noise with RZ_RENDER_ADAPTIVE only");
     if (p->flags & (RZ_RENDER_ACCUMULATE | RZ_RENDER_ADAPTIVE))
         return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_ACCUMULATE and RZ_RENDER_ADAPTIVE do not apply to guide buffers");
+    if (p->flags & RZ_RENDER_PASSES) return rz_fail(RZ_ERR_INVALID_ARG, "guides: RZ_RENDER_PASSES does not apply to guide buffers");
     RenderPlan P;
     if (const int rc = plan_render(ctx, cam, p, ctx->acc, P, "guides")) return rc;
     DeviceGuard guard;

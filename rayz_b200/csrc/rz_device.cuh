@@ -21,6 +21,8 @@
 #include <algorithm>
 #include <vector>
 
+#include "../../include/rayz_cuda.h"   // RZ_MAT_*, RZ_PASS_*
+
 #define RZ_HD __host__ __device__ __forceinline__
 // Rare branches of the shading code are kept OUT of line on the device: the staged kernels are 35-45 KB against a 32 KB L1.5
 // instruction cache, and ncu charged up to 3 stall cycles per issued instruction to `no_instruction` (profiles/).
@@ -166,18 +168,44 @@ struct RzPathArgs {
     // covers list entries [tile * 32, tile * 32 + 32), and lane k's pixel is px_list[entry] instead of the entry itself.
     const uint32_t *px_list;     // local pixel indices in increasing order (rz_adaptive.cu)
     uint32_t n_list;             // entries in px_list
-    uint32_t sobol;              // RZ_SAMPLER_* bits.  != 0 (RZ_RENDER_SOBOL): the launchers run each kernel's SOBOL instance
-                                 // (rz_sampler.cuh's pairs), with RZ_SAMPLER_RQMC its SOBOL = 2 instance
+    uint32_t sobol;              // RZ_SAMPLER_* bits.  RZ_SAMPLER_SOBOL (RZ_RENDER_SOBOL): the launchers run each kernel's SOBOL
+                                 // instance (rz_sampler.cuh's pairs), with RZ_SAMPLER_RQMC its SOBOL = 2 instance; RZ_PATH_PASSES
+                                 // (RZ_RENDER_PASSES): its PASSES instance
 };
+
+// ---------------------------------------------------------------------------------------------
+// Light-path passes (RZ_RENDER_PASSES, include/rayz_cuda.h).  In the PASSES instances a path's `seg` word holds the hits so far
+// in bits 0-28 and the material kind of its first hit in bits 29-30, set on that hit; bit 31 stays the wavefront's
+// dead-on-arrival marker.  Every form a path lives in already stores seg whole (queue entries' q+2.w, the wavefront's C.w), so
+// no queue or slot format changes; rz_shade_segment masks the count before it reads it.  The count reaches max_depth at most,
+// so max_depth <= RZ_PASS_MAX_DEPTH keeps it out of the kind bits (larger is refused).
+// ---------------------------------------------------------------------------------------------
+#define RZ_SEG_HITS 0x1fffffffu
+#define RZ_SEG_KIND_SHIFT 29
+#define RZ_PASS_MAX_DEPTH RZ_SEG_HITS
+RZ_HD uint32_t rz_seg_hits(uint32_t seg) { return seg & RZ_SEG_HITS; }
+RZ_HD uint32_t rz_seg_first_kind(uint32_t seg) { return (seg >> RZ_SEG_KIND_SHIFT) & 3u; }
+// seg after the hit that makes its count `hits + 1`: the first hit also records the kind
+RZ_HD uint32_t rz_seg_after_hit(uint32_t seg, uint32_t kind) { return (rz_seg_hits(seg) == 0u ? seg | (kind << RZ_SEG_KIND_SHIFT) : seg) + 1u; }
+// The pass of a path that reaches the sky after `hits` scattering hits, the first of material kind first_kind (RZ_MAT_*).
+RZ_HD uint32_t rz_pass_of(uint32_t hits, uint32_t first_kind) {
+    return hits == 0u ? (uint32_t)RZ_PASS_ENVIRONMENT : (uint32_t)RZ_PASS_DIFFUSE_DIRECT + 2u * first_kind + (hits >= 2u ? 1u : 0u);
+}
 
 // RzPathArgs::sobol.  RZ_SAMPLER_RQMC (RZ_RENDER_RQMC) rides in the same word, so that the Philox instances see the very
 // arguments they saw before the flag existed; the launchers run the SOBOL = 2 instances for it (rz_pick_sampler): the replicate
 // mapping of rz_sobol_pair, and a sky path also adds its clamped luminance to its replicate's sum (rz_rep_offset).
-enum { RZ_SAMPLER_SOBOL = 1u, RZ_SAMPLER_RQMC = 2u };
+// RZ_PATH_PASSES (RZ_RENDER_PASSES) rides there too, for the same reason: a new field would move the parameters that follow
+// RzPathArgs in the wavefront's and the guides' kernels.  The launchers run the PASSES instances for it (rz_pick_instance).
+enum { RZ_SAMPLER_SOBOL = 1u, RZ_SAMPLER_RQMC = 2u, RZ_PATH_PASSES = 4u };
 // RZ_RENDER_RQMC's replicate sums share the accumulators' allocation: [n_pad][4] accumulators, then [n_pad][2] replicate sums
 // (2^-32 fixed point, slot lp * 2 + (sample & 1)), n_pad = n_local_px rounded up to whole warps.  This is the offset, in words,
 // of the replicate sums.
 RZ_HD size_t rz_rep_offset(uint32_t n_local_px) { return (size_t)((n_local_px + 31u) / 32u) * 32u * 4u; }
+// RZ_RENDER_PASSES' pass sums come after those: [n_pad][RZ_PASS_COUNT][3] (2^-32 fixed point), at this offset in words.
+RZ_HD size_t rz_pass_offset(uint32_t n_local_px, bool rqmc) { return rz_rep_offset(n_local_px) / 4u * (rqmc ? 6u : 4u); }
+// Words of the accumulators' allocation for n_pad = n_tiles * 32 pixels.
+RZ_HD size_t rz_accum_words(size_t n_tiles, bool rqmc, bool passes) { return n_tiles * 32u * ((rqmc ? 6u : 4u) + (passes ? RZ_PASS_COUNT * 3u : 0u)); }
 
 // Guide buffers (rayz_cuda_render_guides, rz_guides_kernel in rz_bvh_trace.cu): the camera segments of a render with these
 // RzPathArgs, each followed to its first hit only.  The outputs are the gather root's buffers at the context's rows (peer

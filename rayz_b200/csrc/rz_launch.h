@@ -46,6 +46,8 @@ struct RzResolveArgs {
 struct RzNoisePartial { double sum, sum2, max; unsigned long long above; };
 
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_passes_resolve(const RzResolveArgs *a, const unsigned long long *passes, float4 *out, size_t plane,
+                                                cudaStream_t stream);
 extern "C" cudaError_t rz_launch_noise_reduce(const unsigned long long *accum, const uint32_t *n_px, const double *gain, const double *pool,
                                               uint32_t n_local_px, uint32_t n, double target, RzNoisePartial *out, cudaStream_t stream);
 extern "C" size_t rz_rqmc_gain_words(uint32_t n_local_px, uint32_t width);

@@ -1,4 +1,4 @@
-// rz_misc.cu — K5 resolve/quantise, the noise summary, the segment pass and K6 FP32 peak microbenchmark.
+// rz_misc.cu — K5 resolve/quantise, the light-path passes' resolve, the noise summary, the segment pass and K6 FP32 peak microbenchmark.
 
 // ---------------------------------------------------------------------------------------------
 // K5.  Fixed-point accumulators -> linear float4 + gamma-2 RGB8.
@@ -16,17 +16,23 @@
 #include "rz_device.cuh"   // rz_pixel_err_of, rz_quantise_rgb8
 #include "rz_launch.h"     // RzResolveArgs, RzNoisePartial
 
-__global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) {
-    const uint32_t lp = blockIdx.x * blockDim.x + threadIdx.x;
-    if (lp >= a.n_local_px) return;
-    const ulonglong2 q0 = *reinterpret_cast<const ulonglong2 *>(a.accum + (size_t)lp * 4);
-    const unsigned long long q1 = a.accum[(size_t)lp * 4 + 2];
+// the gather root's pixel of local pixel lp (its rows of the context's frame)
+__device__ __forceinline__ size_t rz_resolve_dst(const RzResolveArgs &a, uint32_t lp) {
     size_t dst = lp;
     if (a.dev_count > 1u) {
         const uint32_t lr = lp / a.width, i = lp - lr * a.width;
         const uint32_t lb = lr / a.band_rows, within = lr - lb * a.band_rows;
         dst = (size_t)((lb * a.dev_count + a.dev_index) * a.band_rows + within) * a.width + i;
     }
+    return dst;
+}
+
+__global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) {
+    const uint32_t lp = blockIdx.x * blockDim.x + threadIdx.x;
+    if (lp >= a.n_local_px) return;
+    const ulonglong2 q0 = *reinterpret_cast<const ulonglong2 *>(a.accum + (size_t)lp * 4);
+    const unsigned long long q1 = a.accum[(size_t)lp * 4 + 2];
+    const size_t dst = rz_resolve_dst(a, lp);
     const uint32_t n = a.n_px ? a.n_px[lp] : a.spp;
     if (a.out_spp) a.out_spp[dst] = n;
     if (a.out_err) a.out_err[dst] = (float)rz_pixel_err_of(a.accum + (size_t)lp * 4, n, a.gain, a.pool, lp);
@@ -40,6 +46,31 @@ __global__ void __launch_bounds__(256) rz_resolve_kernel(const RzResolveArgs a) 
 extern "C" cudaError_t rz_launch_resolve(const RzResolveArgs *a, cudaStream_t stream) {
     if (a->n_local_px == 0) return cudaSuccess;
     rz_resolve_kernel<<<(a->n_local_px + 255) / 256, 256, 0, stream>>>(*a);
+    return cudaGetLastError();
+}
+
+// RZ_RENDER_PASSES (rayz_cuda_passes only): pass i of local pixel lp -> out[i * plane + dst], rgb = the pass sums over the
+// pixel's count in the resolve's f64 arithmetic, a = 1.  The same addressing as rz_resolve_kernel, so the planes' rows land where
+// the image's do.
+__global__ void __launch_bounds__(256) rz_passes_resolve_kernel(const RzResolveArgs a, const unsigned long long *__restrict__ passes,
+                                                                float4 *__restrict__ out, size_t plane) {
+    const uint32_t lp = blockIdx.x * blockDim.x + threadIdx.x;
+    if (lp >= a.n_local_px) return;
+    const size_t dst = rz_resolve_dst(a, lp);
+    const uint32_t n = a.n_px ? a.n_px[lp] : a.spp;
+    const double inv = 1.0 / (double)n;
+    const double s = 2.3283064365386962890625e-10;  // 2^-32
+    const unsigned long long *q = passes + (size_t)lp * (RZ_PASS_COUNT * 3);
+#pragma unroll
+    for (int i = 0; i < RZ_PASS_COUNT; i++)
+        out[i * plane + dst] = make_float4((float)((double)q[3 * i] * s * inv), (float)((double)q[3 * i + 1] * s * inv),
+                                           (float)((double)q[3 * i + 2] * s * inv), 1.0f);
+}
+
+extern "C" cudaError_t rz_launch_passes_resolve(const RzResolveArgs *a, const unsigned long long *passes, float4 *out, size_t plane,
+                                                cudaStream_t stream) {
+    if (a->n_local_px == 0) return cudaSuccess;
+    rz_passes_resolve_kernel<<<(a->n_local_px + 255) / 256, 256, 0, stream>>>(*a, passes, out, plane);
     return cudaGetLastError();
 }
 

@@ -64,7 +64,7 @@ struct RzStream {
 
 // G = sphere PAIRS per search-loop iteration
 // LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list)
-template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false, int SOBOL = 0>
+template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false, int SOBOL = 0, bool PASSES = false>
 __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -178,7 +178,7 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
             if (!st[r].alive) continue;
             if (STATS) { c_segs++; c_sph += a.set.n; }   // brute force: every sphere of the set
             uint32_t kind;
-            const int res = rz_shade_segment(a, st[r].ray, st[r].thr, st[r].seg, st[r].lp, st[r].gpix, st[r].sample, bk[r], kind, SOBOL);
+            const int res = rz_shade_segment(a, st[r].ray, st[r].thr, st[r].seg, st[r].lp, st[r].gpix, st[r].sample, bk[r], kind, SOBOL, PASSES);
             if (STATS) {
                 if (kind < 3u) c_hit[kind]++;
                 if (res == RZ_END_SKY) c_sky++;
@@ -230,7 +230,7 @@ struct RzSegCounters {
 };
 
 // Shade the two rays of a lane after the search and append the survivors (with their sort keys) to the next queue.
-template <bool STATS, int SOBOL>
+template <bool STATS, int SOBOL, bool PASSES>
 __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRay (&L)[2], unsigned lane, unsigned lt_mask, RzSegCounters &C) {
 #pragma unroll 1
     for (int trip = 0; trip < 2; trip++) {
@@ -239,7 +239,7 @@ __device__ __forceinline__ void rz_shade_and_push2(const RzPathArgs &a, RzLaneRa
         if (Q.live) {
             if (STATS) C.segs++;
             uint32_t kind;
-            const int res = rz_shade_segment(a, Q.ray, Q.thr, Q.seg, Q.lp, Q.gpix, Q.smp, Q.bk, kind, SOBOL);
+            const int res = rz_shade_segment(a, Q.ray, Q.thr, Q.seg, Q.lp, Q.gpix, Q.smp, Q.bk, kind, SOBOL, PASSES);
             if (STATS) {
                 if (kind < 3u) C.hit[kind]++;
                 if (res == RZ_END_SKY) C.sky++;
@@ -303,7 +303,7 @@ __device__ __forceinline__ void rz_flush_counters(const RzPathArgs &a, const RzS
 // Paths that scatter are appended, ballot-compacted, to the HBM queue the sorted stages start from; paths
 // that leave the scene or are absorbed accumulate here.  36 % of all segments are camera segments.  The cull
 // (rz_tile_cone / rz_tile_keep, rz_device.cuh) is host + device and property-tested on the CPU.
-template <bool STATS, int SOBOL = 0>
+template <bool STATS, int SOBOL = 0, bool PASSES = false>
 __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -384,7 +384,7 @@ __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
                 L[0].bk = bk[0]; L[1].bk = bk[1];
             }
             if (STATS) C.sph += (unsigned long long)(n_ls + n_lm) * ((L[0].live ? 1u : 0u) + (L[1].live ? 1u : 0u));
-            rz_shade_and_push2<STATS, SOBOL>(a, L, lane, lt_mask, C);
+            rz_shade_and_push2<STATS, SOBOL, PASSES>(a, L, lane, lt_mask, C);
         }
         __syncwarp();   // the lists are rewritten for the next unit
     }
@@ -475,7 +475,7 @@ __global__ void __launch_bounds__(128) rz_bin_lists_kernel(const RzPathArgs a) {
 // Round 1 sorted on all 16 key bits (two radix passes) and culled each unit with its largest reach; ordering by reach
 // inside the unit costs one global pass less and culls every batch with its OWN reach.  The cull functions are host +
 // device and property-tested on the CPU (tests/test_hostsim_cpu.py).
-template <bool STATS, int SOBOL = 0>
+template <bool STATS, int SOBOL = 0, bool PASSES = false>
 __global__ void RZ_SECOND_BOUNDS rz_second_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -602,7 +602,7 @@ __global__ void RZ_SECOND_BOUNDS rz_second_kernel(const RzPathArgs a) {
                 L[0].bk = bk[0]; L[1].bk = bk[1];
             }
             if (STATS) C.sph += (unsigned long long)(n_ls + n_lm) * ((L[0].live ? 1u : 0u) + (L[1].live ? 1u : 0u));
-            rz_shade_and_push2<STATS, SOBOL>(a, L, lane, lt_mask, C);
+            rz_shade_and_push2<STATS, SOBOL, PASSES>(a, L, lane, lt_mask, C);
         }
         __syncwarp();
     }
@@ -618,18 +618,20 @@ static size_t rz_second_smem_bytes(const RzPathArgs &a) {
 }
 
 static auto rz_second_instance(const RzPathArgs &a, int collect_stats) {
-    return rz_pick_instance(a, collect_stats, [](auto S, auto M) { return rz_second_kernel<decltype(S)::value, decltype(M)::value>; });
+    return rz_pick_instance(a, collect_stats, [](auto S, auto M, auto P) { return rz_second_kernel<decltype(S)::value, decltype(M)::value, decltype(P)::value>; });
 }
 
 // One form of rz_path_kernel on the persistent grid; rays_per_thread in {1,2}.
 template <bool QUEUE, bool LIST>
 static cudaError_t rz_launch_one(const RzPathArgs &a, int rays_per_thread, int collect_stats, int sm_count, cudaStream_t stream,
                                  int *grid_out) {
-    const auto one = rz_pick_instance(a, collect_stats, [](auto S, auto M) { return rz_path_kernel<1, 2, decltype(S)::value, 5, QUEUE, LIST, decltype(M)::value>; });
+    const auto one = rz_pick_instance(a, collect_stats, [](auto S, auto M, auto P) {
+        return rz_path_kernel<1, 2, decltype(S)::value, 5, QUEUE, LIST, decltype(M)::value, decltype(P)::value>;
+    });
     // 8 resident CTAs per SM (64 registers, 232 B of spills outside the search loop) measured 3 % faster than the 5 CTAs the
     // unconstrained 88-register build gets: 1522 vs 1472 Mpaths/s at config 2 / 100 spp.  (The STATS instances keep 5.)
-    const auto two = rz_pick_instance(a, collect_stats, [](auto S, auto M) {
-        return rz_path_kernel<2, 2, decltype(S)::value, decltype(S)::value ? 5 : 8, QUEUE, LIST, decltype(M)::value>;
+    const auto two = rz_pick_instance(a, collect_stats, [](auto S, auto M, auto P) {
+        return rz_path_kernel<2, 2, decltype(S)::value, decltype(S)::value ? 5 : 8, QUEUE, LIST, decltype(M)::value, decltype(P)::value>;
     });
     const auto kern = rays_per_thread == 1 ? one : two;
     const size_t smem = rz_pk_bytes(a);
@@ -658,7 +660,7 @@ extern "C" size_t rz_primary_smem_bytes(const RzPathArgs *a) {
 
 // Stage 1: camera segments of the work units [unit_base, unit_base + n_units) -> queue.
 extern "C" cudaError_t rz_launch_primary(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream) {
-    const auto kern = rz_pick_instance(*a, collect_stats, [](auto S, auto M) { return rz_primary_kernel<decltype(S)::value, decltype(M)::value>; });
+    const auto kern = rz_pick_instance(*a, collect_stats, [](auto S, auto M, auto P) { return rz_primary_kernel<decltype(S)::value, decltype(M)::value, decltype(P)::value>; });
     const size_t smem = rz_primary_smem_bytes(a);
     int grid = 0;
     const cudaError_t e = rz_persistent_grid(kern, smem, sm_count, &grid);

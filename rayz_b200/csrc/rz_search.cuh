@@ -329,19 +329,25 @@ __device__ __forceinline__ const float4 *rz_stage_scene_cv(const RzSphereSet &se
 // as a uniform bit inside the Sobol instances cost plain Sobol 2 to 4 % of its Mpaths/s.
 template <class K>
 static inline K rz_pick_sampler(const RzPathArgs &a, K philox, K sobol, K rqmc) {
-    return (a.sobol & RZ_SAMPLER_RQMC) ? rqmc : a.sobol ? sobol : philox;
+    return (a.sobol & RZ_SAMPLER_RQMC) ? rqmc : (a.sobol & RZ_SAMPLER_SOBOL) ? sobol : philox;
 }
 
-// The instance a launcher runs for (collect_stats, a.sobol).  `inst` names the kernel's instances once, as a generic lambda of
-// (std::integral_constant<bool, STATS>, std::integral_constant<int, SOBOL>), e.g.
-//   [](auto S, auto M) { return rz_second_kernel<decltype(S)::value, decltype(M)::value>; }
+// The instance a launcher runs for (collect_stats, a.sobol).  `inst` names the kernel's instances once, as a
+// generic lambda of (std::integral_constant<bool, STATS>, std::integral_constant<int, SOBOL>, std::integral_constant<bool, PASSES>),
+// e.g.
+//   [](auto S, auto M, auto P) { return rz_second_kernel<decltype(S)::value, decltype(M)::value, decltype(P)::value>; }
+// PASSES (RZ_RENDER_PASSES) is an instance of its own for the reason SOBOL is: the default instances carry no trace of it.
 template <int V> using rz_int_c = std::integral_constant<int, V>;
+template <class F, class S, class P>
+static inline auto rz_pick_sampler_of(const RzPathArgs &a, F inst, S stats, P passes) {
+    return rz_pick_sampler(a, inst(stats, rz_int_c<0>(), passes), inst(stats, rz_int_c<1>(), passes), inst(stats, rz_int_c<2>(), passes));
+}
 template <class F>
 static inline auto rz_pick_instance(const RzPathArgs &a, int collect_stats, F inst) {
     const std::true_type T{};
     const std::false_type N{};
-    return collect_stats ? rz_pick_sampler(a, inst(T, rz_int_c<0>()), inst(T, rz_int_c<1>()), inst(T, rz_int_c<2>()))
-                         : rz_pick_sampler(a, inst(N, rz_int_c<0>()), inst(N, rz_int_c<1>()), inst(N, rz_int_c<2>()));
+    if (a.sobol & RZ_PATH_PASSES) return collect_stats ? rz_pick_sampler_of(a, inst, T, T) : rz_pick_sampler_of(a, inst, N, T);
+    return collect_stats ? rz_pick_sampler_of(a, inst, T, N) : rz_pick_sampler_of(a, inst, N, N);
 }
 
 // Grid of a persistent kernel: as many 128-thread CTAs as fit on every SM with `smem` bytes of dynamic shared memory.  The
@@ -362,9 +368,11 @@ enum { RZ_CONT = 0, RZ_END_SKY = 1, RZ_END_ABSORBED = 2, RZ_END_DEPTH = 3 };
 // One step of bounceRay (renderer.zig:103-126) after the closest-hit query: miss -> sky and
 // accumulate; hit -> refine in f64, scatter, attenuate.  `kind_out` = material kind of the hit.  `sobol`: the kernel's SOBOL
 // template argument (0 Philox, 1 RZ_RENDER_SOBOL, 2 with RZ_RENDER_RQMC), a compile-time constant, so that the Philox instances
-// carry no trace of the other sampler.
+// carry no trace of the other sampler.  `passes`: the kernel's PASSES template argument (RZ_RENDER_PASSES), likewise: seg also
+// carries the first hit's kind (rz_seg_after_hit) and a sky path adds its radiance to its pass too.
 __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray, float3 &thr, uint32_t &seg, uint32_t lp,
-                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, int sobol) {
+                                                uint32_t gpix, uint32_t sample, int bk, uint32_t &kind_out, int sobol,
+                                                bool passes = false) {
     kind_out = 3u;
     if (bk < 0) {
         // miss: background (renderer.zig:124-125), path ends
@@ -379,6 +387,14 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
         if (sobol == 2)
             atomicAdd(a.accum + rz_rep_offset(a.n_local_px) + (size_t)lp * 2u + (sample & 1u),
                       rz_fixed32(rz_clamp_radiance(rz_luma(rz_clamp_radiance(L.x), rz_clamp_radiance(L.y), rz_clamp_radiance(L.z)))));
+        // RZ_RENDER_PASSES: the same three values into the path's pass (the beauty above is never derived from the passes)
+        if (passes) {
+            unsigned long long *ps = a.accum + rz_pass_offset(a.n_local_px, sobol == 2) +
+                                     ((size_t)lp * RZ_PASS_COUNT + rz_pass_of(rz_seg_hits(seg), rz_seg_first_kind(seg))) * 3u;
+            atomicAdd(ps + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.f), 1048576.f) * 4294967296.f));
+            atomicAdd(ps + 1, __float2ull_rn(fminf(fmaxf(L.y, 0.f), 1048576.f) * 4294967296.f));
+            atomicAdd(ps + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.f), 1048576.f) * 4294967296.f));
+        }
         return RZ_END_SKY;
     }
     const int k = bk & ~RZ_FAR_BIT;
@@ -394,15 +410,17 @@ __device__ __forceinline__ int rz_shade_segment(const RzPathArgs &a, RzRay &ray,
     M.inv_scale = __hiloint2double(__float_as_int(m3.y), __float_as_int(m3.x));
     const uint32_t kind = M.kind;
     kind_out = kind < 3u ? kind : 0u;
-    seg++;
-    const uint4 rb = rz_philox(gpix, sample, seg, 0u, a.seed_lo, a.seed_hi);
-    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(seg), sample, sobol == 2)   // u.z, u.w stay Philox
+    if (passes) seg = rz_seg_after_hit(seg, kind_out);
+    else seg++;
+    const uint32_t hits = passes ? rz_seg_hits(seg) : seg;   // the bounce number every draw and the depth test read
+    const uint4 rb = rz_philox(gpix, sample, hits, 0u, a.seed_lo, a.seed_hi);
+    const float2 q = sobol ? rz_sobol_u01(a.seed_lo, a.seed_hi, gpix, rz_pair_bounce(hits), sample, sobol == 2)   // u.z, u.w stay Philox
                            : make_float2(rz_u01(rb.x >> 8), rz_u01(rb.y >> 8));
     const float4 u = make_float4(q.x, q.y, rz_u01(rb.z >> 8), rz_u01(rb.w >> 8));
     float3 att;
     if (!rz_scatter(M, a.texs, h, k, u, ray, att)) return RZ_END_ABSORBED;  // black (renderer.zig:109,120)
     thr = thr * att;
-    if (seg >= a.max_depth) return RZ_END_DEPTH;  // depth == 0 => black (renderer.zig:104-105)
+    if (hits >= a.max_depth) return RZ_END_DEPTH;  // depth == 0 => black (renderer.zig:104-105)
     return RZ_CONT;
 }
 

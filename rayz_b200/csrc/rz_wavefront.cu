@@ -196,7 +196,7 @@ __global__ void wf_after_intersect(WfState s) {
     c->q_total = off;
 }
 
-template <bool STATS, int SOBOL>
+template <bool STATS, int SOBOL, bool PASSES>
 __global__ void __launch_bounds__(256) wf_shade(const RzPathArgs a, WfState s) {
     const WfCounters c = *s.ctr;
     const unsigned int M = s.M;
@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(256) wf_shade(const RzPathArgs a, WfState s) {
             if (doa) { res = RZ_END_DEPTH; kind = 3u; }
             else {
                 if (STATS) c_segs++;
-                res = rz_shade_segment(a, ray, thr, seg, D.x, D.y, D.z, (int)D.w, kind, SOBOL);
+                res = rz_shade_segment(a, ray, thr, seg, D.x, D.y, D.z, (int)D.w, kind, SOBOL, PASSES);
                 if (STATS) {
                     if (kind < 3u) c_hit[kind]++;
                     if (res == RZ_END_SKY) c_sky++;
@@ -328,11 +328,11 @@ extern "C" cudaError_t rz_wavefront_render(const RzPathArgs *a, int sm_count, in
         cudaGraph_t g;
         if ((e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal)) != cudaSuccess) return e;
         for (int it = 0; it < ITERS; it++) {
-            rz_pick_instance(*a, st, [](auto S, auto M) { return wf_generate<decltype(S)::value, decltype(M)::value>; })<<<grid_s, 256, 0, cap>>>(*a, ws->st);
+            rz_pick_instance(*a, st, [](auto S, auto M, auto) { return wf_generate<decltype(S)::value, decltype(M)::value>; })<<<grid_s, 256, 0, cap>>>(*a, ws->st);
             wf_after_generate<<<1, 1, 0, cap>>>(ws->st);
             wf_intersect<2><<<grid_i, 128, smem, cap>>>(*a, ws->st);
             wf_after_intersect<<<1, 1, 0, cap>>>(ws->st);
-            rz_pick_instance(*a, st, [](auto S, auto M) { return wf_shade<decltype(S)::value, decltype(M)::value>; })<<<grid_s, 256, 0, cap>>>(*a, ws->st);
+            rz_pick_instance(*a, st, [](auto S, auto M, auto P) { return wf_shade<decltype(S)::value, decltype(M)::value, decltype(P)::value>; })<<<grid_s, 256, 0, cap>>>(*a, ws->st);
             wf_advance<<<1, 1, 0, cap>>>(ws->st);
         }
         cudaMemcpyAsync(ws->h_done, &ws->st.ctr->done, sizeof(unsigned int), cudaMemcpyDeviceToHost, cap);

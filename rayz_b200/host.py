@@ -278,13 +278,14 @@ class Backend:
     @staticmethod
     def params(width, height, spp, max_depth=50, seed=1, sample_offset=0, variant="auto", t_min=0.0, shard_index=0,
                shard_count=1, band_rows=0, collect_stats=False, serial_passes=False, accumulate=False,
-               moments=False, sobol=False, rqmc=False) -> abi.RzRenderParams:
+               moments=False, sobol=False, rqmc=False, passes=False) -> abi.RzRenderParams:
         """RzRenderParams.  accumulate: add this batch to the previous render's sums (RZ_RENDER_ACCUMULATE; sample_offset must
         continue where they end); moments: also sum each path's luminance squared, so that noise() can estimate the error;
         sobol: draw the camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox (RZ_RENDER_SOBOL);
         rqmc: two independently scrambled Sobol replicates per pixel, so that the noise estimate sees the stratification
         (RZ_RENDER_RQMC).  rqmc does not imply sobol or moments: the library refuses it without both, and with an odd spp or
-        sample_offset."""
+        sample_offset.  passes: also sum each path's radiance into its light-path pass, so that passes() can split the frame
+        (RZ_RENDER_PASSES; no pixel changes)."""
         p = abi.RzRenderParams()
         p.width, p.height, p.spp, p.max_depth = width, height, spp, max_depth
         p.seed, p.sample_offset = seed, sample_offset
@@ -293,7 +294,8 @@ class Backend:
         p.shard_index, p.shard_count, p.band_rows = shard_index, shard_count, band_rows
         p.collect_stats = 1 if collect_stats else 0
         p.flags = ((abi.RENDER_SERIAL_PASSES if serial_passes else 0) | (abi.RENDER_ACCUMULATE if accumulate else 0)
-                   | (abi.RENDER_MOMENTS if moments else 0) | (abi.RENDER_SOBOL if sobol else 0) | (abi.RENDER_RQMC if rqmc else 0))
+                   | (abi.RENDER_MOMENTS if moments else 0) | (abi.RENDER_SOBOL if sobol else 0) | (abi.RENDER_RQMC if rqmc else 0)
+                   | (abi.RENDER_PASSES if passes else 0))
         return p
 
     def reserve(self, p: abi.RzRenderParams):
@@ -365,6 +367,16 @@ class Backend:
         rows, w = int(self.lib.rayz_cuda_context_rows(self._h, self._acc_shape[0], *self._acc_shape[2:])), self._acc_shape[1]
         out = np.empty((rows, w), dtype=np.uint32)
         abi.check(self.lib.rayz_cuda_pixel_samples(self._h, out.ctypes.data))
+        return out
+
+    def passes(self) -> np.ndarray:
+        """rayz_cuda_passes: the light-path passes of the accumulated frame (rendered with passes=True) -> [7,rows,w,4] f32,
+        plane i = pass abi.PASS_NAMES[i], each laid out like render()'s linear; they sum to the linear frame to f32 rounding."""
+        if self._acc_shape is None:   # nothing rendered: the library says why
+            abi.check(self.lib.rayz_cuda_passes(self._h, None))
+        rows, w = int(self.lib.rayz_cuda_context_rows(self._h, self._acc_shape[0], *self._acc_shape[2:])), self._acc_shape[1]
+        out = np.empty((abi.PASS_COUNT, rows, w, 4), dtype=np.float32)
+        abi.check(self.lib.rayz_cuda_passes(self._h, out.ctypes.data))
         return out
 
     def guides(self, cam: abi.RzCamera, p: abi.RzRenderParams):
@@ -480,14 +492,15 @@ class Tracer:
         return self._backend
 
     def render(self, noise_target: float | None = None, max_spp: int = 4096, adaptive: bool = False, moments: bool = False,
-               pooled: bool = False) -> int:
+               pooled: bool = False, passes: bool = False) -> int:
         """noise_target (displayed-value rms error, 1/255 = one 8-bit step): start at samples_per_px and double the samples
         until the frame's rms error reaches it or max_spp samples are in (rayz_cuda_render_to_noise); `self.noise` then holds
         the summary.  adaptive: the target bounds every pixel's error, and only the pixels still above it get more samples;
         `self.pixel_samples` then holds the counts; pooled (with adaptive): each pixel stops on an error pooled with its row
         segment's (RZ_RENDER_ADAPTIVE_POOLED), so that the bound holds for the measured error; the library refuses it
         elsewhere.  Without a target, one render of samples_per_px, as the reference; moments: also sum what the per-pixel
-        noise estimate needs (RZ_RENDER_MOMENTS, no pixel changes), so that denoise() can follow."""
+        noise estimate needs (RZ_RENDER_MOMENTS, no pixel changes), so that denoise() can follow; passes: also sum the
+        light-path passes (RZ_RENDER_PASSES, no pixel changes), so that passes() can follow."""
         b = self.backend
         arrays = self.pool.arrays()
         self._uploaded = None
@@ -498,6 +511,8 @@ class Tracer:
         p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant, **kw)
         if pooled:
             p.flags |= abi.RENDER_ADAPTIVE_POOLED
+        if passes:
+            p.flags |= abi.RENDER_PASSES
         if noise_target is None:
             lin, rgb8, rays = b.render(self.camera.rz, p)
         else:
@@ -507,6 +522,11 @@ class Tracer:
         self.img.rgb8 = rgb8
         return rays
 
+    def passes(self) -> dict:
+        """The light-path passes of the last render(passes=True) (rayz_cuda_passes): pass name (abi.PASS_NAMES) -> linear
+        [h, w, 4] f32 image; the images sum to the render's linear frame to f32 rounding."""
+        planes = self.backend.passes()
+        return {name: planes[i] for i, name in enumerate(abi.PASS_NAMES)}
 
     def render_guides(self):
         """Guide buffers for a denoiser over the camera samples render() traces (samples_per_px, seed): first-hit albedo with

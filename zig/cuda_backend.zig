@@ -77,6 +77,16 @@ pub const RZ_RENDER_ADAPTIVE: u32 = 8; // rayz_cuda_render_to_noise: the target 
 pub const RZ_RENDER_SOBOL: u32 = 0x10; // camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox
 pub const RZ_RENDER_RQMC: u32 = 0x20; // with SOBOL and MOMENTS: two scrambled replicates per pixel, a noise estimate that sees the stratification
 pub const RZ_RENDER_ADAPTIVE_POOLED: u32 = 0x40; // with ADAPTIVE, rayz_cuda_render_to_noise only: stop each pixel on an error pooled over its row segment
+pub const RZ_RENDER_PASSES: u32 = 0x80; // also sum each path's radiance into its light-path pass (rayz_cuda_passes); no pixel changes
+// light-path passes: plane index of rayz_cuda_passes' output (include/rayz_cuda.h "Light-path passes")
+pub const RZ_PASS_ENVIRONMENT: u32 = 0;
+pub const RZ_PASS_DIFFUSE_DIRECT: u32 = 1;
+pub const RZ_PASS_DIFFUSE_INDIRECT: u32 = 2;
+pub const RZ_PASS_GLOSSY_DIRECT: u32 = 3;
+pub const RZ_PASS_GLOSSY_INDIRECT: u32 = 4;
+pub const RZ_PASS_TRANSMISSION_DIRECT: u32 = 5;
+pub const RZ_PASS_TRANSMISSION_INDIRECT: u32 = 6;
+pub const RZ_PASS_COUNT: u32 = 7;
 
 pub const RzNoise = extern struct {
     samples: u64,
@@ -107,6 +117,7 @@ pub extern fn rayz_cuda_primary_ids(ctx: *RzContext, cam: *const RzCamera, width
 pub extern fn rayz_cuda_noise(ctx: *RzContext, target: f32, out_err: ?[*]f32, out: ?*RzNoise) c_int;
 pub extern fn rayz_cuda_render_to_noise(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, target: f32, max_spp: u32, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8, out_paths: ?*u64, out_noise: ?*RzNoise) c_int;
 pub extern fn rayz_cuda_pixel_samples(ctx: *RzContext, out_spp: [*]u32) c_int;
+pub extern fn rayz_cuda_passes(ctx: *RzContext, out_passes: [*]f32) c_int; // RZ_PASS_COUNT planes of rows x width x 4
 // guide buffers for a denoiser: first-hit albedo + coverage, normal + hit distance (rows * width * 4 floats each)
 pub extern fn rayz_cuda_render_guides(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, out_albedo: ?[*]f32, out_normal: ?[*]f32) c_int;
 // the accumulated frame (RZ_RENDER_MOMENTS) denoised with the guides of the last rayz_cuda_render_guides call (rows * width * 4 floats, * 3 bytes)
