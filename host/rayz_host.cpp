@@ -3,7 +3,7 @@
 //     rayz_host <img_w> [out.ppm] [--spp N] [--depth N] [--seed S] [--render-seed S]
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
-//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc] [--pooled] [--passes PREFIX]
+//               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc] [--pooled] [--passes PREFIX] [--mattes PREFIX]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -24,6 +24,9 @@
 // --passes PREFIX renders with RZ_RENDER_PASSES (no pixel changes) and writes the frame's seven light-path passes
 // (rayz_cuda_passes) as 3-channel PFM files PREFIX_<name>.pfm, name = environment, diffuse_direct, diffuse_indirect,
 // glossy_direct, glossy_indirect, transmission_direct, transmission_indirect; they sum to the frame's linear values.
+// --mattes PREFIX also writes the ID mattes of the render's camera samples (rayz_cuda_render_mattes), six ranks, as 3-channel
+// PFM files PREFIX_rank<r>.pfm: the rank's sphere index as a float (-1 the sky, -2 no such rank), its coverage, 0.  Mattes
+// take at most 1024 samples per pixel.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -48,7 +51,8 @@ int main(int argc, char **argv) {
     size_t spp = 10, depth = 50;
     int gpus = 1, grid = 11;
     uint32_t variant = RZ_VARIANT_AUTO;
-    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr, *passes = nullptr;
+    const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr, *passes = nullptr,
+               *mattes = nullptr;
     bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false, rqmc = false, pooled = false;
     float noise_target = 0;
     uint32_t max_spp = 4096;
@@ -73,6 +77,7 @@ int main(int argc, char **argv) {
         else if (a == "--guides") guides = val();
         else if (a == "--denoise") denoise = val();
         else if (a == "--passes") passes = val();
+        else if (a == "--mattes") mattes = val();
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -80,6 +85,7 @@ int main(int argc, char **argv) {
         } else if (!out_fname && a.rfind("--", 0) != 0) out_fname = argv[i];
         else { std::fprintf(stderr, "unknown argument %s\n", a.c_str()); return 2; }
     }
+    if (mattes && spp > RZ_MATTE_MAX_SPP) { std::fprintf(stderr, "--mattes: --spp %zu is above the mattes' %u samples per pixel\n", spp, RZ_MATTE_MAX_SPP); return 2; }
     if (!have_seed) { std::random_device rd; seed = ((uint64_t)rd() << 32) ^ rd(); }  // renderer.zig:55-59: seeded from the OS
 
     try {
@@ -148,6 +154,23 @@ int main(int argc, char **argv) {
             if (!f) { std::perror(denoise); return 1; }
             tracer.denoised.writePPM(f);
             std::fclose(f);
+        }
+        if (mattes) {
+            const uint32_t ranks = 6;
+            tracer.renderMattes(ranks);
+            const size_t npx = tracer.img.w * tracer.img.h;
+            std::vector<float> plane(npx * 3, 0.f);
+            for (uint32_t r = 0; r < ranks; r++) {
+                for (size_t i = 0; i < npx; i++) {
+                    plane[3 * i] = (float)tracer.matte_ids[i * ranks + r];
+                    plane[3 * i + 1] = tracer.matte_coverage[i * ranks + r];
+                }
+                const std::string path = std::string(mattes) + "_rank" + std::to_string(r) + ".pfm";
+                FILE *f = std::fopen(path.c_str(), "wb");
+                if (!f) { std::perror(path.c_str()); return 1; }
+                writePFM(f, plane.data(), tracer.img.w, tracer.img.h, 3, 0, 3);
+                std::fclose(f);
+            }
         }
         if (dump_scene && !dumpScene(tracer, dump_scene)) { std::perror(dump_scene); return 1; }
         if (dump_linear) {

@@ -269,6 +269,8 @@ struct Tracer {
     bool passes = false;          // RZ_RENDER_PASSES (no pixel changes), so that readPasses() can follow
     std::vector<float> pass_planes;   // light-path passes of the last readPasses(): RZ_PASS_COUNT planes of h x w x 4 floats
     Image denoised;               // rgb8 of the last denoise()
+    std::vector<int32_t> matte_ids;      // ID mattes of the last renderMattes(): h x w x ranks caller's sphere indices
+    std::vector<float> matte_coverage;   // ... and the fraction of the pixel's samples each covers
 
     Tracer(size_t img_w, double vfov, double focus_dist, double defocus_angle, V3 look_from, V3 look_at, V3 vup, uint64_t seed)
         : rng(seed) {
@@ -370,6 +372,16 @@ struct Tracer {
         albedo.assign(img.w * img.h * 4, 0.f);
         normal.assign(img.w * img.h * 4, 0.f);
         check(rayz_cuda_render_guides(ctx, &cam, &p, albedo.data(), normal.data()));
+    }
+
+    // ID mattes of the camera samples render() traces, ranked per pixel by coverage (rayz_cuda_render_mattes), after render().
+    void renderMattes(uint32_t ranks) {
+        RzRenderParams p = renderParams();
+        p.flags &= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;   // the render's own camera rays, as renderGuides()
+        const RzCamera cam = camera.flat();
+        matte_ids.assign(img.w * img.h * ranks, 0);
+        matte_coverage.assign(img.w * img.h * ranks, 0.f);
+        check(rayz_cuda_render_mattes(ctx, &cam, &p, ranks, matte_ids.data(), matte_coverage.data()));
     }
 
     // The frame of the last render() (with moments, or a noise target) denoised with the guides of renderGuides(), after it

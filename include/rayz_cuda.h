@@ -436,6 +436,32 @@ int rayz_cuda_passes(RzContext *ctx, float *out_passes);
 int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, float *out_albedo, float *out_normal);
 
 /*
+ * ID mattes, for compositing (the data Cryptomatte stores): per pixel of the context's rows, the spheres its camera samples
+ * [p->sample_offset, p->sample_offset + p->spp) hit first, ranked by exact coverage.  The samples are the SAME camera rays a
+ * render with these parameters traces and rayz_cuda_render_guides follows (jitter, lens point, shutter time, every sampler),
+ * each followed to its first hit by the BVH kernel's search.  A sample's id is the caller's index of that sphere
+ * (RzScene order), or RZ_MATTE_MISS for a miss.  n_id = the pixel's samples with that id.  Ranks are ordered by n_id
+ * descending, then id ascending: a total order, so the result depends on (scene, camera, seed, pixel, sample range) only, not
+ * on shards, devices or launch shape.  Host outputs, each nullable, of rows * width * ranks entries, rank r of local pixel lp at
+ * lp * ranks + r (rows ordered like out_linear_rgba):
+ *   out_ids      : the id of the rank, RZ_MATTE_EMPTY past the pixel's distinct ids
+ *   out_coverage : (float)((double)n_id / (double)spp), 0 past the pixel's distinct ids
+ * Counts are recoverable exactly as rint(coverage * spp); with ranks >= spp the ranks hold the pixel's whole histogram.
+ * max_depth and collect_stats have no effect.  Refused with nothing touched, messages prefixed "mattes:": RZ_ERR_INVALID_ARG for
+ * NULL ctx, cam or p, ranks of 0 or above RZ_MATTE_MAX_RANKS, spp above RZ_MATTE_MAX_SPP, and RZ_RENDER_ACCUMULATE,
+ * RZ_RENDER_ADAPTIVE, RZ_RENDER_ADAPTIVE_POOLED or RZ_RENDER_PASSES in the flags; parameters a render refuses, with its codes.
+ * RZ_ERR_INTERNAL if the traversal stack overflowed (results withheld, the context stays usable).  Leaves the accumulated frame,
+ * its sample counts, the guide buffers, RzStats, RzTiming and rayz_cuda_render_device's buffers untouched (a render enqueued by
+ * rayz_cuda_render_device(sync = 0) is waited for first, as rayz_cuda_render_guides does).
+ */
+#define RZ_MATTE_MISS   (-1)    /* id of a camera sample that hit no sphere (the sky)              */
+#define RZ_MATTE_EMPTY  (-2)    /* id of a rank past the pixel's distinct ids; its coverage is 0   */
+#define RZ_MATTE_MAX_RANKS 16u
+#define RZ_MATTE_MAX_SPP 1024u
+int rayz_cuda_render_mattes(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, uint32_t ranks,
+                            int32_t *out_ids, float *out_coverage);
+
+/*
  * Denoiser parameters (rayz_cuda_denoise).  A zero sigma takes its default.
  */
 typedef struct RzDenoiseParams {

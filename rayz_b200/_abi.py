@@ -26,6 +26,8 @@ RENDER_PASSES = 0x80            # also sum each sky path's radiance into its lig
 PASS_NAMES = ("environment", "diffuse_direct", "diffuse_indirect", "glossy_direct", "glossy_indirect", "transmission_direct",
               "transmission_indirect")
 PASS_COUNT = len(PASS_NAMES)
+# ID mattes (rayz_cuda_render_mattes): the id of a sample that hit no sphere, of a rank past the pixel's distinct ids, and limits
+MATTE_MISS, MATTE_EMPTY, MATTE_MAX_RANKS, MATTE_MAX_SPP = -1, -2, 16, 1024
 
 _dp, _up = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 
@@ -114,6 +116,8 @@ SYMBOLS = {
     "rayz_cuda_pixel_samples": (C.c_int, [C.c_void_p, C.c_void_p]),
     "rayz_cuda_passes": (C.c_int, [C.c_void_p, C.c_void_p]),
     "rayz_cuda_render_guides": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_void_p, C.c_void_p]),
+    "rayz_cuda_render_mattes": (C.c_int, [C.c_void_p, C.POINTER(RzCamera), C.POINTER(RzRenderParams), C.c_uint32, C.c_void_p,
+                                          C.c_void_p]),
     "rayz_cuda_denoise": (C.c_int, [C.c_void_p, C.POINTER(RzDenoiseParams), C.c_void_p, C.c_void_p]),
     "rayz_cuda_shard_rows": (C.c_uint32, [C.c_uint32] * 4),
     "rayz_cuda_context_rows": (C.c_uint32, [C.c_void_p] + [C.c_uint32] * 4),

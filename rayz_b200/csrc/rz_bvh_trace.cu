@@ -579,6 +579,96 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGui
         g.out_normal[dst] = make_float4((float)(nx / n), (float)(ny / n), (float)(nz / n), hits ? (float)(dist / (double)hits) : 0.f);
 }
 
+// ID mattes: the guides' camera samples and walk, each sample's first-hit id (the caller's sphere index, RZ_MATTE_MISS) tallied
+// per pixel and ranked by rz_matte_key.  One warp per pixel, four per CTA: lane l traces samples l, l + 32, ... (the rays of one
+// pixel are more coherent than those of an 8 x 4 block) and stores their ids in the warp's n_pad ints of shared memory.  The
+// warp sorts them (bitonic, n_pad a power of two, padded with INT32_MAX), so every id is one run; lane l owns the run ENDS in
+// positions [l c, l c + c), c = n_pad / 32, and the start of the run it enters from the lane before (a max-scan).  Rank r is the
+// warp's least run key above rank r - 1's.  Exact for any scene: a pixel can see spp distinct ids and every one is a run.
+template <int SOBOL>
+__global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_mattes_kernel(const RzMatteArgs g) {
+    extern __shared__ int32_t rz_matte_ids[];
+    const RzPathArgs &a = g.a;
+    const unsigned lane = threadIdx.x & 31u;
+    const uint32_t n_pad = g.n_pad, spp = a.spp;
+    int32_t *ids = rz_matte_ids + (threadIdx.x >> 5) * n_pad;
+    const uint32_t lp = blockIdx.x * 4u + (threadIdx.x >> 5);
+    if (lp >= a.n_local_px) return;   // the whole warp
+    const float4 *__restrict__ nodes = reinterpret_cast<const float4 *>(a.bvh);
+    uint32_t pi = 0, pj = 0;
+    rz_local_to_global(lp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
+    const uint32_t gpix = pj * a.width + pi;
+    const int descend_min = (int)a.bvh_descend_min;
+    int stack[RZ_STACK];
+    unsigned long long c_none = 0;   // rz_bvh_round's counters: untouched without STATS
+    for (uint32_t s0 = 0; s0 < spp; s0 += 32u) {
+        const uint32_t s = s0 + lane;
+        const bool live = s < spp;
+        RzRay ray;
+        if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL);
+        else { ray.o = f3(0.f, 0.f, 0.f); ray.d = f3(0.f, 1.f, 0.f); ray.time = 0.f; ray.self_k = -1; }
+        const float ix = 1.0f / ray.d.x, iy = 1.0f / ray.d.y, iz = 1.0f / ray.d.z;
+        float bt = 3.0e38f;
+        int bk = -1, sp = 0, cur = live ? 0 : RZ_SENTINEL;
+        while (__any_sync(0xffffffffu, cur != RZ_SENTINEL))
+            rz_bvh_round<false>(a, nodes, ray, ix, iy, iz, cur, sp, stack, bt, bk, descend_min, c_none, c_none);
+        if (live) ids[s] = bk < 0 ? (int32_t)RZ_MATTE_MISS : __ldg(a.set.orig + (bk & ~RZ_FAR_BIT));
+    }
+    for (uint32_t s = spp + lane; s < n_pad; s += 32u) ids[s] = 0x7fffffff;
+    __syncwarp();
+    for (uint32_t k = 2u; k <= n_pad; k <<= 1)
+        for (uint32_t j = k >> 1; j > 0u; j >>= 1) {
+            for (uint32_t t = lane; t < n_pad / 2u; t += 32u) {   // pair t: i = t with a 0 inserted at bit log2(j), and i + j
+                const uint32_t i = ((t & ~(j - 1u)) << 1) | (t & (j - 1u));
+                const int32_t x = ids[i], y = ids[i + j];
+                if ((x > y) == ((i & k) == 0u)) { ids[i] = y; ids[i + j] = x; }
+            }
+            __syncwarp();
+        }
+    // the first spp positions are the ids, sorted; the padding sorts after them
+    const uint32_t c = n_pad / 32u, p0 = lane * c, p1 = min(p0 + c, spp);
+    int last = -1;   // the last run start in this lane's positions
+    for (uint32_t p = p0; p < p1; p++)
+        if (p == 0u || ids[p] != ids[p - 1u]) last = (int)p;
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, last, o);
+        if ((int)lane >= o) last = max(last, v);
+    }
+    int carry = __shfl_up_sync(0xffffffffu, last, 1);   // the start of the run that enters this lane's positions
+    if (lane == 0u) carry = 0;
+    unsigned long long prev = 0ull, mine = ~0ull;       // every key is above 0; ~0ull: no run left (RZ_MATTE_EMPTY)
+    for (uint32_t r = 0; r < g.ranks; r++) {
+        unsigned long long best = ~0ull;
+        int start = carry;
+        for (uint32_t p = p0; p < p1; p++) {
+            const int32_t v = ids[p];
+            if (p == 0u || v != ids[p - 1u]) start = (int)p;
+            if (p + 1u == spp || v != ids[p + 1u]) {
+                const unsigned long long key = rz_matte_key(p + 1u - (uint32_t)start, v);
+                if (key > prev && key < best) best = key;
+            }
+        }
+        for (int o = 16; o > 0; o >>= 1) {
+            const unsigned long long v = __shfl_xor_sync(0xffffffffu, best, o);
+            best = v < best ? v : best;
+        }
+        if (best == ~0ull) break;   // the pixel's distinct ids are all ranked
+        if (lane == r) mine = best;
+        prev = best;
+    }
+    if (lane >= g.ranks) return;
+    size_t dst = lp;
+    if (g.dev_count > 1u) {   // rz_resolve_kernel's band arithmetic
+        const uint32_t lr = lp / a.width, lb = lr / a.band_rows, within = lr - lb * a.band_rows;
+        dst = (size_t)((lb * g.dev_count + g.dev_index) * a.band_rows + within) * a.width + (lp - lr * a.width);
+    }
+    dst = dst * g.ranks + lane;
+    const bool empty = mine == ~0ull;
+    if (g.out_ids) g.out_ids[dst] = empty ? (int32_t)RZ_MATTE_EMPTY : rz_matte_key_id(mine);
+    // f64: this unit is built with --use_fast_math, under which an f32 division is approximate
+    if (g.out_coverage) g.out_coverage[dst] = empty ? 0.f : (float)((double)rz_matte_key_count(mine) / (double)spp);
+}
+
 // inst: the kernel's instances (rz_pick_instance), launched on the persistent grid
 template <class F>
 cudaError_t launch_kernel(F inst, const RzPathArgs &a, int collect_stats, int sm_count, cudaStream_t stream) {
@@ -628,6 +718,18 @@ extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t strea
     const uint32_t blocks = ((b.a.width + 7u) / 8u) * ((rows + 3u) / 4u);
     if (blocks == 0u) return cudaSuccess;
     rz_pick_instance(b.a, 0, [](auto, auto M, auto) { return rz_guides_kernel<decltype(M)::value>; })<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
+    return cudaGetLastError();
+}
+
+// ID mattes of the device's local pixels: one warp per pixel, four per CTA, n_pad ids of shared memory per warp.
+extern "C" cudaError_t rz_launch_mattes(const RzMatteArgs *g, cudaStream_t stream) {
+    RzMatteArgs b = *g;
+    rz_bvh_tuning(b.a);
+    if (b.a.n_local_px == 0u) return cudaSuccess;
+    b.n_pad = 32u;
+    while (b.n_pad < b.a.spp) b.n_pad <<= 1;
+    rz_pick_instance(b.a, 0, [](auto, auto M, auto) { return rz_mattes_kernel<decltype(M)::value>; })
+        <<<(b.a.n_local_px + 3u) / 4u, 128, 4u * b.n_pad * sizeof(int32_t), stream>>>(b);
     return cudaGetLastError();
 }
 

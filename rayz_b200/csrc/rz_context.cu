@@ -129,6 +129,8 @@ struct Dev {
     DBuf<uint32_t> out_spp;           // rayz_cuda_pixel_samples: per-pixel sample counts of the context's rows (gather root only)
     DBuf<float4> out_passes;          // rayz_cuda_passes: RZ_PASS_COUNT planes of the context's rows (gather root only)
     DBuf<float4> out_guides;          // rayz_cuda_render_guides: albedo, then normal + depth, of the context's rows (gather root only)
+    DBuf<int32_t> out_matte_ids;      // rayz_cuda_render_mattes: [rows * width][ranks] ids and coverage of the context's rows
+    DBuf<float> out_matte_cov;        // (gather root only; grown for a larger ranks)
     // rayz_cuda_denoise (gather root only): the resolved frame, then the denoised one; the per-pixel error; the ping-pong pair of
     // (demodulated rgb, variance); the depth gradient; the denoised rgb8.  Never Dev::out_linear / out_rgb8, which a
     // rayz_cuda_render_device caller may still hold.
@@ -1544,6 +1546,53 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
     GuideRecord &G = ctx->guides;
     G.frame = P.frame; G.cam = *cam; G.seed = p->seed; G.first_offset = p->sample_offset; G.samples = p->spp;
     G.valid = true;
+    return RZ_OK;
+}
+
+// ID mattes (include/rayz_cuda.h): every device ranks its rows' first-hit ids with rz_mattes_kernel, which stores straight into
+// the gather root's buffers as rz_guides_kernel does; the error words are read behind every stream, then the root's buffers
+// are copied out.  The accumulators, their record, the per-pixel counts, the guide buffers, stats and timing stay as they are.
+extern "C" int rayz_cuda_render_mattes(RzContext *ctx, const RzCamera *cam, const RzRenderParams *p, uint32_t ranks,
+                                       int32_t *out_ids, float *out_coverage) {
+    if (!ctx || !cam || !p) return rz_fail(RZ_ERR_INVALID_ARG, "mattes: NULL argument");
+    if (ranks == 0 || ranks > RZ_MATTE_MAX_RANKS) return rz_fail(RZ_ERR_INVALID_ARG, "mattes: ranks %u outside 1..%u", ranks, RZ_MATTE_MAX_RANKS);
+    if (p->spp > RZ_MATTE_MAX_SPP) return rz_fail(RZ_ERR_INVALID_ARG, "mattes: spp %u above RZ_MATTE_MAX_SPP (%u)", p->spp, RZ_MATTE_MAX_SPP);
+    if (p->flags & (RZ_RENDER_ACCUMULATE | RZ_RENDER_ADAPTIVE | RZ_RENDER_ADAPTIVE_POOLED))
+        return rz_fail(RZ_ERR_INVALID_ARG, "mattes: RZ_RENDER_ACCUMULATE, RZ_RENDER_ADAPTIVE and RZ_RENDER_ADAPTIVE_POOLED do not apply to mattes");
+    if (p->flags & RZ_RENDER_PASSES) return rz_fail(RZ_ERR_INVALID_ARG, "mattes: RZ_RENDER_PASSES does not apply to mattes");
+    RenderPlan P;
+    if (const int rc = plan_render(ctx, cam, p, ctx->acc, P, "mattes")) return rc;
+    DeviceGuard guard;
+    // a render enqueued by rayz_cuda_render_device(sync = 0) reports through the error words this call clears: read them first
+    { const int rc = settle_accumulation(ctx); if (rc) return rc; }
+    const uint32_t ND = (uint32_t)ctx->devs.size();
+    const size_t n = P.split.npx * ranks;
+    Dev &D0 = ctx->devs[0];
+    int rc;
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if ((rc = D0.out_matte_ids.alloc(n)) || (rc = D0.out_matte_cov.alloc(n))) return rc;
+    rc = for_each_device(ctx, [&](uint32_t d) -> int {
+        Dev &D = ctx->devs[d];
+        RZ_CUDA(cudaSetDevice(D.id));
+        int r;
+        if ((r = D.errword.alloc(4))) return r;
+        RZ_CUDA(cudaMemsetAsync(D.errword.p, 0, 4 * sizeof(unsigned int), D.stream));
+        RzMatteArgs g;
+        memset(&g, 0, sizeof g);
+        g.a = path_args(ctx, P, d);
+        g.out_ids = D0.out_matte_ids.p;
+        g.out_coverage = D0.out_matte_cov.p;
+        g.ranks = ranks;
+        g.dev_index = d; g.dev_count = ND;
+        RZ_CUDA(rz_launch_mattes(&g, D.stream));
+        return RZ_OK;
+    });
+    if (rc) return rc;
+    if ((rc = read_error_words(ctx, "mattes"))) return rc;   // behind every device's stream: the root's buffers are complete
+    RZ_CUDA(cudaSetDevice(D0.id));
+    if (out_ids) RZ_CUDA(cudaMemcpyAsync(out_ids, D0.out_matte_ids.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, D0.stream));
+    if (out_coverage) RZ_CUDA(cudaMemcpyAsync(out_coverage, D0.out_matte_cov.p, n * sizeof(float), cudaMemcpyDeviceToHost, D0.stream));
+    RZ_CUDA(cudaStreamSynchronize(D0.stream));
     return RZ_OK;
 }
 

@@ -218,6 +218,24 @@ struct RzGuideArgs {
     uint32_t dev_index, dev_count;   // local row lr -> context row ((lr / band_rows) * dev_count + dev_index) * band_rows + lr % band_rows
 };
 
+// ID mattes (rayz_cuda_render_mattes, rz_mattes_kernel in rz_bvh_trace.cu): the same camera segments as the guides, each
+// sample's first-hit id tallied per pixel and ranked.  The outputs are the gather root's buffers, addressed like the guides'.
+struct RzMatteArgs {
+    RzPathArgs a;                 // read as RzGuideArgs::a is (a.spp <= RZ_MATTE_MAX_SPP)
+    int32_t *out_ids;             // [context rows * width][ranks]: caller's sphere index, RZ_MATTE_MISS or RZ_MATTE_EMPTY
+    float *out_coverage;          // [context rows * width][ranks]: n_id / spp, 0 for RZ_MATTE_EMPTY
+    uint32_t ranks;               // 1..RZ_MATTE_MAX_RANKS
+    uint32_t dev_index, dev_count;   // as RzGuideArgs'
+    uint32_t n_pad;               // ids each warp sorts: the least power of two >= max(spp, 32) (set by rz_launch_mattes)
+};
+// Rank order of a (count, id) run as one 64-bit key: ascending keys are count descending, then id ascending.  Counts are at
+// most RZ_MATTE_MAX_SPP; ids are any int32 (the sign bit flipped keeps their order as unsigned).
+RZ_HD unsigned long long rz_matte_key(uint32_t count, int32_t id) {
+    return ((unsigned long long)(0xffffffffu - count) << 32) | (unsigned long long)((uint32_t)id ^ 0x80000000u);
+}
+RZ_HD uint32_t rz_matte_key_count(unsigned long long key) { return 0xffffffffu - (uint32_t)(key >> 32); }
+RZ_HD int32_t rz_matte_key_id(unsigned long long key) { return (int32_t)((uint32_t)key ^ 0x80000000u); }
+
 // ---------------------------------------------------------------------------------------------
 // Per-pixel noise (RZ_RENDER_MOMENTS, DESIGN.md "Progressive rendering").  Slot 3 of a pixel's accumulator sums Y^2 over its
 // paths in the 2^-32 fixed point of slots 0..2, Y = Rec. 709 luminance of the same clamped radiance the three colour atomics

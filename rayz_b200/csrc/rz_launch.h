@@ -6,7 +6,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-struct RzPathArgs; struct RzGuideArgs; struct RzDenoiseArgs; struct RzBvhNode;   // rz_device.cuh, rz_denoise.cuh: by pointer only
+struct RzPathArgs; struct RzGuideArgs; struct RzMatteArgs; struct RzDenoiseArgs; struct RzBvhNode;   // rz_device.cuh, rz_denoise.cuh: by pointer only
 
 // ------------------------------------------------------------------------------ K0 (rz_ids.cu)
 struct RzRefNode { double low[3], high[3]; int32_t left, right, start, end; };   // BVH of hit.zig:101-108, children by index (RefBuilder)
@@ -92,6 +92,7 @@ extern "C" cudaError_t rz_bvh_warm(void);
 extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream);
 extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t stream);
+extern "C" cudaError_t rz_launch_mattes(const RzMatteArgs *g, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------ K4 (rz_bvh_build.cu)
 extern "C" size_t rz_lbvh_scratch_bytes(uint32_t n);

@@ -389,6 +389,17 @@ class Backend:
         abi.check(self.lib.rayz_cuda_render_guides(self._h, C.byref(cam), C.byref(p), albedo.ctypes.data, normal.ctypes.data))
         return albedo, normal
 
+    def mattes(self, cam: abi.RzCamera, p: abi.RzRenderParams, ranks: int = 6):
+        """rayz_cuda_render_mattes: the first-hit ids of the camera samples a render with these parameters traces, ranked per
+        pixel by count descending, then id ascending -> (ids [rows,w,ranks] int32: caller's sphere index, abi.MATTE_MISS for the
+        sky, abi.MATTE_EMPTY past the pixel's distinct ids; coverage [rows,w,ranks] f32: count / spp).  Leaves the accumulated
+        frame, the guides, stats and timing as they were."""
+        rows = self.shard_rows(p)
+        ids = np.empty((rows, p.width, max(int(ranks), 1)), dtype=np.int32)
+        cov = np.empty(ids.shape, dtype=np.float32)
+        abi.check(self.lib.rayz_cuda_render_mattes(self._h, C.byref(cam), C.byref(p), ranks, ids.ctypes.data, cov.ctypes.data))
+        return ids, cov
+
     def denoise(self, iterations: int = 5, sigma_luminance: float = 4.0, sigma_normal: float = 128.0, sigma_depth: float = 1.0):
         """rayz_cuda_denoise: the accumulated frame (needs moments=True) filtered by the edge-avoiding à-trous filter, steered by
         its noise estimate and the guides of the last guides() call of the same frame, camera and seed ->
@@ -474,6 +485,8 @@ class Tracer:
         self.albedo = None         # [h, w, 4] guide buffers of the last render_guides(): rgb albedo + coverage
         self.normal = None         # [h, w, 4] ... unit normal + hit distance
         self.denoised = None       # (linear [h, w, 4], rgb8 [h, w, 3]) of the last denoise()
+        self.matte_ids = None      # [h, w, ranks] ID mattes of the last render_mattes(): caller's sphere indices by rank
+        self.matte_coverage = None  # [h, w, ranks] ... the fraction of the pixel's samples each covers
         self._backend = None
         self._uploaded = None      # the pool arrays of the backend's last scene upload
 
@@ -534,6 +547,21 @@ class Tracer:
         self.albedo and self.normal.  The scene is uploaded only when the pool differs from the one this tracer last uploaded,
         so that the frame of a previous render() stays accumulated for denoise() (it used to be uploaded on every call, which
         ended that frame).  An upload made directly through self.backend is not seen: call render() after one."""
+        b = self._backend_with_scene()
+        self.albedo, self.normal = b.guides(self.camera.rz, self._first_hit_params())
+        return self.albedo, self.normal
+
+    def render_mattes(self, ranks: int = 6):
+        """ID mattes over the camera samples render() traces (samples_per_px, seed, at most 1024): per pixel, the caller's
+        indices of the spheres its samples hit first, ranked by coverage (rayz_cuda_render_mattes).  Returns (ids [h, w, ranks]
+        int32, coverage [h, w, ranks] f32), also kept as self.matte_ids and self.matte_coverage.  The scene is uploaded as
+        render_guides() uploads it: only when the pool changed."""
+        b = self._backend_with_scene()
+        self.matte_ids, self.matte_coverage = b.mattes(self.camera.rz, self._first_hit_params(), ranks)
+        return self.matte_ids, self.matte_coverage
+
+    def _backend_with_scene(self) -> Backend:
+        """The backend, with the pool uploaded unless it equals the one this tracer last uploaded."""
         b = self.backend
         arrays = self.pool.arrays()
         # the scene render() uploaded stays: uploading it again would end the accumulated frame that denoise() filters
@@ -542,10 +570,12 @@ class Tracer:
             self._uploaded = None
             b.upload_scene(arrays)
             self._uploaded = arrays
-        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
-                           **self._sampler())
-        self.albedo, self.normal = b.guides(self.camera.rz, p)
-        return self.albedo, self.normal
+        return b
+
+    def _first_hit_params(self) -> abi.RzRenderParams:
+        """The parameters of render()'s camera samples, for the first-hit calls (guides, mattes)."""
+        return Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
+                              **self._sampler())
 
     def denoise(self, iterations: int = 5, sigma_luminance: float = 4.0, sigma_normal: float = 128.0, sigma_depth: float = 1.0):
         """The frame of the last render() (with moments=True, or a noise target) denoised with the guides of render_guides(),

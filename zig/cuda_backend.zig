@@ -87,6 +87,11 @@ pub const RZ_PASS_GLOSSY_INDIRECT: u32 = 4;
 pub const RZ_PASS_TRANSMISSION_DIRECT: u32 = 5;
 pub const RZ_PASS_TRANSMISSION_INDIRECT: u32 = 6;
 pub const RZ_PASS_COUNT: u32 = 7;
+// ID mattes (rayz_cuda_render_mattes): ids of a sample that hit no sphere and of a rank past the pixel's distinct ids; limits
+pub const RZ_MATTE_MISS: i32 = -1;
+pub const RZ_MATTE_EMPTY: i32 = -2;
+pub const RZ_MATTE_MAX_RANKS: u32 = 16;
+pub const RZ_MATTE_MAX_SPP: u32 = 1024;
 
 pub const RzNoise = extern struct {
     samples: u64,
@@ -120,6 +125,8 @@ pub extern fn rayz_cuda_pixel_samples(ctx: *RzContext, out_spp: [*]u32) c_int;
 pub extern fn rayz_cuda_passes(ctx: *RzContext, out_passes: [*]f32) c_int; // RZ_PASS_COUNT planes of rows x width x 4
 // guide buffers for a denoiser: first-hit albedo + coverage, normal + hit distance (rows * width * 4 floats each)
 pub extern fn rayz_cuda_render_guides(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, out_albedo: ?[*]f32, out_normal: ?[*]f32) c_int;
+// first-hit ids of the same camera samples ranked per pixel by coverage: rows * width * ranks ids and coverages
+pub extern fn rayz_cuda_render_mattes(ctx: *RzContext, cam: *const RzCamera, params: *const RzRenderParams, ranks: u32, out_ids: ?[*]i32, out_coverage: ?[*]f32) c_int;
 // the accumulated frame (RZ_RENDER_MOMENTS) denoised with the guides of the last rayz_cuda_render_guides call (rows * width * 4 floats, * 3 bytes)
 pub extern fn rayz_cuda_denoise(ctx: *RzContext, dp: ?*const RzDenoiseParams, out_linear_rgba: ?[*]f32, out_rgb8: ?[*]u8) c_int;
 pub extern fn rayz_cuda_last_error() [*:0]const u8;
