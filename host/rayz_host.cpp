@@ -4,6 +4,7 @@
 //               [--variant auto|mega|wavefront|bvh] [--gpus N] [--grid G] [--scene bouncing|penultimate]
 //               [--dump-scene file] [--dump-linear file] [--ppm-bench] [--noise-target X [--max-spp N] [--adaptive]]
 //               [--guides PREFIX] [--denoise FILE] [--sobol] [--rqmc] [--pooled] [--passes PREFIX] [--mattes PREFIX]
+//               [--filter box|tent|gaussian|blackman-harris[:WIDTH]]
 //
 // Same argv contract (img_w required, optional output path, else stdout), same report line
 // ("Finished render (…s): … rps and … us per ray", rays = primary samples), same ASCII P3 output.
@@ -27,6 +28,9 @@
 // --mattes PREFIX also writes the ID mattes of the render's camera samples (rayz_cuda_render_mattes), six ranks, as 3-channel
 // PFM files PREFIX_rank<r>.pfm: the rank's sphere index as a float (-1 the sky, -2 no such rank), its coverage, 0.  Mattes
 // take at most 1024 samples per pixel.
+// --filter KIND[:WIDTH] draws each camera sample's offset from a reconstruction filter (RZ_RENDER_FILTER) in every one of these
+// runs, guides and mattes included: tent, gaussian or blackman-harris, WIDTH its full width in px (1 to 4, a multiple of
+// 1/16; default 2, 3 and 1.5).  The default, box, is the reference's uniform jitter.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -54,6 +58,7 @@ int main(int argc, char **argv) {
     const char *dump_scene = nullptr, *dump_linear = nullptr, *guides = nullptr, *denoise = nullptr, *passes = nullptr,
                *mattes = nullptr;
     bool ppm_bench = false, penultimate = false, adaptive = false, sobol = false, rqmc = false, pooled = false;
+    uint32_t pixel_filter = 0;
     float noise_target = 0;
     uint32_t max_spp = 4096;
     for (int i = 2; i < argc; i++) {
@@ -78,6 +83,19 @@ int main(int argc, char **argv) {
         else if (a == "--denoise") denoise = val();
         else if (a == "--passes") passes = val();
         else if (a == "--mattes") mattes = val();
+        else if (a == "--filter") {
+            const std::string v = val(), kind = v.substr(0, v.find(':'));
+            const uint32_t k = kind == "box" ? RZ_FILTER_BOX : kind == "tent" ? RZ_FILTER_TENT : kind == "gaussian" ? RZ_FILTER_GAUSSIAN
+                               : kind == "blackman-harris" ? RZ_FILTER_BLACKMAN_HARRIS : 99u;
+            double width = 0;
+            if (v.find(':') != std::string::npos) width = std::strtod(v.c_str() + v.find(':') + 1, nullptr);
+            const double w16 = width * 16.0;
+            if (k == 99u || !(w16 >= 0 && w16 <= 255 && w16 == std::floor(w16))) {
+                std::fprintf(stderr, "--filter: expected box, tent, gaussian or blackman-harris, optionally :WIDTH in px (a multiple of 1/16), got %s\n", v.c_str());
+                return 2;
+            }
+            pixel_filter = RZ_RENDER_FILTER(k, (uint32_t)w16);   // the library refuses widths outside 1..4 px, and a width with the box
+        }
         else if (a == "--scene") penultimate = std::string(val()) == "penultimate";
         else if (a == "--variant") {
             const std::string v = val();
@@ -103,6 +121,7 @@ int main(int argc, char **argv) {
         tracer.rqmc = rqmc;
         tracer.pooled = pooled;
         tracer.passes = passes != nullptr;
+        tracer.pixel_filter = pixel_filter;
         tracer.devices.clear();
         for (int g = 0; g < gpus; g++) tracer.devices.push_back(g);
         if (pen) penultimateScene(tracer); else randomBouncing(tracer, -grid, grid);

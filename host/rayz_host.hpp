@@ -267,6 +267,7 @@ struct Tracer {
     bool rqmc = false;            // RZ_RENDER_RQMC (with SOBOL and MOMENTS): two Sobol replicates per pixel, a noise estimate that sees them
     bool pooled = false;          // RZ_RENDER_ADAPTIVE_POOLED, passed through: with adaptive, each pixel stops on an error pooled over its row segment
     bool passes = false;          // RZ_RENDER_PASSES (no pixel changes), so that readPasses() can follow
+    uint32_t pixel_filter = 0;    // the RZ_RENDER_FILTER field (kind and width) of render(), renderGuides() and renderMattes()
     std::vector<float> pass_planes;   // light-path passes of the last readPasses(): RZ_PASS_COUNT planes of h x w x 4 floats
     Image denoised;               // rgb8 of the last denoise()
     std::vector<int32_t> matte_ids;      // ID mattes of the last renderMattes(): h x w x ranks caller's sphere indices
@@ -309,6 +310,7 @@ struct Tracer {
         if (rqmc) p.flags |= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;
         if (pooled) p.flags |= RZ_RENDER_ADAPTIVE_POOLED;   // the library refuses it without RZ_RENDER_ADAPTIVE
         if (passes) p.flags |= RZ_RENDER_PASSES;
+        p.flags |= pixel_filter;
         return p;
     }
 
@@ -367,7 +369,7 @@ struct Tracer {
     // Guide buffers for a denoiser over the camera samples render() traces (rayz_cuda_render_guides), after render().
     void renderGuides() {
         RzRenderParams p = renderParams();
-        p.flags &= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;   // the render's own camera rays (RQMC needs MOMENTS beside it)
+        p.flags &= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS | RZ_RENDER_FILTER_MASK | RZ_RENDER_FILTER_WIDTH_MASK;   // the render's own camera rays (RQMC needs MOMENTS beside it)
         const RzCamera cam = camera.flat();
         albedo.assign(img.w * img.h * 4, 0.f);
         normal.assign(img.w * img.h * 4, 0.f);
@@ -377,7 +379,7 @@ struct Tracer {
     // ID mattes of the camera samples render() traces, ranked per pixel by coverage (rayz_cuda_render_mattes), after render().
     void renderMattes(uint32_t ranks) {
         RzRenderParams p = renderParams();
-        p.flags &= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS;   // the render's own camera rays, as renderGuides()
+        p.flags &= RZ_RENDER_SOBOL | RZ_RENDER_RQMC | RZ_RENDER_MOMENTS | RZ_RENDER_FILTER_MASK | RZ_RENDER_FILTER_WIDTH_MASK;   // the render's own camera rays, as renderGuides()
         const RzCamera cam = camera.flat();
         matte_ids.assign(img.w * img.h * ranks, 0);
         matte_coverage.assign(img.w * img.h * ranks, 0.f);

@@ -254,6 +254,41 @@ typedef struct RzRenderParams {
                                     * PASSES bit differs from the accumulated render's is refused, the sums untouched;
                                     * rayz_cuda_render_guides refuses the flag; max_depth > 2^29 - 1 is refused with
                                     * RZ_ERR_INVALID_ARG (the first hit's kind rides in the top bits of a path's hit count). */
+/* Pixel reconstruction filter (DESIGN.md "Pixel filters"), a field of flags: the kind in bits 8-9, the width in bits 16-23.
+ * Filter importance sampling: each camera sample's offset from the pixel centre is drawn from the filter, and the sample keeps
+ * weight 1.  Sample (px, py) with jitter uniforms (ux, uy) (Philox, or Sobol's camera-jitter pair) starts at
+ * (px + w(ux), py + w(uy)), w the inverse CDF of the filter's normalised marginal g; lens, time and scatter uniforms are
+ * unchanged.  The filters are separable, f(x, y) = g(x) g(y), with support |x| <= R = W / 2 for the full width W:
+ *   RZ_FILTER_BOX              w(u) = u - 0.5 (the reference's getRay jitter, bit for bit the code path without the field)
+ *   RZ_FILTER_TENT             g(x) = 1 - |x| / R                                                       default W = 2 px
+ *   RZ_FILTER_GAUSSIAN         g(x) = exp(-x^2 / 2 s^2) - exp(-R^2 / 2 s^2), s = W / 6 (pbrt-v4's form)  default W = 3 px
+ *   RZ_FILTER_BLACKMAN_HARRIS  g(x) = 0.35875 + 0.48829 cos(2 pi x / W) + 0.14128 cos(4 pi x / W)
+ *                                     + 0.01168 cos(6 pi x / W) (Cycles' form)                          default W = 1.5 px
+ * The width field is W in 1/16 px: 0 is the kind's default, otherwise 16..64 (1 to 4 px).  w is monotone in u, inside [-R, R]
+ * and odd about u = 1/2, and within 1e-5 px of the exact inverse CDF at every 24-bit u (interpolated in f64 from exact tables
+ * of the unit-width filter, rounded to f32 once).
+ * Every sample keeps weight 1 and a pixel stays the mean of its own samples: batches, shards, devices, adaptive counts, passes
+ * and the noise estimate keep every guarantee they have with the box.  Under RZ_RENDER_SOBOL the warp is monotone per axis, so
+ * each stratum of the jitter pair maps to a box of equal filter mass.  Honoured by rayz_cuda_render, rayz_cuda_render_device,
+ * rayz_cuda_render_to_noise (plain, adaptive and pooled), rayz_cuda_render_guides and rayz_cuda_render_mattes, with every
+ * variant and sampler; rayz_cuda_primary_ids (pixel centres) ignores it.  Refused with RZ_ERR_INVALID_ARG, the message naming
+ * the rule and nothing touched: a width of 1..15 or above 64, a nonzero width with RZ_FILTER_BOX, and an RZ_RENDER_ACCUMULATE
+ * batch whose field (kind or width) differs from the accumulated render's.  rayz_cuda_denoise refuses guide buffers rendered
+ * with another field than the accumulated frame. */
+#define RZ_RENDER_FILTER_SHIFT 8
+#define RZ_RENDER_FILTER_MASK 0x300u
+#define RZ_RENDER_FILTER_WIDTH_SHIFT 16
+#define RZ_RENDER_FILTER_WIDTH_MASK 0xff0000u
+#define RZ_FILTER_BOX 0u
+#define RZ_FILTER_TENT 1u
+#define RZ_FILTER_GAUSSIAN 2u
+#define RZ_FILTER_BLACKMAN_HARRIS 3u
+#define RZ_FILTER_WIDTH_MIN 16u   /* 1 px, in 1/16 px */
+#define RZ_FILTER_WIDTH_MAX 64u   /* 4 px */
+/* the flags of a filter: kind RZ_FILTER_*, width16 the full width in 1/16 px (0: the kind's default) */
+#define RZ_RENDER_FILTER(kind, width16) \
+    ((((uint32_t)(kind) << RZ_RENDER_FILTER_SHIFT) & RZ_RENDER_FILTER_MASK) | \
+     (((uint32_t)(width16) << RZ_RENDER_FILTER_WIDTH_SHIFT) & RZ_RENDER_FILTER_WIDTH_MASK))
 
 /*
  * Light-path passes (RZ_RENDER_PASSES).  A path that ends in the sky with h scattering hits before it adds its clamped

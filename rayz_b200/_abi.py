@@ -22,6 +22,19 @@ VARIANTS = {"auto": 0, "mega": 1, "wavefront": 2, "bvh": 3, "mega_single": 4}
 RENDER_SERIAL_PASSES, RENDER_MOMENTS, RENDER_ACCUMULATE, RENDER_ADAPTIVE, RENDER_SOBOL, RENDER_RQMC = 1, 2, 4, 8, 0x10, 0x20   # RzRenderParams.flags (RZ_RENDER_*)
 RENDER_ADAPTIVE_POOLED = 0x40   # with RENDER_ADAPTIVE in render_to_noise: stop each pixel on an error pooled over its row segment
 RENDER_PASSES = 0x80            # also sum each sky path's radiance into its light-path pass (rayz_cuda_passes)
+# pixel reconstruction filter, a field of RzRenderParams.flags (RZ_RENDER_FILTER): kind in bits 8-9, full width in 1/16 px in
+# bits 16-23 (0: the kind's default; else 16..64)
+RENDER_FILTER_SHIFT, RENDER_FILTER_MASK, RENDER_FILTER_WIDTH_SHIFT, RENDER_FILTER_WIDTH_MASK = 8, 0x300, 16, 0xFF0000
+FILTER_BOX, FILTER_TENT, FILTER_GAUSSIAN, FILTER_BLACKMAN_HARRIS = 0, 1, 2, 3
+FILTER_WIDTH_MIN, FILTER_WIDTH_MAX = 16, 64
+FILTERS = {"box": FILTER_BOX, "tent": FILTER_TENT, "gaussian": FILTER_GAUSSIAN, "blackman-harris": FILTER_BLACKMAN_HARRIS}
+
+
+def render_filter(kind: int, width16: int = 0) -> int:
+    """RZ_RENDER_FILTER(kind, width16): the flags of a filter."""
+    return ((kind << RENDER_FILTER_SHIFT) & RENDER_FILTER_MASK) | ((width16 << RENDER_FILTER_WIDTH_SHIFT) & RENDER_FILTER_WIDTH_MASK)
+
+
 # RZ_PASS_*: index -> name of the light-path passes rayz_cuda_passes returns, in plane order
 PASS_NAMES = ("environment", "diffuse_direct", "diffuse_indirect", "glossy_direct", "glossy_indirect", "transmission_direct",
               "transmission_indirect")

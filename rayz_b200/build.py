@@ -33,7 +33,7 @@ UNITS = {
     "rz_bvh_trace.cu": ["--use_fast_math"],
     "rz_context.cu": [],
 }
-HEADERS = ["rz_device.cuh", "rz_sampler.cuh", "rz_search.cuh", "rz_denoise.cuh", "rz_launch.h", os.path.join("..", "..", "include", "rayz_cuda.h")]
+HEADERS = ["rz_device.cuh", "rz_filter_table.h", "rz_sampler.cuh", "rz_search.cuh", "rz_denoise.cuh", "rz_launch.h", os.path.join("..", "..", "include", "rayz_cuda.h")]
 
 
 def _nvcc() -> str:

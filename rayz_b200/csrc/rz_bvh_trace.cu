@@ -132,7 +132,7 @@ __device__ __forceinline__ void rz_bvh_round(const RzPathArgs &a, const float4 *
 }
 
 // LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list).
-template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false, int SOBOL = 0, bool PASSES = false>
+template <bool STATS, bool QUEUE, int UNIT = 512, bool LIST = false, int SOBOL = 0, bool PASSES = false, bool FILTER = false>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -231,7 +231,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
                             lp = nlp;
                             gpix = pj * a.width + pi;
                             sample = a.sample_offset + unit_s0 + (k >> 5);
-                            ray = rz_camera_ray(a.cam, pi, pj, gpix, sample, a.seed_lo, a.seed_hi, SOBOL);
+                            ray = rz_camera_ray(a.cam, pi, pj, gpix, sample, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
                             thr = f3(1.f, 1.f, 1.f);
                             seg = 0;
                             alive = a.max_depth > 0u;
@@ -271,7 +271,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_bvh_kernel(const RzPathAr
 // in L1; survivors go to the next queue, and the tail of the paths to the persistent kernel above (QUEUE).
 // CAMERA: the camera rays of a work unit — an 8 x 4-pixel block x `chunk` samples — do not walk the tree one by one; the warp
 // culls the tree once against the block's cone and the rays search the surviving spheres as a list (below).  The sorted stages (CAMERA = false) are off by default (RzTuning::bvh_stages = 0: measured as a loss).
-template <bool STATS, bool CAMERA, int SOBOL = 0, bool PASSES = false>
+template <bool STATS, bool CAMERA, int SOBOL = 0, bool PASSES = false, bool FILTER = false>
 __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB) rz_bvh_stage_kernel(const RzPathArgs a) {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -339,7 +339,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                     ax.x += __shfl_xor_sync(0xffffffffu, ax.x, o); ax.y += __shfl_xor_sync(0xffffffffu, ax.y, o); ax.z += __shfl_xor_sync(0xffffffffu, ax.z, o);
                 }
                 const bool has_axis = rz_tile_axis(ax);
-                float cmin = valid ? rz_tile_corner_cos(a.cam, pc, ax) : 1.0f;
+                float cmin = valid ? rz_tile_corner_cos(a.cam, pc, ax, FILTER ? rz_filter_reach(a.sobol) : 0.5f) : 1.0f;   // a filter's support
                 for (int o = 16; o > 0; o >>= 1) cmin = fminf(cmin, __shfl_xor_sync(0xffffffffu, cmin, o));
                 const RzTileCone cone = rz_tile_cone(a.cam, ax, has_axis, cmin, a.focus_dist, a.lens_radius);
                 unsigned head = 0u, tail = 1u;
@@ -408,7 +408,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                         const bool have = valid && (b + (uint32_t)r < n_batches);
                         live[r] = have && a.max_depth > 0u;
                         if (STATS && have) { c_paths++; if (!live[r]) c_depth++; }
-                        if (live[r]) rays[r] = rz_camera_ray(a.cam, pi, pj, gpix0, smp[r], a.seed_lo, a.seed_hi, SOBOL);
+                        if (live[r]) rays[r] = rz_camera_ray(a.cam, pi, pj, gpix0, smp[r], a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
                         else { rays[r].o = f3(0.f, 0.f, 0.f); rays[r].d = f3(0.f, 1.f, 0.f); rays[r].time = 0.f; rays[r].self_k = -1; }
                     }
                     float bt[2] = {3.0e38f, 3.0e38f};
@@ -457,7 +457,7 @@ __global__ void __launch_bounds__(128, CAMERA ? RZ_BVH_CAMERA_MINB : RZ_BVH_MINB
                 smp = a.sample_offset + s0 + b;
                 live = valid && a.max_depth > 0u;
                 if (STATS && valid) { c_paths++; if (!live) c_depth++; }
-                if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, smp, a.seed_lo, a.seed_hi, SOBOL);
+                if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, smp, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
             } else {
                 const uint32_t i = b * 32u + lane;
                 live = i < ne;
@@ -526,7 +526,7 @@ __device__ __forceinline__ float3 rz_guide_albedo(const RzPathArgs &a, int k, co
 // samples in lockstep: a block's rays fan out over a third of the angle of 32 pixels of a row (the camera stage's reason for
 // the same blocks), so the lanes visit more of the same nodes.  Each lane sums its pixel's samples in f64, in sample order, and
 // divides once: the result depends on (scene, camera, seed, pixel, sample range) only.
-template <int SOBOL>
+template <int SOBOL, bool FILTER = false>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGuideArgs g) {
     const RzPathArgs &a = g.a;
     const unsigned lane = threadIdx.x & 31u;
@@ -546,7 +546,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGui
     uint32_t hits = 0;
     for (uint32_t s = 0; s < a.spp; s++) {
         RzRay ray;
-        if (valid) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL);
+        if (valid) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
         else { ray.o = f3(0.f, 0.f, 0.f); ray.d = f3(0.f, 1.f, 0.f); ray.time = 0.f; ray.self_k = -1; }
         const float ix = 1.0f / ray.d.x, iy = 1.0f / ray.d.y, iz = 1.0f / ray.d.z;
         float bt = 3.0e38f;
@@ -585,7 +585,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_guides_kernel(const RzGui
 // warp sorts them (bitonic, n_pad a power of two, padded with INT32_MAX), so every id is one run; lane l owns the run ENDS in
 // positions [l c, l c + c), c = n_pad / 32, and the start of the run it enters from the lane before (a max-scan).  Rank r is the
 // warp's least run key above rank r - 1's.  Exact for any scene: a pixel can see spp distinct ids and every one is a run.
-template <int SOBOL>
+template <int SOBOL, bool FILTER = false>
 __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_mattes_kernel(const RzMatteArgs g) {
     extern __shared__ int32_t rz_matte_ids[];
     const RzPathArgs &a = g.a;
@@ -605,7 +605,7 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_mattes_kernel(const RzMat
         const uint32_t s = s0 + lane;
         const bool live = s < spp;
         RzRay ray;
-        if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL);
+        if (live) ray = rz_camera_ray(a.cam, pi, pj, gpix, a.sample_offset + s, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
         else { ray.o = f3(0.f, 0.f, 0.f); ray.d = f3(0.f, 1.f, 0.f); ray.time = 0.f; ray.self_k = -1; }
         const float ix = 1.0f / ray.d.x, iy = 1.0f / ray.d.y, iz = 1.0f / ray.d.z;
         float bt = 3.0e38f;
@@ -670,14 +670,22 @@ __global__ void __launch_bounds__(128, RZ_BVH_MINB) rz_mattes_kernel(const RzMat
 }
 
 // inst: the kernel's instances (rz_pick_instance), launched on the persistent grid
-template <class F>
-cudaError_t launch_kernel(F inst, const RzPathArgs &a, int collect_stats, int sm_count, cudaStream_t stream) {
-    const auto kern = rz_pick_instance(a, collect_stats, inst);
+template <class K>
+cudaError_t launch_grid(K kern, const RzPathArgs &a, int sm_count, cudaStream_t stream) {
     int grid = 0;
     const cudaError_t e = rz_persistent_grid(kern, 0, sm_count, &grid);
     if (e != cudaSuccess) return e;
     kern<<<grid, 128, 0, stream>>>(a);
     return cudaGetLastError();
+}
+template <class F>
+cudaError_t launch_kernel(F inst, const RzPathArgs &a, int collect_stats, int sm_count, cudaStream_t stream) {
+    return launch_grid(rz_pick_instance(a, collect_stats, inst), a, sm_count, stream);
+}
+// the same for a kernel that generates camera rays: `inst` also takes FILTER (rz_pick_camera_instance)
+template <class F>
+cudaError_t launch_camera_kernel(F inst, const RzPathArgs &a, int collect_stats, int sm_count, cudaStream_t stream) {
+    return launch_grid(rz_pick_camera_instance(a, collect_stats, inst), a, sm_count, stream);
 }
 
 }  // namespace
@@ -706,8 +714,8 @@ extern "C" cudaError_t rz_launch_bvh(const RzPathArgs *a, int collect_stats, int
     if (b.q_in)
         return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, true, 512, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
     if (b.px_list)
-        return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, false, 512, true, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
-    return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_kernel<decltype(S)::value, false, 512, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
+        return launch_camera_kernel([](auto S, auto M, auto P, auto F) { return rz_bvh_kernel<decltype(S)::value, false, 512, true, decltype(M)::value, decltype(P)::value, decltype(F)::value>; }, b, collect_stats, sm_count, stream);
+    return launch_camera_kernel([](auto S, auto M, auto P, auto F) { return rz_bvh_kernel<decltype(S)::value, false, 512, false, decltype(M)::value, decltype(P)::value, decltype(F)::value>; }, b, collect_stats, sm_count, stream);
 }
 
 // Guide buffers of the device's local pixels: one warp per 8 x 4 block, four per CTA.
@@ -717,7 +725,7 @@ extern "C" cudaError_t rz_launch_guides(const RzGuideArgs *g, cudaStream_t strea
     const uint32_t rows = b.a.width ? b.a.n_local_px / b.a.width : 0u;
     const uint32_t blocks = ((b.a.width + 7u) / 8u) * ((rows + 3u) / 4u);
     if (blocks == 0u) return cudaSuccess;
-    rz_pick_instance(b.a, 0, [](auto, auto M, auto) { return rz_guides_kernel<decltype(M)::value>; })<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
+    rz_pick_camera_instance(b.a, 0, [](auto, auto M, auto, auto F) { return rz_guides_kernel<decltype(M)::value, decltype(F)::value>; })<<<(blocks + 3u) / 4u, 128, 0, stream>>>(b);
     return cudaGetLastError();
 }
 
@@ -728,7 +736,7 @@ extern "C" cudaError_t rz_launch_mattes(const RzMatteArgs *g, cudaStream_t strea
     if (b.a.n_local_px == 0u) return cudaSuccess;
     b.n_pad = 32u;
     while (b.n_pad < b.a.spp) b.n_pad <<= 1;
-    rz_pick_instance(b.a, 0, [](auto, auto M, auto) { return rz_mattes_kernel<decltype(M)::value>; })
+    rz_pick_camera_instance(b.a, 0, [](auto, auto M, auto, auto F) { return rz_mattes_kernel<decltype(M)::value, decltype(F)::value>; })
         <<<(b.a.n_local_px + 3u) / 4u, 128, 4u * b.n_pad * sizeof(int32_t), stream>>>(b);
     return cudaGetLastError();
 }
@@ -738,6 +746,6 @@ extern "C" cudaError_t rz_launch_bvh_stage(const RzPathArgs *a, int collect_stat
     RzPathArgs b = *a;
     rz_bvh_tuning(b);
     if (!b.q_in)
-        return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_stage_kernel<decltype(S)::value, true, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
+        return launch_camera_kernel([](auto S, auto M, auto P, auto F) { return rz_bvh_stage_kernel<decltype(S)::value, true, decltype(M)::value, decltype(P)::value, decltype(F)::value>; }, b, collect_stats, sm_count, stream);
     return launch_kernel([](auto S, auto M, auto P) { return rz_bvh_stage_kernel<decltype(S)::value, false, decltype(M)::value, decltype(P)::value>; }, b, collect_stats, sm_count, stream);
 }

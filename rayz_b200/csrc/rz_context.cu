@@ -190,6 +190,7 @@ struct AccumRecord {
     uint32_t max_depth = 0, moments = 0, sobol = 0, rqmc = 0;
     uint32_t pooled = 0;       // RZ_RENDER_ADAPTIVE_POOLED: every consumer of the error reads the pooled e* (Dev::px_pool)
     uint32_t passes = 0;       // RZ_RENDER_PASSES: the pass sums behind the accumulators hold the frame's light-path passes
+    uint32_t filter = 0;       // the flags' pixel-filter field (RZ_RENDER_FILTER), as given
     uint64_t seed = 0;
     float t_min = 0;
     RzCamera cam{};
@@ -206,6 +207,7 @@ struct GuideRecord {
     Frame frame;
     RzCamera cam{};
     uint64_t seed = 0;
+    uint32_t filter = 0;   // the pixel-filter field the guides were traced with (RZ_RENDER_FILTER)
     uint32_t first_offset = 0, samples = 0;
 };
 
@@ -918,6 +920,18 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         P.refused = true;
         return rz_fail(RZ_ERR_INVALID_ARG, "%s: RZ_RENDER_ADAPTIVE_POOLED requires RZ_RENDER_ADAPTIVE (rayz_cuda_render_to_noise only)", who);
     }
+    {   // the pixel filter's field (RZ_RENDER_FILTER): refused before anything is touched
+        const uint32_t kind = rz_filter_kind(p->flags), w16 = (p->flags & RZ_RENDER_FILTER_WIDTH_MASK) >> RZ_RENDER_FILTER_WIDTH_SHIFT;
+        if (kind == RZ_FILTER_BOX && w16 != 0u) {
+            P.refused = true;
+            return rz_fail(RZ_ERR_INVALID_ARG, "%s: RZ_FILTER_BOX takes no width (the width field must be 0; got %u/16 px)", who, w16);
+        }
+        if (w16 != 0u && (w16 < RZ_FILTER_WIDTH_MIN || w16 > RZ_FILTER_WIDTH_MAX)) {
+            P.refused = true;
+            return rz_fail(RZ_ERR_INVALID_ARG, "%s: a pixel filter's width must be 0 (the kind's default) or 16..64 sixteenths of a pixel (1 to 4 px; got %u)",
+                           who, w16);
+        }
+    }
     if ((p->flags & RZ_RENDER_PASSES) && p->max_depth > RZ_PASS_MAX_DEPTH) {   // the count must stay out of the kind bits (rz_seg_after_hit)
         P.refused = true;
         return rz_fail(RZ_ERR_INVALID_ARG, "%s: RZ_RENDER_PASSES requires max_depth <= 2^29 - 1 (the first hit's kind rides in the top bits of a path's hit count; got %u)",
@@ -932,6 +946,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
         next.rqmc = (p->flags & RZ_RENDER_RQMC) ? 1u : 0u;
         next.pooled = (p->flags & RZ_RENDER_ADAPTIVE_POOLED) ? 1u : 0u;
         next.passes = (p->flags & RZ_RENDER_PASSES) ? 1u : 0u;
+        next.filter = p->flags & RZ_PATH_FILTER_BITS;
         next.t_min = p->t_min > 0 ? p->t_min : 1e-4f; next.cam = *cam;
         next.first_offset = p->sample_offset; next.samples = p->spp;
         next.adaptive = (p->flags & RZ_RENDER_ADAPTIVE) != 0;
@@ -948,6 +963,7 @@ static int plan_render(const RzContext *ctx, const RzCamera *cam, const RzRender
             if (prev.sobol != next.sobol) return refuse("the RZ_RENDER_SOBOL bit differs from the accumulated render");
             if (prev.rqmc != next.rqmc) return refuse("the RZ_RENDER_RQMC bit differs from the accumulated render");
             if (prev.passes != next.passes) return refuse("the RZ_RENDER_PASSES bit differs from the accumulated render");
+            if (prev.filter != next.filter) return refuse("the pixel filter (RZ_RENDER_FILTER kind or width) differs from the accumulated render");
             if ((uint64_t)p->sample_offset != (uint64_t)prev.first_offset + prev.samples)
                 return refuse("sample_offset must continue where the accumulated samples end (previous sample_offset + spp)");
             if (prev.samples + p->spp > 0xFFFFFFFFull) return refuse("the cumulative sample count would pass 2^32 - 1");
@@ -1151,7 +1167,7 @@ static RzPathArgs path_args(const RzContext *ctx, const RenderPlan &P, uint32_t 
     a.shard_index = P.frame.s * ND + d; a.shard_count = P.frame.S * ND; a.band_rows = P.frame.band;
     a.seed_lo = (uint32_t)p->seed; a.seed_hi = (uint32_t)(p->seed >> 32);
     a.sobol = ((p->flags & RZ_RENDER_SOBOL) ? RZ_SAMPLER_SOBOL : 0u) | ((p->flags & RZ_RENDER_RQMC) ? RZ_SAMPLER_RQMC : 0u) |
-              ((p->flags & RZ_RENDER_PASSES) ? RZ_PATH_PASSES : 0u);
+              ((p->flags & RZ_RENDER_PASSES) ? RZ_PATH_PASSES : 0u) | (p->flags & RZ_PATH_FILTER_BITS);
     a.t_min = P.next.t_min;   // plan_render applied the default
     a.err = D.errword.p;
     a.unit_entries = ctx->tun.unit_entries;
@@ -1544,7 +1560,7 @@ extern "C" int rayz_cuda_render_guides(RzContext *ctx, const RzCamera *cam, cons
     if (out_normal) RZ_CUDA(cudaMemcpyAsync(out_normal, D0.out_guides.p + npx, npx * sizeof(float4), cudaMemcpyDeviceToHost, D0.stream));
     RZ_CUDA(cudaStreamSynchronize(D0.stream));
     GuideRecord &G = ctx->guides;
-    G.frame = P.frame; G.cam = *cam; G.seed = p->seed; G.first_offset = p->sample_offset; G.samples = p->spp;
+    G.frame = P.frame; G.cam = *cam; G.seed = p->seed; G.filter = p->flags & RZ_PATH_FILTER_BITS; G.first_offset = p->sample_offset; G.samples = p->spp;
     G.valid = true;
     return RZ_OK;
 }
@@ -1628,6 +1644,8 @@ extern "C" int rayz_cuda_denoise(RzContext *ctx, const RzDenoiseParams *dp, floa
         return rz_fail(RZ_ERR_INVALID_ARG, "denoise: no guide buffers (none, the last rayz_cuda_render_guides failed, or a scene upload or reserve came in between)");
     if (G.frame != A->frame || memcmp(&G.cam, &A->cam, sizeof(RzCamera)) != 0 || G.seed != A->seed)
         return rz_fail(RZ_ERR_INVALID_ARG, "denoise: the guide buffers' frame, camera or seed differ from the accumulated frame's");
+    if (G.filter != A->filter)
+        return rz_fail(RZ_ERR_INVALID_ARG, "denoise: the guide buffers' pixel filter (RZ_RENDER_FILTER kind or width) differs from the accumulated frame's");
     const uint32_t ND = (uint32_t)ctx->devs.size();
     Dev &D0 = ctx->devs[0];
     const FrameSplit sp(ctx, A->frame);

@@ -17,6 +17,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#include <string.h>
 
 #include <algorithm>
 #include <vector>
@@ -197,7 +198,10 @@ RZ_HD uint32_t rz_pass_of(uint32_t hits, uint32_t first_kind) {
 // mapping of rz_sobol_pair, and a sky path also adds its clamped luminance to its replicate's sum (rz_rep_offset).
 // RZ_PATH_PASSES (RZ_RENDER_PASSES) rides there too, for the same reason: a new field would move the parameters that follow
 // RzPathArgs in the wavefront's and the guides' kernels.  The launchers run the PASSES instances for it (rz_pick_instance).
+// The pixel filter's field (RZ_RENDER_FILTER) rides there at the flags' own bits, RZ_PATH_FILTER_BITS; a kind other than the
+// box runs the FILTER instances of the kernels that generate camera rays (rz_pick_camera_instance).
 enum { RZ_SAMPLER_SOBOL = 1u, RZ_SAMPLER_RQMC = 2u, RZ_PATH_PASSES = 4u };
+#define RZ_PATH_FILTER_BITS (RZ_RENDER_FILTER_MASK | RZ_RENDER_FILTER_WIDTH_MASK)
 // RZ_RENDER_RQMC's replicate sums share the accumulators' allocation: [n_pad][4] accumulators, then [n_pad][2] replicate sums
 // (2^-32 fixed point, slot lp * 2 + (sample & 1)), n_pad = n_local_px rounded up to whole warps.  This is the offset, in words,
 // of the replicate sums.
@@ -509,12 +513,76 @@ RZ_HD void rz_consider(int k, float nb, float nd, int self_k, float t_min, float
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Pixel filters (RZ_RENDER_FILTER, include/rayz_cuda.h; DESIGN.md "Pixel filters").  The kernels' FILTER instances read the
+// flags' filter field from RzPathArgs::sobol, where it sits at the same bits (RZ_PATH_FILTER_BITS).
+// ---------------------------------------------------------------------------------------------
+RZ_HD uint32_t rz_filter_kind(uint32_t bits) { return (bits & RZ_RENDER_FILTER_MASK) >> RZ_RENDER_FILTER_SHIFT; }
+// the full width in 1/16 px, the kind's default for a width field of 0 (box: 16, the pixel)
+RZ_HD uint32_t rz_filter_width16(uint32_t bits) {
+    const uint32_t w = (bits & RZ_RENDER_FILTER_WIDTH_MASK) >> RZ_RENDER_FILTER_WIDTH_SHIFT, k = rz_filter_kind(bits);
+    return w ? w : k == RZ_FILTER_TENT ? 32u : k == RZ_FILTER_GAUSSIAN ? 48u : k == RZ_FILTER_BLACKMAN_HARRIS ? 24u : 16u;
+}
+// Half-width in px of the offsets a pixel's camera samples reach: max(0.5, R).  What the camera-stage cones widen to.
+RZ_HD float rz_filter_reach(uint32_t bits) { return fmaxf(0.5f, (float)rz_filter_width16(bits) * 0.03125f); }
+
+// The warp's tables (scripts/gen_filter_table.py): per kind of unit width, at the nodes of a grid over the mass v from the left
+// edge with RZ_FILTER_CELLS cells per binade of v, the node's distance d from that edge and the slope dd/dv, both exact to f64.
+#include "rz_filter_table.h"
+static __device__ const double rz_filter_table_dev[3][RZ_FILTER_NODES][2] = RZ_FILTER_TABLE_INIT;
+static const double rz_filter_table_host[3][RZ_FILTER_NODES][2] = RZ_FILTER_TABLE_INIT;
+
+// The warp w(u): a sample's offset in px from the pixel centre along one axis, for a jitter uniform u in [0, 1).  The inverse
+// CDF of the filter's normalised marginal: monotone non-decreasing, inside [-R, R] and odd about 1/2 (w(1 - u) = -w(u) exactly:
+// it is evaluated for v = min(u, 1 - u), the mass from the nearer edge, and mirrored), so the tails, where the density goes to
+// 0 and an f32 CDF would move x by a lot, are never a difference of near-equal numbers.  Box: u - 0.5 in f32, rz_lens_ray's
+// jitter.  The other kinds: cubic Hermite interpolation of the table of the unit filter in the cell of v (a cell spans 1/32 of
+// its v, where the warp is a smooth power law of v: the interpolation is exact to ~1e-9 of d), in f64, scaled by the width and
+// rounded to f32 once.  No transcendental function and no iteration: the f64 Newton solve this replaced cost more than the
+// camera segment itself on the B200 (DESIGN.md "Pixel filters").
+RZ_HD float rz_filter_warp(uint32_t kind, uint32_t width16, float u) {
+    if (kind == RZ_FILTER_BOX) return u - 0.5f;
+    const bool upper = u >= 0.5f;
+    const float v = upper ? 1.0f - u : u;   // exact (Sterbenz)
+#ifdef __CUDA_ARCH__
+    const uint32_t b = __float_as_uint(v);
+    const double (*T)[2] = rz_filter_table_dev[kind - 1u];
+#else
+    uint32_t b;
+    memcpy(&b, &v, sizeof b);
+    const double (*T)[2] = rz_filter_table_host[kind - 1u];
+#endif
+    const int e = (int)(b >> 23) - 127;     // v in [2^e, 2^(e + 1))
+    double d;
+    if (e < -24) {                          // below the samplers' smallest nonzero uniform: linear to d(0) = 0
+        d = T[0][0] * ((double)v * 16777216.0);
+    } else {
+        const uint32_t n = (uint32_t)(e + 24) * (uint32_t)RZ_FILTER_CELLS + ((b >> 18) & 31u);
+        const double t = (double)(b & 0x3ffffu) * (1.0 / 262144.0);   // position in the cell, exact
+        const double h = ldexp(1.0, e - 5);                             // the cell's width in v
+        const double t2 = t * t, t3 = t2 * t;
+        d = (2.0 * t3 - 3.0 * t2 + 1.0) * T[n][0] + (t3 - 2.0 * t2 + t) * h * T[n][1] + (3.0 * t2 - 2.0 * t3) * T[n + 1u][0] +
+            (t3 - t2) * h * T[n + 1u][1];
+    }
+    const double x = (double)width16 * 0.0625 * (0.5 - d);
+    return (float)(upper ? x : -x);
+}
+
 // Camera.getRay with rng (camera.zig:59-77) from its five uniforms: jittered pixel position, thin-lens origin on the defocus
 // disk, time in [0,1).  Disk sample is polar instead of rejection (same distribution, and area-preserving: strata of (ur, ua)
-// stay strata of the disk).
-RZ_HD RzRay rz_lens_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, float ux, float uy, float ut, float ur, float ua) {
-    const float x = (float)px + (ux - 0.5f);
-    const float y = (float)py + (uy - 0.5f);
+// stay strata of the disk).  filter != 0 (the FILTER instances pass RzPathArgs::sobol; only when its filter field is not the
+// box): the jitter goes through rz_filter_warp.
+RZ_HD RzRay rz_lens_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, float ux, float uy, float ut, float ur, float ua,
+                        uint32_t filter = 0u) {
+    float x, y;
+    if (filter) {
+        const uint32_t kind = rz_filter_kind(filter), w16 = rz_filter_width16(filter);
+        x = (float)px + rz_filter_warp(kind, w16, ux);
+        y = (float)py + rz_filter_warp(kind, w16, uy);
+    } else {
+        x = (float)px + (ux - 0.5f);
+        y = (float)py + (uy - 0.5f);
+    }
     RzRay ray;
     ray.o = cam.look_from;
     if (cam.defocus) {
@@ -533,19 +601,20 @@ RZ_HD RzRay rz_lens_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, float ux,
 // One Philox block gives the five uniforms: 4 x 24 high bits + 3 x 8 low bits.  With `sobol` != 0 (RZ_RENDER_SOBOL; the kernels
 // pass their SOBOL template argument) three Sobol pairs give them instead (rz_sampler.cuh): jitter, lens (radius, angle) and the
 // shutter time (first coordinate of the third pair); `sobol` = 2 (RZ_RENDER_RQMC) draws them from the sample's replicate.
+// `filter`: rz_lens_ray's (0 in every instance but the FILTER ones).
 RZ_HD RzRay rz_camera_ray(const RzCamF32 &cam, uint32_t px, uint32_t py, uint32_t gpix, uint32_t sample,
-                          uint32_t k0, uint32_t k1, int sobol = 0) {
+                          uint32_t k0, uint32_t k1, int sobol = 0, uint32_t filter = 0u) {
     if (sobol) {
         const bool rqmc = sobol == 2;
         const float2 j = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_JITTER, sample, rqmc);
         const float2 l = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_LENS, sample, rqmc);
         const float t = rz_sobol_u01(k0, k1, gpix, RZ_PAIR_CAMERA_TIME, sample, rqmc).x;
-        return rz_lens_ray(cam, px, py, j.x, j.y, t, l.x, l.y);
+        return rz_lens_ray(cam, px, py, j.x, j.y, t, l.x, l.y, filter);
     }
     const uint4 r = rz_philox(gpix, sample, 0u, 0u, k0, k1);
     const float ux = rz_u01(r.x >> 8), uy = rz_u01(r.y >> 8), ut = rz_u01(r.z >> 8), ur = rz_u01(r.w >> 8);
     const float ua = rz_u01(((r.x & 0xffu) << 16) | ((r.y & 0xffu) << 8) | (r.z & 0xffu));
-    return rz_lens_ray(cam, px, py, ux, uy, ut, ur, ua);
+    return rz_lens_ray(cam, px, py, ux, uy, ut, ur, ua, filter);
 }
 
 // Sky of bounceRay's miss branch (renderer.zig:124-125): ((1-t)*1 + (0.5,0.7,1.0)) * t — not a lerp.
@@ -856,12 +925,13 @@ RZ_HD float3 rz_tile_pixel_dir(const RzCamF32 &cam, uint32_t pi, uint32_t pj) {
     return cam.px_origin + cam.px_du * (float)pi + cam.px_dv * (float)pj - cam.look_from;
 }
 
-// smallest cosine between the axis and the four corners of the pixel whose centre direction is pc
-RZ_HD float rz_tile_corner_cos(const RzCamF32 &cam, float3 pc, float3 ax) {
+// smallest cosine between the axis and the four corners of the square of half-width `half` px around the pixel whose centre
+// direction is pc: the pixel itself, or under a pixel filter the support its samples reach (rz_filter_reach)
+RZ_HD float rz_tile_corner_cos(const RzCamF32 &cam, float3 pc, float3 ax, float half = 0.5f) {
     float cmin = 1.0f;
 #pragma unroll
     for (int c = 0; c < 4; c++) {
-        const float3 q = pc + cam.px_du * ((c & 1) ? 0.5f : -0.5f) + cam.px_dv * ((c & 2) ? 0.5f : -0.5f);
+        const float3 q = pc + cam.px_du * ((c & 1) ? half : -half) + cam.px_dv * ((c & 2) ? half : -half);
         cmin = fminf(cmin, dot3(ax, normalize3(q)));
     }
     return cmin;

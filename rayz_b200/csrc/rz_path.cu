@@ -64,7 +64,7 @@ struct RzStream {
 
 // G = sphere PAIRS per search-loop iteration
 // LIST (not with QUEUE): the adaptive rounds' form, paths of the pixels a.px_list names (RzPathArgs::px_list)
-template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false, int SOBOL = 0, bool PASSES = false>
+template <int R, int G, bool STATS, int MB, bool QUEUE, bool LIST = false, int SOBOL = 0, bool PASSES = false, bool FILTER = false>
 __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -143,7 +143,7 @@ __global__ void __launch_bounds__(128, MB) rz_path_kernel(const RzPathArgs a) {
                             st[r].lp = lp;
                             st[r].gpix = pj * a.width + pi;
                             st[r].sample = a.sample_offset + unit_s0 + (k >> 5);
-                            st[r].ray = rz_camera_ray(a.cam, pi, pj, st[r].gpix, st[r].sample, a.seed_lo, a.seed_hi, SOBOL);
+                            st[r].ray = rz_camera_ray(a.cam, pi, pj, st[r].gpix, st[r].sample, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
                             st[r].thr = f3(1.f, 1.f, 1.f);
                             st[r].seg = 0;
                             st[r].alive = a.max_depth > 0u;
@@ -303,7 +303,7 @@ __device__ __forceinline__ void rz_flush_counters(const RzPathArgs &a, const RzS
 // Paths that scatter are appended, ballot-compacted, to the HBM queue the sorted stages start from; paths
 // that leave the scene or are absorbed accumulate here.  36 % of all segments are camera segments.  The cull
 // (rz_tile_cone / rz_tile_keep, rz_device.cuh) is host + device and property-tested on the CPU.
-template <bool STATS, int SOBOL = 0, bool PASSES = false>
+template <bool STATS, int SOBOL = 0, bool PASSES = false, bool FILTER = false>
 __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
     extern __shared__ __align__(16) unsigned char rz_smem[];
     __shared__ __align__(8) uint64_t s_bar;
@@ -331,14 +331,15 @@ __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
         if (valid) rz_local_to_global(lp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
         const uint32_t gpix = pj * a.width + pi;
 
-        // ---- cone around the tile's camera rays: axis = mean pixel direction, half-angle from the pixel corners
+        // ---- cone around the tile's camera rays: axis = mean pixel direction, half-angle from the pixel corners (under a pixel
+        // filter, the corners of the support its samples reach)
         const float3 pc = rz_tile_pixel_dir(a.cam, pi, pj);
         float3 ax = valid ? normalize3(pc) : f3(0.f, 0.f, 0.f);
         for (int o = 16; o > 0; o >>= 1) {
             ax.x += __shfl_xor_sync(0xffffffffu, ax.x, o); ax.y += __shfl_xor_sync(0xffffffffu, ax.y, o); ax.z += __shfl_xor_sync(0xffffffffu, ax.z, o);
         }
         const bool has_axis = rz_tile_axis(ax);
-        float cmin = valid ? rz_tile_corner_cos(a.cam, pc, ax) : 1.0f;
+        float cmin = valid ? rz_tile_corner_cos(a.cam, pc, ax, FILTER ? rz_filter_reach(a.sobol) : 0.5f) : 1.0f;
         for (int o = 16; o > 0; o >>= 1) cmin = fminf(cmin, __shfl_xor_sync(0xffffffffu, cmin, o));
         const RzTileCone cone = rz_tile_cone(a.cam, ax, has_axis, cmin, a.focus_dist, a.lens_radius);
         // one lane per sphere, stationary and moving through the same code; the lists keep set order (= search order)
@@ -370,7 +371,7 @@ __global__ void RZ_PRIMARY_BOUNDS rz_primary_kernel(const RzPathArgs a) {
                 const bool have = valid && (s + (uint32_t)trip < ns);
                 Q.live = have && a.max_depth > 0u;
                 if (STATS && have) { C.paths++; if (!Q.live) C.depth++; }
-                if (Q.live) Q.ray = rz_camera_ray(a.cam, pi, pj, gpix, Q.smp, a.seed_lo, a.seed_hi, SOBOL);
+                if (Q.live) Q.ray = rz_camera_ray(a.cam, pi, pj, gpix, Q.smp, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
                 else { Q.ray.o = f3(0.f, 0.f, 0.f); Q.ray.d = f3(0.f, 1.f, 0.f); Q.ray.time = 0.f; Q.ray.self_k = -1; }
                 Q.thr = f3(1.f, 1.f, 1.f); Q.seg = 0u; Q.lp = lp; Q.gpix = gpix; Q.bk = -1; Q.cont = false; Q.key = 0u;
                 if (trip == 0) L[1] = L[0];   // slot 0 is rewritten by the second trip
@@ -625,13 +626,18 @@ static auto rz_second_instance(const RzPathArgs &a, int collect_stats) {
 template <bool QUEUE, bool LIST>
 static cudaError_t rz_launch_one(const RzPathArgs &a, int rays_per_thread, int collect_stats, int sm_count, cudaStream_t stream,
                                  int *grid_out) {
-    const auto one = rz_pick_instance(a, collect_stats, [](auto S, auto M, auto P) {
-        return rz_path_kernel<1, 2, decltype(S)::value, 5, QUEUE, LIST, decltype(M)::value, decltype(P)::value>;
+    // the forms that generate camera rays have FILTER instances (rz_pick_camera_instance); the queue-fed form does not
+    auto pick = [&](auto inst) {
+        if constexpr (QUEUE) return rz_pick_instance(a, collect_stats, [inst](auto S, auto M, auto P) { return inst(S, M, P, std::false_type{}); });
+        else return rz_pick_camera_instance(a, collect_stats, inst);
+    };
+    const auto one = pick([](auto S, auto M, auto P, auto F) {
+        return rz_path_kernel<1, 2, decltype(S)::value, 5, QUEUE, LIST, decltype(M)::value, decltype(P)::value, decltype(F)::value>;
     });
     // 8 resident CTAs per SM (64 registers, 232 B of spills outside the search loop) measured 3 % faster than the 5 CTAs the
     // unconstrained 88-register build gets: 1522 vs 1472 Mpaths/s at config 2 / 100 spp.  (The STATS instances keep 5.)
-    const auto two = rz_pick_instance(a, collect_stats, [](auto S, auto M, auto P) {
-        return rz_path_kernel<2, 2, decltype(S)::value, decltype(S)::value ? 5 : 8, QUEUE, LIST, decltype(M)::value, decltype(P)::value>;
+    const auto two = pick([](auto S, auto M, auto P, auto F) {
+        return rz_path_kernel<2, 2, decltype(S)::value, decltype(S)::value ? 5 : 8, QUEUE, LIST, decltype(M)::value, decltype(P)::value, decltype(F)::value>;
     });
     const auto kern = rays_per_thread == 1 ? one : two;
     const size_t smem = rz_pk_bytes(a);
@@ -660,7 +666,9 @@ extern "C" size_t rz_primary_smem_bytes(const RzPathArgs *a) {
 
 // Stage 1: camera segments of the work units [unit_base, unit_base + n_units) -> queue.
 extern "C" cudaError_t rz_launch_primary(const RzPathArgs *a, int collect_stats, int sm_count, cudaStream_t stream) {
-    const auto kern = rz_pick_instance(*a, collect_stats, [](auto S, auto M, auto P) { return rz_primary_kernel<decltype(S)::value, decltype(M)::value, decltype(P)::value>; });
+    const auto kern = rz_pick_camera_instance(*a, collect_stats, [](auto S, auto M, auto P, auto F) {
+        return rz_primary_kernel<decltype(S)::value, decltype(M)::value, decltype(P)::value, decltype(F)::value>;
+    });
     const size_t smem = rz_primary_smem_bytes(a);
     int grid = 0;
     const cudaError_t e = rz_persistent_grid(kern, smem, sm_count, &grid);

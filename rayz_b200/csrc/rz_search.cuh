@@ -349,6 +349,14 @@ static inline auto rz_pick_instance(const RzPathArgs &a, int collect_stats, F in
     if (a.sobol & RZ_PATH_PASSES) return collect_stats ? rz_pick_sampler_of(a, inst, T, T) : rz_pick_sampler_of(a, inst, N, T);
     return collect_stats ? rz_pick_sampler_of(a, inst, T, N) : rz_pick_sampler_of(a, inst, N, N);
 }
+// The same for a kernel that generates camera rays: `inst` takes a fourth argument, std::integral_constant<bool, FILTER>, and
+// FILTER (a pixel filter other than the box in a.sobol, RZ_RENDER_FILTER) is an instance of its own for the same reason.
+template <class F>
+static inline auto rz_pick_camera_instance(const RzPathArgs &a, int collect_stats, F inst) {
+    if (rz_filter_kind(a.sobol) != RZ_FILTER_BOX)
+        return rz_pick_instance(a, collect_stats, [inst](auto S, auto M, auto P) { return inst(S, M, P, std::true_type{}); });
+    return rz_pick_instance(a, collect_stats, [inst](auto S, auto M, auto P) { return inst(S, M, P, std::false_type{}); });
+}
 
 // Grid of a persistent kernel: as many 128-thread CTAs as fit on every SM with `smem` bytes of dynamic shared memory.  The
 // attribute that admits that much is set only when smem > 0 (the BVH kernels take none).

@@ -73,7 +73,7 @@ __device__ __forceinline__ void wf_decode(const RzPathArgs &a, unsigned long lon
     sample = r >> 5;
 }
 
-template <bool STATS, int SOBOL>
+template <bool STATS, int SOBOL, bool FILTER = false>
 __global__ void __launch_bounds__(256) wf_generate(const RzPathArgs a, WfState s) {
     const WfCounters c = *s.ctr;
     const unsigned long long remaining = c.total_paths - c.next_path;
@@ -91,7 +91,7 @@ __global__ void __launch_bounds__(256) wf_generate(const RzPathArgs a, WfState s
             uint32_t pi, pj;
             rz_local_to_global(lp, a.width, a.shard_index, a.shard_count, a.band_rows, pi, pj);
             d.y = pj * a.width + pi;
-            const RzRay ray = rz_camera_ray(a.cam, pi, pj, d.y, d.z, a.seed_lo, a.seed_hi, SOBOL);
+            const RzRay ray = rz_camera_ray(a.cam, pi, pj, d.y, d.z, a.seed_lo, a.seed_hi, SOBOL, FILTER ? a.sobol : 0u);
             A = make_float4(ray.o.x, ray.o.y, ray.o.z, ray.time);
             B = make_float4(ray.d.x, ray.d.y, ray.d.z, __int_as_float(ray.self_k));
             C = make_float4(1.f, 1.f, 1.f, __uint_as_float(0u));
@@ -328,7 +328,7 @@ extern "C" cudaError_t rz_wavefront_render(const RzPathArgs *a, int sm_count, in
         cudaGraph_t g;
         if ((e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal)) != cudaSuccess) return e;
         for (int it = 0; it < ITERS; it++) {
-            rz_pick_instance(*a, st, [](auto S, auto M, auto) { return wf_generate<decltype(S)::value, decltype(M)::value>; })<<<grid_s, 256, 0, cap>>>(*a, ws->st);
+            rz_pick_camera_instance(*a, st, [](auto S, auto M, auto, auto F) { return wf_generate<decltype(S)::value, decltype(M)::value, decltype(F)::value>; })<<<grid_s, 256, 0, cap>>>(*a, ws->st);
             wf_after_generate<<<1, 1, 0, cap>>>(ws->st);
             wf_intersect<2><<<grid_i, 128, smem, cap>>>(*a, ws->st);
             wf_after_intersect<<<1, 1, 0, cap>>>(ws->st);

@@ -278,14 +278,24 @@ class Backend:
     @staticmethod
     def params(width, height, spp, max_depth=50, seed=1, sample_offset=0, variant="auto", t_min=0.0, shard_index=0,
                shard_count=1, band_rows=0, collect_stats=False, serial_passes=False, accumulate=False,
-               moments=False, sobol=False, rqmc=False, passes=False) -> abi.RzRenderParams:
+               moments=False, sobol=False, rqmc=False, passes=False, pixel_filter="box", filter_width=None) -> abi.RzRenderParams:
         """RzRenderParams.  accumulate: add this batch to the previous render's sums (RZ_RENDER_ACCUMULATE; sample_offset must
         continue where they end); moments: also sum each path's luminance squared, so that noise() can estimate the error;
         sobol: draw the camera and scatter samples from Owen-scrambled Sobol pairs instead of Philox (RZ_RENDER_SOBOL);
         rqmc: two independently scrambled Sobol replicates per pixel, so that the noise estimate sees the stratification
         (RZ_RENDER_RQMC).  rqmc does not imply sobol or moments: the library refuses it without both, and with an odd spp or
         sample_offset.  passes: also sum each path's radiance into its light-path pass, so that passes() can split the frame
-        (RZ_RENDER_PASSES; no pixel changes)."""
+        (RZ_RENDER_PASSES; no pixel changes).  pixel_filter: the reconstruction filter each camera sample's offset is drawn
+        from, "box" (the default: the reference's uniform jitter), "tent", "gaussian" or "blackman-harris" (RZ_RENDER_FILTER);
+        filter_width: its full width in px, None for the kind's default (2, 3 and 1.5 px), else 1 to 4 px in steps of 1/16
+        (a width with the box is refused by the library)."""
+        if pixel_filter not in abi.FILTERS:
+            raise ValueError(f"pixel_filter must be one of {sorted(abi.FILTERS)}, not {pixel_filter!r}")
+        w16 = 0
+        if filter_width is not None:
+            w16 = int(round(float(filter_width) * 16))
+            if w16 != float(filter_width) * 16 or not 0 <= w16 <= 255:
+                raise ValueError(f"filter_width must be a multiple of 1/16 px, not {filter_width!r}")
         p = abi.RzRenderParams()
         p.width, p.height, p.spp, p.max_depth = width, height, spp, max_depth
         p.seed, p.sample_offset = seed, sample_offset
@@ -295,7 +305,7 @@ class Backend:
         p.collect_stats = 1 if collect_stats else 0
         p.flags = ((abi.RENDER_SERIAL_PASSES if serial_passes else 0) | (abi.RENDER_ACCUMULATE if accumulate else 0)
                    | (abi.RENDER_MOMENTS if moments else 0) | (abi.RENDER_SOBOL if sobol else 0) | (abi.RENDER_RQMC if rqmc else 0)
-                   | (abi.RENDER_PASSES if passes else 0))
+                   | (abi.RENDER_PASSES if passes else 0) | abi.render_filter(abi.FILTERS[pixel_filter], w16))
         return p
 
     def reserve(self, p: abi.RzRenderParams):
@@ -476,6 +486,8 @@ class Tracer:
         self.pool = MemPool()
         self.seed = seed           # the reference seeds from the OS (renderer.zig:55-59)
         self.variant = "auto"
+        self.pixel_filter = "box"  # reconstruction filter of render(), render_guides(), render_mattes() and so denoise():
+        self.filter_width = None   # "tent", "gaussian" or "blackman-harris", width in px (None: the kind's default)
         self.sampler = "philox"    # or "sobol": low-discrepancy camera and scatter samples (RZ_RENDER_SOBOL) in render(),
                                    # render_guides() and so the denoised frame; or "sobol-rqmc": the same with two replicates
                                    # per pixel and the noise estimate they allow (RZ_RENDER_RQMC, with moments)
@@ -497,6 +509,10 @@ class Tracer:
         if self.sampler not in self.SAMPLERS:
             raise ValueError(f"Tracer.sampler must be 'philox', 'sobol' or 'sobol-rqmc', not {self.sampler!r}")
         return dict(self.SAMPLERS[self.sampler])
+
+    def _filter(self) -> dict:
+        """Backend.params keywords of the pixel filter."""
+        return {"pixel_filter": self.pixel_filter, "filter_width": self.filter_width}
 
     @property
     def backend(self) -> Backend:
@@ -521,7 +537,8 @@ class Tracer:
         self._uploaded = arrays
         kw = self._sampler()
         kw["moments"] = moments or kw.get("moments", False)
-        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant, **kw)
+        p = Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant, **kw,
+                           **self._filter())
         if pooled:
             p.flags |= abi.RENDER_ADAPTIVE_POOLED
         if passes:
@@ -575,7 +592,7 @@ class Tracer:
     def _first_hit_params(self) -> abi.RzRenderParams:
         """The parameters of render()'s camera samples, for the first-hit calls (guides, mattes)."""
         return Backend.params(self.img.w, self.img.h, self.samples_per_px, self.max_bounces, self.seed, variant=self.variant,
-                              **self._sampler())
+                              **self._sampler(), **self._filter())
 
     def denoise(self, iterations: int = 5, sigma_luminance: float = 4.0, sigma_normal: float = 128.0, sigma_depth: float = 1.0):
         """The frame of the last render() (with moments=True, or a noise target) denoised with the guides of render_guides(),

@@ -78,6 +78,20 @@ pub const RZ_RENDER_SOBOL: u32 = 0x10; // camera and scatter samples from Owen-s
 pub const RZ_RENDER_RQMC: u32 = 0x20; // with SOBOL and MOMENTS: two scrambled replicates per pixel, a noise estimate that sees the stratification
 pub const RZ_RENDER_ADAPTIVE_POOLED: u32 = 0x40; // with ADAPTIVE, rayz_cuda_render_to_noise only: stop each pixel on an error pooled over its row segment
 pub const RZ_RENDER_PASSES: u32 = 0x80; // also sum each path's radiance into its light-path pass (rayz_cuda_passes); no pixel changes
+// pixel reconstruction filter, a field of RzRenderParams.flags: kind in bits 8-9, full width in 1/16 px in bits 16-23 (0: default)
+pub const RZ_RENDER_FILTER_SHIFT: u32 = 8;
+pub const RZ_RENDER_FILTER_MASK: u32 = 0x300;
+pub const RZ_RENDER_FILTER_WIDTH_SHIFT: u32 = 16;
+pub const RZ_RENDER_FILTER_WIDTH_MASK: u32 = 0xff0000;
+pub const RZ_FILTER_BOX: u32 = 0;
+pub const RZ_FILTER_TENT: u32 = 1;
+pub const RZ_FILTER_GAUSSIAN: u32 = 2;
+pub const RZ_FILTER_BLACKMAN_HARRIS: u32 = 3;
+pub const RZ_FILTER_WIDTH_MIN: u32 = 16; // 1 px
+pub const RZ_FILTER_WIDTH_MAX: u32 = 64; // 4 px
+pub fn RZ_RENDER_FILTER(kind: u32, width16: u32) u32 {
+    return ((kind << RZ_RENDER_FILTER_SHIFT) & RZ_RENDER_FILTER_MASK) | ((width16 << RZ_RENDER_FILTER_WIDTH_SHIFT) & RZ_RENDER_FILTER_WIDTH_MASK);
+}
 // light-path passes: plane index of rayz_cuda_passes' output (include/rayz_cuda.h "Light-path passes")
 pub const RZ_PASS_ENVIRONMENT: u32 = 0;
 pub const RZ_PASS_DIFFUSE_DIRECT: u32 = 1;
